@@ -2,7 +2,7 @@
 """bench.py -- headline measurement (BASELINE.json): 1080p frame-pairs/s (detect + LK flow + velocity solve) and
 Monte-Carlo trials/s, plus the other three BASELINE configurations, all in the ONE JSON line of the default run.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path (pyramids -> Shi-Tomasi -> pyramidal LK -> velocity solve) over one batch of
@@ -61,7 +61,9 @@ def log(msg):
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps of every leg (default: 10, and 50 samples / 400 resident steps in the C1 / C4 "
+                         "latency legs, whose percentiles and per-frame means want more)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=128, help="frame pairs per step per GPU")
@@ -75,7 +77,25 @@ def parse():
                     help="internal: run one multi-process CPU baseline in this (CUDA-free) process and print its JSON")
     ap.add_argument("--workload", default="all", choices=["all", "c1", "c2", "c4", "c5"],
                     help="all (default: every BASELINE configuration in one line) or a single configuration")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result records of the last timed C2 step (rank 0) as DIR/<field>.npy, float64")
+    args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    args.latency_samples, args.latency_reps = (50, 400) if args.steps is None else (args.steps, args.steps)
+    if args.steps is None:
+        args.steps = 10
+    if args.dump_outputs and (args.impl == "reference" or args.workload not in ("all", "c2")):
+        ap.error("--dump-outputs writes what the C2 headline path computed: use it with --workload all or c2")
+    return args
+
+
+def dump_outputs(out_dir, rec):
+    """One float64 array per field of the result records (the integer fields are exact in float64). The inputs are
+    seeded synthetic frames, so two builds run with the same arguments can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name in rec.dtype.names:
+        np.save(os.path.join(out_dir, name + ".npy"), rec[name].astype(np.float64))
 
 
 def bind_near_gpu(index):
@@ -449,7 +469,7 @@ def leg_latency(args, ofb200, torch, ctx, name, rank):
         step()
     ctx.sync()
     lat = []
-    for _ in range(max(args.steps, 50)):
+    for _ in range(args.latency_samples):
         ctx.timer_start(); step(); lat.append(ctx.timer_stop())
     res = np.zeros(1, ofb200._lib.RESULT_DTYPE); ctx.memcpy(res, d_res, res.nbytes)
     ctx.set_profile(True)
@@ -465,7 +485,7 @@ def leg_latency(args, ofb200, torch, ctx, name, rank):
     for _ in range(5):
         ofb200.frame_pairs(ha[None], hb[None], imu[:1], cfg, ctx=ctx)
     e2e_lat = []
-    for _ in range(max(args.steps, 50)):
+    for _ in range(args.latency_samples):
         t0 = time.perf_counter(); ofb200.frame_pairs(ha[None], hb[None], imu[:1], cfg, ctx=ctx); e2e_lat.append((time.perf_counter() - t0) * 1e3)
     # the same camera through the device-resident feature lifecycle: (i) what velocity_measurment_node's image callback
     # would run, one pageable host frame in, one result record out per call; (ii) resident frames, asynchronous calls
@@ -476,12 +496,12 @@ def leg_latency(args, ofb200, torch, ctx, name, rank):
     for k in range(6):
         tres = trk.step(hb if k & 1 else ha, imu[:1])
     trk_lat = []
-    for k in range(max(args.steps, 50)):
+    for k in range(args.latency_samples):
         t0 = time.perf_counter(); tres = trk.step(hb if k & 1 else ha, imu[:1]); trk_lat.append((time.perf_counter() - t0) * 1e3)
     trk.close()
     trk = ofb200.StreamTracker(w, h, borrow_frames=True, **kw)
     d_tres = torch.zeros(ofb200._lib.TRACK_RESULT_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
-    nrep = max(args.steps, 400)          # (a 50-step run is dominated by its first steps: 46 vs 41 us per 640x480 frame)
+    nrep = args.latency_reps             # (a short run is dominated by its first steps: 46 us per 640x480 frame over 50, 41 over 400)
 
     # (the argument objects are built once: at ~40 us per step the per-call conversion of three tensors to pointers shows)
     step_fn, chk = ctx.lib.ofb_tracker_step, ofb200._lib.check
@@ -822,6 +842,8 @@ def main():
     # correctness of what was timed: results must be plausible velocities (forward pairs have an exact truth)
     res = np.zeros(B, ofb200._lib.RESULT_DTYPE)
     ctx.memcpy(res, d_res, res.nbytes)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res)
     verr = max(np.abs(res["v"][k] - pairs[(k // 2) % len(pairs)][2]["v"]).max() for k in range(0, B, 2))
     tracked = int(res["n_tracked"].min())
     # the same number of pairs as independent (prev, next) buffers: both frames of every pair uploaded / pyramided

@@ -1,20 +1,23 @@
 """Loads the REFERENCE's own functions (verbatim, at run time) for pinning the oracle.
 
-Test infrastructure only. Works only where /root/reference exists (this container, not the
-GPU box): simulation.py / velocity_measurment_node / evaluate_exp.py cannot be imported
-(matplotlib / rospy missing, sweeps run at import), so their FunctionDefs are AST-extracted
-and exec'd in a namespace holding numpy. Nothing is copied into the repo.
+Test infrastructure only. Works only where OFB_REFERENCE_DIR names a checkout of the original
+Python project. The repository does not carry it: without it the live comparisons skip and the
+committed golden outputs under tests/golden/ pin the oracle. simulation.py /
+velocity_measurment_node / evaluate_exp.py cannot be imported (matplotlib / rospy missing, sweeps
+run at import), so their FunctionDefs are AST-extracted and exec'd in a namespace holding numpy.
+Nothing is copied into the repo.
 """
 import ast
 import os
 
 import numpy as np
 
-REF = os.environ.get("OFB_REFERENCE_DIR", "/root/reference")
+REF = os.environ.get("OFB_REFERENCE_DIR", "")
+MISSING = "needs OFB_REFERENCE_DIR (a checkout of the original project)"
 
 
 def available():
-    return os.path.isfile(os.path.join(REF, "numerical_simulation", "simulation.py"))
+    return bool(REF) and os.path.isfile(os.path.join(REF, "numerical_simulation", "simulation.py"))
 
 
 def load_functions(relpath, names=None, extra_globals=None):

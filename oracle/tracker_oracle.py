@@ -1,6 +1,6 @@
 """CPU ORACLE (test infrastructure, NOT product code) for the feature lifecycle around the tracker
 (SURVEY 8f-2). Restates, step by step, what the reference's per-frame loops do (paths relative to
-/root/reference):
+the original project's checkout):
 
 * track + status filter      flight_experiments/evaluate_exp.py:97-99, velocity_measurment_node:133-136
 * static_immobile            of_library.py:88-92

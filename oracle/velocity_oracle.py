@@ -1,7 +1,7 @@
 """CPU ORACLE (test infrastructure, NOT product code) for stages 4-5 of the hot path.
 
 Plain NumPy restatement of the reference's own arithmetic; every function cites the
-reference lines it follows (paths relative to /root/reference):
+reference lines it follows (paths relative to the original project's checkout):
 
 * generate_test_data   numerical_simulation/simulation.py:7-12, velocity_measurment_node:25-29
 * solve_lgs (3 variants) simulation.py:15-30 (S), velocity_measurment_node:30-42 (N),
@@ -21,9 +21,9 @@ reference lines it follows (paths relative to /root/reference):
 * body -> world        velocity_measurment_node:258
 
 PARITY PIN: tests/test_oracle_velocity.py runs the reference's functions themselves
-(AST-extracted from /root/reference and exec'd, when that directory exists) against this
+(AST-extracted and exec'd where OFB_REFERENCE_DIR names a checkout of it) against this
 restatement, and tests/golden/velocity_golden.npz (made by tools/make_golden.py from the
-reference functions) pins it where /root/reference is absent (the GPU box).
+reference functions) pins it everywhere else.
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline leg may import this.
 """

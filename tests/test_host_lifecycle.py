@@ -83,9 +83,9 @@ def test_ros_yaml_without_ros_classes():
 
 
 def test_reference_recordings_load():
+    if not ref_loader.available():
+        pytest.skip(ref_loader.MISSING)
     path = os.path.join(ref_loader.REF, "flight_experiments", "hgtData.yaml")
-    if not os.path.isfile(path):
-        pytest.skip("needs /root/reference")
     with open(path) as f:
         head = "".join(f.readline() for _ in range(13 * 200))
     msgs = replay.load_ros_yaml(io.StringIO(head))

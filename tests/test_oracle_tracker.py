@@ -1,6 +1,6 @@
 """Pins oracle/tracker_oracle.py (the lifecycle restatement, SURVEY 8f-2): against tests/golden/tracker_golden.npz
 (made by tools/make_golden_tracker.py with the real cv2 4.13 operators and the reference's own static_immobile /
-r_tilde / solve_lgs) and, where cv2 and /root/reference exist, against those run live."""
+r_tilde / solve_lgs) and, where cv2 and a checkout of the reference (OFB_REFERENCE_DIR) exist, against those run live."""
 import os
 
 import numpy as np
@@ -100,10 +100,10 @@ def test_static_immobile_equals_reference():
 
 
 def test_golden_is_what_cv2_and_the_reference_produce_here(g):
-    """Fixture freshness: where cv2 and /root/reference exist the golden file is regenerated live and compared."""
+    """Fixture freshness: where cv2 and the reference exist the golden file is regenerated live and compared."""
     cv2 = pytest.importorskip("cv2")
     if not ref_loader.available() or not cv2.__version__.startswith("4.13"):
-        pytest.skip("needs /root/reference and cv2 4.13")
+        pytest.skip(ref_loader.MISSING + " and cv2 4.13")
     eng = tc.cv2_engine()
     for name in tc.SCENARIOS:
         frames, imus, kw = tc.build(name)
@@ -111,29 +111,22 @@ def test_golden_is_what_cv2_and_the_reference_produce_here(g):
         compare_with_golden(g, name, res, 0.0, 1e-12)
 
 
-@pytest.mark.parametrize("seed", [21, 22, 23])
+@pytest.mark.parametrize("seed", tc.RANDOM_SEEDS)
 def test_oracle_vs_live_cv2_on_random_sequences(seed):
     """Beyond the committed fixture: random drift / rotation / occlusion / parameters, the oracle step against the same
-    step made of the real cv2 operators and the reference's functions, teacher-forced on the cv2 chain."""
+    step made of the real cv2 operators (tests/golden/tracker_random_golden.npz, made by tools/make_golden_tracker.py;
+    run live, with the reference's own functions, where cv2 4.13 and the reference exist), teacher-forced on the cv2
+    chain."""
     cv2 = pytest.importorskip("cv2")
-    if not ref_loader.available() or not cv2.__version__.startswith("4.13"):
-        pytest.skip("needs /root/reference and cv2 4.13")
-    rng = np.random.default_rng(seed)
-    T = 6
-    step = tuple(rng.uniform(-8, 8, 2))
-    occl = (int(rng.integers(2, 5)), int(rng.integers(0, 150)), int(rng.integers(0, 100)), 120, 100)
-    frames = [tc._sequence(seed, T, step, float(rng.uniform(-0.005, 0.005)), occl)]
-    mode = ["exp", "node", "module"][seed % 3]
-    kw = dict(max_features=int(rng.integers(30, 80)), topup=mode, mask_radius=int(rng.integers(5, 40)),
-              variant=["exp", "node", "sim"][seed % 3], scaling=1.0 / tc.F,
-              gate=None if seed % 2 else ("le", -0.9), max_speed=0.0 if seed % 3 else 12.0, dummy_value=-1.0,
-              feature_params=dict(qualityLevel=float(rng.uniform(0.02, 0.2)), minDistance=int(rng.integers(5, 15)),
-                                  blockSize=int(rng.choice([3, 5, 7, 12]))))
-    kw["min_features"] = kw["max_features"] - int(rng.integers(3, 10))
-    imus = [tc._imu(seed, T, step, (0.8, 3.0), (1.0, 0.2))]
-    eng = tc.cv2_engine()
-    ref = tc.run_oracle_tracker(lambda: tracker_oracle.TrackerOracle(tc.W, tc.H, engine=eng, **kw), frames, imus)
-    g = {"live_" + k: v for k, v in tc.pack(ref, kw["max_features"] + kw["min_features"]).items()}
+    frames, imus, kw = tc.random_case(seed)
+    if ref_loader.available() and cv2.__version__.startswith("4.13"):
+        eng = tc.cv2_engine()
+        ref = tc.run_oracle_tracker(lambda: tracker_oracle.TrackerOracle(tc.W, tc.H, engine=eng, **kw), frames, imus)
+        g = {"live_" + k: v for k, v in tc.pack(ref, kw["max_features"] + kw["min_features"]).items()}
+    else:
+        stored = np.load(os.path.join(GOLDEN, "tracker_random_golden.npz"))
+        g = {"live_" + k[len("s%d_" % seed):]: stored[k] for k in stored.files if k.startswith("s%d_" % seed)}
+        assert g, "no stored sequence for seed %d" % seed
 
     class OwnSelectionOnCv2Map(tracker_oracle.Engine):
         """the oracle's selection on cv2's lambda_min map: two correct fp32 maps may order near-ties differently (the

@@ -1,6 +1,6 @@
 """Pins the numpy oracle (oracle/velocity_oracle.py) to the REFERENCE: against the committed golden
 outputs of the reference's own functions (tests/golden/velocity_golden.npz, made by
-tools/make_golden.py) and, where /root/reference exists, against those functions run live."""
+tools/make_golden.py) and, where OFB_REFERENCE_DIR names a checkout of it, against those functions run live."""
 import os
 import warnings
 
@@ -97,7 +97,7 @@ def test_philox_known_answer():
     assert abs(z.mean()) < 0.01 and abs(z.std() - 1) < 0.01
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not present (GPU box)")
+@pytest.mark.skipif(not ref_loader.available(), reason=ref_loader.MISSING)
 def test_oracle_against_live_reference():
     sim = ref_loader.simulation()
     node = ref_loader.node()
@@ -160,7 +160,7 @@ def test_live_sorting_scenario_matches_reference(g2, points200):
     np.testing.assert_allclose(tf, g2["live_true_flow"], rtol=1e-11, atol=1e-12)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="needs /root/reference")
+@pytest.mark.skipif(not ref_loader.available(), reason=ref_loader.MISSING)
 def test_module_system_live_reference():
     """Where the reference exists: regenerate one module case through the AST-extracted statements and compare."""
     import importlib.util

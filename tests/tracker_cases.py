@@ -138,16 +138,36 @@ def pack(results, cap):
     return g
 
 
-def cv2_engine():
+RANDOM_SEEDS = (21, 22, 23)
+
+
+def random_case(seed):
+    """A random drift / rotation / occlusion / parameter draw for one stream: -> (frames, imus, tracker kwargs)"""
+    rng = np.random.default_rng(seed)
+    T = 6
+    step = tuple(rng.uniform(-8, 8, 2))
+    occl = (int(rng.integers(2, 5)), int(rng.integers(0, 150)), int(rng.integers(0, 100)), 120, 100)
+    frames = [_sequence(seed, T, step, float(rng.uniform(-0.005, 0.005)), occl)]
+    mode = ["exp", "node", "module"][seed % 3]
+    kw = dict(max_features=int(rng.integers(30, 80)), topup=mode, mask_radius=int(rng.integers(5, 40)),
+              variant=["exp", "node", "sim"][seed % 3], scaling=1.0 / F,
+              gate=None if seed % 2 else ("le", -0.9), max_speed=0.0 if seed % 3 else 12.0, dummy_value=-1.0,
+              feature_params=dict(qualityLevel=float(rng.uniform(0.02, 0.2)), minDistance=int(rng.integers(5, 15)),
+                                  blockSize=int(rng.choice([3, 5, 7, 12]))))
+    kw["min_features"] = kw["max_features"] - int(rng.integers(3, 10))
+    imus = [_imu(seed, T, step, (0.8, 3.0), (1.0, 0.2))]
+    return frames, imus, kw
+
+
+def cv2_engine(reference=True):
     """The same step operators backed by the REAL cv2 and the reference's own functions (AST-extracted by
-    oracle/ref_loader.py). Only available in the build container (cv2 + /root/reference)."""
+    oracle/ref_loader.py; needs OFB_REFERENCE_DIR). reference=False keeps the oracle's restatements of the three
+    arithmetic functions instead: solve_lgs and r_tilde (pinned to the reference's stored outputs by
+    tests/test_oracle_velocity.py) and static_immobile (pinned by tests/test_oracle_tracker.py)."""
     import cv2
     from oracle import ref_loader, tracker_oracle
-    lib = ref_loader.of_library("root")
-    solvers = {"node": ref_loader.node()["solve_lgs"], "exp": ref_loader.evaluate_exp()["solve_lgs"],
-               "sim": ref_loader.simulation()["solve_lgs"]}
 
-    class Cv2Engine(tracker_oracle.Engine):
+    class Cv2Operators(tracker_oracle.Engine):
         def good_features(self, img, max_corners, quality, min_distance, block_size, mask=None):
             return cv2.goodFeaturesToTrack(img, mask=mask, maxCorners=max_corners, qualityLevel=quality,
                                            minDistance=min_distance, blockSize=block_size)
@@ -165,6 +185,13 @@ def cv2_engine():
         def bgr2gray(self, bgr):
             return cv2.cvtColor(bgr, cv2.COLOR_BGR2GRAY)
 
+    if not reference:
+        return Cv2Operators()
+    lib = ref_loader.of_library("root")
+    solvers = {"node": ref_loader.node()["solve_lgs"], "exp": ref_loader.evaluate_exp()["solve_lgs"],
+               "sim": ref_loader.simulation()["solve_lgs"]}
+
+    class Cv2Engine(Cv2Operators):
         def solve(self, x, u, d, n, w, t, variant):
             if variant == "node":
                 v, res, rank, s = solvers["node"](x, u, d, n, w)

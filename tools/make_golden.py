@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Generates tests/golden/* from the REFERENCE ITSELF (run in the build container, where
-/root/reference and cv2 4.13.0 exist; the GPU box only reads the committed fixtures).
+"""Generates tests/golden/* from the REFERENCE ITSELF (needs cv2 4.13.0 and
+OFB_REFERENCE_DIR naming a checkout of the original project; the tests only read the committed fixtures).
 
 * velocity_golden.npz : outputs of the reference's own functions, AST-extracted from
   numerical_simulation/simulation.py, velocity_measurment_node, flight_experiments/evaluate_exp.py
@@ -202,7 +202,7 @@ def cv2_golden():
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
     if not ref_loader.available():
-        sys.exit("needs /root/reference")
+        sys.exit(ref_loader.MISSING)
     velocity_golden()
     cv2_golden()
     for f in sorted(os.listdir(OUT)):

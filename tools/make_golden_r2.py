@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Round-2 fixtures, generated from the REFERENCE ITSELF in the build container (where /root/reference exists; the GPU
-box only reads the committed file): tests/golden/velocity_golden_r2.npz.
+"""Round-2 fixtures, generated from the REFERENCE ITSELF (needs OFB_REFERENCE_DIR naming a checkout of the original
+project; the tests only read the committed file): tests/golden/velocity_golden_r2.npz.
 
 * module_*   : the inline least-squares system of optical_flow_experiments/of_module.py:136-146. The statements
   (A = ..., B = ..., the `for` loop, `np.linalg.lstsq(A, B)`) are AST-extracted from the script's `while` body and exec'd
@@ -187,7 +187,7 @@ def live_sorting_golden(g):
 
 if __name__ == "__main__":
     if not ref_loader.available():
-        sys.exit("needs /root/reference")
+        sys.exit(ref_loader.MISSING)
     g = {}
     module_golden(g)
     time_evolution_golden(g)

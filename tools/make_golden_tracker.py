@@ -1,9 +1,13 @@
 #!/usr/bin/env python
 """Generates tests/golden/tracker_golden.npz: the scenarios of tests/tracker_cases.py run through the lifecycle
 steps with the REAL cv2 4.13 operators (calcOpticalFlowPyrLK, goodFeaturesToTrack, circle, cvtColor) and the
-reference's own of_library.static_immobile / of_library.r_tilde / solve_lgs (AST-extracted from /root/reference).
-Run in the build container; the GPU box only reads the committed fixture. Also stores cv2.circle masks for a set
-of radii / centres (the exclusion mask of velocity_measurment_node:159-161)."""
+reference's own of_library.static_immobile / of_library.r_tilde / solve_lgs (AST-extracted from the checkout that
+OFB_REFERENCE_DIR names). Also stores cv2.circle masks for a set of radii / centres (the exclusion mask of
+velocity_measurment_node:159-161).
+
+Generates tests/golden/tracker_random_golden.npz: the random sequences of tracker_cases.random_case through the
+same cv2 operators, with the reference's three functions where the reference is available and otherwise with the
+oracle's pinned restatements of them; the file's `arithmetic` entry records which."""
 import os
 import sys
 
@@ -14,11 +18,31 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 sys.dont_write_bytecode = True
 import tracker_cases as tc  # noqa: E402
-from oracle import tracker_oracle  # noqa: E402
+from oracle import ref_loader, tracker_oracle  # noqa: E402
+
+
+def random_golden():
+    import cv2
+    assert cv2.__version__.startswith("4.13"), cv2.__version__
+    reference = ref_loader.available()
+    eng = tc.cv2_engine(reference=reference)
+    g = {"arithmetic": np.array("reference" if reference else "oracle")}
+    for seed in tc.RANDOM_SEEDS:
+        frames, imus, kw = tc.random_case(seed)
+        res = tc.run_oracle_tracker(lambda: tracker_oracle.TrackerOracle(tc.W, tc.H, engine=eng, **kw), frames, imus)
+        for k, v in tc.pack(res, kw["max_features"] + kw["min_features"]).items():
+            g["s%d_%s" % (seed, k)] = v
+        print("seed", seed, "n_points", g["s%d_n_points" % seed].tolist(), "added", g["s%d_n_added" % seed].tolist())
+    out = os.path.join(ROOT, "tests", "golden", "tracker_random_golden.npz")
+    np.savez_compressed(out, **g)
+    print("wrote", out, os.path.getsize(out), "bytes, arithmetic:", g["arithmetic"])
 
 
 def main():
     import cv2
+    random_golden()
+    if not ref_loader.available():
+        sys.exit("tracker_golden.npz not rewritten: " + ref_loader.MISSING)
     eng = tc.cv2_engine()
     g = {}
     for name in tc.SCENARIOS:

@@ -1,5 +1,6 @@
-import sys, time, numpy as np, torch
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tests')
+import os, sys, time, numpy as np, torch
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import ofb200, synth
 ctx = ofb200.Context(0)
 w, h = (int(sys.argv[1]), int(sys.argv[2])) if len(sys.argv) > 2 else (640, 480)

@@ -18,7 +18,8 @@ from .of_library import pix_trans, r_tilde, static_immobile, initialize_ft
 from .velocity import (solve_lgs, solve_full, solve_lgs_batched, solve_lgs_module, generate_test_data, feasibility,
                        quaternion_to_rotation, plane_normal, body_to_world)
 from .vision import (goodFeaturesToTrack, calcOpticalFlowPyrLK, cornerMinEigenVal, buildPyramid, pyrDown, cvtColor,
-                     Pyramid, make_pair_cfg, frame_pairs, frame_sequence, COLOR_BGR2GRAY, TERM_CRITERIA_COUNT, TERM_CRITERIA_EPS)
+                     Pyramid, make_pair_cfg, frame_pairs, frame_sequence, COLOR_BGR2GRAY, TERM_CRITERIA_COUNT, TERM_CRITERIA_EPS,
+                     undistortPoints, undistortPointsIter, make_camera, CAMERA_ITERATIONS)
 from .tracker import StreamTracker, FleetTracker, exclusion_mask
 from .simulation import of_simulation, feas_simulation, overlap, run_named_sweep, run_sweep, sorting_study, advect_points
 

@@ -12,7 +12,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libofb200.so")
-SOURCES = ["api.cu", "pyramid.cu", "features.cu", "pyrlk.cu", "velocity.cu", "montecarlo.cu", "pairs.cu", "tracker.cu"]
+SOURCES = ["api.cu", "pyramid.cu", "features.cu", "pyrlk.cu", "velocity.cu", "montecarlo.cu", "pairs.cu", "tracker.cu", "camera.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]

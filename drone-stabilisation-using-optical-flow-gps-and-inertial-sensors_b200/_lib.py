@@ -32,6 +32,13 @@ class PairCfg(C.Structure):
                 ("detect", C.c_int)]
 
 
+class Camera(C.Structure):
+    """ofb_camera: K without skew, OpenCV's distortion coefficients (k1 k2 p1 p2 k3 k4 k5 k6), the fixed-point
+    iteration count of the inverse lens model and the flow rate (u = (x_new - x_old) * rate)."""
+    _fields_ = [("fx", C.c_double), ("fy", C.c_double), ("cx", C.c_double), ("cy", C.c_double), ("dist", C.c_double * 8),
+                ("n_dist", C.c_int), ("iterations", C.c_int), ("rate", C.c_double)]
+
+
 class ImuSample(C.Structure):
     _fields_ = [("d", C.c_double), ("n", C.c_double * 3), ("w", C.c_double * 3), ("t", C.c_double * 3)]
 
@@ -129,6 +136,9 @@ _SIGNATURES = {
     "ofb_tracker_step": (i32, [vp, vp, i32, sz, vp, vp, vp, vp, vp, vp, vp]),
     "ofb_tracker_graph_info": (i32, [vp, C.POINTER(u64), C.POINTER(i32)]),
     "ofb_tracker_render_mask": (i32, [vp, vp, i32, i32, i32, i32, vp]),
+    "ofb_tracker_set_camera": (i32, [vp, C.POINTER(Camera)]),
+    "ofb_undistort_points": (i32, [vp, C.POINTER(Camera), vp, i32, vp, vp]),
+    "ofb_frame_pairs_cam": (i32, [vp, C.POINTER(PairCfg), C.POINTER(Camera), i32, vp, vp, i32, sz, vp, vp, vp, vp, vp, vp, vp]),
     "ofb_mc_sweep": (i32, [vp, vp, i32, i32, vp, vp, i32, u64, u64, u64, i32, vp, vp, vp]),
     "ofb_mc_sweep_multi": (i32, [vp, i32, vp, i32, i32, vp, vp, i32, u64, u64, u64, i32, vp]),
     "ofb_mc_feas": (i32, [vp, vp, i32, vp, vp, u64, u64, u64, vp]),

@@ -87,7 +87,7 @@ struct PinBuf {
 #define OFB_DEV_ASSERT(c) ((void)0)
 #endif
 
-enum { OFB_NSCRATCH = 25, OFB_NSTAGES = 5, OFB_NSTAGE_EV = 6, OFB_NFUNC_SLOTS = 32 };
+enum { OFB_NSCRATCH = 26, OFB_NSTAGES = 5, OFB_NSTAGE_EV = 6, OFB_NFUNC_SLOTS = 32 };
 
 struct ofb_ctx {
     int device = 0;
@@ -140,7 +140,8 @@ enum {
     SC_OUT0, SC_OUT1, SC_OUT2, SC_OUT3,                      // staged outputs
     SC_CAND, SC_CANDCNT, SC_SEL, SC_GRID, SC_PTS0, SC_PTS1, SC_STAT, SC_ERR,
     SC_MC0, SC_MC1, SC_MC2, SC_TMP0, SC_TMP1, SC_TMP2,
-    SC_FRAMES                                                // device staging of host frames (ofb_frame_pairs)
+    SC_FRAMES,                                               // device staging of host frames (ofb_frame_pairs)
+    SC_CALIB                                                 // calibrated tracks of ofb_frame_pairs_cam
 };
 
 struct ofb_pyr {

@@ -14,6 +14,7 @@
 #include "features.cuh"
 #include "pyrlk.cuh"
 #include "velocity_device.cuh"
+#include "camera.cuh"
 
 namespace {
 
@@ -35,9 +36,9 @@ struct TrackLoader {
     __device__ bool dist(int, int, double&) const { return false; }
 };
 
-__global__ void __launch_bounds__(OFB_SOLVE_THREADS)
-pair_solve_kernel(TrackLoader ld, int variant, const ofb_imu_sample* __restrict__ imu, ofb_pair_result* __restrict__ out,
-                  const FeatImageState* __restrict__ det)
+template <class Loader>
+__device__ __forceinline__ void pair_solve(const Loader& ld, int variant, const ofb_imu_sample* __restrict__ imu,
+                                           ofb_pair_result* __restrict__ out, const FeatImageState* __restrict__ det)
 {
     int f = blockIdx.x;
     const ofb_imu_sample& s = imu[f];
@@ -53,12 +54,35 @@ pair_solve_kernel(TrackLoader ld, int variant, const ofb_imu_sample* __restrict_
     }
 }
 
+__global__ void __launch_bounds__(OFB_SOLVE_THREADS)
+pair_solve_kernel(TrackLoader ld, int variant, const ofb_imu_sample* __restrict__ imu, ofb_pair_result* __restrict__ out,
+                  const FeatImageState* __restrict__ det)
+{
+    pair_solve(ld, variant, imu, out, det);
+}
+
+// With a calibrated camera: every tracked point is undistorted once into xu (the solve reads each point twice), then
+// solved from there.
+__global__ void __launch_bounds__(OFB_SOLVE_THREADS)
+pair_solve_cam_kernel(TrackLoader tl, ofb_camera cam, double4* __restrict__ xu, int variant,
+                      const ofb_imu_sample* __restrict__ imu, ofb_pair_result* __restrict__ out,
+                      const FeatImageState* __restrict__ det)
+{
+    const int f = blockIdx.x, n = tl.end(f);
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        const size_t o = (size_t)f * tl.stride + i;
+        if (tl.status[o]) xu[o] = ofb_calibrate(cam, tl.next[2 * o], tl.next[2 * o + 1], tl.prev[2 * o], tl.prev[2 * o + 1]);
+    }
+    __syncthreads();
+    pair_solve(CalibLoader{xu, tl.stride, tl.status, tl.counts, tl.counts_stride, 0}, variant, imu, out, det);
+}
+
 }  // namespace
 
 // Stages 1b-4 for pairs [c0, c0+n) whose level-0 frames already sit in pp/pn (images 0..n-1 of each).
 // Sequence layout (pn == pp): pp holds n+1 consecutive frames of one stream, pair i = (image i, image i+1), so every
 // interior frame's pyramid is built once and serves as "next" of one pair and "prev" of the following one.
-static int run_pairs_chunk(ofb_ctx* ctx, const ofb_pair_cfg* cfg, ofb_pyr* pp, ofb_pyr* pn, int n, int c0,
+static int run_pairs_chunk(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, ofb_pyr* pp, ofb_pyr* pn, int n, int c0,
                            const ofb_imu_sample* dimu, const int* counts_in, float* d_prev, float* d_next, uint8_t* d_stat,
                            ofb_pair_result* d_res, bool mark)
 {
@@ -121,7 +145,13 @@ static int run_pairs_chunk(ofb_ctx* ctx, const ofb_pair_cfg* cfg, ofb_pyr* pp, o
                           cfg->max_level, cfg->max_count, cfg->eps, 0, cfg->min_eig_thr, cn, cs, ctx->scratch[SC_ERR].as<float>()));
     STAGE_MARK(4);
     TrackLoader ld{cp, cn, cs, counts, counts_stride, (size_t)K, cfg->cx, cfg->cy, cfg->pos_scale, cfg->flow_scale};
-    pair_solve_kernel<<<n, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, cfg->variant, dimu + c0, d_res + c0, st);
+    if (cam) {
+        OFB_TRY(ctx->scratch[SC_CALIB].reserve(sizeof(double4) * (size_t)n * K));
+        pair_solve_cam_kernel<<<n, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, *cam, ctx->scratch[SC_CALIB].as<double4>(), cfg->variant,
+                                                                       dimu + c0, d_res + c0, st);
+    } else {
+        pair_solve_kernel<<<n, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, cfg->variant, dimu + c0, d_res + c0, st);
+    }
     OFB_LAUNCH_CHECK(ctx);
     STAGE_MARK(5);
 #undef STAGE_MARK
@@ -133,7 +163,17 @@ extern "C" int ofb_frame_pairs(ofb_ctx* ctx, const ofb_pair_cfg* cfg, int n_pair
                                const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
                                ofb_pair_result* results, float* prev_pts, float* next_pts, uint8_t* status)
 {
+    return ofb_frame_pairs_cam(ctx, cfg, nullptr, n_pairs, prev, next, pitch, image_stride, imu, pts_in, n_in, results, prev_pts,
+                               next_pts, status);
+}
+
+extern "C" int ofb_frame_pairs_cam(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, int n_pairs,
+                                   const uint8_t* prev, const uint8_t* next, int pitch, size_t image_stride,
+                                   const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
+                                   ofb_pair_result* results, float* prev_pts, float* next_pts, uint8_t* status)
+{
     OFB_REQUIRE(ctx && cfg && prev && next && imu && results, "frame_pairs: null argument");
+    if (cam) OFB_TRY(ofb_camera_check(cam, "frame_pairs"));
     OFB_REQUIRE(n_pairs > 0 && n_pairs <= 65535, "frame_pairs: n_pairs must be in 1..65535");
     const int w = cfg->width, h = cfg->height, K = cfg->max_corners;
     OFB_REQUIRE(w > 0 && h > 0 && pitch >= w, "frame_pairs: bad image geometry");
@@ -237,7 +277,7 @@ extern "C" int ofb_frame_pairs(ofb_ctx* ctx, const ofb_pair_cfg* cfg, int n_pair
             if (!seq)
                 OFB_TRY(ofb_pyr_prepare(c, &c->pair_pyr[slot][1], d_nextf + (size_t)c0 * stride_d, w, h, pitch_d, stride_d, n,
                                         chunk, cfg->max_level, false));
-            OFB_TRY(run_pairs_chunk(c, cfg, c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
+            OFB_TRY(run_pairs_chunk(c, cfg, cam, c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
                                     (const ofb_imu_sample*)dimu, counts_in, d_prev, d_next, d_stat, (ofb_pair_result*)o[3].dev, false));
             c0 += n;
         }
@@ -273,7 +313,7 @@ extern "C" int ofb_frame_pairs(ofb_ctx* ctx, const ofb_pair_cfg* cfg, int n_pair
             if (!seq)
                 OFB_TRY(ofb_pyr_prepare(c, &c->pair_pyr[slot][1], next + (size_t)c0 * image_stride, w, h, pitch, image_stride, n, per,
                                         cfg->max_level, false));
-            OFB_TRY(run_pairs_chunk(c, cfg, c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
+            OFB_TRY(run_pairs_chunk(c, cfg, cam, c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
                                     (const ofb_imu_sample*)dimu, counts_in, d_prev, d_next, d_stat, (ofb_pair_result*)o[3].dev, false));
         }
         ctx->launches += tw->launches - tw0;
@@ -286,7 +326,7 @@ extern "C" int ofb_frame_pairs(ofb_ctx* ctx, const ofb_pair_cfg* cfg, int n_pair
                             seq ? n_pairs + 1 : n_pairs, cfg->max_level, false));
     if (!seq)
         OFB_TRY(ofb_pyr_prepare(ctx, &ctx->pair_pyr[0][1], next, w, h, pitch, image_stride, n_pairs, n_pairs, cfg->max_level, false));
-    OFB_TRY(run_pairs_chunk(ctx, cfg, ctx->pair_pyr[0][0], seq ? ctx->pair_pyr[0][0] : ctx->pair_pyr[0][1], n_pairs, 0,
+    OFB_TRY(run_pairs_chunk(ctx, cfg, cam, ctx->pair_pyr[0][0], seq ? ctx->pair_pyr[0][0] : ctx->pair_pyr[0][1], n_pairs, 0,
                             (const ofb_imu_sample*)dimu, counts_in, d_prev, d_next, d_stat, (ofb_pair_result*)o[3].dev, ctx->profile));
     int rc = ofb_finish_out(ctx, o, 4);
     if (rc == OFB_OK && ctx->profile) {

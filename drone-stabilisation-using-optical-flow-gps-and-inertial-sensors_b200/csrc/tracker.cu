@@ -19,6 +19,7 @@
 #include "features.cuh"
 #include "pyrlk.cuh"
 #include "velocity_device.cuh"
+#include "camera.cuh"
 
 struct ofb_tracker {
     ofb_ctx* ctx = nullptr;
@@ -65,6 +66,11 @@ struct ofb_tracker {
     cudaEvent_t ev_filt = nullptr, ev_sol = nullptr, ev_sol_join = nullptr;
     bool sol_pending = false;
     int plain_steps = 0;               // steps run launch by launch since creation (scratch arenas are sized by them)
+    // calibrated camera (ofb_tracker_set_camera): the filter kernel reads it from cam_dev, which is written in stream order,
+    // so a graph captured with a camera replays whatever camera is current; calib holds the kept points' (x, y, ux, uy)
+    bool has_cam = false;
+    ofb_camera cam_host;
+    DevBuf cam_dev, calib;
     uint64_t graph_steps = 0;
 };
 
@@ -80,6 +86,7 @@ struct TrackerDev {
     double* vlast;                                                  // [S][3]
     int cap;
     int variant; double cx, cy, ps, fs;
+    const ofb_camera* cam; double4* calib;                          // calibrated camera (NULL: the pinhole cx, cy, ps, fs)
     double max_speed, dummy; int gate_mode; double gate_T;
     int min_solve, min_features, topup_mode, max_features;
     int have_prev;
@@ -164,8 +171,14 @@ track_filter_solve_kernel(TrackerDev T, const ofb_imu_sample* __restrict__ imu, 
             }
             if (keep && T.have_prev && T.gate_mode != OFB_GATE_NONE && have_prior) { // node:238-245, of_module.py:125-131
                 const float dx = qx - px, dy = qy - py;
-                const double r = r_tilde_point(((double)qx - T.cx) * T.ps, ((double)qy - T.cy) * T.ps, (double)dx * T.fs,
-                                               (double)dy * T.fs, n3, vp);
+                double r;
+                if (T.cam) {
+                    const double4 xu = ofb_calibrate(*T.cam, qx, qy, px, py);
+                    r = r_tilde_point(xu.x, xu.y, xu.z, xu.w, n3, vp);
+                } else {
+                    r = r_tilde_point(((double)qx - T.cx) * T.ps, ((double)qy - T.cy) * T.ps, (double)dx * T.fs, (double)dy * T.fs,
+                                      n3, vp);
+                }
                 keep = T.gate_mode == OFB_GATE_R_GE ? r >= T.gate_T : r <= T.gate_T;
             }
         }
@@ -186,6 +199,13 @@ track_filter_solve_kernel(TrackerDev T, const ofb_imu_sample* __restrict__ imu, 
         kept += tot;
         __syncthreads();
     }
+    // calibrated camera: the kept points are undistorted once more, in their compacted order, for the solve (it reads
+    // every point twice); keeping the gate's values instead would hold them across the compaction and spill
+    if (PART != 2 && T.cam && T.have_prev)
+        for (int i = tid; i < kept; i += OFB_SOLVE_THREADS) {
+            const size_t o = base + i;
+            T.calib[o] = ofb_calibrate(*T.cam, T.kept_next[2 * o], T.kept_next[2 * o + 1], T.kept_prev[2 * o], T.kept_prev[2 * o + 1]);
+        }
     if (PART != 2) {
         // tracked: every lane of a warp holds its warp's total; sum over warps
         if (lane == 0) wtot[warp] = tracked;
@@ -197,9 +217,13 @@ track_filter_solve_kernel(TrackerDev T, const ofb_imu_sample* __restrict__ imu, 
     }
     OfbSolveOut o;
     const bool solve = T.have_prev && kept >= T.min_solve && kept > 0;
-    if (PART != 1 && solve) {
-        KeptLoader ld{T.kept_prev, T.kept_next, kept, (size_t)T.cap, T.cx, T.cy, T.ps, T.fs};
-        o = ofb_block_solve(ld, s, T.variant, im.d, im.n, im.w, im.t, vp);    // vp: MODULE's per-point distances (of_module.py:125)
+    if (PART != 1 && solve) {                                         // vp: MODULE's per-point distances (of_module.py:125)
+        if (T.cam) {
+            o = ofb_block_solve(CalibLoader{T.calib, (size_t)T.cap, nullptr, nullptr, 0, kept}, s, T.variant, im.d, im.n, im.w, im.t, vp);
+        } else {
+            KeptLoader ld{T.kept_prev, T.kept_next, kept, (size_t)T.cap, T.cx, T.cy, T.ps, T.fs};
+            o = ofb_block_solve(ld, s, T.variant, im.d, im.n, im.w, im.t, vp);
+        }
     }
     // the detector's per-image state and (for streams that will top up) its min-distance cell grid start clean
     if (PART != 2 && kept <= T.min_features)
@@ -444,7 +468,8 @@ extern "C" int ofb_tracker_destroy(ofb_tracker* t)
     if (t->ev_join) cudaEventDestroy(t->ev_join);
     if (t->ev_lk) cudaEventDestroy(t->ev_lk);
     if (t->ev_pyr) cudaEventDestroy(t->ev_pyr);
-    DevBuf* bufs[] = {&t->counts, &t->nxt, &t->status, &t->err, &t->kept_prev, &t->det, &t->vlast, &t->mask, &t->hw, &t->bgr, &t->dev_io};
+    DevBuf* bufs[] = {&t->counts, &t->nxt, &t->status, &t->err, &t->kept_prev, &t->det, &t->vlast, &t->mask, &t->hw, &t->bgr, &t->dev_io,
+                      &t->cam_dev, &t->calib};
     for (DevBuf* b : bufs) b->release();
     delete t;
     return OFB_OK;
@@ -622,6 +647,7 @@ static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitc
     T.kept_prev = t->kept_prev.as<float>(); T.kept_next = Pn;
     T.count = count; T.need = need; T.kept = keptn; T.count0 = count + 3 * S; T.vlast = t->vlast.as<double>();
     T.cap = cap; T.variant = pc.variant; T.cx = pc.cx; T.cy = pc.cy; T.ps = pc.pos_scale; T.fs = pc.flow_scale;
+    T.cam = t->has_cam ? t->cam_dev.as<ofb_camera>() : nullptr; T.calib = t->calib.as<double4>();
     T.max_speed = cfg.max_speed; T.dummy = cfg.dummy_value; T.gate_mode = cfg.gate_mode; T.gate_T = cfg.gate_T;
     T.min_solve = cfg.min_solve; T.min_features = cfg.min_features; T.topup_mode = cfg.topup_mode; T.max_features = K;
     T.have_prev = t->have_prev ? 1 : 0;
@@ -887,6 +913,33 @@ extern "C" int ofb_tracker_step(ofb_tracker* t, const uint8_t* frames, int pitch
     }
     t->plain_steps++;
     return tracker_step_launches(t, frames, pitch, image_stride, imu, v_prior, results, pts_out, n_out, kept_prev, kept_next);
+}
+
+extern "C" int ofb_tracker_set_camera(ofb_tracker* t, const ofb_camera* cam)
+{
+    OFB_REQUIRE(t, "tracker_set_camera: null tracker");
+    if (cam) OFB_TRY(ofb_camera_check(cam, "tracker_set_camera"));
+    ofb_ctx* ctx = t->ctx;
+    OFB_CUDA(cudaSetDevice(ctx->device));
+    if (cam) {
+        OFB_TRY(t->cam_dev.reserve(sizeof(ofb_camera)));
+        OFB_TRY(t->calib.reserve(sizeof(double4) * (size_t)t->cfg.n_streams * t->cap));
+        // Stream order on the context's stream places the update behind the filter kernels of every step enqueued so far
+        // (the only readers of the camera; a split solve reads the calibrated points its filter wrote) and in front of
+        // the next step's, whether that step is launched or replayed from a graph. A pageable source is staged before
+        // cudaMemcpyAsync returns.
+        t->cam_host = *cam;
+        OFB_CUDA(cudaMemcpyAsync(t->cam_dev.p, &t->cam_host, sizeof(ofb_camera), cudaMemcpyHostToDevice, ctx->stream));
+    }
+    if (t->has_cam != (cam != nullptr)) {
+        // attaching or detaching changes the filter kernel's arguments: graphs captured before are rebuilt (no graph is in
+        // flight: a replayed step synchronises before it returns)
+        for (int i = 0; i < 2; ++i)
+            for (int j = 0; j < 2; ++j)
+                if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
+        t->has_cam = cam != nullptr;
+    }
+    return OFB_OK;
 }
 
 /* steps replayed from a CUDA graph so far (0 when graphs are off or were never eligible); *conditional_out = 1 when

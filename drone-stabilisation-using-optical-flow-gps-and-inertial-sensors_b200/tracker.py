@@ -13,7 +13,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from .vision import make_pair_cfg
+from .vision import as_camera, make_pair_cfg
 
 
 class StreamTracker:
@@ -30,12 +30,13 @@ class StreamTracker:
           while it is exactly zero the gate is skipped (r_tilde is 1 for every point then).
     max_speed > 0 enables of.static_immobile(new, old, max_speed, d, dummy_value).
     borrow_frames: device-resident grey frames (CUDA tensors) are tracked in place instead of being copied into the
-    tracker; pass a NEW tensor every step (the tracker keeps the previous one alive; do not overwrite it)."""
+    tracker; pass a NEW tensor every step (the tracker keeps the previous one alive; do not overwrite it).
+    camera: (K, D, rate[, iterations]) or vision.make_camera(...) -- see set_camera."""
 
     def __init__(self, width, height, max_features=100, min_features=20, n_streams=1, feature_params=None,
                  lk_params=None, topup="exp", mask_radius=30, bgr=False, variant="exp", principal=None,
                  scaling=1.0, flow_scaling=None, max_speed=0.0, dummy_value=float("nan"), gate=None, min_solve=3,
-                 min_eig_thr=1e-4, borrow_frames=False, v_init=None, ctx=None):
+                 min_eig_thr=1e-4, borrow_frames=False, v_init=None, camera=None, ctx=None):
         fp = dict(qualityLevel=0.01, minDistance=10, blockSize=7)
         fp.update(feature_params or {})
         lk = dict(winSize=(15, 15), maxLevel=3, criteria=(3, 20, 0.03))
@@ -71,6 +72,8 @@ class StreamTracker:
         cap = C.c_int()
         _lib.check(self.ctx.lib.ofb_tracker_capacity(self.h, C.byref(cap)))
         self.capacity = cap.value
+        if camera is not None:
+            self.set_camera(camera)
 
     def close(self):
         if getattr(self, "h", None) and getattr(self.ctx, "h", None):
@@ -95,6 +98,13 @@ class StreamTracker:
 
     def reset(self):
         _lib.check(self.ctx.lib.ofb_tracker_reset(self.h))
+
+    def set_camera(self, camera):
+        """Calibrated camera of every stream from the next step on: the gate and the solve see
+        x = undistort(p_new), u = (undistort(p_new) - undistort(p_old)) * rate (OpenCV's lens model, iterations default to
+        vision.CAMERA_ITERATIONS) instead of the pinhole principal / scaling / flow_scaling. None detaches it."""
+        cam = as_camera(camera)
+        _lib.check(self.ctx.lib.ofb_tracker_set_camera(self.h, C.byref(cam) if cam is not None else None))
 
     def set_points(self, points):
         """points: one (N,2)/(N,1,2) array per stream (or a single array when n_streams == 1)."""
@@ -201,6 +211,11 @@ class FleetTracker:
         out = self.local.step(frames_local, imu_local, **kw)
         self.last = out[0] if isinstance(out, tuple) else out
         return out
+
+    def set_camera(self, camera):
+        """StreamTracker.set_camera on this rank's streams"""
+        if self.local is not None:
+            self.local.set_camera(camera)
 
     def gather_velocities(self):
         """(n_streams, 3) velocities of the last step on every rank; rows of streams that did not solve (or have not

@@ -7,6 +7,8 @@ module (SURVEY 8b):
         velocity_measurment_node:133; evaluate_exp.py:98; of_module.py:88; of_library.py:249
     cvtColor(img, COLOR_BGR2GRAY)  velocity_measurment_node:113
     frame_pairs(...)               the per-frame dataflow of node:224-267 / evaluate_exp.py:77-120, batched
+    undistortPoints(src, cameraMatrix, distCoeffs, R=None, P=None)    cv2.undistortPoints (5 iterations)
+    undistortPointsIter(src, cameraMatrix, distCoeffs, R, P, criteria) with the COUNT criterion
 """
 import ctypes as C
 
@@ -179,6 +181,96 @@ def calcOpticalFlowPyrLK(prevImg, nextImg, prevPts, nextPts=None, status=None, e
             p.close()
 
 
+# The velocity paths iterate the inverse lens model 20 times by default, cv2.undistortPoints 5 times. For a wide-angle
+# k1 = -0.3 lens (1280x720, fx = 900 px) 5 iterations leave up to 0.48 px of error at the image edge against the
+# converged inverse, 10 leave 1.3e-3 px and 20 leave 1e-8 px. A bias of 0.48 px enters x and u directly and with them
+# the velocity, so the velocity paths pay for the converged inverse (the cost is a few hundred fp64 operations per point).
+CAMERA_ITERATIONS = 20
+
+
+def make_camera(cameraMatrix, distCoeffs, rate=1.0, iterations=CAMERA_ITERATIONS):
+    """ofb_camera from OpenCV's K (3x3, no skew) and D (None or 4, 5 or 8 coefficients: plumb_bob /
+    rational_polynomial). rate: u = (x_new - x_old) * rate (the frame rate 1/dt for a velocity in m/s)."""
+    K = np.asarray(cameraMatrix, dtype=np.float64)
+    if K.size != 9:
+        raise ValueError("cameraMatrix must be 3x3")
+    K = K.reshape(3, 3)
+    D = np.zeros(0) if distCoeffs is None else np.asarray(distCoeffs, dtype=np.float64).ravel()
+    if len(D) not in (0, 4, 5, 8):
+        raise ValueError("distCoeffs must have 0, 4, 5 or 8 entries (got %d)" % len(D))
+    if not (np.isfinite(K).all() and np.isfinite(D).all() and np.isfinite(rate)):
+        raise ValueError("non-finite camera parameter")
+    if K[0, 1] != 0 or K[1, 0] != 0 or K[2, 0] != 0 or K[2, 1] != 0 or K[2, 2] != 1:
+        raise ValueError("cameraMatrix must be [[fx, 0, cx], [0, fy, cy], [0, 0, 1]] (no skew)")
+    if K[0, 0] <= 0 or K[1, 1] <= 0:
+        raise ValueError("fx and fy must be positive")
+    if not rate > 0:
+        raise ValueError("rate must be positive")
+    if int(iterations) != iterations or not 1 <= int(iterations) <= 1000:
+        raise ValueError("iterations must be an integer in 1..1000")
+    cam = _lib.Camera()
+    cam.fx, cam.fy, cam.cx, cam.cy = K[0, 0], K[1, 1], K[0, 2], K[1, 2]
+    cam.dist[:len(D)] = [float(d) for d in D]
+    cam.n_dist, cam.iterations, cam.rate = len(D), int(iterations), float(rate)
+    return cam
+
+
+def as_camera(camera):
+    """The `camera=` argument of the velocity paths: None, an _lib.Camera, or (K, D, rate[, iterations])."""
+    if camera is None or isinstance(camera, _lib.Camera):
+        return camera
+    if not isinstance(camera, (tuple, list)) or len(camera) not in (3, 4):
+        raise ValueError("camera must be (K, D, rate) or (K, D, rate, iterations)")
+    return make_camera(*camera)
+
+
+def _rectification(R, P):
+    """H = P[:, :3] @ R as cvUndistortPointsInternal forms it (sums in index order), None for the identity."""
+    if R is None and P is None:
+        return None
+    Rm = np.eye(3) if R is None else np.asarray(R, dtype=np.float64)
+    if Rm.size != 9:
+        raise ValueError("R must be 3x3")
+    Rm = Rm.reshape(3, 3)
+    if P is None:
+        H = Rm.copy()
+    else:
+        Pm = np.asarray(P, dtype=np.float64)
+        if Pm.shape not in ((3, 3), (3, 4)):
+            raise ValueError("P must be 3x3 or 3x4")
+        H = np.zeros((3, 3))
+        for i in range(3):
+            for j in range(3):
+                H[i, j] = Pm[i, 0] * Rm[0, j] + Pm[i, 1] * Rm[1, j] + Pm[i, 2] * Rm[2, j]
+    if not np.isfinite(H).all():
+        raise ValueError("non-finite entry in R or P")
+    return np.ascontiguousarray(H)
+
+
+def undistortPointsIter(src, cameraMatrix, distCoeffs, R, P, criteria, ctx=None):
+    """cv2.undistortPointsIter with the COUNT criterion: src (N,2) / (N,1,2) float32 or float64 pixels ->
+    (N,1,2) of src's dtype (normalised coordinates, or rectified / projected by P @ R)."""
+    typ, count, _ = criteria
+    if int(typ) & TERM_CRITERIA_EPS or not int(typ) & TERM_CRITERIA_COUNT:
+        raise ValueError("only the TERM_CRITERIA_COUNT criterion is supported")
+    a = np.asarray(src)
+    if a.dtype not in (np.float32, np.float64) or a.ndim not in (2, 3) or a.shape[-1] != 2 or (a.ndim == 3 and a.shape[1] != 1):
+        raise ValueError("src must be an (N,2) or (N,1,2) float32 / float64 array")
+    cam = make_camera(cameraMatrix, distCoeffs, 1.0, count)
+    H = _rectification(R, P)
+    pts = np.ascontiguousarray(a.reshape(-1, 2), dtype=np.float64)
+    out = np.empty_like(pts)
+    if len(pts):
+        ctx = ctx or _lib.default_context()
+        _lib.check(ctx.lib.ofb_undistort_points(ctx.h, C.byref(cam), _lib.ptr(pts), len(pts), _lib.ptr(H), _lib.ptr(out)))
+    return out.astype(a.dtype).reshape(-1, 1, 2)
+
+
+def undistortPoints(src, cameraMatrix, distCoeffs, R=None, P=None, ctx=None):
+    """cv2.undistortPoints: 5 fixed-point iterations of the inverse lens model."""
+    return undistortPointsIter(src, cameraMatrix, distCoeffs, R, P, (TERM_CRITERIA_COUNT, 5, 0), ctx=ctx)
+
+
 def make_pair_cfg(width, height, max_corners, quality=0.01, min_distance=10.0, block_size=7, win=(15, 15),
                   max_level=3, criteria=(3, 20, 0.03), min_eig_thr=1e-4, variant="node", principal=None,
                   pos_scale=1.0, flow_scale=1.0, detect=True):
@@ -197,13 +289,17 @@ def make_pair_cfg(width, height, max_corners, quality=0.01, min_distance=10.0, b
     return cfg
 
 
-def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, ctx=None, on_overflow="raise"):
+def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, ctx=None, on_overflow="raise", camera=None):
     """Batched detect(+)track+solve. prev/nxt: (N,H,W) uint8 numpy arrays (host) or CUDA tensors;
     imu: structured array _lib.IMU_DTYPE (N,). Returns a structured array _lib.RESULT_DTYPE (N,)
     (and prev_pts, next_pts, status when want_tracks).
     A pair whose detector ran out of candidate slots (plateau images: more than w*h/4 + 1024 local maxima above the
     quality threshold) carries `flags & PAIR_OVERFLOW`; its feature list is truncated, so by default that raises
-    OfbError (on_overflow="ignore" returns the flagged records instead)."""
+    OfbError (on_overflow="ignore" returns the flagged records instead).
+    camera: (K, D, rate[, iterations]) or make_camera(...): the solve sees x = undistort(p_new) and
+    u = (undistort(p_new) - undistort(p_old)) * rate instead of cfg's pinhole (cx, cy, pos_scale, flow_scale);
+    iterations default to CAMERA_ITERATIONS."""
+    cam = as_camera(camera)
     ctx = ctx or _lib.default_context()
     n = int(prev.shape[0])
     h, w = int(prev.shape[1]), int(prev.shape[2])
@@ -225,9 +321,9 @@ def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, 
     if pts_in is not None:
         pts_in = np.ascontiguousarray(pts_in, dtype=np.float32)
         n_in = np.ascontiguousarray(n_in, dtype=np.int32)
-    _lib.check(ctx.lib.ofb_frame_pairs(ctx.h, C.byref(cfg), n, _lib.ptr(prev), _lib.ptr(nxt), w, w * h, _lib.ptr(imu),
-                                       _lib.ptr(pts_in), _lib.ptr(n_in), _lib.ptr(res), _lib.ptr(pp), _lib.ptr(pn),
-                                       _lib.ptr(st)))
+    _lib.check(ctx.lib.ofb_frame_pairs_cam(ctx.h, C.byref(cfg), C.byref(cam) if cam is not None else None, n, _lib.ptr(prev),
+                                           _lib.ptr(nxt), w, w * h, _lib.ptr(imu), _lib.ptr(pts_in), _lib.ptr(n_in), _lib.ptr(res),
+                                           _lib.ptr(pp), _lib.ptr(pn), _lib.ptr(st)))
     if on_overflow == "raise" and (res["flags"] & _lib.PAIR_OVERFLOW).any():
         bad = np.nonzero(res["flags"] & _lib.PAIR_OVERFLOW)[0]
         raise _lib.OfbError("frame_pairs: detector candidate buffer overflowed for pair(s) %s: the image has more than "
@@ -237,12 +333,13 @@ def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, 
     return res
 
 
-def frame_sequence(frames, imu, cfg, want_tracks=False, ctx=None, on_overflow="raise"):
+def frame_sequence(frames, imu, cfg, want_tracks=False, ctx=None, on_overflow="raise", camera=None):
     """One camera stream: frames (N+1,H,W) uint8 -> N consecutive pairs (frame i, frame i+1), as
     velocity_measurment_node:224-267 sees them (it keeps the previous callback's image). Passing the two views
     of ONE buffer lets the library upload every frame and build its pyramid once (`next == prev + image_stride`
     is the C ABI's sequence layout, include/ofb200.h)."""
     if isinstance(frames, np.ndarray):
         frames = np.ascontiguousarray(frames, dtype=np.uint8)
-    return frame_pairs(frames[:-1], frames[1:], imu, cfg, want_tracks=want_tracks, ctx=ctx, on_overflow=on_overflow)
+    return frame_pairs(frames[:-1], frames[1:], imu, cfg, want_tracks=want_tracks, ctx=ctx, on_overflow=on_overflow,
+                       camera=camera)
 

@@ -212,6 +212,38 @@ int ofb_frame_pairs(ofb_ctx* ctx, const ofb_pair_cfg* cfg, int n_pairs,
                     const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
                     ofb_pair_result* results, float* prev_pts, float* next_pts, uint8_t* status);
 
+/* ---- calibrated camera: OpenCV's pinhole + lens model (plumb_bob / rational_polynomial), no skew.
+ *      Replaces the ideal pinhole of velocity_measurment_node:229-235 (one focal length, no distortion) with what a
+ *      caller of the reference's style does with cv2.undistortPoints before the solve. Per point, in fp64 and in
+ *      OpenCV's operation order (cvUndistortPointsInternal):
+ *        x0 = (px - cx) * (1/fx), y0 = (py - cy) * (1/fy); x = x0, y = y0;
+ *        `iterations` times (none when n_dist == 0): r2 = x^2 + y^2,
+ *          icdist = (1 + ((k6 r2 + k5) r2 + k4) r2) / (1 + ((k3 r2 + k2) r2 + k1) r2)  (icdist < 0: x = x0, y = y0, stop)
+ *          x = (x0 - (2 p1 x y + p2 (r2 + 2 x^2))) icdist,  y = (y0 - (p1 (r2 + 2 y^2) + 2 p2 x y)) icdist
+ *      A ROS camera_info maps as fx = K[0], fy = K[4], cx = K[2], cy = K[5], dist = D (plumb_bob: 5 coefficients,
+ *      rational_polynomial: 8). cv2.undistortPoints iterates 5 times; wide-angle lenses need more to converge (a
+ *      k1 = -0.3 lens: 0.48 px left after 5, 1e-8 px after 20), so the struct carries the count explicitly. */
+typedef struct {
+    double fx, fy, cx, cy;   /* camera matrix K (no skew); fx, fy > 0 */
+    double dist[8];          /* k1 k2 p1 p2 k3 k4 k5 k6 (OpenCV order); entries past n_dist are ignored */
+    int    n_dist;           /* 0, 4, 5 or 8 */
+    int    iterations;       /* fixed-point iterations of the inverse lens model, 1..1000 */
+    double rate;             /* > 0: u = (x_new - x_old) * rate, e.g. the frame rate 1/dt */
+} ofb_camera;
+
+/* cv2.undistortPointsIter(src, K, D, R, P, (TERM_CRITERIA_COUNT, iterations, 0)): pts and out are n x 2 float64 (host
+ * or device; out may equal pts). H = P[:, :3] @ R as 9 row-major doubles, applied as OpenCV does
+ * (x, y) <- ((H0 x + H1 y + H2) w, (H3 x + H4 y + H5) w), w = 1 / (H6 x + H7 y + H8); NULL = identity.
+ * cam->rate is not used here. */
+int ofb_undistort_points(ofb_ctx* ctx, const ofb_camera* cam, const double* pts, int n, const double* H, double* out);
+
+/* ofb_frame_pairs with a calibrated camera: x = undistort(p_new), u = (undistort(p_new) - undistort(p_old)) * rate
+ * (cfg->cx / cy / pos_scale / flow_scale are not used). cam == NULL is exactly ofb_frame_pairs. */
+int ofb_frame_pairs_cam(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, int n_pairs,
+                        const uint8_t* prev, const uint8_t* next, int pitch, size_t image_stride,
+                        const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
+                        ofb_pair_result* results, float* prev_pts, float* next_pts, uint8_t* status);
+
 /* ---- feature lifecycle around the tracker (SURVEY 8f-2): the point set of every camera stream stays on the
  *      device between frames. One step does what the reference's per-frame loops do around the tracker
  *      (flight_experiments/evaluate_exp.py:97-120, velocity_measurment_node:129-172 and 224-260,
@@ -309,6 +341,11 @@ int ofb_tracker_step(ofb_tracker* trk, const uint8_t* frames, int pitch, size_t 
  * measured slower than letting its kernels exit at once, hence opt-in. *steps_out = steps replayed from a graph so
  * far; *conditional_out (may be NULL) = 1 when those graphs use the conditional node. */
 int ofb_tracker_graph_info(const ofb_tracker* trk, uint64_t* steps_out, int* conditional_out);
+/* Attach a calibrated camera to every stream of the tracker (cam == NULL detaches it: back to cfg.pair's pinhole).
+ * From the next ofb_tracker_step on, the r_tilde gate, the MODULE variant's per-point distances and the solve see
+ * x = undistort(p_new), u = (undistort(p_new) - undistort(p_old)) * rate; static_immobile stays in pixels. A step
+ * already enqueued (split solve, deferred top-up, graph replay) keeps the camera it was enqueued with. */
+int ofb_tracker_set_camera(ofb_tracker* trk, const ofb_camera* cam);
 /* the exclusion mask OFB_TOPUP_APPEND_MASKED would use for `n` points (n x 2 float32): mask_out h x w u8
  * (1 = allowed, 0 = inside a circle). Exposed for parity tests against cv2.circle. */
 int ofb_tracker_render_mask(ofb_ctx* ctx, const float* pts, int n, int radius, int w, int h, uint8_t* mask_out);

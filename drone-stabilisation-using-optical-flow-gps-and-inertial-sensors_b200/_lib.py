@@ -139,6 +139,9 @@ _SIGNATURES = {
     "ofb_tracker_set_camera": (i32, [vp, C.POINTER(Camera)]),
     "ofb_undistort_points": (i32, [vp, C.POINTER(Camera), vp, i32, vp, vp]),
     "ofb_frame_pairs_cam": (i32, [vp, C.POINTER(PairCfg), C.POINTER(Camera), i32, vp, vp, i32, sz, vp, vp, vp, vp, vp, vp, vp]),
+    "ofb_pyrlk_fb": (i32, [vp, vp, i32, vp, i32, vp, i32, i32, i32, i32, i32, f64, f64, f64, vp, vp, vp, vp]),
+    "ofb_frame_pairs_fb": (i32, [vp, C.POINTER(PairCfg), C.POINTER(Camera), f64, i32, vp, vp, i32, sz, vp, vp, vp, vp, vp, vp, vp]),
+    "ofb_tracker_set_fb_check": (i32, [vp, f64]),
     "ofb_mc_sweep": (i32, [vp, vp, i32, i32, vp, vp, i32, u64, u64, u64, i32, vp, vp, vp]),
     "ofb_mc_sweep_multi": (i32, [vp, i32, vp, i32, i32, vp, vp, i32, u64, u64, u64, i32, vp]),
     "ofb_mc_feas": (i32, [vp, vp, i32, vp, vp, u64, u64, u64, vp]),

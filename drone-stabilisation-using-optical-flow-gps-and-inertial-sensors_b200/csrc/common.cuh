@@ -230,7 +230,8 @@ enum {
     FS_LK = 17,
     FS_PYR_TOP = 18,
     FS_SELECT16 = 19,        // + {256, 512, 1024 threads}: non-portable cluster size (16) allowed     (3 slots)
-    FS_MARCH_LEAN = 22       // + 2 * {bs 3, 7, 12} + write_map: the marching kernel without the general row loop (6 slots)
+    FS_MARCH_LEAN = 22,      // + 2 * {bs 3, 7, 12} + write_map: the marching kernel without the general row loop (6 slots)
+    FS_LK_FB = 28            // the generic LK kernel with the forward-backward check
 };
 // Raises a kernel's dynamic shared-memory limit on the context's device when this context has not done so yet.
 template <class F>

@@ -82,7 +82,8 @@ pair_solve_cam_kernel(TrackLoader tl, ofb_camera cam, double4* __restrict__ xu, 
 // Stages 1b-4 for pairs [c0, c0+n) whose level-0 frames already sit in pp/pn (images 0..n-1 of each).
 // Sequence layout (pn == pp): pp holds n+1 consecutive frames of one stream, pair i = (image i, image i+1), so every
 // interior frame's pyramid is built once and serves as "next" of one pair and "prev" of the following one.
-static int run_pairs_chunk(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, ofb_pyr* pp, ofb_pyr* pn, int n, int c0,
+static int run_pairs_chunk(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, double fb_max_err, ofb_pyr* pp, ofb_pyr* pn,
+                           int n, int c0,
                            const ofb_imu_sample* dimu, const int* counts_in, float* d_prev, float* d_next, uint8_t* d_stat,
                            ofb_pair_result* d_res, bool mark)
 {
@@ -142,7 +143,8 @@ static int run_pairs_chunk(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_came
     STAGE_MARK(3);
     OFB_TRY(ctx->scratch[SC_ERR].reserve(sizeof(float) * (size_t)n * K));
     OFB_TRY(ofb_lk_device(ctx, pp, 0, 1, pn, seq ? 1 : 0, 1, n, cp, counts, counts_stride, K, (size_t)K, cfg->win_w, cfg->win_h,
-                          cfg->max_level, cfg->max_count, cfg->eps, 0, cfg->min_eig_thr, cn, cs, ctx->scratch[SC_ERR].as<float>()));
+                          cfg->max_level, cfg->max_count, cfg->eps, 0, cfg->min_eig_thr, cn, cs, ctx->scratch[SC_ERR].as<float>(),
+                          fb_max_err));
     STAGE_MARK(4);
     TrackLoader ld{cp, cn, cs, counts, counts_stride, (size_t)K, cfg->cx, cfg->cy, cfg->pos_scale, cfg->flow_scale};
     if (cam) {
@@ -172,8 +174,18 @@ extern "C" int ofb_frame_pairs_cam(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const 
                                    const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
                                    ofb_pair_result* results, float* prev_pts, float* next_pts, uint8_t* status)
 {
+    return ofb_frame_pairs_fb(ctx, cfg, cam, 0.0, n_pairs, prev, next, pitch, image_stride, imu, pts_in, n_in, results, prev_pts,
+                              next_pts, status);
+}
+
+extern "C" int ofb_frame_pairs_fb(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, double fb_max_err, int n_pairs,
+                                  const uint8_t* prev, const uint8_t* next, int pitch, size_t image_stride,
+                                  const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
+                                  ofb_pair_result* results, float* prev_pts, float* next_pts, uint8_t* status)
+{
     OFB_REQUIRE(ctx && cfg && prev && next && imu && results, "frame_pairs: null argument");
     if (cam) OFB_TRY(ofb_camera_check(cam, "frame_pairs"));
+    OFB_REQUIRE(ofb_fb_thr_ok(fb_max_err), "frame_pairs: fb_max_err must be >= 0 (0 = no forward-backward check)");
     OFB_REQUIRE(n_pairs > 0 && n_pairs <= 65535, "frame_pairs: n_pairs must be in 1..65535");
     const int w = cfg->width, h = cfg->height, K = cfg->max_corners;
     OFB_REQUIRE(w > 0 && h > 0 && pitch >= w, "frame_pairs: bad image geometry");
@@ -277,7 +289,7 @@ extern "C" int ofb_frame_pairs_cam(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const 
             if (!seq)
                 OFB_TRY(ofb_pyr_prepare(c, &c->pair_pyr[slot][1], d_nextf + (size_t)c0 * stride_d, w, h, pitch_d, stride_d, n,
                                         chunk, cfg->max_level, false));
-            OFB_TRY(run_pairs_chunk(c, cfg, cam, c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
+            OFB_TRY(run_pairs_chunk(c, cfg, cam, fb_max_err, c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
                                     (const ofb_imu_sample*)dimu, counts_in, d_prev, d_next, d_stat, (ofb_pair_result*)o[3].dev, false));
             c0 += n;
         }
@@ -313,7 +325,7 @@ extern "C" int ofb_frame_pairs_cam(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const 
             if (!seq)
                 OFB_TRY(ofb_pyr_prepare(c, &c->pair_pyr[slot][1], next + (size_t)c0 * image_stride, w, h, pitch, image_stride, n, per,
                                         cfg->max_level, false));
-            OFB_TRY(run_pairs_chunk(c, cfg, cam, c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
+            OFB_TRY(run_pairs_chunk(c, cfg, cam, fb_max_err, c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
                                     (const ofb_imu_sample*)dimu, counts_in, d_prev, d_next, d_stat, (ofb_pair_result*)o[3].dev, false));
         }
         ctx->launches += tw->launches - tw0;
@@ -326,7 +338,7 @@ extern "C" int ofb_frame_pairs_cam(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const 
                             seq ? n_pairs + 1 : n_pairs, cfg->max_level, false));
     if (!seq)
         OFB_TRY(ofb_pyr_prepare(ctx, &ctx->pair_pyr[0][1], next, w, h, pitch, image_stride, n_pairs, n_pairs, cfg->max_level, false));
-    OFB_TRY(run_pairs_chunk(ctx, cfg, cam, ctx->pair_pyr[0][0], seq ? ctx->pair_pyr[0][0] : ctx->pair_pyr[0][1], n_pairs, 0,
+    OFB_TRY(run_pairs_chunk(ctx, cfg, cam, fb_max_err, ctx->pair_pyr[0][0], seq ? ctx->pair_pyr[0][0] : ctx->pair_pyr[0][1], n_pairs, 0,
                             (const ofb_imu_sample*)dimu, counts_in, d_prev, d_next, d_stat, (ofb_pair_result*)o[3].dev, ctx->profile));
     int rc = ofb_finish_out(ctx, o, 4);
     if (rc == OFB_OK && ctx->profile) {

@@ -65,10 +65,13 @@ __device__ __forceinline__ void bil_weights(float a, float b, int& w00, int& w01
     w11 = 16384 - w00 - w01 - w10;
 }
 
+// FB: the forward-backward check, as lk_track_fast2_kernel<true>.
+template <bool FB>
 __global__ void __launch_bounds__(LK_WARPS * 32)
 lk_track_kernel(LKParams P, const float* __restrict__ prev_pts, float* __restrict__ next_pts,
                 uint8_t* __restrict__ status, float* __restrict__ err, const int* __restrict__ counts,
-                int counts_stride, int n_uniform, size_t pts_stride, size_t warp_smem)
+                int counts_stride, int n_uniform, size_t pts_stride, size_t warp_smem, double fb_thr,
+                float* __restrict__ fb_err)
 {
     extern __shared__ __align__(16) unsigned char lk_smem[];
     int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -94,127 +97,153 @@ lk_track_kernel(LKParams P, const float* __restrict__ prev_pts, float* __restric
     float errv = 0.f;
     int pimg = P.prev_image0 + pair * P.prev_image_step, nimg = P.next_image0 + pair * P.next_image_step;
 
-    for (int level = P.nlev - 1; level >= 0; --level) {
-        const uint8_t* I = P.prev.base[level] + (size_t)pimg * P.prev.stride[level];
-        const uint8_t* J = P.next.base[level] + (size_t)nimg * P.next.stride[level];
-        const int w = P.prev.w[level], h = P.prev.h[level];
-        const int ipitch = P.prev.pitch[level], jpitch = P.next.pitch[level];
-        float sc = 1.f / (float)(1 << level);
-        float ppx = ptx * sc, ppy = pty * sc;
-        if (level == P.nlev - 1) {
-            if (P.flags & OFB_LK_USE_INITIAL_FLOW) { nx = nx * sc; ny = ny * sc; }
-            else { nx = ppx; ny = ppy; }
-        } else { nx = nx * 2.f; ny = ny * 2.f; }
-        float px = ppx - hwx, py = ppy - hwy;
-        int ix = __float2int_rd(px), iy = __float2int_rd(py);
-        if (ix < -winW || ix >= w || iy < -winH || iy >= h) {
-            if (level == 0) { st = false; errv = 0.f; }
-            continue;
-        }
-        float a = px - (float)ix, b = py - (float)iy;
-        int w00, w01, w10, w11;
-        bil_weights(a, b, w00, w01, w10, w11);
-        // ---- template: stage I neighbourhood, Scharr under the window, interpolated patches ----
-        __syncwarp();
-        stage_block(I, w, h, ipitch, ix - 1, iy - 1, RW, RH, reg, RP, lane);
-        __syncwarp();
-        for (int i = lane; i < DW * DH; i += 32) {
-            int r = i / DW, c = i - r * DW;
-            int X = ix + c, Y = iy + r;
-            short gx = 0, gy = 0;
-            if ((unsigned)X < (unsigned)w && (unsigned)Y < (unsigned)h) {
-                const uint8_t* r0 = reg + r * RP + c;          // (X-1, Y-1)
-                const uint8_t* r1 = r0 + RP;
-                const uint8_t* r2 = r1 + RP;
-                gx = (short)(3 * ((int)r0[2] - (int)r0[0]) + 10 * ((int)r1[2] - (int)r1[0]) + 3 * ((int)r2[2] - (int)r2[0]));
-                gy = (short)(3 * ((int)r2[0] - (int)r0[0]) + 10 * ((int)r2[1] - (int)r0[1]) + 3 * ((int)r2[2] - (int)r0[2]));
+#pragma unroll
+    for (int pass = 0; pass < (FB ? 2 : 1); ++pass) {
+        const bool bwd = FB && pass == 1;
+        for (int level = P.nlev - 1; level >= 0; --level) {
+            const uint8_t* I = bwd ? P.next.base[level] + (size_t)nimg * P.next.stride[level]
+                                   : P.prev.base[level] + (size_t)pimg * P.prev.stride[level];
+            const uint8_t* J = bwd ? P.prev.base[level] + (size_t)pimg * P.prev.stride[level]
+                                   : P.next.base[level] + (size_t)nimg * P.next.stride[level];
+            const int w = P.prev.w[level], h = P.prev.h[level];
+            const int ipitch = bwd ? P.next.pitch[level] : P.prev.pitch[level], jpitch = bwd ? P.prev.pitch[level] : P.next.pitch[level];
+            float sc = 1.f / (float)(1 << level);
+            float ppx = ptx * sc, ppy = pty * sc;
+            if (level == P.nlev - 1) {
+                if (!bwd && (P.flags & OFB_LK_USE_INITIAL_FLOW)) { nx = nx * sc; ny = ny * sc; }
+                else { nx = ppx; ny = ppy; }
+            } else { nx = nx * 2.f; ny = ny * 2.f; }
+            float px = ppx - hwx, py = ppy - hwy;
+            int ix = __float2int_rd(px), iy = __float2int_rd(py);
+            if (ix < -winW || ix >= w || iy < -winH || iy >= h) {
+                if (level == 0) { st = false; errv = 0.f; }
+                continue;
             }
-            ders[i] = gx; ders[DW * DH + i] = gy;
-        }
-        __syncwarp();
-        int iA11 = 0, iA12 = 0, iA22 = 0;
-        for (int i = lane; i < npx; i += 32) {
-            int y = i / winW, x = i - y * winW;
-            const uint8_t* s0 = reg + (y + 1) * RP + x + 1;
-            const uint8_t* s1 = s0 + RP;
-            int iv = ((int)s0[0] * w00 + (int)s0[1] * w01 + (int)s1[0] * w10 + (int)s1[1] * w11 + (1 << 8)) >> 9;
-            const short* d0 = ders + y * DW + x;
-            const short* d1 = d0 + DW;
-            int gx = ((int)d0[0] * w00 + (int)d0[1] * w01 + (int)d1[0] * w10 + (int)d1[1] * w11 + (1 << 13)) >> 14;
-            const short* e0 = d0 + DW * DH;
-            const short* e1 = e0 + DW;
-            int gy = ((int)e0[0] * w00 + (int)e0[1] * w01 + (int)e1[0] * w10 + (int)e1[1] * w11 + (1 << 13)) >> 14;
-            pat[i] = (short)iv; pat[npx + i] = (short)gx; pat[2 * npx + i] = (short)gy;
-            iA11 += gx * gx; iA12 += gx * gy; iA22 += gy * gy;
-        }
-        float A11 = (float)warp_sum_ll(iA11) * FLT_SCALE;
-        float A12 = (float)warp_sum_ll(iA12) * FLT_SCALE;
-        float A22 = (float)warp_sum_ll(iA22) * FLT_SCALE;
-        float D = __fsub_rn(__fmul_rn(A11, A22), __fmul_rn(A12, A12));
-        float dd = A11 - A22;
-        float minEig = (A22 + A11 - sqrtf(__fadd_rn(__fmul_rn(dd, dd), __fmul_rn(__fmul_rn(4.f, A12), A12)))) /
-                       (float)(2 * winW * winH);
-        if ((double)minEig < P.min_eig_thr || D < 1.1920928955078125e-7f) {
-            if (level == 0) st = false;
-            continue;
-        }
-        D = 1.f / D;
-        float qx = nx - hwx, qy = ny - hwy;
-        float pdx = 0.f, pdy = 0.f;
-        bool lost = false;
-        for (int j = 0; j < P.max_count; ++j) {
-            int jx = __float2int_rd(qx), jy = __float2int_rd(qy);
-            if (jx < -winW || jx >= w || jy < -winH || jy >= h) { lost = true; break; }
-            a = qx - (float)jx; b = qy - (float)jy;
+            float a = px - (float)ix, b = py - (float)iy;
+            int w00, w01, w10, w11;
             bil_weights(a, b, w00, w01, w10, w11);
+            // ---- template: stage I neighbourhood, Scharr under the window, interpolated patches ----
             __syncwarp();
-            stage_block(J, w, h, jpitch, jx, jy, DW, DH, reg, RP, lane);
+            stage_block(I, w, h, ipitch, ix - 1, iy - 1, RW, RH, reg, RP, lane);
             __syncwarp();
-            int ib1 = 0, ib2 = 0;
+            for (int i = lane; i < DW * DH; i += 32) {
+                int r = i / DW, c = i - r * DW;
+                int X = ix + c, Y = iy + r;
+                short gx = 0, gy = 0;
+                if ((unsigned)X < (unsigned)w && (unsigned)Y < (unsigned)h) {
+                    const uint8_t* r0 = reg + r * RP + c;          // (X-1, Y-1)
+                    const uint8_t* r1 = r0 + RP;
+                    const uint8_t* r2 = r1 + RP;
+                    gx = (short)(3 * ((int)r0[2] - (int)r0[0]) + 10 * ((int)r1[2] - (int)r1[0]) + 3 * ((int)r2[2] - (int)r2[0]));
+                    gy = (short)(3 * ((int)r2[0] - (int)r0[0]) + 10 * ((int)r2[1] - (int)r0[1]) + 3 * ((int)r2[2] - (int)r0[2]));
+                }
+                ders[i] = gx; ders[DW * DH + i] = gy;
+            }
+            __syncwarp();
+            int iA11 = 0, iA12 = 0, iA22 = 0;
             for (int i = lane; i < npx; i += 32) {
                 int y = i / winW, x = i - y * winW;
-                const uint8_t* s0 = reg + y * RP + x;
+                const uint8_t* s0 = reg + (y + 1) * RP + x + 1;
                 const uint8_t* s1 = s0 + RP;
-                int jv = ((int)s0[0] * w00 + (int)s0[1] * w01 + (int)s1[0] * w10 + (int)s1[1] * w11 + (1 << 8)) >> 9;
-                int diff = jv - (int)pat[i];
-                ib1 += diff * (int)pat[npx + i];
-                ib2 += diff * (int)pat[2 * npx + i];
+                int iv = ((int)s0[0] * w00 + (int)s0[1] * w01 + (int)s1[0] * w10 + (int)s1[1] * w11 + (1 << 8)) >> 9;
+                const short* d0 = ders + y * DW + x;
+                const short* d1 = d0 + DW;
+                int gx = ((int)d0[0] * w00 + (int)d0[1] * w01 + (int)d1[0] * w10 + (int)d1[1] * w11 + (1 << 13)) >> 14;
+                const short* e0 = d0 + DW * DH;
+                const short* e1 = e0 + DW;
+                int gy = ((int)e0[0] * w00 + (int)e0[1] * w01 + (int)e1[0] * w10 + (int)e1[1] * w11 + (1 << 13)) >> 14;
+                pat[i] = (short)iv; pat[npx + i] = (short)gx; pat[2 * npx + i] = (short)gy;
+                iA11 += gx * gx; iA12 += gx * gy; iA22 += gy * gy;
             }
-            float b1 = (float)warp_sum_ll(ib1) * FLT_SCALE;
-            float b2 = (float)warp_sum_ll(ib2) * FLT_SCALE;
-            float dx = __fmul_rn(__fsub_rn(__fmul_rn(A12, b2), __fmul_rn(A22, b1)), D);
-            float dy = __fmul_rn(__fsub_rn(__fmul_rn(A12, b1), __fmul_rn(A11, b2)), D);
-            qx += dx; qy += dy;
-            nx = qx + hwx; ny = qy + hwy;
-            if ((double)dx * (double)dx + (double)dy * (double)dy <= P.eps) break;
-            if (j > 0 && fabsf(dx + pdx) < 0.01f && fabsf(dy + pdy) < 0.01f) {
-                nx -= dx * 0.5f; ny -= dy * 0.5f;
-                break;
+            float A11 = (float)warp_sum_ll(iA11) * FLT_SCALE;
+            float A12 = (float)warp_sum_ll(iA12) * FLT_SCALE;
+            float A22 = (float)warp_sum_ll(iA22) * FLT_SCALE;
+            float D = __fsub_rn(__fmul_rn(A11, A22), __fmul_rn(A12, A12));
+            float dd = A11 - A22;
+            float minEig = (A22 + A11 - sqrtf(__fadd_rn(__fmul_rn(dd, dd), __fmul_rn(__fmul_rn(4.f, A12), A12)))) /
+                           (float)(2 * winW * winH);
+            if ((double)minEig < P.min_eig_thr || D < 1.1920928955078125e-7f) {
+                if (level == 0) st = false;
+                continue;
             }
-            pdx = dx; pdy = dy;
-        }
-        if (lost && level == 0) st = false;
-        if (st && level == 0) {
-            float rx = nx - hwx, ry = ny - hwy;
-            int jx = __float2int_rd(rx), jy = __float2int_rd(ry);
-            if (jx < -winW || jx >= w || jy < -winH || jy >= h) { st = false; }
-            else {
-                a = rx - (float)jx; b = ry - (float)jy;
+            D = 1.f / D;
+            float qx = nx - hwx, qy = ny - hwy;
+            float pdx = 0.f, pdy = 0.f;
+            bool lost = false;
+            for (int j = 0; j < P.max_count; ++j) {
+                int jx = __float2int_rd(qx), jy = __float2int_rd(qy);
+                if (jx < -winW || jx >= w || jy < -winH || jy >= h) { lost = true; break; }
+                a = qx - (float)jx; b = qy - (float)jy;
                 bil_weights(a, b, w00, w01, w10, w11);
                 __syncwarp();
                 stage_block(J, w, h, jpitch, jx, jy, DW, DH, reg, RP, lane);
                 __syncwarp();
-                int ie = 0;
+                int ib1 = 0, ib2 = 0;
                 for (int i = lane; i < npx; i += 32) {
                     int y = i / winW, x = i - y * winW;
                     const uint8_t* s0 = reg + y * RP + x;
                     const uint8_t* s1 = s0 + RP;
                     int jv = ((int)s0[0] * w00 + (int)s0[1] * w01 + (int)s1[0] * w10 + (int)s1[1] * w11 + (1 << 8)) >> 9;
-                    ie += abs(jv - (int)pat[i]);
+                    int diff = jv - (int)pat[i];
+                    ib1 += diff * (int)pat[npx + i];
+                    ib2 += diff * (int)pat[2 * npx + i];
                 }
-                errv = (float)__reduce_add_sync(0xffffffffu, ie) * (1.f / (float)(32 * winW * winH));
+                float b1 = (float)warp_sum_ll(ib1) * FLT_SCALE;
+                float b2 = (float)warp_sum_ll(ib2) * FLT_SCALE;
+                float dx = __fmul_rn(__fsub_rn(__fmul_rn(A12, b2), __fmul_rn(A22, b1)), D);
+                float dy = __fmul_rn(__fsub_rn(__fmul_rn(A12, b1), __fmul_rn(A11, b2)), D);
+                qx += dx; qy += dy;
+                nx = qx + hwx; ny = qy + hwy;
+                if ((double)dx * (double)dx + (double)dy * (double)dy <= P.eps) break;
+                if (j > 0 && fabsf(dx + pdx) < 0.01f && fabsf(dy + pdy) < 0.01f) {
+                    nx -= dx * 0.5f; ny -= dy * 0.5f;
+                    break;
+                }
+                pdx = dx; pdy = dy;
+            }
+            if (lost && level == 0) st = false;
+            if (st && level == 0) {
+                float rx = nx - hwx, ry = ny - hwy;
+                int jx = __float2int_rd(rx), jy = __float2int_rd(ry);
+                if (jx < -winW || jx >= w || jy < -winH || jy >= h) { st = false; }
+                else if (!bwd) {                  // (the backward pass only needs the status of this bounds test)
+                    a = rx - (float)jx; b = ry - (float)jy;
+                    bil_weights(a, b, w00, w01, w10, w11);
+                    __syncwarp();
+                    stage_block(J, w, h, jpitch, jx, jy, DW, DH, reg, RP, lane);
+                    __syncwarp();
+                    int ie = 0;
+                    for (int i = lane; i < npx; i += 32) {
+                        int y = i / winW, x = i - y * winW;
+                        const uint8_t* s0 = reg + y * RP + x;
+                        const uint8_t* s1 = s0 + RP;
+                        int jv = ((int)s0[0] * w00 + (int)s0[1] * w01 + (int)s1[0] * w10 + (int)s1[1] * w11 + (1 << 8)) >> 9;
+                        ie += abs(jv - (int)pat[i]);
+                    }
+                    errv = (float)__reduce_add_sync(0xffffffffu, ie) * (1.f / (float)(32 * winW * winH));
+                }
             }
         }
+        if (FB && pass == 0) {
+            // the forward result is stored now and the starting point re-read at the end, so that neither stays in
+            // registers across the backward pass
+            if (lane == 0) {
+                OFB_DEV_ASSERT(feat >= 0 && feat < n && (gridDim.y == 1 || po < (size_t)(pair + 1) * pts_stride));
+                next_pts[2 * po] = nx; next_pts[2 * po + 1] = ny;
+                if (err) err[po] = st ? errv : 0.f;
+                if (!st) { status[po] = 0; if (fb_err) fb_err[po] = INFINITY; }
+            }
+            if (!st) return;
+            ptx = nx; pty = ny;
+        }
+    }
+    if (FB) {
+        if (lane == 0) {
+            const float d = fmaxf(fabsf(prev_pts[2 * po] - nx), fabsf(prev_pts[2 * po + 1] - ny));
+            status[po] = st && (double)d < fb_thr ? 1 : 0;
+            if (fb_err) fb_err[po] = st ? d : INFINITY;
+        }
+        return;
     }
     if (lane == 0) {
         OFB_DEV_ASSERT(feat >= 0 && feat < n && (gridDim.y == 1 || po < (size_t)(pair + 1) * pts_stride));   // (one pair: the stride is unused)
@@ -517,10 +546,15 @@ lk_track_fast_kernel(LKParams P, const float* __restrict__ prev_pts, float* __re
 //     evaluation OpenCV uses is only needed there).
 __device__ __forceinline__ unsigned int prmt(unsigned int a, unsigned int b, unsigned int sel) { return __byte_perm(a, b, sel); }
 
+// FB = the forward-backward check (ofb_pyrlk_fb): a feature whose forward track has status 1 is tracked back from
+// where it landed, in the same warp, and keeps status 1 only when the backward track has status 1 too and ends within
+// fb_thr of the starting point (max-norm of the fp32 difference, compared in fp64). next_pts and err are the forward
+// pass's. FB = false is the plain LK kernel.
+template <bool FB>
 __global__ void __launch_bounds__(LKF_WARPS * 32, 32 / LKF_WARPS)
 lk_track_fast2_kernel(const __grid_constant__ LKParams P, const float* __restrict__ prev_pts, float* __restrict__ next_pts,
                       uint8_t* __restrict__ status, float* __restrict__ err, const int* __restrict__ counts,
-                      int counts_stride, int n_uniform, size_t pts_stride)
+                      int counts_stride, int n_uniform, size_t pts_stride, double fb_thr, float* __restrict__ fb_err)
 {
     const int lane = threadIdx.x & 31;
     const int pair = blockIdx.y;
@@ -531,7 +565,7 @@ lk_track_fast2_kernel(const __grid_constant__ LKParams P, const float* __restric
     const int winW = P.win_w, winH = P.win_h;
     const int r = lane >> 1, hh = lane & 1;
     const size_t po = (size_t)pair * pts_stride + feat;
-    const float ptx = prev_pts[2 * po], pty = prev_pts[2 * po + 1];
+    float ptx = prev_pts[2 * po], pty = prev_pts[2 * po + 1];
     float nx = 0.f, ny = 0.f;
     if (P.flags & OFB_LK_USE_INITIAL_FLOW) { nx = next_pts[2 * po]; ny = next_pts[2 * po + 1]; }
     const float hwx = P.hwx, hwy = P.hwy;
@@ -543,182 +577,208 @@ lk_track_fast2_kernel(const __grid_constant__ LKParams P, const float* __restric
     float errv = 0.f;
     const int pimg = P.prev_image0 + pair * P.prev_image_step, nimg = P.next_image0 + pair * P.next_image_step;
 
-    for (int level = P.nlev - 1; level >= 0; --level) {
-        const LKLevel& L = P.lv[level];
-        const int w = L.w, h = L.h, ipitch = L.ipitch, jpitch = L.jpitch;
-        const uint8_t* __restrict__ I = L.I + (size_t)pimg * L.istride;
-        const uint8_t* __restrict__ J = L.J + (size_t)nimg * L.jstride;
-        const int ilow = ((((unsigned long long)I) & 3ull) == 0 && (ipitch & 3) == 0) ? 0 : 4;   // see load12
-        const int jlow = ((((unsigned long long)J) & 3ull) == 0 && (jpitch & 3) == 0) ? 0 : 4;
-        const float sc = __int_as_float((127 - level) << 23);        // 2^-level
-        const float ppx = ptx * sc, ppy = pty * sc;
-        if (level == P.nlev - 1) {
-            if (P.flags & OFB_LK_USE_INITIAL_FLOW) { nx = nx * sc; ny = ny * sc; }
-            else { nx = ppx; ny = ppy; }
-        } else { nx = nx * 2.f; ny = ny * 2.f; }
-        const float px = ppx - hwx, py = ppy - hwy;
-        const int ix = __float2int_rd(px), iy = __float2int_rd(py);
-        if (ix < -winW || ix >= w || iy < -winH || iy >= h) {
-            if (level == 0) { st = false; errv = 0.f; }
-            continue;
-        }
-        float a = px - (float)ix, b = py - (float)iy;
-        int w00, w01, w10, w11;
-        bil_weights(a, b, w00, w01, w10, w11);
-        // ---- template ---------------------------------------------------------------------------------
-        // rows iy+r-1 (A), iy+r (B), iy+r+1 (C); byte j of a row segment <-> column ix + 8hh - 1 + j, j = 0..11
-        const bool icol = ix - 1 >= ilow && ix + 8 + 15 <= w, irow = iy - 1 >= 0 && iy + 16 < h;
-        const bool ifast = icol && irow;
-        const int X0 = ix - 1 + 8 * hh;
-        unsigned int A0, A1, A2, B0, B1, B2, C0, C1, C2;
-        {
-            int ya = iy + r - 1, yb = iy + r, yc = iy + r + 1;
-            if (!irow) { ya = refl101(ya, h); yb = refl101(yb, h); yc = refl101(yc, h); }
-            load12(I, w, ipitch, X0, ya, icol, A0, A1, A2);
-            load12(I, w, ipitch, X0, yb, icol, B0, B1, B2);
-            load12(I, w, ipitch, X0, yc, icol, C0, C1, C2);
-        }
-        // Scharr, two columns per word. pa/pb/pc[i] = columns (2i, 2i+1) of rows A/B/C as 16-bit halves.
-        //   t0 = 3 (A + C) + 10 B            <= 4080                      (vertical smoothing, for gx)
-        //   t1 = C - A + 256                 in [1, 511]                  (vertical difference, for gy)
-        //   gx[k] + 4096 = t0[k+2] - t0[k] + 4096,   gy[k] + 4096 = 3 (t1[k] + t1[k+2]) + 10 t1[k+1]
-        unsigned int GX[5], GY[5];                   // (g[2i], g[2i+1]) + 4096 per half, Scharr at column ix + 8hh + k
-        {
-            unsigned int t0[6], t1[6];
-            const unsigned int aw[3] = {A0, A1, A2}, bw[3] = {B0, B1, B2}, cw[3] = {C0, C1, C2};
+    // FB: pass 1 tracks back from the forward result (I and J swap roles; the level geometry is shared, both pyramids
+    // have one size), with no initial flow
 #pragma unroll
-            for (int i = 0; i < 6; ++i) {
-                const unsigned int sel = (i & 1) ? 0x4342u : 0x4140u;
-                const unsigned int pa = prmt(aw[i >> 1], 0u, sel), pb = prmt(bw[i >> 1], 0u, sel), pc = prmt(cw[i >> 1], 0u, sel);
-                t0[i] = 3u * (pa + pc) + 10u * pb;
-                t1[i] = pc + 0x01000100u - pa;
+    for (int pass = 0; pass < (FB ? 2 : 1); ++pass) {
+        const bool bwd = FB && pass == 1;
+        for (int level = P.nlev - 1; level >= 0; --level) {
+            const LKLevel& L = P.lv[level];
+            const int w = L.w, h = L.h, ipitch = bwd ? L.jpitch : L.ipitch, jpitch = bwd ? L.ipitch : L.jpitch;
+            const uint8_t* __restrict__ I = bwd ? L.J + (size_t)nimg * L.jstride : L.I + (size_t)pimg * L.istride;
+            const uint8_t* __restrict__ J = bwd ? L.I + (size_t)pimg * L.istride : L.J + (size_t)nimg * L.jstride;
+            const int ilow = ((((unsigned long long)I) & 3ull) == 0 && (ipitch & 3) == 0) ? 0 : 4;   // see load12
+            const int jlow = ((((unsigned long long)J) & 3ull) == 0 && (jpitch & 3) == 0) ? 0 : 4;
+            const float sc = __int_as_float((127 - level) << 23);        // 2^-level
+            const float ppx = ptx * sc, ppy = pty * sc;
+            if (level == P.nlev - 1) {
+                if (!bwd && (P.flags & OFB_LK_USE_INITIAL_FLOW)) { nx = nx * sc; ny = ny * sc; }
+                else { nx = ppx; ny = ppy; }
+            } else { nx = nx * 2.f; ny = ny * 2.f; }
+            const float px = ppx - hwx, py = ppy - hwy;
+            const int ix = __float2int_rd(px), iy = __float2int_rd(py);
+            if (ix < -winW || ix >= w || iy < -winH || iy >= h) {
+                if (level == 0) { st = false; errv = 0.f; }
+                continue;
             }
-#pragma unroll
-            for (int i = 0; i < 5; ++i) {
-                GX[i] = t0[i + 1] + 0x10001000u - t0[i];
-                const unsigned int mid = prmt(t1[i], t1[i + 1], 0x5432u);            // (t1[2i+1], t1[2i+2])
-                GY[i] = 3u * (t1[i] + t1[i + 1]) + 10u * mid;
+            float a = px - (float)ix, b = py - (float)iy;
+            int w00, w01, w10, w11;
+            bil_weights(a, b, w00, w01, w10, w11);
+            // ---- template ---------------------------------------------------------------------------------
+            // rows iy+r-1 (A), iy+r (B), iy+r+1 (C); byte j of a row segment <-> column ix + 8hh - 1 + j, j = 0..11
+            const bool icol = ix - 1 >= ilow && ix + 8 + 15 <= w, irow = iy - 1 >= 0 && iy + 16 < h;
+            const bool ifast = icol && irow;
+            const int X0 = ix - 1 + 8 * hh;
+            unsigned int A0, A1, A2, B0, B1, B2, C0, C1, C2;
+            {
+                int ya = iy + r - 1, yb = iy + r, yc = iy + r + 1;
+                if (!irow) { ya = refl101(ya, h); yb = refl101(yb, h); yc = refl101(yc, h); }
+                load12(I, w, ipitch, X0, ya, icol, A0, A1, A2);
+                load12(I, w, ipitch, X0, yb, icol, B0, B1, B2);
+                load12(I, w, ipitch, X0, yc, icol, C0, C1, C2);
             }
-        }
-        if (!ifast) {       // OpenCV's derivative images are ZERO outside the image (a zero gradient is 4096 here)
-            const bool rowin = (unsigned)(iy + r) < (unsigned)h;
+            // Scharr, two columns per word. pa/pb/pc[i] = columns (2i, 2i+1) of rows A/B/C as 16-bit halves.
+            //   t0 = 3 (A + C) + 10 B            <= 4080                      (vertical smoothing, for gx)
+            //   t1 = C - A + 256                 in [1, 511]                  (vertical difference, for gy)
+            //   gx[k] + 4096 = t0[k+2] - t0[k] + 4096,   gy[k] + 4096 = 3 (t1[k] + t1[k+2]) + 10 t1[k+1]
+            unsigned int GX[5], GY[5];                   // (g[2i], g[2i+1]) + 4096 per half, Scharr at column ix + 8hh + k
+            {
+                unsigned int t0[6], t1[6];
+                const unsigned int aw[3] = {A0, A1, A2}, bw[3] = {B0, B1, B2}, cw[3] = {C0, C1, C2};
 #pragma unroll
-            for (int i = 0; i < 5; ++i) {
-                const bool okl = rowin && (unsigned)(ix + 8 * hh + 2 * i) < (unsigned)w;
-                const bool okh = rowin && (unsigned)(ix + 8 * hh + 2 * i + 1) < (unsigned)w;
-                const unsigned int keep = (okl ? 0x0000ffffu : 0u) | (okh ? 0xffff0000u : 0u);
-                const unsigned int zero = (okl ? 0u : 0x00001000u) | (okh ? 0u : 0x10000000u);
-                GX[i] = (GX[i] & keep) | zero; GY[i] = (GY[i] & keep) | zero;
-            }
-        }
-        int Cp[8], Gx[8], Gy[8];
-        int iA11 = 0, iA12 = 0, iA22 = 0;
-        {
-            // biased gradients of rows r (own) and r+1 (lane + 2), one value per column k = 0..8
-            int gxa[9], gya[9], gxb[9], gyb[9];
+                for (int i = 0; i < 6; ++i) {
+                    const unsigned int sel = (i & 1) ? 0x4342u : 0x4140u;
+                    const unsigned int pa = prmt(aw[i >> 1], 0u, sel), pb = prmt(bw[i >> 1], 0u, sel), pc = prmt(cw[i >> 1], 0u, sel);
+                    t0[i] = 3u * (pa + pc) + 10u * pb;
+                    t1[i] = pc + 0x01000100u - pa;
+                }
 #pragma unroll
-            for (int i = 0; i < 5; ++i) {
-                const unsigned int nxp = __shfl_down_sync(0xffffffffu, GX[i], 2), nyp = __shfl_down_sync(0xffffffffu, GY[i], 2);
-                gxa[2 * i] = (int)(GX[i] & 0xffffu); gya[2 * i] = (int)(GY[i] & 0xffffu);
-                gxb[2 * i] = (int)(nxp & 0xffffu); gyb[2 * i] = (int)(nyp & 0xffffu);
-                if (i < 4) {
-                    gxa[2 * i + 1] = (int)(GX[i] >> 16); gya[2 * i + 1] = (int)(GY[i] >> 16);
-                    gxb[2 * i + 1] = (int)(nxp >> 16); gyb[2 * i + 1] = (int)(nyp >> 16);
+                for (int i = 0; i < 5; ++i) {
+                    GX[i] = t0[i + 1] + 0x10001000u - t0[i];
+                    const unsigned int mid = prmt(t1[i], t1[i + 1], 0x5432u);            // (t1[2i+1], t1[2i+2])
+                    GY[i] = 3u * (t1[i] + t1[i + 1]) + 10u * mid;
                 }
             }
-            // template value: rows B, C from column ix + 8hh on = byte 1 of the segments; the same dp2a taps as the
-            // Newton loop (pixel k reads bytes k, k+1 of both rows)
-            const int Wt = (w00 & 0xffff) | (w01 << 16), Wb = (w10 & 0xffff) | (w11 << 16);
-            const unsigned int tt[4] = {__funnelshift_r(B0, B1, 8), __funnelshift_r(B0, B1, 16), __funnelshift_r(B1, B2, 8), __funnelshift_r(B1, B2, 16)};
-            const unsigned int uu[4] = {__funnelshift_r(C0, C1, 8), __funnelshift_r(C0, C1, 16), __funnelshift_r(C1, C2, 8), __funnelshift_r(C1, C2, 16)};
-            const int c0 = (1 << 13) - (4096 << 14);          // rounding constant minus the bias times the weight sum 2^14
+            if (!ifast) {       // OpenCV's derivative images are ZERO outside the image (a zero gradient is 4096 here)
+                const bool rowin = (unsigned)(iy + r) < (unsigned)h;
 #pragma unroll
-            for (int k = 0; k < 8; ++k) {
-                const int s_ = ((k >> 2) << 1) | (k & 1);
-                int iv;
-                if ((k & 2) == 0) { iv = dp2a_lo(Wt, tt[s_], 1 << 8); iv = dp2a_lo(Wb, uu[s_], iv); }
-                else { iv = dp2a_hi(Wt, tt[s_], 1 << 8); iv = dp2a_hi(Wb, uu[s_], iv); }
-                iv >>= 9;
-                int gx = (gxa[k] * w00 + gxa[k + 1] * w01 + gxb[k] * w10 + gxb[k + 1] * w11 + c0) >> 14;
-                int gy = (gya[k] * w00 + gya[k + 1] * w01 + gyb[k] * w10 + gyb[k + 1] * w11 + c0) >> 14;
-                if (!((vmask >> k) & 1u)) { gx = 0; gy = 0; }
-                Cp[k] = 256 - 512 * iv; Gx[k] = gx; Gy[k] = gy;
-                iA11 += gx * gx; iA12 += gx * gy; iA22 += gy * gy;
+                for (int i = 0; i < 5; ++i) {
+                    const bool okl = rowin && (unsigned)(ix + 8 * hh + 2 * i) < (unsigned)w;
+                    const bool okh = rowin && (unsigned)(ix + 8 * hh + 2 * i + 1) < (unsigned)w;
+                    const unsigned int keep = (okl ? 0x0000ffffu : 0u) | (okh ? 0xffff0000u : 0u);
+                    const unsigned int zero = (okl ? 0u : 0x00001000u) | (okh ? 0u : 0x10000000u);
+                    GX[i] = (GX[i] & keep) | zero; GY[i] = (GY[i] & keep) | zero;
+                }
             }
-        }
-        const float A11 = warp_sum_exact_f(iA11) * FLT_SCALE;
-        const float A12 = warp_sum_exact_f(iA12) * FLT_SCALE;
-        const float A22 = warp_sum_exact_f(iA22) * FLT_SCALE;
-        float D2 = __fsub_rn(__fmul_rn(A11, A22), __fmul_rn(A12, A12));
-        const float dd = A11 - A22;
-        const float minEig = (A22 + A11 - sqrtf(__fadd_rn(__fmul_rn(dd, dd), __fmul_rn(__fmul_rn(4.f, A12), A12)))) /
-                             (float)(2 * winW * winH);
-        if ((double)minEig < P.min_eig_thr || D2 < 1.1920928955078125e-7f) {
-            if (level == 0) st = false;
-            continue;
-        }
-        D2 = 1.f / D2;
-        float qx = nx - hwx, qy = ny - hwy;
-        float pdx = 0.f, pdy = 0.f;
-        bool lost = false;
-        unsigned int T0 = 0, T1 = 0, T2 = 0, U0 = 0, U1 = 0, U2 = 0;
-        int cjx = INT_MIN, cjy = INT_MIN;
-        for (int j = 0; j < P.max_count; ++j) {
-            const int jx = __float2int_rd(qx), jy = __float2int_rd(qy);
-            if (jx < -winW || jx >= w || jy < -winH || jy >= h) { lost = true; break; }
-            a = qx - (float)jx; b = qy - (float)jy;
-            bil_weights(a, b, w00, w01, w10, w11);
-            const int Wt = (w00 & 0xffff) | (w01 << 16), Wb = (w10 & 0xffff) | (w11 << 16);
-            if (jx != cjx || jy != cjy) {               // the patch rows stay in registers while the integer position holds
-                const bool jcol = jx >= jlow && jx + 8 + 16 <= w, jrow = jy >= 0 && jy + 15 < h;
-                OFB_DEV_ASSERT(!jrow || (jy + r >= 0 && jy + r < h)); load12(J, w, jpitch, jx + 8 * hh, jrow ? jy + r : refl101(jy + r, h), jcol, T0, T1, T2);
-                U0 = __shfl_down_sync(0xffffffffu, T0, 2); U1 = __shfl_down_sync(0xffffffffu, T1, 2);
-                U2 = __shfl_down_sync(0xffffffffu, T2, 2);
-                cjx = jx; cjy = jy;
+            int Cp[8], Gx[8], Gy[8];
+            int iA11 = 0, iA12 = 0, iA22 = 0;
+            {
+                // biased gradients of rows r (own) and r+1 (lane + 2), one value per column k = 0..8
+                int gxa[9], gya[9], gxb[9], gyb[9];
+#pragma unroll
+                for (int i = 0; i < 5; ++i) {
+                    const unsigned int nxp = __shfl_down_sync(0xffffffffu, GX[i], 2), nyp = __shfl_down_sync(0xffffffffu, GY[i], 2);
+                    gxa[2 * i] = (int)(GX[i] & 0xffffu); gya[2 * i] = (int)(GY[i] & 0xffffu);
+                    gxb[2 * i] = (int)(nxp & 0xffffu); gyb[2 * i] = (int)(nyp & 0xffffu);
+                    if (i < 4) {
+                        gxa[2 * i + 1] = (int)(GX[i] >> 16); gya[2 * i + 1] = (int)(GY[i] >> 16);
+                        gxb[2 * i + 1] = (int)(nxp >> 16); gyb[2 * i + 1] = (int)(nyp >> 16);
+                    }
+                }
+                // template value: rows B, C from column ix + 8hh on = byte 1 of the segments; the same dp2a taps as the
+                // Newton loop (pixel k reads bytes k, k+1 of both rows)
+                const int Wt = (w00 & 0xffff) | (w01 << 16), Wb = (w10 & 0xffff) | (w11 << 16);
+                const unsigned int tt[4] = {__funnelshift_r(B0, B1, 8), __funnelshift_r(B0, B1, 16), __funnelshift_r(B1, B2, 8), __funnelshift_r(B1, B2, 16)};
+                const unsigned int uu[4] = {__funnelshift_r(C0, C1, 8), __funnelshift_r(C0, C1, 16), __funnelshift_r(C1, C2, 8), __funnelshift_r(C1, C2, 16)};
+                const int c0 = (1 << 13) - (4096 << 14);          // rounding constant minus the bias times the weight sum 2^14
+#pragma unroll
+                for (int k = 0; k < 8; ++k) {
+                    const int s_ = ((k >> 2) << 1) | (k & 1);
+                    int iv;
+                    if ((k & 2) == 0) { iv = dp2a_lo(Wt, tt[s_], 1 << 8); iv = dp2a_lo(Wb, uu[s_], iv); }
+                    else { iv = dp2a_hi(Wt, tt[s_], 1 << 8); iv = dp2a_hi(Wb, uu[s_], iv); }
+                    iv >>= 9;
+                    int gx = (gxa[k] * w00 + gxa[k + 1] * w01 + gxb[k] * w10 + gxb[k + 1] * w11 + c0) >> 14;
+                    int gy = (gya[k] * w00 + gya[k + 1] * w01 + gyb[k] * w10 + gyb[k + 1] * w11 + c0) >> 14;
+                    if (!((vmask >> k) & 1u)) { gx = 0; gy = 0; }
+                    Cp[k] = 256 - 512 * iv; Gx[k] = gx; Gy[k] = gy;
+                    iA11 += gx * gx; iA12 += gx * gy; iA22 += gy * gy;
+                }
             }
-            int ib1 = 0, ib2 = 0;
-            LKF_FOR_PIXELS(T0, T1, T2, U0, U1, U2, Wt, Wb, {
-                ib1 += diff * Gx[k]; ib2 += diff * Gy[k];
-            })
-            const float b1 = warp_sum_exact_f(ib1) * FLT_SCALE;
-            const float b2 = warp_sum_exact_f(ib2) * FLT_SCALE;
-            const float dx = __fmul_rn(__fsub_rn(__fmul_rn(A12, b2), __fmul_rn(A22, b1)), D2);
-            const float dy = __fmul_rn(__fsub_rn(__fmul_rn(A12, b1), __fmul_rn(A11, b2)), D2);
-            qx += dx; qy += dy;
-            nx = qx + hwx; ny = qy + hwy;
-            // delta.ddot(delta) <= eps^2, evaluated in double by OpenCV: fp32 decides unless it is within 1e-6 of the bound
-            const float s2 = __fmaf_rn(dx, dx, __fmul_rn(dy, dy));
-            bool conv = s2 < P.eps_lo;
-            if (!conv && !(s2 > P.eps_hi)) conv = (double)dx * (double)dx + (double)dy * (double)dy <= P.eps;
-            if (conv) break;
-            if (j > 0 && fabsf(dx + pdx) < 0.01f && fabsf(dy + pdy) < 0.01f) {
-                nx -= dx * 0.5f; ny -= dy * 0.5f;
-                break;
+            const float A11 = warp_sum_exact_f(iA11) * FLT_SCALE;
+            const float A12 = warp_sum_exact_f(iA12) * FLT_SCALE;
+            const float A22 = warp_sum_exact_f(iA22) * FLT_SCALE;
+            float D2 = __fsub_rn(__fmul_rn(A11, A22), __fmul_rn(A12, A12));
+            const float dd = A11 - A22;
+            const float minEig = (A22 + A11 - sqrtf(__fadd_rn(__fmul_rn(dd, dd), __fmul_rn(__fmul_rn(4.f, A12), A12)))) /
+                                 (float)(2 * winW * winH);
+            if ((double)minEig < P.min_eig_thr || D2 < 1.1920928955078125e-7f) {
+                if (level == 0) st = false;
+                continue;
             }
-            pdx = dx; pdy = dy;
-        }
-        if (lost && level == 0) st = false;
-        if (st && level == 0) {
-            const float rx = nx - hwx, ry = ny - hwy;
-            const int jx = __float2int_rd(rx), jy = __float2int_rd(ry);
-            if (jx < -winW || jx >= w || jy < -winH || jy >= h) { st = false; }
-            else {
-                a = rx - (float)jx; b = ry - (float)jy;
+            D2 = 1.f / D2;
+            float qx = nx - hwx, qy = ny - hwy;
+            float pdx = 0.f, pdy = 0.f;
+            bool lost = false;
+            unsigned int T0 = 0, T1 = 0, T2 = 0, U0 = 0, U1 = 0, U2 = 0;
+            int cjx = INT_MIN, cjy = INT_MIN;
+            for (int j = 0; j < P.max_count; ++j) {
+                const int jx = __float2int_rd(qx), jy = __float2int_rd(qy);
+                if (jx < -winW || jx >= w || jy < -winH || jy >= h) { lost = true; break; }
+                a = qx - (float)jx; b = qy - (float)jy;
                 bil_weights(a, b, w00, w01, w10, w11);
                 const int Wt = (w00 & 0xffff) | (w01 << 16), Wb = (w10 & 0xffff) | (w11 << 16);
-                if (jx != cjx || jy != cjy) {
+                if (jx != cjx || jy != cjy) {               // the patch rows stay in registers while the integer position holds
                     const bool jcol = jx >= jlow && jx + 8 + 16 <= w, jrow = jy >= 0 && jy + 15 < h;
                     OFB_DEV_ASSERT(!jrow || (jy + r >= 0 && jy + r < h)); load12(J, w, jpitch, jx + 8 * hh, jrow ? jy + r : refl101(jy + r, h), jcol, T0, T1, T2);
                     U0 = __shfl_down_sync(0xffffffffu, T0, 2); U1 = __shfl_down_sync(0xffffffffu, T1, 2);
                     U2 = __shfl_down_sync(0xffffffffu, T2, 2);
+                    cjx = jx; cjy = jy;
                 }
-                int ie = 0;
+                int ib1 = 0, ib2 = 0;
                 LKF_FOR_PIXELS(T0, T1, T2, U0, U1, U2, Wt, Wb, {
-                    if ((vmask >> k) & 1u) ie += abs(diff);
+                    ib1 += diff * Gx[k]; ib2 += diff * Gy[k];
                 })
-                errv = (float)__reduce_add_sync(0xffffffffu, ie) * (1.f / (float)(32 * winW * winH));
+                const float b1 = warp_sum_exact_f(ib1) * FLT_SCALE;
+                const float b2 = warp_sum_exact_f(ib2) * FLT_SCALE;
+                const float dx = __fmul_rn(__fsub_rn(__fmul_rn(A12, b2), __fmul_rn(A22, b1)), D2);
+                const float dy = __fmul_rn(__fsub_rn(__fmul_rn(A12, b1), __fmul_rn(A11, b2)), D2);
+                qx += dx; qy += dy;
+                nx = qx + hwx; ny = qy + hwy;
+                // delta.ddot(delta) <= eps^2, evaluated in double by OpenCV: fp32 decides unless it is within 1e-6 of the bound
+                const float s2 = __fmaf_rn(dx, dx, __fmul_rn(dy, dy));
+                bool conv = s2 < P.eps_lo;
+                if (!conv && !(s2 > P.eps_hi)) conv = (double)dx * (double)dx + (double)dy * (double)dy <= P.eps;
+                if (conv) break;
+                if (j > 0 && fabsf(dx + pdx) < 0.01f && fabsf(dy + pdy) < 0.01f) {
+                    nx -= dx * 0.5f; ny -= dy * 0.5f;
+                    break;
+                }
+                pdx = dx; pdy = dy;
+            }
+            if (lost && level == 0) st = false;
+            if (st && level == 0) {
+                const float rx = nx - hwx, ry = ny - hwy;
+                const int jx = __float2int_rd(rx), jy = __float2int_rd(ry);
+                if (jx < -winW || jx >= w || jy < -winH || jy >= h) { st = false; }
+                else if (!bwd) {                  // (the backward pass only needs the status of this bounds test)
+                    a = rx - (float)jx; b = ry - (float)jy;
+                    bil_weights(a, b, w00, w01, w10, w11);
+                    const int Wt = (w00 & 0xffff) | (w01 << 16), Wb = (w10 & 0xffff) | (w11 << 16);
+                    if (jx != cjx || jy != cjy) {
+                        const bool jcol = jx >= jlow && jx + 8 + 16 <= w, jrow = jy >= 0 && jy + 15 < h;
+                        OFB_DEV_ASSERT(!jrow || (jy + r >= 0 && jy + r < h)); load12(J, w, jpitch, jx + 8 * hh, jrow ? jy + r : refl101(jy + r, h), jcol, T0, T1, T2);
+                        U0 = __shfl_down_sync(0xffffffffu, T0, 2); U1 = __shfl_down_sync(0xffffffffu, T1, 2);
+                        U2 = __shfl_down_sync(0xffffffffu, T2, 2);
+                    }
+                    int ie = 0;
+                    LKF_FOR_PIXELS(T0, T1, T2, U0, U1, U2, Wt, Wb, {
+                        if ((vmask >> k) & 1u) ie += abs(diff);
+                    })
+                    errv = (float)__reduce_add_sync(0xffffffffu, ie) * (1.f / (float)(32 * winW * winH));
+                }
             }
         }
+        if (FB && pass == 0) {
+            // the forward result is stored now and the starting point re-read at the end, so that neither stays in
+            // registers across the backward pass
+            if (lane == 0) {
+                OFB_DEV_ASSERT(feat >= 0 && feat < n && (gridDim.y == 1 || po < (size_t)(pair + 1) * pts_stride));
+                next_pts[2 * po] = nx; next_pts[2 * po + 1] = ny;
+                if (err) err[po] = st ? errv : 0.f;
+                if (!st) { status[po] = 0; if (fb_err) fb_err[po] = INFINITY; }
+            }
+            if (!st) return;
+            ptx = nx; pty = ny;
+        }
+    }
+    if (FB) {
+        if (lane == 0) {
+            const float d = fmaxf(fabsf(prev_pts[2 * po] - nx), fabsf(prev_pts[2 * po + 1] - ny));
+            status[po] = st && (double)d < fb_thr ? 1 : 0;
+            if (fb_err) fb_err[po] = st ? d : INFINITY;
+        }
+        return;
     }
     if (lane == 0) {
         OFB_DEV_ASSERT(feat >= 0 && feat < n && (gridDim.y == 1 || po < (size_t)(pair + 1) * pts_stride));   // (one pair: the stride is unused)
@@ -726,6 +786,12 @@ lk_track_fast2_kernel(const __grid_constant__ LKParams P, const float* __restric
         status[po] = st ? 1 : 0;
         if (err) err[po] = st ? errv : 0.f;
     }
+}
+
+__global__ void fill_inf_kernel(float* __restrict__ out, int n)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) out[i] = INFINITY;
 }
 
 }  // namespace
@@ -750,9 +816,10 @@ static void fill_levels(LKLevelSet* s, const ofb_pyr* p)
 int ofb_lk_device(ofb_ctx* ctx, const ofb_pyr* prev, int prev_image0, int prev_step, const ofb_pyr* next, int next_image0,
                   int next_step, int n_pairs, const float* prev_pts, const int* counts, int counts_stride, int n_uniform,
                   size_t pts_stride, int win_w, int win_h, int max_level, int max_count, double eps, int flags,
-                  double min_eig_thr, float* next_pts, uint8_t* status, float* err)
+                  double min_eig_thr, float* next_pts, uint8_t* status, float* err, double fb_thr, float* fb_err)
 {
     OFB_REQUIRE(win_w > 2 && win_h > 2, "pyrlk: winSize must be larger than 2x2");
+    const bool fb = fb_thr > 0.0;
     OFB_REQUIRE(win_w * win_h <= 64 * 64, "pyrlk: winSize too large (max 4096 pixels)");
     OFB_REQUIRE(prev->w[0] == next->w[0] && prev->h[0] == next->h[0], "pyrlk: prev/next size mismatch");
     LKParams P;
@@ -790,23 +857,35 @@ int ofb_lk_device(ofb_ctx* ctx, const ofb_pyr* prev, int prev_image0, int prev_s
     const char* env = getenv("OFB_LK_GENERIC");      // parity tests cross-check the two kernels
     if (win_w <= 16 && win_h <= 15 && !(env && env[0] == '1')) {
         dim3 fgrid(ofb_div_up(n_uniform, LKF_WARPS), n_pairs);
-        const char* v1 = getenv("OFB_LK_V1");            // first-generation register-resident kernel (cross-check / A-B timing)
-        if (v1 && v1[0] == '1')
+        // first-generation register-resident kernel (cross-check / A-B timing of the plain path; the forward-backward
+        // check always runs in the second-generation kernel)
+        const char* v1 = getenv("OFB_LK_V1");
+        if (fb)
+            lk_track_fast2_kernel<true><<<fgrid, LKF_WARPS * 32, 0, ctx->stream>>>(P, prev_pts, next_pts, status, err, counts,
+                                                                                  counts_stride, n_uniform, pts_stride,
+                                                                                  fb_thr, fb_err);
+        else if (v1 && v1[0] == '1')
             lk_track_fast_kernel<<<fgrid, LKF_WARPS * 32, 0, ctx->stream>>>(P, prev_pts, next_pts, status, err, counts,
                                                                            counts_stride, n_uniform, pts_stride);
         else
-            lk_track_fast2_kernel<<<fgrid, LKF_WARPS * 32, 0, ctx->stream>>>(P, prev_pts, next_pts, status, err, counts,
-                                                                            counts_stride, n_uniform, pts_stride);
+            lk_track_fast2_kernel<false><<<fgrid, LKF_WARPS * 32, 0, ctx->stream>>>(P, prev_pts, next_pts, status, err, counts,
+                                                                                   counts_stride, n_uniform, pts_stride,
+                                                                                   0.0, nullptr);
         OFB_LAUNCH_CHECK(ctx);
         return OFB_OK;
     }
     size_t wsm = ofb_lk_warp_smem(win_w, win_h);
     size_t smem = wsm * LK_WARPS;
-    OFB_TRY(ofb_ensure_smem(ctx, FS_LK, lk_track_kernel, smem));
+    if (fb) OFB_TRY(ofb_ensure_smem(ctx, FS_LK_FB, lk_track_kernel<true>, smem));
+    else OFB_TRY(ofb_ensure_smem(ctx, FS_LK, lk_track_kernel<false>, smem));
     if (n_uniform <= 0) return OFB_OK;
     dim3 grid(ofb_div_up(n_uniform, LK_WARPS), n_pairs);
-    lk_track_kernel<<<grid, LK_WARPS * 32, smem, ctx->stream>>>(P, prev_pts, next_pts, status, err, counts, counts_stride,
-                                                               n_uniform, pts_stride, wsm);
+    if (fb)
+        lk_track_kernel<true><<<grid, LK_WARPS * 32, smem, ctx->stream>>>(P, prev_pts, next_pts, status, err, counts, counts_stride,
+                                                                         n_uniform, pts_stride, wsm, fb_thr, fb_err);
+    else
+        lk_track_kernel<false><<<grid, LK_WARPS * 32, smem, ctx->stream>>>(P, prev_pts, next_pts, status, err, counts, counts_stride,
+                                                                          n_uniform, pts_stride, wsm, 0.0, nullptr);
     OFB_LAUNCH_CHECK(ctx);
     return OFB_OK;
 }
@@ -835,4 +914,33 @@ extern "C" int ofb_pyrlk(ofb_ctx* ctx, const ofb_pyr* prev, int prev_image, cons
                           max_level, max_count, eps, flags, min_eig_thr, (float*)o[0].dev, (uint8_t*)o[1].dev,
                           (float*)o[2].dev));
     return ofb_finish_out(ctx, o, 3);
+}
+
+extern "C" int ofb_pyrlk_fb(ofb_ctx* ctx, const ofb_pyr* prev, int prev_image, const ofb_pyr* next, int next_image,
+                            const float* prev_pts, int n, int win_w, int win_h, int max_level, int max_count, double eps,
+                            double min_eig_thr, double fb_max_err, float* next_pts, uint8_t* status, float* err, float* fb_err)
+{
+    OFB_REQUIRE(ctx && prev && next && next_pts && status, "pyrlk_fb: null argument");
+    OFB_REQUIRE(ofb_fb_thr_ok(fb_max_err), "pyrlk_fb: fb_max_err must be >= 0 (0 = no check)");
+    OFB_REQUIRE(n >= 0, "pyrlk_fb: negative point count");
+    OFB_REQUIRE(prev_image >= 0 && prev_image < prev->n_images && next_image >= 0 && next_image < next->n_images,
+                "pyrlk_fb: image index out of range");
+    if (n == 0) return OFB_OK;
+    OFB_REQUIRE(prev_pts, "pyrlk_fb: null prevPts");
+    OFB_CUDA(cudaSetDevice(ctx->device));
+    const void* dpts;
+    OFB_TRY(ofb_stage_in(ctx, SC_PTS0, prev_pts, sizeof(float) * 2 * (size_t)n, &dpts));
+    OutStage o[4];
+    OFB_TRY(ofb_stage_out(ctx, SC_PTS1, next_pts, sizeof(float) * 2 * (size_t)n, &o[0]));
+    OFB_TRY(ofb_stage_out(ctx, SC_STAT, status, (size_t)n, &o[1]));
+    OFB_TRY(ofb_stage_out(ctx, SC_ERR, err, sizeof(float) * (size_t)n, &o[2]));
+    OFB_TRY(ofb_stage_out(ctx, SC_OUT0, fb_err, sizeof(float) * (size_t)n, &o[3]));
+    if (fb_max_err == 0.0 && o[3].dev) {     // no check, no backward pass: no distance either
+        fill_inf_kernel<<<ofb_div_up(n, 256), 256, 0, ctx->stream>>>((float*)o[3].dev, n);
+        OFB_LAUNCH_CHECK(ctx);
+    }
+    OFB_TRY(ofb_lk_device(ctx, prev, prev_image, 0, next, next_image, 0, 1, (const float*)dpts, nullptr, 0, n, 0, win_w, win_h,
+                          max_level, max_count, eps, 0, min_eig_thr, (float*)o[0].dev, (uint8_t*)o[1].dev, (float*)o[2].dev,
+                          fb_max_err, (float*)o[3].dev));
+    return ofb_finish_out(ctx, o, 4);
 }

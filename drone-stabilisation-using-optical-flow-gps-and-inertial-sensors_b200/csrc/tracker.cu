@@ -71,6 +71,9 @@ struct ofb_tracker {
     bool has_cam = false;
     ofb_camera cam_host;
     DevBuf cam_dev, calib;
+    // forward-backward check of the LK tracks (ofb_tracker_set_fb_check), 0 = off: a kernel argument, so captured graphs
+    // hold the value they were captured with
+    double fb_max_err = 0.0;
     uint64_t graph_steps = 0;
 };
 
@@ -671,7 +674,7 @@ static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitc
         ctx->lk_lo = lo;
         const int rc = ofb_lk_device(ctx, t->pyr[t->cur ^ 1], 0, 1, t->pyr[t->cur], 0, 1, S, P, hi, 1, cap, (size_t)cap, pc.win_w,
                                      pc.win_h, pc.max_level, pc.max_count, pc.eps, 0, pc.min_eig_thr, t->nxt.as<float>(),
-                                     t->status.as<uint8_t>(), t->err.as<float>());
+                                     t->status.as<uint8_t>(), t->err.as<float>(), t->fb_max_err);
         ctx->lk_lo = nullptr;
         return rc;
     };
@@ -938,6 +941,21 @@ extern "C" int ofb_tracker_set_camera(ofb_tracker* t, const ofb_camera* cam)
             for (int j = 0; j < 2; ++j)
                 if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
         t->has_cam = cam != nullptr;
+    }
+    return OFB_OK;
+}
+
+extern "C" int ofb_tracker_set_fb_check(ofb_tracker* t, double fb_max_err)
+{
+    OFB_REQUIRE(t, "tracker_set_fb_check: null tracker");
+    OFB_REQUIRE(ofb_fb_thr_ok(fb_max_err), "tracker_set_fb_check: fb_max_err must be >= 0 (0 = off)");
+    if (fb_max_err != t->fb_max_err) {
+        // the threshold is an argument of the LK launch: graphs captured with the old value are rebuilt (no graph is in
+        // flight: a replayed step synchronises before it returns)
+        for (int i = 0; i < 2; ++i)
+            for (int j = 0; j < 2; ++j)
+                if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
+        t->fb_max_err = fb_max_err;
     }
     return OFB_OK;
 }

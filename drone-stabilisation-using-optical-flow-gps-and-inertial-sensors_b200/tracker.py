@@ -13,7 +13,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from .vision import as_camera, make_pair_cfg
+from .vision import _fb_threshold, as_camera, make_pair_cfg
 
 
 class StreamTracker:
@@ -31,12 +31,14 @@ class StreamTracker:
     max_speed > 0 enables of.static_immobile(new, old, max_speed, d, dummy_value).
     borrow_frames: device-resident grey frames (CUDA tensors) are tracked in place instead of being copied into the
     tracker; pass a NEW tensor every step (the tracker keeps the previous one alive; do not overwrite it).
-    camera: (K, D, rate[, iterations]) or vision.make_camera(...) -- see set_camera."""
+    camera: (K, D, rate[, iterations]) or vision.make_camera(...) -- see set_camera.
+    fb_threshold: None / 0 = off, T > 0 = forward-backward check of the LK tracks -- see set_fb_threshold."""
 
     def __init__(self, width, height, max_features=100, min_features=20, n_streams=1, feature_params=None,
                  lk_params=None, topup="exp", mask_radius=30, bgr=False, variant="exp", principal=None,
                  scaling=1.0, flow_scaling=None, max_speed=0.0, dummy_value=float("nan"), gate=None, min_solve=3,
-                 min_eig_thr=1e-4, borrow_frames=False, v_init=None, camera=None, ctx=None):
+                 min_eig_thr=1e-4, borrow_frames=False, v_init=None, camera=None, fb_threshold=None, ctx=None):
+        fb = _fb_threshold(fb_threshold)
         fp = dict(qualityLevel=0.01, minDistance=10, blockSize=7)
         fp.update(feature_params or {})
         lk = dict(winSize=(15, 15), maxLevel=3, criteria=(3, 20, 0.03))
@@ -74,6 +76,8 @@ class StreamTracker:
         self.capacity = cap.value
         if camera is not None:
             self.set_camera(camera)
+        if fb:
+            _lib.check(self.ctx.lib.ofb_tracker_set_fb_check(self.h, fb))
 
     def close(self):
         if getattr(self, "h", None) and getattr(self.ctx, "h", None):
@@ -105,6 +109,12 @@ class StreamTracker:
         vision.CAMERA_ITERATIONS) instead of the pinhole principal / scaling / flow_scaling. None detaches it."""
         cam = as_camera(camera)
         _lib.check(self.ctx.lib.ofb_tracker_set_camera(self.h, C.byref(cam) if cam is not None else None))
+
+    def set_fb_threshold(self, threshold):
+        """Forward-backward check of every stream's LK tracks from the next step on (vision.track_forward_backward): a
+        point that does not return within `threshold` px of where it started counts as lost (status 0). None or 0
+        turns it off."""
+        _lib.check(self.ctx.lib.ofb_tracker_set_fb_check(self.h, _fb_threshold(threshold)))
 
     def set_points(self, points):
         """points: one (N,2)/(N,1,2) array per stream (or a single array when n_streams == 1)."""
@@ -216,6 +226,12 @@ class FleetTracker:
         """StreamTracker.set_camera on this rank's streams"""
         if self.local is not None:
             self.local.set_camera(camera)
+
+    def set_fb_threshold(self, threshold):
+        """StreamTracker.set_fb_threshold on this rank's streams"""
+        t = _fb_threshold(threshold)
+        if self.local is not None:
+            self.local.set_fb_threshold(t)
 
     def gather_velocities(self):
         """(n_streams, 3) velocities of the last step on every rank; rows of streams that did not solve (or have not

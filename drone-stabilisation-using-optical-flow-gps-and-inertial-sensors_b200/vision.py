@@ -9,8 +9,10 @@ module (SURVEY 8b):
     frame_pairs(...)               the per-frame dataflow of node:224-267 / evaluate_exp.py:77-120, batched
     undistortPoints(src, cameraMatrix, distCoeffs, R=None, P=None)    cv2.undistortPoints (5 iterations)
     undistortPointsIter(src, cameraMatrix, distCoeffs, R, P, criteria) with the COUNT criterion
+    track_forward_backward(prevImg, nextImg, prevPts, threshold, ...)  LK forwards + backwards, lk_track.py's check
 """
 import ctypes as C
+import numbers
 
 import numpy as np
 
@@ -181,6 +183,56 @@ def calcOpticalFlowPyrLK(prevImg, nextImg, prevPts, nextPts=None, status=None, e
             p.close()
 
 
+def _fb_threshold(threshold):
+    """The forward-backward check's threshold as the C ABI takes it: None or 0 = off (0.0), else a positive number of
+    pixels (+inf allowed). Raises ValueError for a negative, NaN or non-numeric value."""
+    if threshold is None:
+        return 0.0
+    if isinstance(threshold, (bool, np.bool_)) or not isinstance(threshold, numbers.Real):
+        raise ValueError("fb threshold must be a number of pixels, got %r" % (threshold,))
+    t = float(threshold)
+    if not t >= 0.0:
+        raise ValueError("fb threshold must be >= 0 (0 or None = off), got %r" % (threshold,))
+    return t
+
+
+def track_forward_backward(prevImg, nextImg, prevPts, threshold=1.0, winSize=(21, 21), maxLevel=3,
+                           criteria=(TERM_CRITERIA_COUNT | TERM_CRITERIA_EPS, 30, 0.01), minEigThreshold=1e-4, ctx=None):
+    """calcOpticalFlowPyrLK forwards, then backwards from the forward result, in one launch (the check of OpenCV's
+    samples/python/lk_track.py). -> (nextPts (N,1,2) f32, status (N,1) u8, err (N,1) f32, fbErr (N,) f32).
+    nextPts and err are the forward call's; status is 1 where the forward and the backward status are 1 and
+    fbErr = max(|x0 - x0r|, |y0 - y0r|) < threshold; fbErr is +inf where either pass lost the point (everywhere
+    when threshold is 0 or None: then status is the forward one). Defaults are calcOpticalFlowPyrLK's; prevImg /
+    nextImg may be Pyramid objects."""
+    thr = _fb_threshold(threshold)
+    ctx = ctx or _lib.default_context()
+    pts = np.ascontiguousarray(np.asarray(prevPts, dtype=np.float32).reshape(-1, 2))
+    n = len(pts)
+    own = []
+    pp = prevImg if isinstance(prevImg, Pyramid) else Pyramid(_gray(prevImg, "prevImg"), maxLevel, ctx)
+    if pp is not prevImg:
+        own.append(pp)
+    pn = nextImg if isinstance(nextImg, Pyramid) else Pyramid(_gray(nextImg, "nextImg"), maxLevel, ctx)
+    if pn is not nextImg:
+        own.append(pn)
+    try:
+        if pp.sizes[0] != pn.sizes[0]:
+            raise ValueError("prevImg and nextImg must have the same size")
+        out = np.zeros((n, 2), np.float32)
+        st = np.zeros(n, np.uint8)
+        er = np.zeros(n, np.float32)
+        fb = np.full(n, np.inf, np.float32)
+        count, eps = _criteria(criteria)
+        if n:
+            _lib.check(ctx.lib.ofb_pyrlk_fb(ctx.h, pp.h, 0, pn.h, 0, _lib.ptr(pts), n, int(winSize[0]), int(winSize[1]),
+                                            int(maxLevel), count, eps, float(minEigThreshold), thr, _lib.ptr(out),
+                                            _lib.ptr(st), _lib.ptr(er), _lib.ptr(fb)))
+        return out.reshape(-1, 1, 2), st.reshape(-1, 1), er.reshape(-1, 1), fb
+    finally:
+        for p in own:
+            p.close()
+
+
 # The velocity paths iterate the inverse lens model 20 times by default, cv2.undistortPoints 5 times. For a wide-angle
 # k1 = -0.3 lens (1280x720, fx = 900 px) 5 iterations leave up to 0.48 px of error at the image edge against the
 # converged inverse, 10 leave 1.3e-3 px and 20 leave 1e-8 px. A bias of 0.48 px enters x and u directly and with them
@@ -289,7 +341,8 @@ def make_pair_cfg(width, height, max_corners, quality=0.01, min_distance=10.0, b
     return cfg
 
 
-def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, ctx=None, on_overflow="raise", camera=None):
+def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, ctx=None, on_overflow="raise", camera=None,
+                fb_threshold=None):
     """Batched detect(+)track+solve. prev/nxt: (N,H,W) uint8 numpy arrays (host) or CUDA tensors;
     imu: structured array _lib.IMU_DTYPE (N,). Returns a structured array _lib.RESULT_DTYPE (N,)
     (and prev_pts, next_pts, status when want_tracks).
@@ -298,7 +351,11 @@ def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, 
     OfbError (on_overflow="ignore" returns the flagged records instead).
     camera: (K, D, rate[, iterations]) or make_camera(...): the solve sees x = undistort(p_new) and
     u = (undistort(p_new) - undistort(p_old)) * rate instead of cfg's pinhole (cx, cy, pos_scale, flow_scale);
-    iterations default to CAMERA_ITERATIONS."""
+    iterations default to CAMERA_ITERATIONS.
+    fb_threshold: None / 0 = off; T > 0 = forward-backward check of every track (track_forward_backward): a track that
+    does not return within T px counts as lost (status 0, not in n_tracked, not in the solve). It runs on pixel
+    positions, before the camera model."""
+    thr = _fb_threshold(fb_threshold)
     cam = as_camera(camera)
     ctx = ctx or _lib.default_context()
     n = int(prev.shape[0])
@@ -321,9 +378,9 @@ def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, 
     if pts_in is not None:
         pts_in = np.ascontiguousarray(pts_in, dtype=np.float32)
         n_in = np.ascontiguousarray(n_in, dtype=np.int32)
-    _lib.check(ctx.lib.ofb_frame_pairs_cam(ctx.h, C.byref(cfg), C.byref(cam) if cam is not None else None, n, _lib.ptr(prev),
-                                           _lib.ptr(nxt), w, w * h, _lib.ptr(imu), _lib.ptr(pts_in), _lib.ptr(n_in), _lib.ptr(res),
-                                           _lib.ptr(pp), _lib.ptr(pn), _lib.ptr(st)))
+    _lib.check(ctx.lib.ofb_frame_pairs_fb(ctx.h, C.byref(cfg), C.byref(cam) if cam is not None else None, thr, n,
+                                          _lib.ptr(prev), _lib.ptr(nxt), w, w * h, _lib.ptr(imu), _lib.ptr(pts_in), _lib.ptr(n_in),
+                                          _lib.ptr(res), _lib.ptr(pp), _lib.ptr(pn), _lib.ptr(st)))
     if on_overflow == "raise" and (res["flags"] & _lib.PAIR_OVERFLOW).any():
         bad = np.nonzero(res["flags"] & _lib.PAIR_OVERFLOW)[0]
         raise _lib.OfbError("frame_pairs: detector candidate buffer overflowed for pair(s) %s: the image has more than "
@@ -333,7 +390,7 @@ def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, 
     return res
 
 
-def frame_sequence(frames, imu, cfg, want_tracks=False, ctx=None, on_overflow="raise", camera=None):
+def frame_sequence(frames, imu, cfg, want_tracks=False, ctx=None, on_overflow="raise", camera=None, fb_threshold=None):
     """One camera stream: frames (N+1,H,W) uint8 -> N consecutive pairs (frame i, frame i+1), as
     velocity_measurment_node:224-267 sees them (it keeps the previous callback's image). Passing the two views
     of ONE buffer lets the library upload every frame and build its pyramid once (`next == prev + image_stride`
@@ -341,5 +398,5 @@ def frame_sequence(frames, imu, cfg, want_tracks=False, ctx=None, on_overflow="r
     if isinstance(frames, np.ndarray):
         frames = np.ascontiguousarray(frames, dtype=np.uint8)
     return frame_pairs(frames[:-1], frames[1:], imu, cfg, want_tracks=want_tracks, ctx=ctx, on_overflow=on_overflow,
-                       camera=camera)
+                       camera=camera, fb_threshold=fb_threshold)
 

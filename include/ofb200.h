@@ -195,7 +195,7 @@ typedef struct {
     double res;
     int    rank;
     int    n_features;   /* detected (or given) */
-    int    n_tracked;    /* status==1 */
+    int    n_tracked;    /* status==1 (ofb_frame_pairs_fb: and passed the forward-backward check) */
     int    flags;        /* OFB_PAIR_* (occupies what used to be tail padding: the record is still 72 bytes) */
 } ofb_pair_result;
 
@@ -243,6 +243,28 @@ int ofb_frame_pairs_cam(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera*
                         const uint8_t* prev, const uint8_t* next, int pitch, size_t image_stride,
                         const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
                         ofb_pair_result* results, float* prev_pts, float* next_pts, uint8_t* status);
+
+/* ---- forward-backward check of the LK tracks (OpenCV's samples/python/lk_track.py): every point with forward status 1
+ *      is tracked back from next to prev, starting at its forward result, with the same window, levels, criteria and
+ *      min_eig_thr and no initial flow. fb_err = max(|x0 - x0r|, |y0 - y0r|) in fp32; the point keeps status 1 iff the
+ *      forward and the backward status are 1 and (double)fb_err < fb_max_err. LK's status only says that the window
+ *      was well conditioned and stayed inside the image: a point that is covered or uncovered between the frames, a
+ *      patch that changes appearance or a window that slides along an edge is tracked with status 1 to a wrong place,
+ *      and rarely returns to where it started. Both passes run in one launch, in the warp that owns the feature.
+ *      fb_max_err > 0 (+inf allowed) enables the check, 0 disables it; negative values and NaN return OFB_E_INVALID. */
+/* calcOpticalFlowPyrLK + the check, without initial flow: next_pts and err are exactly ofb_pyrlk's, status is the
+ * combined decision, fb_err (n floats, may be NULL) the distance where both passes had status 1 and +inf elsewhere
+ * (everywhere when fb_max_err == 0). */
+int ofb_pyrlk_fb(ofb_ctx* ctx, const ofb_pyr* prev, int prev_image, const ofb_pyr* next, int next_image,
+                 const float* prev_pts, int n, int win_w, int win_h, int max_level, int max_count, double eps,
+                 double min_eig_thr, double fb_max_err, float* next_pts, uint8_t* status, float* err, float* fb_err);
+/* ofb_frame_pairs_cam with the check folded into the track status: the solve, ofb_pair_result.n_tracked and the
+ * optional status output see only the points that passed it. The check runs on pixel positions, before any camera
+ * model. fb_max_err == 0 is exactly ofb_frame_pairs_cam. */
+int ofb_frame_pairs_fb(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, double fb_max_err, int n_pairs,
+                       const uint8_t* prev, const uint8_t* next, int pitch, size_t image_stride,
+                       const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
+                       ofb_pair_result* results, float* prev_pts, float* next_pts, uint8_t* status);
 
 /* ---- feature lifecycle around the tracker (SURVEY 8f-2): the point set of every camera stream stays on the
  *      device between frames. One step does what the reference's per-frame loops do around the tracker
@@ -299,7 +321,7 @@ typedef struct {
     int    rank;
     int    flags;
     int    n_prev;           /* points tracked from (count before the step) */
-    int    n_tracked;        /* status == 1 */
+    int    n_tracked;        /* status == 1 (with ofb_tracker_set_fb_check: and passed the forward-backward check) */
     int    n_kept;           /* after the gates = points the solve used */
     int    n_added;          /* appended by the top-up */
     int    n_points;         /* count after the step */
@@ -346,6 +368,10 @@ int ofb_tracker_graph_info(const ofb_tracker* trk, uint64_t* steps_out, int* con
  * x = undistort(p_new), u = (undistort(p_new) - undistort(p_old)) * rate; static_immobile stays in pixels. A step
  * already enqueued (split solve, deferred top-up, graph replay) keeps the camera it was enqueued with. */
 int ofb_tracker_set_camera(ofb_tracker* trk, const ofb_camera* cam);
+/* Forward-backward check of every stream's LK tracks (see ofb_pyrlk_fb) from the next ofb_tracker_step on; 0 turns it
+ * off (the default). A point that fails it counts as lost (status 0): it leaves the set before the gates, the solve
+ * and the top-up. A change of the value rebuilds the captured CUDA graphs. */
+int ofb_tracker_set_fb_check(ofb_tracker* trk, double fb_max_err);
 /* the exclusion mask OFB_TOPUP_APPEND_MASKED would use for `n` points (n x 2 float32): mask_out h x w u8
  * (1 = allowed, 0 = inside a circle). Exposed for parity tests against cv2.circle. */
 int ofb_tracker_render_mask(ofb_ctx* ctx, const float* pts, int n, int radius, int w, int h, uint8_t* mask_out);

@@ -100,8 +100,7 @@ struct ofb_ctx {
     // ingest to an internal stream only when neither happened since its previous step (see tracker_step_launches).
     uint64_t async_writes = 0;
     bool stream_exported = false;
-    const int* lk_lo = nullptr;         // set around an ofb_lk_device call: per-pair first feature to track (LKParams::counts_lo)
-    // streams of objects living on this context (a tracker's deferred top-up) that must be joined before the context's
+    // streams of objects living on this context (a tracker's split solve) that must be joined before the context's
     // stream counts as "done": ofb_ctx_sync, ofb_timer_stop and the memcpy calls wait for them (ofb_join_aux)
     std::vector<std::pair<cudaStream_t, cudaEvent_t>> aux_join;
     // cudaFuncAttributeMaxDynamicSharedMemorySize is a per-DEVICE attribute of a kernel: what this context has already

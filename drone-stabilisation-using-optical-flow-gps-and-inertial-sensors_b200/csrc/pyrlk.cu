@@ -79,19 +79,20 @@ lk_track_kernel(LKParams P, const float* __restrict__ prev_pts, float* __restric
     int n = counts ? counts[(size_t)pair * counts_stride] : n_uniform;
     int feat = blockIdx.x * LK_WARPS + warp;
     if (feat >= n) return;
-    if (P.counts_lo && feat < P.counts_lo[(size_t)pair * counts_stride]) return;
     const int winW = P.win_w, winH = P.win_h, npx = winW * winH;
     const int RW = winW + 3, RH = winH + 3, RP = (RW + 3) & ~3;
     const int DW = winW + 1, DH = winH + 1;
-    unsigned char* base = lk_smem + (size_t)warp * warp_smem;
-    uint8_t* reg = base;                                       // RP x RH staged image bytes
-    short* ders = (short*)(base + (((size_t)RP * RH + 15) & ~(size_t)15));   // Ix, Iy over DW x DH
-    short* pat = ders + 2 * DW * DH;                           // Ipatch, dIx, dIy over npx
     size_t po = (size_t)pair * pts_stride + feat;
     float ptx = prev_pts[2 * po], pty = prev_pts[2 * po + 1];
     float nx = 0.f, ny = 0.f;
     if (P.flags & OFB_LK_USE_INITIAL_FLOW) { nx = next_pts[2 * po]; ny = next_pts[2 * po + 1]; }
-    const float hwx = (winW - 1) * 0.5f, hwy = (winH - 1) * 0.5f;
+    // (the point is loaded before the slices are set up: in this order ptxas spills 20 / 20 bytes for FB = false and
+    // 16 / 32 for FB = true, the least of the orders tried)
+    unsigned char* base = lk_smem + (size_t)warp * warp_smem;
+    uint8_t* reg = base;                                       // RP x RH staged image bytes
+    short* ders = (short*)(base + (((size_t)RP * RH + 15) & ~(size_t)15));   // Ix, Iy over DW x DH
+    short* pat = ders + 2 * DW * DH;                           // Ipatch, dIx, dIy over npx
+    const float hwx = P.hwx, hwy = P.hwy;
     const float FLT_SCALE = 1.f / (1 << 20);
     bool st = true;
     float errv = 0.f;
@@ -101,12 +102,11 @@ lk_track_kernel(LKParams P, const float* __restrict__ prev_pts, float* __restric
     for (int pass = 0; pass < (FB ? 2 : 1); ++pass) {
         const bool bwd = FB && pass == 1;
         for (int level = P.nlev - 1; level >= 0; --level) {
-            const uint8_t* I = bwd ? P.next.base[level] + (size_t)nimg * P.next.stride[level]
-                                   : P.prev.base[level] + (size_t)pimg * P.prev.stride[level];
-            const uint8_t* J = bwd ? P.prev.base[level] + (size_t)pimg * P.prev.stride[level]
-                                   : P.next.base[level] + (size_t)nimg * P.next.stride[level];
-            const int w = P.prev.w[level], h = P.prev.h[level];
-            const int ipitch = bwd ? P.next.pitch[level] : P.prev.pitch[level], jpitch = bwd ? P.prev.pitch[level] : P.next.pitch[level];
+            const LKLevel& L = P.lv[level];
+            const uint8_t* I = bwd ? L.J + (size_t)nimg * L.jstride : L.I + (size_t)pimg * L.istride;
+            const uint8_t* J = bwd ? L.I + (size_t)pimg * L.istride : L.J + (size_t)nimg * L.jstride;
+            const int w = L.w, h = L.h;
+            const int ipitch = bwd ? L.jpitch : L.ipitch, jpitch = bwd ? L.ipitch : L.jpitch;
             float sc = 1.f / (float)(1 << level);
             float ppx = ptx * sc, ppy = pty * sc;
             if (level == P.nlev - 1) {
@@ -254,14 +254,6 @@ lk_track_kernel(LKParams P, const float* __restrict__ prev_pts, float* __restric
 }
 
 // ================= register-resident fast path: winW <= 16, winH <= 15 (the reference uses 15x15) ============
-// lane = (row r = lane>>1, half hh = lane&1): the lane owns the 8 window pixels (8hh+k, r), k=0..7, for the
-// whole track. Everything a lane needs sits in 12-byte row segments (three 32-bit words after re-alignment with
-// funnel shifts): no shared memory, no byte-granular traffic. Row r+1 of the window comes from lane+2 by
-// shuffle (the two lanes of row 15 only feed their neighbours). The Q14 bilinear taps of the image are two
-// dp2a (16-bit weights x u8 pixels) per pixel; a funnel shift yields the byte pairs of pixels k and k+2 at once.
-// One feature = one warp = one CTA: the fast kernels use no shared memory and no block barrier, and features differ in
-// their number of Newton steps -- with four warps per CTA the three that finished early kept their slots until the
-// slowest one was done (0.854 -> 0.805 ms per 128 pairs with one; -DOFB_LKF_WARPS=n for A/B builds). 32 CTAs per SM.
 #ifndef OFB_LKF_WARPS
 #define OFB_LKF_WARPS 1
 #endif
@@ -312,12 +304,6 @@ __device__ __forceinline__ void load12(const uint8_t* __restrict__ img, int w, i
     }
 }
 
-__device__ __forceinline__ int byte_of(unsigned int w0, unsigned int w1, unsigned int w2, int j)
-{   // j is a compile-time constant after unrolling
-    unsigned int w = j < 4 ? w0 : (j < 8 ? w1 : w2);
-    return (int)((w >> (8 * (j & 3))) & 0xffu);
-}
-
 // Exact warp sum of int32 lane values, returned as the correctly rounded float of the 64-bit total: two REDUX
 // (low 16 bits unsigned, high part signed; neither can overflow over 32 lanes) instead of a 5-level shuffle chain.
 __device__ __forceinline__ float warp_sum_exact_f(int v)
@@ -345,207 +331,24 @@ __device__ __forceinline__ float warp_sum_exact_f(int v)
         }                                                                                         \
     }
 
-__global__ void __launch_bounds__(LKF_WARPS * 32, 32 / LKF_WARPS)
-lk_track_fast_kernel(LKParams P, const float* __restrict__ prev_pts, float* __restrict__ next_pts,
-                     uint8_t* __restrict__ status, float* __restrict__ err, const int* __restrict__ counts,
-                     int counts_stride, int n_uniform, size_t pts_stride)
-{
-    const int lane = threadIdx.x & 31;
-    const int pair = blockIdx.y;
-    const int n = counts ? counts[(size_t)pair * counts_stride] : n_uniform;
-    const int feat = blockIdx.x * LKF_WARPS + (threadIdx.x >> 5);
-    if (feat >= n) return;
-    if (P.counts_lo && feat < P.counts_lo[(size_t)pair * counts_stride]) return;
-    const int winW = P.win_w, winH = P.win_h;
-    const int r = lane >> 1, hh = lane & 1;
-    const size_t po = (size_t)pair * pts_stride + feat;
-    const float ptx = prev_pts[2 * po], pty = prev_pts[2 * po + 1];
-    float nx = 0.f, ny = 0.f;
-    if (P.flags & OFB_LK_USE_INITIAL_FLOW) { nx = next_pts[2 * po]; ny = next_pts[2 * po + 1]; }
-    const float hwx = (winW - 1) * 0.5f, hwy = (winH - 1) * 0.5f;
-    const float FLT_SCALE = 1.f / (1 << 20);
-    // validity of the lane's pixels: column 8hh+k < winW, row r < winH
-    unsigned int vmask = 0;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) if (8 * hh + k < winW && r < winH) vmask |= 1u << k;
-    bool st = true;
-    float errv = 0.f;
-    const int pimg = P.prev_image0 + pair * P.prev_image_step, nimg = P.next_image0 + pair * P.next_image_step;
+__device__ __forceinline__ unsigned int prmt(unsigned int a, unsigned int b, unsigned int sel) { return __byte_perm(a, b, sel); }
 
-    for (int level = P.nlev - 1; level >= 0; --level) {
-        const uint8_t* I = P.prev.base[level] + (size_t)pimg * P.prev.stride[level];
-        const uint8_t* J = P.next.base[level] + (size_t)nimg * P.next.stride[level];
-        const int w = P.prev.w[level], h = P.prev.h[level];
-        const int ipitch = P.prev.pitch[level], jpitch = P.next.pitch[level];
-        const int ilow = ((((unsigned long long)I) & 3ull) == 0 && (ipitch & 3) == 0) ? 0 : 4;   // see load12
-        const int jlow = ((((unsigned long long)J) & 3ull) == 0 && (jpitch & 3) == 0) ? 0 : 4;
-        const float sc = 1.f / (float)(1 << level);
-        const float ppx = ptx * sc, ppy = pty * sc;
-        if (level == P.nlev - 1) {
-            if (P.flags & OFB_LK_USE_INITIAL_FLOW) { nx = nx * sc; ny = ny * sc; }
-            else { nx = ppx; ny = ppy; }
-        } else { nx = nx * 2.f; ny = ny * 2.f; }
-        const float px = ppx - hwx, py = ppy - hwy;
-        const int ix = __float2int_rd(px), iy = __float2int_rd(py);
-        if (ix < -winW || ix >= w || iy < -winH || iy >= h) {
-            if (level == 0) { st = false; errv = 0.f; }
-            continue;
-        }
-        float a = px - (float)ix, b = py - (float)iy;
-        int w00, w01, w10, w11;
-        bil_weights(a, b, w00, w01, w10, w11);
-        // ---- template ---------------------------------------------------------------------------------
-        // rows iy+r-1, iy+r, iy+r+1, bytes j=0..11 <-> columns ix+8hh-1+j
-        // warp-uniform: all columns / all rows of the patch (plus the Scharr ring) inside the image
-        const bool icol = ix - 1 >= ilow && ix + 8 + 15 <= w, irow = iy - 1 >= 0 && iy + 16 < h;
-        const bool ifast = icol && irow;
-        const int X0 = ix - 1 + 8 * hh;
-        unsigned int A0, A1, A2, B0, B1, B2, C0, C1, C2;
-        {
-            int ya = iy + r - 1, yb = iy + r, yc = iy + r + 1;
-            if (!irow) { ya = refl101(ya, h); yb = refl101(yb, h); yc = refl101(yc, h); }
-            load12(I, w, ipitch, X0, ya, icol, A0, A1, A2);
-            load12(I, w, ipitch, X0, yb, icol, B0, B1, B2);
-            load12(I, w, ipitch, X0, yc, icol, C0, C1, C2);
-        }
-        int t0[11], t1[11];
-#pragma unroll
-        for (int j = 0; j < 11; ++j) {
-            int av = byte_of(A0, A1, A2, j), bv = byte_of(B0, B1, B2, j), cv = byte_of(C0, C1, C2, j);
-            t0[j] = 3 * (av + cv) + 10 * bv;
-            t1[j] = cv - av;
-        }
-        // Scharr at row iy+r, columns ix+8hh+k, k=0..8; zero outside the image (OpenCV pads derivatives with 0)
-        unsigned int D[9];
-        const bool rowin = (unsigned)(iy + r) < (unsigned)h;
-#pragma unroll
-        for (int k = 0; k < 9; ++k) {
-            int gx = t0[k + 2] - t0[k];
-            int gy = 3 * (t1[k] + t1[k + 2]) + 10 * t1[k + 1];
-            D[k] = ((unsigned int)gx & 0xffffu) | ((unsigned int)gy << 16);
-        }
-        if (!ifast) {
-#pragma unroll
-            for (int k = 0; k < 9; ++k)
-                if (!(rowin && (unsigned)(ix + 8 * hh + k) < (unsigned)w)) D[k] = 0u;
-        }
-        int Cp[8], Gx[8], Gy[8];
-        int iA11 = 0, iA12 = 0, iA22 = 0;
-        {
-            int gxa = (int)(short)(D[0] & 0xffffu), gya = (int)D[0] >> 16;
-            unsigned int Db = __shfl_down_sync(0xffffffffu, D[0], 2);
-            int gxc = (int)(short)(Db & 0xffffu), gyc = (int)Db >> 16;
-#pragma unroll
-            for (int k = 0; k < 8; ++k) {
-                int gxb = (int)(short)(D[k + 1] & 0xffffu), gyb = (int)D[k + 1] >> 16;
-                unsigned int Dn = __shfl_down_sync(0xffffffffu, D[k + 1], 2);
-                int gxd = (int)(short)(Dn & 0xffffu), gyd = (int)Dn >> 16;
-                int iv = (byte_of(B0, B1, B2, k + 1) * w00 + byte_of(B0, B1, B2, k + 2) * w01 +
-                          byte_of(C0, C1, C2, k + 1) * w10 + byte_of(C0, C1, C2, k + 2) * w11 + (1 << 8)) >> 9;
-                int gx = (gxa * w00 + gxb * w01 + gxc * w10 + gxd * w11 + (1 << 13)) >> 14;
-                int gy = (gya * w00 + gyb * w01 + gyc * w10 + gyd * w11 + (1 << 13)) >> 14;
-                if (!((vmask >> k) & 1u)) { gx = 0; gy = 0; }
-                Cp[k] = 256 - 512 * iv; Gx[k] = gx; Gy[k] = gy;
-                iA11 += gx * gx; iA12 += gx * gy; iA22 += gy * gy;
-                gxa = gxb; gya = gyb; gxc = gxd; gyc = gyd;
-            }
-        }
-        const float A11 = warp_sum_exact_f(iA11) * FLT_SCALE;
-        const float A12 = warp_sum_exact_f(iA12) * FLT_SCALE;
-        const float A22 = warp_sum_exact_f(iA22) * FLT_SCALE;
-        float D2 = __fsub_rn(__fmul_rn(A11, A22), __fmul_rn(A12, A12));
-        const float dd = A11 - A22;
-        const float minEig = (A22 + A11 - sqrtf(__fadd_rn(__fmul_rn(dd, dd), __fmul_rn(__fmul_rn(4.f, A12), A12)))) /
-                             (float)(2 * winW * winH);
-        if ((double)minEig < P.min_eig_thr || D2 < 1.1920928955078125e-7f) {
-            if (level == 0) st = false;
-            continue;
-        }
-        D2 = 1.f / D2;
-        float qx = nx - hwx, qy = ny - hwy;
-        float pdx = 0.f, pdy = 0.f;
-        bool lost = false;
-        unsigned int T0 = 0, T1 = 0, T2 = 0, U0 = 0, U1 = 0, U2 = 0;
-        int cjx = INT_MIN, cjy = INT_MIN;
-        for (int j = 0; j < P.max_count; ++j) {
-            const int jx = __float2int_rd(qx), jy = __float2int_rd(qy);
-            if (jx < -winW || jx >= w || jy < -winH || jy >= h) { lost = true; break; }
-            a = qx - (float)jx; b = qy - (float)jy;
-            bil_weights(a, b, w00, w01, w10, w11);
-            const int Wt = (w00 & 0xffff) | (w01 << 16), Wb = (w10 & 0xffff) | (w11 << 16);
-            // the patch rows stay in registers while the integer position does not move (most Newton steps are
-            // sub-pixel): only the bilinear weights change then
-            if (jx != cjx || jy != cjy) {
-                const bool jcol = jx >= jlow && jx + 8 + 16 <= w, jrow = jy >= 0 && jy + 15 < h;
-                OFB_DEV_ASSERT(!jrow || (jy + r >= 0 && jy + r < h)); load12(J, w, jpitch, jx + 8 * hh, jrow ? jy + r : refl101(jy + r, h), jcol, T0, T1, T2);
-                U0 = __shfl_down_sync(0xffffffffu, T0, 2); U1 = __shfl_down_sync(0xffffffffu, T1, 2);
-                U2 = __shfl_down_sync(0xffffffffu, T2, 2);
-                cjx = jx; cjy = jy;
-            }
-            int ib1 = 0, ib2 = 0;
-            LKF_FOR_PIXELS(T0, T1, T2, U0, U1, U2, Wt, Wb, {
-                ib1 += diff * Gx[k]; ib2 += diff * Gy[k];
-            })
-            const float b1 = warp_sum_exact_f(ib1) * FLT_SCALE;
-            const float b2 = warp_sum_exact_f(ib2) * FLT_SCALE;
-            const float dx = __fmul_rn(__fsub_rn(__fmul_rn(A12, b2), __fmul_rn(A22, b1)), D2);
-            const float dy = __fmul_rn(__fsub_rn(__fmul_rn(A12, b1), __fmul_rn(A11, b2)), D2);
-            qx += dx; qy += dy;
-            nx = qx + hwx; ny = qy + hwy;
-            if ((double)dx * (double)dx + (double)dy * (double)dy <= P.eps) break;
-            if (j > 0 && fabsf(dx + pdx) < 0.01f && fabsf(dy + pdy) < 0.01f) {
-                nx -= dx * 0.5f; ny -= dy * 0.5f;
-                break;
-            }
-            pdx = dx; pdy = dy;
-        }
-        if (lost && level == 0) st = false;
-        if (st && level == 0) {
-            const float rx = nx - hwx, ry = ny - hwy;
-            const int jx = __float2int_rd(rx), jy = __float2int_rd(ry);
-            if (jx < -winW || jx >= w || jy < -winH || jy >= h) { st = false; }
-            else {
-                a = rx - (float)jx; b = ry - (float)jy;
-                bil_weights(a, b, w00, w01, w10, w11);
-                const int Wt = (w00 & 0xffff) | (w01 << 16), Wb = (w10 & 0xffff) | (w11 << 16);
-                if (jx != cjx || jy != cjy) {
-                    const bool jcol = jx >= jlow && jx + 8 + 16 <= w, jrow = jy >= 0 && jy + 15 < h;
-                    OFB_DEV_ASSERT(!jrow || (jy + r >= 0 && jy + r < h)); load12(J, w, jpitch, jx + 8 * hh, jrow ? jy + r : refl101(jy + r, h), jcol, T0, T1, T2);
-                    U0 = __shfl_down_sync(0xffffffffu, T0, 2); U1 = __shfl_down_sync(0xffffffffu, T1, 2);
-                    U2 = __shfl_down_sync(0xffffffffu, T2, 2);
-                }
-                int ie = 0;
-                LKF_FOR_PIXELS(T0, T1, T2, U0, U1, U2, Wt, Wb, {
-                    if ((vmask >> k) & 1u) ie += abs(diff);
-                })
-                errv = (float)__reduce_add_sync(0xffffffffu, ie) * (1.f / (float)(32 * winW * winH));
-            }
-        }
-    }
-    if (lane == 0) {
-        OFB_DEV_ASSERT(feat >= 0 && feat < n && (gridDim.y == 1 || po < (size_t)(pair + 1) * pts_stride));   // (one pair: the stride is unused)
-        next_pts[2 * po] = nx; next_pts[2 * po + 1] = ny;
-        status[po] = st ? 1 : 0;
-        if (err) err[po] = st ? errv : 0.f;
-    }
-}
-
-// ================= register-resident kernel, second generation ===========================================
-// Same mapping and the same integer arithmetic as lk_track_fast_kernel (which stays as the cross-check, OFB_LK_V1=1);
-// what changed is what its per-source-line profile flagged (profiles/r2_before_lk_by_line.txt: 7.0 k warp
-// instructions per feature, ~920 per pyramid level before the first Newton step):
+// Register-resident LK kernel. lane = (row r = lane>>1, half hh = lane&1): the lane owns the 8 window pixels (8hh+k, r),
+// k=0..7, for the whole track. Everything a lane needs sits in 12-byte row segments (three 32-bit words after re-alignment
+// with funnel shifts): no shared memory, no byte-granular traffic. Row r+1 of the window comes from lane+2 by shuffle (the
+// two lanes of row 15 only feed their neighbours). Per level:
 //   * Scharr under the window with two columns per instruction (packed 16-bit halves, biased so that no half ever
-//     borrows from its neighbour) instead of 33 byte extractions and scalar arithmetic per level; the gradients stay
-//     biased by +4096 through the bilinear interpolation, whose weights sum to exactly 2^14, so the bias leaves in the
-//     rounding constant;
-//   * the row below comes through 10 shuffles of column PAIRS (was 9 shuffles of packed (gx, gy) words plus their
-//     packing and unpacking);
-//   * the template value uses the dp2a taps of the Newton loop (no byte extraction at all);
+//     borrows from its neighbour); the gradients stay biased by +4096 through the bilinear interpolation, whose weights
+//     sum to exactly 2^14, so the bias leaves in the rounding constant;
+//   * the row below comes through 10 shuffles of column PAIRS;
+//   * the template value and the Newton steps use the same Q14 bilinear taps: two dp2a (16-bit weights x u8 pixels) per
+//     pixel, a funnel shift yields the byte pairs of pixels k and k+2 at once;
 //   * per-level parameters are one packed record in constant memory, the level scale is built from its exponent, and
 //     the convergence test |delta|^2 <= eps^2 is decided in fp32 unless it falls within 1e-6 of the threshold (the fp64
 //     evaluation OpenCV uses is only needed there).
-__device__ __forceinline__ unsigned int prmt(unsigned int a, unsigned int b, unsigned int sel) { return __byte_perm(a, b, sel); }
-
+// One feature = one warp = one CTA: no shared memory and no block barrier, and features differ in their number of Newton
+// steps -- with four warps per CTA the three that finished early kept their slots until the slowest one was done
+// (0.854 -> 0.805 ms per 128 pairs with one; -DOFB_LKF_WARPS=n for A/B builds). 32 CTAs per SM.
 // FB = the forward-backward check (ofb_pyrlk_fb): a feature whose forward track has status 1 is tracked back from
 // where it landed, in the same warp, and keeps status 1 only when the backward track has status 1 too and ends within
 // fb_thr of the starting point (max-norm of the fp32 difference, compared in fp64). next_pts and err are the forward
@@ -561,7 +364,6 @@ lk_track_fast2_kernel(const __grid_constant__ LKParams P, const float* __restric
     const int n = counts ? counts[(size_t)pair * counts_stride] : n_uniform;
     const int feat = blockIdx.x * LKF_WARPS + (threadIdx.x >> 5);
     if (feat >= n) return;
-    if (P.counts_lo && feat < P.counts_lo[(size_t)pair * counts_stride]) return;
     const int winW = P.win_w, winH = P.win_h;
     const int r = lane >> 1, hh = lane & 1;
     const size_t po = (size_t)pair * pts_stride + feat;
@@ -804,15 +606,6 @@ size_t ofb_lk_warp_smem(int win_w, int win_h)
     return (b + 15) & ~(size_t)15;
 }
 
-static void fill_levels(LKLevelSet* s, const ofb_pyr* p)
-{
-    for (int l = 0; l < p->n_levels; ++l) {
-        if (l == 0) { s->base[0] = p->level0; s->stride[0] = p->level0_stride; s->pitch[0] = p->level0_pitch; }
-        else { s->base[l] = p->base + p->level_off[l]; s->stride[l] = p->image_stride[l]; s->pitch[l] = p->pitch[l]; }
-        s->w[l] = p->w[l]; s->h[l] = p->h[l];
-    }
-}
-
 int ofb_lk_device(ofb_ctx* ctx, const ofb_pyr* prev, int prev_image0, int prev_step, const ofb_pyr* next, int next_image0,
                   int next_step, int n_pairs, const float* prev_pts, const int* counts, int counts_stride, int n_uniform,
                   size_t pts_stride, int win_w, int win_h, int max_level, int max_count, double eps, int flags,
@@ -833,13 +626,16 @@ int ofb_lk_device(ofb_ctx* ctx, const ofb_pyr* prev, int prev_image0, int prev_s
         eff = l + 1;
     }
     P.nlev = eff;
-    P.counts_lo = ctx->lk_lo;
-    fill_levels(&P.prev, prev);
-    fill_levels(&P.next, next);
     for (int l = 0; l < eff; ++l) {
         LKLevel& L = P.lv[l];
-        L.I = P.prev.base[l]; L.J = P.next.base[l]; L.istride = P.prev.stride[l]; L.jstride = P.next.stride[l];
-        L.w = P.prev.w[l]; L.h = P.prev.h[l]; L.ipitch = P.prev.pitch[l]; L.jpitch = P.next.pitch[l];
+        if (l == 0) {
+            L.I = prev->level0; L.istride = prev->level0_stride; L.ipitch = prev->level0_pitch;
+            L.J = next->level0; L.jstride = next->level0_stride; L.jpitch = next->level0_pitch;
+        } else {
+            L.I = prev->base + prev->level_off[l]; L.istride = prev->image_stride[l]; L.ipitch = prev->pitch[l];
+            L.J = next->base + next->level_off[l]; L.jstride = next->image_stride[l]; L.jpitch = next->pitch[l];
+        }
+        L.w = prev->w[l]; L.h = prev->h[l];
     }
     P.win_w = win_w; P.win_h = win_h;
     P.hwx = (win_w - 1) * 0.5f; P.hwy = (win_h - 1) * 0.5f;
@@ -857,16 +653,10 @@ int ofb_lk_device(ofb_ctx* ctx, const ofb_pyr* prev, int prev_image0, int prev_s
     const char* env = getenv("OFB_LK_GENERIC");      // parity tests cross-check the two kernels
     if (win_w <= 16 && win_h <= 15 && !(env && env[0] == '1')) {
         dim3 fgrid(ofb_div_up(n_uniform, LKF_WARPS), n_pairs);
-        // first-generation register-resident kernel (cross-check / A-B timing of the plain path; the forward-backward
-        // check always runs in the second-generation kernel)
-        const char* v1 = getenv("OFB_LK_V1");
         if (fb)
             lk_track_fast2_kernel<true><<<fgrid, LKF_WARPS * 32, 0, ctx->stream>>>(P, prev_pts, next_pts, status, err, counts,
                                                                                   counts_stride, n_uniform, pts_stride,
                                                                                   fb_thr, fb_err);
-        else if (v1 && v1[0] == '1')
-            lk_track_fast_kernel<<<fgrid, LKF_WARPS * 32, 0, ctx->stream>>>(P, prev_pts, next_pts, status, err, counts,
-                                                                           counts_stride, n_uniform, pts_stride);
         else
             lk_track_fast2_kernel<false><<<fgrid, LKF_WARPS * 32, 0, ctx->stream>>>(P, prev_pts, next_pts, status, err, counts,
                                                                                    counts_stride, n_uniform, pts_stride,

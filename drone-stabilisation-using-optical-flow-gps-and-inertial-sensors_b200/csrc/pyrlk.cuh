@@ -2,12 +2,6 @@
 #pragma once
 #include "common.cuh"
 
-struct LKLevelSet {
-    const uint8_t* base[OFB_MAX_LEVELS];
-    unsigned long long stride[OFB_MAX_LEVELS];   // bytes between images of the batch at this level
-    int w[OFB_MAX_LEVELS], h[OFB_MAX_LEVELS], pitch[OFB_MAX_LEVELS];
-};
-
 // one pyramid level of both images, packed so that the register-resident kernel fetches it with three 16-byte loads
 struct LKLevel {
     const uint8_t* I; const uint8_t* J;          // image 0 of the batch at this level
@@ -16,7 +10,6 @@ struct LKLevel {
 };
 
 struct LKParams {
-    LKLevelSet prev, next;
     LKLevel lv[OFB_MAX_LEVELS];
     int nlev;                     // levels actually used (after OpenCV's window-size cut)
     int win_w, win_h, max_count, flags;
@@ -25,7 +18,6 @@ struct LKParams {
     float eps_lo, eps_hi;         // fp32 brackets of eps: |delta|^2 below eps_lo / above eps_hi decides without fp64
     float hwx, hwy;               // (win - 1) / 2
     int prev_image0, prev_image_step, next_image0, next_image_step;   // image of pair p = image0 + p*step
-    const int* counts_lo;         // optional: features below counts_lo[pair * counts_stride] are skipped (ofb_ctx::lk_lo)
 };
 
 // Device-pointer core. counts (optional): per-pair feature count at counts[pair*counts_stride];

@@ -33,7 +33,7 @@ struct ofb_tracker {
     bool have_prev = false;
     DevBuf pts[2];                     // float2 [S][cap]; pts[pcur] = current point sets
     int pcur = 0;
-    DevBuf counts;                     // int [4][S]: count, need (top-up flag), kept (count after the gates), count0 (before the top-up)
+    DevBuf counts;                     // int [3][S]: count, need (top-up flag), kept (count after the gates)
     DevBuf nxt, status, err, kept_prev, det, vlast, mask, hw, bgr;
     // CUDA-graph replay of the steady-state step for small fleets fed from host memory (the launch-bound case: a
     // step is ~15 tiny launches/copies). Inputs are staged in pinned buffers at fixed addresses, so one captured
@@ -44,22 +44,13 @@ struct ofb_tracker {
     uint64_t glaunches[2][2] = {{0, 0}, {0, 0}};
     uint64_t gsig[2][2] = {{0, 0}, {0, 0}};   // signature of the context's scratch arenas the graph's pointers refer to
     bool graph_ok = true;
-    bool cond_ok = true;               // the top-up path may sit in a conditional (IF) node of the graph (opt-in)
-    bool capturing = false, capture_cond = false, cond_used = false;
-    cudaStream_t side_stream = nullptr;   // captures the body of the conditional node
+    bool capturing = false;
     // the new frame's ingest + pyramid run on their own stream: they only have to wait for the LK of the previous step (it
     // read the pyramid slot that is overwritten), so they overlap the previous step's filter / solve / top-up kernels
     cudaStream_t pyr_stream = nullptr;
     cudaEvent_t ev_lk = nullptr, ev_pyr = nullptr;
     bool lk_recorded = false;          // ev_lk marks the LK launch of the previous step
     uint64_t launches_end = ~0ull, async_end = 0;   // the context's counters when the previous step returned
-    // deferred top-up: with device-resident results and no point read-back the top-up path (mask, lambda_min, selection,
-    // append: four launches that exit at once on most frames) runs in a child context -- own stream, own detector
-    // scratch -- and the NEXT step tracks the surviving points (they do not depend on it) before it joins and tracks
-    // what the top-up appended. The parent context's sync / timer / memcpy calls join the child stream (aux_join).
-    ofb_ctx* top_ctx = nullptr;
-    cudaEvent_t ev_filter = nullptr, ev_top = nullptr, ev_join = nullptr;
-    bool top_pending = false;          // a deferred top-up has not been joined into the context's stream yet
     // split solve: with device-resident inputs and result records the fp64 solve of a step runs on its own stream beside
     // the next frame's LK (track_filter_solve_kernel<1> / <2>); the next filter and the context's sync points wait for it
     cudaStream_t sol_stream = nullptr;
@@ -77,7 +68,6 @@ struct ofb_tracker {
     uint64_t graph_steps = 0;
 };
 
-static cudaError_t tracker_join_topup(ofb_tracker* t);
 static cudaError_t tracker_join_solve(ofb_tracker* t);
 
 namespace {
@@ -85,7 +75,7 @@ namespace {
 struct TrackerDev {
     const float* prev; const float* next; const uint8_t* status;   // [S][cap] LK input / output
     float* kept_prev; float* kept_next;                             // [S][cap] compacted
-    int* count; int* need; int* kept; int* count0;
+    int* count; int* need; int* kept;
     double* vlast;                                                  // [S][3]
     int cap;
     int variant; double cx, cy, ps, fs;
@@ -93,7 +83,6 @@ struct TrackerDev {
     double max_speed, dummy; int gate_mode; double gate_T;
     int min_solve, min_features, topup_mode, max_features;
     int have_prev;
-    int use_cond; cudaGraphConditionalHandle cond;                  // graph replay: switch the top-up branch on
     FeatImageState* feat_state; int* cell_grid; size_t cell_stride; // detector scratch, reset here instead of by memsets
 };
 
@@ -244,11 +233,9 @@ track_filter_solve_kernel(TrackerDev T, const ofb_imu_sample* __restrict__ imu, 
             T.feat_state[s] = z;
             r.n_prev = n; r.n_tracked = tracked; r.n_kept = kept; r.n_added = 0; r.n_points = kept;
             const int need = kept <= T.min_features;
-            if (need && T.use_cond) cudaGraphSetConditional(T.cond, 1u);  // any stream that needs a top-up enables the branch
             T.kept[s] = kept;
             T.need[s] = need;
             T.count[s] = (need && T.topup_mode == OFB_TOPUP_REPLACE) ? 0 : kept;    // of_module.py:86 replaces the set
-            T.count0[s] = T.count[s];                                                // (the top-up appends behind this)
         }
     }
 }
@@ -410,7 +397,7 @@ extern "C" int ofb_tracker_create(ofb_ctx* ctx, const ofb_tracker_cfg* cfg, ofb_
     R(t->pts[0], sizeof(float) * 2 * np); R(t->pts[1], sizeof(float) * 2 * np);
     R(t->nxt, sizeof(float) * 2 * np); R(t->kept_prev, sizeof(float) * 2 * np);
     R(t->status, np); R(t->err, sizeof(float) * np);
-    R(t->counts, sizeof(int) * 4 * S); R(t->det, sizeof(float) * 2 * (size_t)S * K);
+    R(t->counts, sizeof(int) * 3 * S); R(t->det, sizeof(float) * 2 * (size_t)S * K);
     R(t->vlast, sizeof(double) * 3 * S);
     if (cfg->topup_mode == OFB_TOPUP_APPEND_MASKED && cfg->mask_radius > 0) {
         R(t->mask, t->stride_d * S);
@@ -424,7 +411,7 @@ extern "C" int ofb_tracker_create(ofb_ctx* ctx, const ofb_tracker_cfg* cfg, ofb_
         ce = cudaMemcpyAsync(t->hw.p, hw.data(), sizeof(int) * hw.size(), cudaMemcpyHostToDevice, ctx->stream);
         if (ce == cudaSuccess) ce = cudaStreamSynchronize(ctx->stream);      // hw is a local
     }
-    if (ce == cudaSuccess) ce = cudaMemsetAsync(t->counts.p, 0, sizeof(int) * 4 * S, ctx->stream);
+    if (ce == cudaSuccess) ce = cudaMemsetAsync(t->counts.p, 0, sizeof(int) * 3 * S, ctx->stream);
     if (ce == cudaSuccess) ce = tracker_seed_prior(t);
     if (ce != cudaSuccess) {
         ofb_set_error("tracker_create: %s", cudaGetErrorString(ce));
@@ -446,7 +433,6 @@ extern "C" int ofb_tracker_destroy(ofb_tracker* t)
     for (int i = 0; i < 2; ++i)
         for (int j = 0; j < 2; ++j) if (t->gexec[i][j]) cudaGraphExecDestroy(t->gexec[i][j]);
     t->pin_in.release(); t->pin_out.release();
-    if (t->side_stream) cudaStreamDestroy(t->side_stream);
     if (t->pyr_stream) { cudaStreamSynchronize(t->pyr_stream); cudaStreamDestroy(t->pyr_stream); }
     if (t->sol_stream) {
         cudaStreamSynchronize(t->sol_stream);
@@ -458,17 +444,6 @@ extern "C" int ofb_tracker_destroy(ofb_tracker* t)
     if (t->ev_filt) cudaEventDestroy(t->ev_filt);
     if (t->ev_sol) cudaEventDestroy(t->ev_sol);
     if (t->ev_sol_join) cudaEventDestroy(t->ev_sol_join);
-    if (t->top_ctx) {
-        cudaStreamSynchronize(t->top_ctx->stream);
-        if (t->ctx)
-            for (size_t i = 0; i < t->ctx->aux_join.size(); ++i)
-                if (t->ctx->aux_join[i].first == t->top_ctx->stream) { t->ctx->aux_join.erase(t->ctx->aux_join.begin() + i); break; }
-        ofb_ctx_destroy(t->top_ctx);
-        if (t->ctx) cudaSetDevice(t->ctx->device);
-    }
-    if (t->ev_filter) cudaEventDestroy(t->ev_filter);
-    if (t->ev_top) cudaEventDestroy(t->ev_top);
-    if (t->ev_join) cudaEventDestroy(t->ev_join);
     if (t->ev_lk) cudaEventDestroy(t->ev_lk);
     if (t->ev_pyr) cudaEventDestroy(t->ev_pyr);
     DevBuf* bufs[] = {&t->counts, &t->nxt, &t->status, &t->err, &t->kept_prev, &t->det, &t->vlast, &t->mask, &t->hw, &t->bgr, &t->dev_io,
@@ -484,8 +459,8 @@ extern "C" int ofb_tracker_reset(ofb_tracker* t)
     OFB_CUDA(cudaSetDevice(t->ctx->device));
     t->have_prev = false;
     t->lk_recorded = false;
-    OFB_CUDA(tracker_join_topup(t));
-    OFB_CUDA(cudaMemsetAsync(t->counts.p, 0, sizeof(int) * 4 * t->cfg.n_streams, t->ctx->stream));
+    OFB_CUDA(tracker_join_solve(t));
+    OFB_CUDA(cudaMemsetAsync(t->counts.p, 0, sizeof(int) * 3 * t->cfg.n_streams, t->ctx->stream));
     OFB_CUDA(tracker_seed_prior(t));
     return OFB_OK;
 }
@@ -502,7 +477,7 @@ extern "C" int ofb_tracker_set_points(ofb_tracker* t, const float* pts, const in
     OFB_REQUIRE(t && pts && counts, "tracker_set_points: null argument");
     ofb_ctx* ctx = t->ctx;
     OFB_CUDA(cudaSetDevice(ctx->device));
-    OFB_CUDA(tracker_join_topup(t));
+    OFB_CUDA(tracker_join_solve(t));
     const int S = t->cfg.n_streams;
     if (!ofb_is_device_ptr(counts))
         for (int s = 0; s < S; ++s)
@@ -513,23 +488,12 @@ extern "C" int ofb_tracker_set_points(ofb_tracker* t, const float* pts, const in
     return OFB_OK;
 }
 
-// order the context's stream behind a deferred top-up that is still pending (see ofb_tracker::top_ctx)
+// order the context's stream behind a split solve that is still pending (see ofb_tracker::sol_stream)
 static cudaError_t tracker_join_solve(ofb_tracker* t)
 {
     if (!t->sol_pending) return cudaSuccess;
     t->sol_pending = false;
     return cudaStreamWaitEvent(t->ctx->stream, t->ev_sol, 0);
-}
-static cudaError_t tracker_join_topup_only(ofb_tracker* t)
-{
-    if (!t->top_pending) return cudaSuccess;
-    t->top_pending = false;
-    return cudaStreamWaitEvent(t->ctx->stream, t->ev_top, 0);
-}
-static cudaError_t tracker_join_topup(ofb_tracker* t)             // the whole previous step: deferred top-up and split solve
-{
-    const cudaError_t e = tracker_join_solve(t);
-    return e != cudaSuccess ? e : tracker_join_topup_only(t);
 }
 
 // One step, launch by launch, on ctx->stream (also the body that is captured into a graph).
@@ -571,24 +535,6 @@ static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitc
         if (early && !cfg.bgr_input && (size_t)S * w * h > ((size_t)32 << 20) && !(ee && ee[0] == '1')) early = false;
     }
     if (ctx->launches != t->launches_end || ctx->async_writes != t->async_end) t->lk_recorded = false;
-    // deferred top-up (opt-in, OFB_TRACKER_DEFER_TOPUP=1): only when nothing of this call is read back on the host and no
-    // output of the call depends on the top-up except the device-resident result records. Measured on B200 (one stream,
-    // device frames, asynchronous calls): it shortens the GPU chain of a 1080p step from 50.7 to <= 45 us, but the second
-    // LK launch and four more event operations raise the host's enqueue time from 30 to 45 us per step -- a 1080p
-    // stream gains 11 %, a 640x480 stream (host bound) loses 20 %, a 256-stream fleet loses 2.5 %: off by default.
-    bool defer = false;
-    {
-        const char* de = getenv("OFB_TRACKER_DEFER_TOPUP");
-        defer = early && ofb_is_device_ptr(results) && !pts_out && !n_out && de && de[0] == '1';
-    }
-    if (defer && !t->top_ctx) {
-        OFB_TRY(ofb_ctx_create(ctx->device, &t->top_ctx));
-        OFB_CUDA(cudaEventCreateWithFlags(&t->ev_filter, cudaEventDisableTiming));
-        OFB_CUDA(cudaEventCreateWithFlags(&t->ev_top, cudaEventDisableTiming));
-        OFB_CUDA(cudaEventCreateWithFlags(&t->ev_join, cudaEventDisableTiming));
-        ctx->aux_join.push_back(std::make_pair(t->top_ctx->stream, t->ev_join));
-    }
-    ofb_ctx* const fctx = defer ? t->top_ctx : ctx;                   // the context the top-up path runs in
     if (early) {
         if (!t->pyr_stream) {
             OFB_CUDA(cudaStreamCreateWithFlags(&t->pyr_stream, cudaStreamNonBlocking));
@@ -648,46 +594,18 @@ static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitc
     TrackerDev T;
     T.prev = P; T.next = t->nxt.as<float>(); T.status = t->status.as<uint8_t>();
     T.kept_prev = t->kept_prev.as<float>(); T.kept_next = Pn;
-    T.count = count; T.need = need; T.kept = keptn; T.count0 = count + 3 * S; T.vlast = t->vlast.as<double>();
+    T.count = count; T.need = need; T.kept = keptn; T.vlast = t->vlast.as<double>();
     T.cap = cap; T.variant = pc.variant; T.cx = pc.cx; T.cy = pc.cy; T.ps = pc.pos_scale; T.fs = pc.flow_scale;
     T.cam = t->has_cam ? t->cam_dev.as<ofb_camera>() : nullptr; T.calib = t->calib.as<double4>();
     T.max_speed = cfg.max_speed; T.dummy = cfg.dummy_value; T.gate_mode = cfg.gate_mode; T.gate_T = cfg.gate_T;
     T.min_solve = cfg.min_solve; T.min_features = cfg.min_features; T.topup_mode = cfg.topup_mode; T.max_features = K;
     T.have_prev = t->have_prev ? 1 : 0;
-    OFB_TRY(ofb_features_scratch(fctx, w, h, pc.min_distance, S, &T.feat_state, &T.cell_grid, &T.cell_stride));
-    // graph capture: the top-up path goes into the body of an IF node whose condition the filter kernel sets, so a
-    // steady-state replay does not even launch the five kernels and two memsets that would exit at once
-    T.use_cond = 0; T.cond = 0;
-    cudaGraph_t cap_graph = nullptr;
-    if (t->capturing && t->capture_cond) {
-        cudaStreamCaptureStatus cs; const cudaGraphNode_t* deps = nullptr; size_t nd = 0;
-        if (cudaStreamGetCaptureInfo_v2(ctx->stream, &cs, nullptr, &cap_graph, &deps, &nd) != cudaSuccess ||
-            cs != cudaStreamCaptureStatusActive ||
-            cudaGraphConditionalHandleCreate(&T.cond, cap_graph, 0, cudaGraphCondAssignDefault) != cudaSuccess) {
-            cudaGetLastError();
-            return OFB_E_UNSUPPORTED;
-        }
-        T.use_cond = 1;
-    }
+    OFB_TRY(ofb_features_scratch(ctx, w, h, pc.min_distance, S, &T.feat_state, &T.cell_grid, &T.cell_stride));
     // 2. track the stream's points from the kept frame into the new one
-    auto lk = [&](const int* hi, const int* lo) -> int {
-        ctx->lk_lo = lo;
-        const int rc = ofb_lk_device(ctx, t->pyr[t->cur ^ 1], 0, 1, t->pyr[t->cur], 0, 1, S, P, hi, 1, cap, (size_t)cap, pc.win_w,
-                                     pc.win_h, pc.max_level, pc.max_count, pc.eps, 0, pc.min_eig_thr, t->nxt.as<float>(),
-                                     t->status.as<uint8_t>(), t->err.as<float>(), t->fb_max_err);
-        ctx->lk_lo = nullptr;
-        return rc;
-    };
-    if (t->have_prev && t->top_pending && early) {
-        // the previous step's top-up may still be running in the child context: the points that survived that step are
-        // tracked now, what the top-up appended (positions count0 .. count) once it has finished
-        OFB_TRY(lk(T.count0, nullptr));
-        OFB_CUDA(tracker_join_topup_only(t));
-        OFB_TRY(lk(count, T.count0));
-    } else {
-        OFB_CUDA(tracker_join_topup_only(t));
-        if (t->have_prev) OFB_TRY(lk(count, nullptr));
-    }
+    if (t->have_prev)
+        OFB_TRY(ofb_lk_device(ctx, t->pyr[t->cur ^ 1], 0, 1, t->pyr[t->cur], 0, 1, S, P, count, 1, cap, (size_t)cap, pc.win_w,
+                              pc.win_h, pc.max_level, pc.max_count, pc.eps, 0, pc.min_eig_thr, t->nxt.as<float>(),
+                              t->status.as<uint8_t>(), t->err.as<float>(), t->fb_max_err));
     t->lk_recorded = false;
     if (early && t->have_prev) { OFB_CUDA(cudaEventRecord(t->ev_lk, ctx->stream)); t->lk_recorded = true; }
     // 3.+4. status filter, gates, solve; the compacted new positions become the point set (Pn)
@@ -732,68 +650,27 @@ static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitc
     OFB_TRY(copy_out(kept_prev, t->kept_prev.as<float>()));
     OFB_TRY(copy_out(kept_next, Pn));                                 // the head of the new point set, before any top-up
     // 5. top-up on the current frame; streams that do not need it are skipped inside the kernels (no host sync)
-    cudaStream_t main_stream = ctx->stream;
-    const uint64_t top_l0 = fctx->launches;
-    if (defer) {
-        OFB_CUDA(cudaEventRecord(t->ev_filter, main_stream));
-        OFB_CUDA(cudaStreamWaitEvent(fctx->stream, t->ev_filter, 0));
-    }
-    cudaGraphNode_t cond_node = nullptr;
-    if (T.use_cond) {
-        cudaStreamCaptureStatus cs; const cudaGraphNode_t* deps = nullptr; size_t nd = 0;
-        cudaGraphNodeParams gp = {};
-        gp.type = cudaGraphNodeTypeConditional;
-        gp.conditional.handle = T.cond; gp.conditional.type = cudaGraphCondTypeIf; gp.conditional.size = 1;
-        if (cudaStreamGetCaptureInfo_v2(main_stream, &cs, nullptr, &cap_graph, &deps, &nd) != cudaSuccess ||
-            cudaGraphAddNode(&cond_node, cap_graph, deps, nd, &gp) != cudaSuccess || !gp.conditional.phGraph_out ||
-            cudaStreamBeginCaptureToGraph(t->side_stream, gp.conditional.phGraph_out[0], nullptr, nullptr, 0,
-                                          cudaStreamCaptureModeRelaxed) != cudaSuccess) {
-            cudaGetLastError();
-            return OFB_E_UNSUPPORTED;
-        }
-        ctx->stream = t->side_stream;                                 // the top-up launches below land in the IF body
-    }
-    auto end_body = [&](int rc) -> int {
-        if (!T.use_cond) return rc;
-        ctx->stream = main_stream;
-        cudaGraph_t body = nullptr;
-        const cudaError_t e = cudaStreamEndCapture(t->side_stream, &body);
-        if (rc != OFB_OK) { cudaGetLastError(); return rc; }
-        if (e != cudaSuccess ||
-            cudaStreamUpdateCaptureDependencies(main_stream, &cond_node, 1, cudaStreamSetCaptureDependencies) != cudaSuccess) {
-            cudaGetLastError();
-            return OFB_E_UNSUPPORTED;
-        }
-        return OFB_OK;
-    };
     const uint8_t* mask = nullptr;
     if (cfg.topup_mode == OFB_TOPUP_APPEND_MASKED && cfg.mask_radius > 0) {
-        const int mr = render_mask_device(fctx, t->mask.as<uint8_t>(), w, h, t->pitch_d, t->stride_d, S, Pn, (size_t)cap, cap, count,
-                                          need, t->hw.as<int>(), cfg.mask_radius);
-        if (mr != OFB_OK) return end_body(mr);
+        OFB_TRY(render_mask_device(ctx, t->mask.as<uint8_t>(), w, h, t->pitch_d, t->stride_d, S, Pn, (size_t)cap, cap, count,
+                                   need, t->hw.as<int>(), cfg.mask_radius));
         mask = t->mask.as<uint8_t>();
     }
     FeatImageState* st = nullptr;
     const unsigned int cand_cap = (unsigned int)(((size_t)w * h) / 4 + 1024);
-    fctx->feat_active = need;
-    fctx->feat_prezeroed = true;                                      // done by track_filter_solve_kernel
-    int fr = ofb_features_device(fctx, f, w, h, fpitch, (S == 1 ? 0 : fstride), S, mask, t->pitch_d, t->stride_d, K, pc.quality,
+    ctx->feat_active = need;
+    ctx->feat_prezeroed = true;                                       // done by track_filter_solve_kernel
+    int fr = ofb_features_device(ctx, f, w, h, fpitch, (S == 1 ? 0 : fstride), S, mask, t->pitch_d, t->stride_d, K, pc.quality,
                                  pc.min_distance, pc.block_size, cand_cap, t->det.as<float>(), (size_t)2 * K, K, &st);
-    fctx->feat_active = nullptr;
-    fctx->feat_prezeroed = false;
-    if (fr != OFB_OK) return end_body(fr);
-    topup_append_kernel<<<S, 128, 0, fctx->stream>>>(T, st, t->det.as<float>(), Pn, (ofb_track_result*)o[0].dev);
-    fctx->launches++;
-    if (defer) {
-        OFB_CUDA(cudaEventRecord(t->ev_top, fctx->stream));
-        t->top_pending = true;
-        ctx->launches += fctx->launches - top_l0;                     // (bench.py's gpu_launches reads the parent's counter)
-    }
+    ctx->feat_active = nullptr;
+    ctx->feat_prezeroed = false;
+    if (fr != OFB_OK) return fr;
+    topup_append_kernel<<<S, 128, 0, ctx->stream>>>(T, st, t->det.as<float>(), Pn, (ofb_track_result*)o[0].dev);
+    ctx->launches++;
     {
         const cudaError_t le = cudaGetLastError();
-        if (le != cudaSuccess) { ofb_set_error("tracker_step: topup_append launch -> %s", cudaGetErrorString(le)); return end_body(OFB_E_CUDA); }
+        if (le != cudaSuccess) { ofb_set_error("tracker_step: topup_append launch -> %s", cudaGetErrorString(le)); return OFB_E_CUDA; }
     }
-    OFB_TRY(end_body(OFB_OK));
     if (o[1].dev) OFB_CUDA(cudaMemcpyAsync(o[1].dev, count, sizeof(int) * S, cudaMemcpyDeviceToDevice, ctx->stream));
     OFB_TRY(copy_out(pts_out, Pn));
     t->pcur ^= 1;
@@ -840,23 +717,18 @@ static int tracker_step_graph(ofb_tracker* t, const uint8_t* frames, int pitch, 
     memcpy(pin + off_imu, imu, sizeof(ofb_imu_sample) * S);
     if (v_prior) memcpy(pin + off_vp, v_prior, sizeof(double) * 3 * S);
     const int par = t->cur, hp = v_prior ? 1 : 0;
-    if (!t->side_stream) OFB_CUDA(cudaStreamCreateWithFlags(&t->side_stream, cudaStreamNonBlocking));
     if (t->gexec[par][hp] && t->gsig[par][hp] != scratch_signature(ctx)) {
         cudaGraphExecDestroy(t->gexec[par][hp]);
         t->gexec[par][hp] = nullptr;
     }
-    for (int attempt = 0; attempt < 2 && !t->gexec[par][hp]; ++attempt) {
+    if (!t->gexec[par][hp]) {
         // capture = a dry run of the launch-by-launch body: it advances the host-side ping-pong state, which is
         // restored afterwards (the graph launch below is what executes the step)
         const int cur0 = t->cur, pcur0 = t->pcur; const bool hp0 = t->have_prev; const uint64_t l0 = ctx->launches;
         cudaGraph_t g = nullptr;
         if (cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeRelaxed) != cudaSuccess) { cudaGetLastError(); return OFB_E_UNSUPPORTED; }
         int rc = OFB_OK;
-        // OFB_TRACKER_COND=1 puts the top-up path into a conditional node. Measured on B200 (640x480, 200 features): the
-        // IF node costs more (97 us per step) than the seven nodes it skips, which exit at once (93 us) -- so the
-        // default keeps them inline.
-        const char* ce = getenv("OFB_TRACKER_COND");
-        t->capturing = true; t->capture_cond = t->cond_ok && ce && ce[0] == '1';
+        t->capturing = true;
         if (cudaMemcpyAsync(dio, pin + off_imu, sizeof(ofb_imu_sample) * S, cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess) rc = OFB_E_CUDA;
         if (rc == OFB_OK && v_prior &&
             cudaMemcpyAsync(dio + d_vp, pin + off_vp, sizeof(double) * 3 * S, cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess) rc = OFB_E_CUDA;
@@ -867,8 +739,7 @@ static int tracker_step_graph(ofb_tracker* t, const uint8_t* frames, int pitch, 
                                             ctx->stream) != cudaSuccess) rc = OFB_E_CUDA;
         const cudaError_t e = cudaStreamEndCapture(ctx->stream, &g);
         const uint64_t captured = ctx->launches - l0;
-        const bool with_cond = t->capture_cond;
-        t->capturing = false; t->capture_cond = false;
+        t->capturing = false;
         t->cur = cur0; t->pcur = pcur0; t->have_prev = hp0; ctx->launches = l0;
         cudaGraphExec_t ex = nullptr;
         bool ok = rc == OFB_OK && e == cudaSuccess && g;
@@ -876,15 +747,12 @@ static int tracker_step_graph(ofb_tracker* t, const uint8_t* frames, int pitch, 
         if (g) cudaGraphDestroy(g);
         if (!ok) {
             cudaGetLastError();
-            if (with_cond) { t->cond_ok = false; continue; }         // retry with the top-up path inline
             return OFB_E_UNSUPPORTED;
         }
         t->gexec[par][hp] = ex; t->glaunches[par][hp] = captured;
         t->gsig[par][hp] = scratch_signature(ctx);                    // (the dry run cannot grow an arena: three plain steps sized them)
-        if (with_cond) t->cond_used = true;
     }
-    if (!t->gexec[par][hp]) return OFB_E_UNSUPPORTED;
-    OFB_CUDA(tracker_join_topup(t));
+    OFB_CUDA(tracker_join_solve(t));
     OFB_CUDA(cudaGraphLaunch(t->gexec[par][hp], ctx->stream));
     t->lk_recorded = false;             // (a later launch-by-launch step orders its ingest behind this graph)
     ctx->launches += t->glaunches[par][hp];
@@ -960,13 +828,13 @@ extern "C" int ofb_tracker_set_fb_check(ofb_tracker* t, double fb_max_err)
     return OFB_OK;
 }
 
-/* steps replayed from a CUDA graph so far (0 when graphs are off or were never eligible); *conditional_out = 1 when
- * the top-up path sits in a conditional node of those graphs */
+/* steps replayed from a CUDA graph so far (0 when graphs are off or were never eligible); *conditional_out is always 0
+ * (the captured graphs hold no conditional node) */
 extern "C" int ofb_tracker_graph_info(const ofb_tracker* t, uint64_t* steps_out, int* conditional_out)
 {
     OFB_REQUIRE(t && steps_out, "tracker_graph_info: null argument");
     *steps_out = t->graph_steps;
-    if (conditional_out) *conditional_out = t->cond_used ? 1 : 0;
+    if (conditional_out) *conditional_out = 0;
     return OFB_OK;
 }
 

@@ -95,7 +95,7 @@ class StreamTracker:
         return self.graph_info()[0]
 
     def graph_info(self):
-        """(steps replayed from a graph, whether the top-up path is a conditional node of it)"""
+        """(steps replayed from a graph, False): the second element is always False, the graphs hold no conditional node"""
         n, c = C.c_uint64(), C.c_int()
         _lib.check(self.ctx.lib.ofb_tracker_graph_info(self.h, C.byref(n), C.byref(c)))
         return n.value, bool(c.value)

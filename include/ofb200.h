@@ -358,15 +358,13 @@ int ofb_tracker_step(ofb_tracker* trk, const uint8_t* frames, int pitch, size_t 
 /* Small fleets fed from host memory (<= 16 MB of frames per step, host imu/results, no optional outputs) are
  * launch bound: from the fourth step on such a step is replayed from a captured CUDA graph (inputs staged in
  * pinned buffers at fixed addresses; one graph per ping-pong parity). Results are identical to the launch-by-launch
- * path; OFB_TRACKER_GRAPH=0 in the environment disables the graph. With OFB_TRACKER_COND=1 the top-up path becomes the
- * body of a conditional (IF) node whose condition the filter kernel sets on the device (cudaGraphSetConditional);
- * measured slower than letting its kernels exit at once, hence opt-in. *steps_out = steps replayed from a graph so
- * far; *conditional_out (may be NULL) = 1 when those graphs use the conditional node. */
+ * path; OFB_TRACKER_GRAPH=0 in the environment disables the graph. *steps_out = steps replayed from a graph so far;
+ * *conditional_out (may be NULL) is always 0: the graphs hold no conditional node. */
 int ofb_tracker_graph_info(const ofb_tracker* trk, uint64_t* steps_out, int* conditional_out);
 /* Attach a calibrated camera to every stream of the tracker (cam == NULL detaches it: back to cfg.pair's pinhole).
  * From the next ofb_tracker_step on, the r_tilde gate, the MODULE variant's per-point distances and the solve see
  * x = undistort(p_new), u = (undistort(p_new) - undistort(p_old)) * rate; static_immobile stays in pixels. A step
- * already enqueued (split solve, deferred top-up, graph replay) keeps the camera it was enqueued with. */
+ * already enqueued (split solve, graph replay) keeps the camera it was enqueued with. */
 int ofb_tracker_set_camera(ofb_tracker* trk, const ofb_camera* cam);
 /* Forward-backward check of every stream's LK tracks (see ofb_pyrlk_fb) from the next ofb_tracker_step on; 0 turns it
  * off (the default). A point that fails it counts as lost (status 0): it leaves the set before the gates, the solve

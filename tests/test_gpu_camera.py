@@ -206,18 +206,17 @@ SWITCH = {5: "B", 9: None, 12: "A"}          # step -> camera set before it
 def run_switching(ofb200, kw, frames, imus, mode, monkeypatch):
     """One stream through the sequence forwards and backwards, switching cameras at the SWITCH steps. mode: "graph"
     (host frames: graph replay from the fourth step), "plain" (OFB_TRACKER_GRAPH=0), "kept" (host frames with the kept
-    tracks read back), "split" / "nosplit" / "defer" (device frames, IMU samples and result records: split solve
-    default on, OFB_TRACKER_SPLIT_SOLVE=0, OFB_TRACKER_DEFER_TOPUP=1)."""
+    tracks read back), "split" / "nosplit" (device frames, IMU samples and result records: split solve default on,
+    OFB_TRACKER_SPLIT_SOLVE=0)."""
     import torch
     monkeypatch.setenv("OFB_TRACKER_GRAPH", "0" if mode == "plain" else "1")
     monkeypatch.setenv("OFB_TRACKER_SPLIT_SOLVE", "0" if mode == "nosplit" else "1")
-    monkeypatch.setenv("OFB_TRACKER_DEFER_TOPUP", "1" if mode == "defer" else "0")
     cams = {"A": cam_for(kw), "B": cam_for(kw, [0.05, -0.01, 0.002, 0.001, 0.0, 0.02, 0.0, 0.001])}
     ctx = ofb200.Context(0)                 # a context that owns its stream: the tracker may use its side streams
     trk = ofb200.StreamTracker(tc.W, tc.H, ctx=ctx, camera=cams["A"], **kw)
     order = list(range(len(frames))) + list(range(len(frames) - 2, -1, -1))
     out, kept = [], []
-    dev = mode in ("split", "nosplit", "defer")
+    dev = mode in ("split", "nosplit")
     d_res = torch.zeros(C.sizeof(ofb200._lib.TrackResult), dtype=torch.uint8, device="cuda") if dev else None
     try:
         for j, k in enumerate(order):
@@ -266,7 +265,7 @@ def test_camera_switch_identical_in_every_mode(ofb200, monkeypatch):
         v = vo.solve_lgs(x, u, im["d"], im["n"], im["w"], im["t"], kw["variant"])[0]
         assert relerr(ref[j]["v"][0], v) <= 1e-9, j
     assert solved >= 8
-    for mode in ("graph", "plain", "split", "nosplit", "defer"):
+    for mode in ("graph", "plain", "split", "nosplit"):
         got, _, graph_steps, _, _ = run_switching(ofb200, kw, frames, imus, mode, monkeypatch)
         if mode == "graph":
             assert graph_steps >= len(order) - 3 - 1, graph_steps

@@ -1,7 +1,7 @@
 """GPU side of the forward-backward check (include/ofb200.h `ofb_pyrlk_fb`, `ofb_frame_pairs_fb`,
 `ofb_tracker_set_fb_check`): the fused kernel against the composition of two LK calls and the NumPy fold, bit for bit;
 against cv2 4.13 (golden file and live); the frame-pair routes, the camera and the solve; the tracker against
-TrackerOracle with oracle/fb_oracle.FBEngine, graph replay, switching and the deferred paths; the outlier scene; and
+TrackerOracle with oracle/fb_oracle.FBEngine, graph replay, switching and the split solve; the outlier scene; and
 the argument checks."""
 import ctypes as C
 
@@ -240,12 +240,11 @@ def run_switching(ofb200, kw, frames, imus, mode, monkeypatch, camera=None, swit
     import torch
     monkeypatch.setenv("OFB_TRACKER_GRAPH", "0" if mode == "plain" else "1")
     monkeypatch.setenv("OFB_TRACKER_SPLIT_SOLVE", "0" if mode == "nosplit" else "1")
-    monkeypatch.setenv("OFB_TRACKER_DEFER_TOPUP", "1" if mode == "defer" else "0")
     ctx = ofb200.Context(0)
     trk = ofb200.StreamTracker(tc.W, tc.H, ctx=ctx, camera=camera, fb_threshold=start, **kw)
     order = list(range(len(frames))) + list(range(len(frames) - 2, -1, -1))
     out = []
-    dev = mode in ("split", "nosplit", "defer")
+    dev = mode in ("split", "nosplit")
     d_res = torch.zeros(C.sizeof(ofb200._lib.TrackResult), dtype=torch.uint8, device="cuda") if dev else None
     try:
         for j, k in enumerate(order):
@@ -270,13 +269,13 @@ def run_switching(ofb200, kw, frames, imus, mode, monkeypatch, camera=None, swit
 
 @pytest.mark.parametrize("scenario,camera", [("exp", False), ("node", True)])
 def test_tracker_fb_switch_identical_in_every_mode(ofb200, monkeypatch, scenario, camera):
-    """on / off / on / off mid-sequence: graph replay, plain launches, split solve and the deferred top-up give the
+    """on / off / on / off mid-sequence: graph replay, the split solve and one kernel for filter and solve give the
     records of plain launches; with the check, with a camera and with the masked top-up ("node")"""
     frames, imus, kw = tc.build(scenario)
     frames, imus = frames[0], imus[0]
     cam = cam_for(kw) if camera else None
     ref, _, order = run_switching(ofb200, kw, frames, imus, "plain", monkeypatch, cam)
-    for mode in ("graph", "split", "nosplit", "defer"):
+    for mode in ("graph", "split", "nosplit"):
         got, graph_steps, _ = run_switching(ofb200, kw, frames, imus, mode, monkeypatch, cam)
         if mode == "graph":
             assert graph_steps >= 6, graph_steps
@@ -309,7 +308,7 @@ def test_tracker_fb_switch_matches_oracle(ofb200, ctx):
 def test_tracker_threshold_zero_is_no_check(ofb200, monkeypatch):
     frames, imus, kw = tc.build("node")
     frames, imus = frames[0], imus[0]
-    for mode in ("graph", "defer"):
+    for mode in ("graph", "split"):
         never, _, order = run_switching(ofb200, kw, frames, imus, mode, monkeypatch, switch={}, start=None)
         zero, _, _ = run_switching(ofb200, kw, frames, imus, mode, monkeypatch, switch={1: 0.0, 5: 0.0}, start=0.0)
         for j in range(len(order)):

@@ -342,8 +342,7 @@ def test_tracker_bgr_fused_equals_separate_conversion(ctx):
 
 def test_tracker_stream_overlap_modes_are_identical(ctx):
     """ofb_tracker_step with device-resident frames / IMU / result records runs the ingest + pyramid on its own stream, the
-    fp64 solve on another one beside the next frame's LK, and (opt-in) defers the top-up path to a child context (the next
-    step tracks the surviving points before it joins). All of that is scheduling only: the records of every step and the final point sets must equal the single-stream schedule
+    fp64 solve on another one beside the next frame's LK. That is scheduling only: the records of every step and the final point sets must equal the single-stream schedule
     (OFB_TRACKER_EARLY_PYR=0), with frequent top-ups (min_features close to max_features), for one stream and a small fleet."""
     import torch
     import ofb200
@@ -367,8 +366,8 @@ def test_tracker_stream_overlap_modes_are_identical(ctx):
                   principal=(mo["cx"], mo["cy"]), scaling=1.0 / mo["f"], flow_scaling=1.0 / (mo["f"] * mo["dt"]),
                   borrow_frames=True, ctx=ctx)
 
-        def run(early, defer, split="0"):
-            os.environ["OFB_TRACKER_EARLY_PYR"], os.environ["OFB_TRACKER_DEFER_TOPUP"] = early, defer
+        def run(early, split="0"):
+            os.environ["OFB_TRACKER_EARLY_PYR"] = early
             os.environ["OFB_TRACKER_SPLIT_SOLVE"] = split
             try:
                 trk = ofb200.StreamTracker(w, h, **kw)
@@ -385,15 +384,14 @@ def test_tracker_stream_overlap_modes_are_identical(ctx):
                 trk.close()
                 return res, last, pts
             finally:
-                os.environ.pop("OFB_TRACKER_EARLY_PYR", None); os.environ.pop("OFB_TRACKER_DEFER_TOPUP", None)
-                os.environ.pop("OFB_TRACKER_SPLIT_SOLVE", None)
-        ref = run("0", "0")
+                os.environ.pop("OFB_TRACKER_EARLY_PYR", None); os.environ.pop("OFB_TRACKER_SPLIT_SOLVE", None)
+        ref = run("0")
         assert ref[0]["n_added"].sum() > 0, "the case must exercise the top-up"
         # (split: the fp64 solve of a step on its own stream beside the next frame's LK, track_filter_solve_kernel<1> / <2>)
-        for early, defer, split in (("1", "0", "0"), ("1", "1", "0"), ("1", "0", "1"), ("1", "1", "1")):
-            got = run(early, defer, split)
+        for early, split in (("1", "0"), ("1", "1")):
+            got = run(early, split)
             for f in ("v", "s", "res", "rank", "n_prev", "n_tracked", "n_kept", "n_added", "n_points", "flags"):
-                assert np.array_equal(got[0][f], ref[0][f], equal_nan=True), (S, early, defer, split, f)
-                assert np.array_equal(got[1][f], ref[1][f], equal_nan=True), (S, early, defer, split, f, "last")
+                assert np.array_equal(got[0][f], ref[0][f], equal_nan=True), (S, early, split, f)
+                assert np.array_equal(got[1][f], ref[1][f], equal_nan=True), (S, early, split, f, "last")
             for s in range(S):
-                assert np.array_equal(got[2][s], ref[2][s]), (S, early, defer, split, s)
+                assert np.array_equal(got[2][s], ref[2][s]), (S, early, split, s)

@@ -138,7 +138,7 @@ enum {
     SC_IN0 = 0, SC_IN1, SC_IN2, SC_IN3, SC_IN4, SC_IN5,      // staged host inputs
     SC_OUT0, SC_OUT1, SC_OUT2, SC_OUT3,                      // staged outputs
     SC_CAND, SC_CANDCNT, SC_SEL, SC_GRID, SC_PTS0, SC_PTS1, SC_STAT, SC_ERR,
-    SC_MC0, SC_MC1, SC_MC2, SC_TMP0, SC_TMP1, SC_TMP2,
+    SC_MC0, SC_MC1, SC_MC2, SC_TMP0, SC_TMP1,
     SC_FRAMES,                                               // device staging of host frames (ofb_frame_pairs)
     SC_CALIB                                                 // calibrated tracks of ofb_frame_pairs_cam
 };

@@ -216,65 +216,80 @@ extern "C" int ofb_frame_pairs_fb(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const o
         if ((const float*)pts_in != d_prev)
             OFB_CUDA(cudaMemcpyAsync(d_prev, pts_in, sizeof(float) * 2 * npts, cudaMemcpyDefault, ctx->stream));
     }
-    const bool host_frames = !ofb_is_device_ptr(prev) && !ofb_is_device_ptr(next);
-    // consecutive frames of one stream in one buffer: each frame is uploaded and its pyramid built once per sub-batch
+    const bool dev_prev = ofb_is_device_ptr(prev), dev_next = ofb_is_device_ptr(next);
+    // consecutive frames of one stream in one buffer: each frame is uploaded and its pyramid built once per chunk
     const bool seq = next == prev + image_stride && n_pairs > 1;
-    const int chunk = 8;
-    if (host_frames && n_pairs > chunk && !ctx->profile) {
-        // Host frames: pipeline sub-batches. The frames of the whole call are staged in one device buffer by
-        // back-to-back H2D copies on a copy stream (the PCIe copy is the bound: nothing else is ever queued between
-        // two copies); a sub-batch starts as soon as its frames have landed and then runs exactly the resident path
-        // (level 0 aliases the staging buffer; in the sequence layout a frame shared by two sub-batches is simply
-        // read by both). Sub-batches compute alternately on this context and on its twin (own stream and scratch),
-        // so the one-CTA-per-image selection of sub-batch i runs beside the lambda_min kernel of sub-batch i+1. The
-        // last sub-batches are smaller: what remains after the last copy is one short chain.
-        if (!ctx->twin) {
-            OFB_TRY(ofb_ctx_create(ctx->device, &ctx->twin));
-            OFB_CUDA(cudaEventCreateWithFlags(&ctx->ev_twin_fork, cudaEventDisableTiming));
-            OFB_CUDA(cudaEventCreateWithFlags(&ctx->ev_twin_join, cudaEventDisableTiming));
-        }
-        ofb_ctx* tw = ctx->twin;
+    const int extra = seq ? 1 : 0;                  // a chunk of n pairs holds n + extra prev frames
+    // Chunk schedule. Chunks of at most `cap` pairs (the capacity of their pyramids) alternate between this context and a
+    // twin context with its own stream and scratch, so the lambda_min kernel (shared-memory heavy, issue bound) of one
+    // chunk and the selection and LK kernels of the other are co-resident on the SMs instead of running back to back.
+    //   * host frames (staged): the frames of the whole call are staged in one device buffer by back-to-back H2D copies on
+    //     a copy stream (the PCIe copy is the bound: nothing else is ever queued between two copies); a chunk of 8 pairs
+    //     starts as soon as its frames have landed, with level 0 aliasing the staging buffer (in the sequence layout a
+    //     frame shared by two chunks is simply read by both). The last chunks are smaller (8, ..., 8, 4, 2, 2): what
+    //     remains after the last copy is one short chain.
+    //   * device frames: two halves of the batch, level 0 is the caller's buffer.
+    //   * otherwise (a small batch, mixed host / device frames, stage timing): one pass over the whole batch.
+    const bool staged = !dev_prev && !dev_next && n_pairs > 8 && !ctx->profile;
+    int cap = n_pairs;
+    if (staged) cap = 8;
+    else if (dev_prev && dev_next && n_pairs >= 2 && !ctx->profile) cap = (n_pairs + 1) / 2;
+    const bool use_twin = n_pairs > cap;
+    if (use_twin && !ctx->twin) {
+        OFB_TRY(ofb_ctx_create(ctx->device, &ctx->twin));
+        OFB_CUDA(cudaEventCreateWithFlags(&ctx->ev_twin_fork, cudaEventDisableTiming));
+        OFB_CUDA(cudaEventCreateWithFlags(&ctx->ev_twin_join, cudaEventDisableTiming));
+    }
+    // level 0 of the chunk pyramids: prev frame i at fprev + i * fstride, next frame i at fnext + i * fstride
+    const uint8_t* fprev = prev; const uint8_t* fnext = next;
+    int fpitch = pitch; size_t fstride = image_stride;
+    uint8_t* frames = nullptr;                      // staging buffer: the prev frames, then (unless seq) the next frames
+    if (staged) {
         if (!ctx->copy_stream) OFB_CUDA(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
         if (!ctx->ev_free[0]) OFB_CUDA(cudaEventCreateWithFlags(&ctx->ev_free[0], cudaEventDisableTiming));
-        const int pitch_d = (w + 15) & ~15;
-        const size_t stride_d = (((size_t)pitch_d * h) + 255) & ~(size_t)255;
-        const size_t n_frames = seq ? (size_t)n_pairs + 1 : 2 * (size_t)n_pairs;
-        OFB_TRY(ctx->scratch[SC_FRAMES].reserve(stride_d * n_frames + 256));
-        uint8_t* d_frames = ctx->scratch[SC_FRAMES].as<uint8_t>();
-        uint8_t* d_prevf = d_frames;
-        uint8_t* d_nextf = seq ? d_frames + stride_d : d_frames + stride_d * (size_t)n_pairs;
-        auto upload = [&](uint8_t* dst, const uint8_t* src, int count) -> int {
-            if (count <= 0) return OFB_OK;
-            if (pitch == pitch_d && image_stride == stride_d) {            // same layout on both sides: one copy
-                OFB_CUDA(cudaMemcpyAsync(dst, src, stride_d * (size_t)(count - 1) + (size_t)pitch * (h - 1) + w,
-                                         cudaMemcpyHostToDevice, ctx->copy_stream));
-                return OFB_OK;
-            }
-            for (int i = 0; i < count; ++i)
-                OFB_CUDA(cudaMemcpy2DAsync(dst + (size_t)i * stride_d, pitch_d, src + (size_t)i * image_stride, pitch, w, h,
-                                           cudaMemcpyHostToDevice, ctx->copy_stream));
-            return OFB_OK;
-        };
+        fpitch = (w + 15) & ~15;
+        fstride = (((size_t)fpitch * h) + 255) & ~(size_t)255;
+        OFB_TRY(ctx->scratch[SC_FRAMES].reserve(fstride * (seq ? (size_t)n_pairs + 1 : 2 * (size_t)n_pairs) + 256));
+        frames = ctx->scratch[SC_FRAMES].as<uint8_t>();
+        fprev = frames;
+        fnext = frames + fstride * (seq ? 1 : (size_t)n_pairs);
         // the staging buffer may still be read by work enqueued earlier (a previous call with device-side outputs)
         OFB_CUDA(cudaEventRecord(ctx->ev_free[0], ctx->stream));
         OFB_CUDA(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_free[0], 0));
+    }
+    auto upload = [&](uint8_t* dst, const uint8_t* src, int count) -> int {
+        if (count <= 0) return OFB_OK;
+        if (pitch == fpitch && image_stride == fstride) {            // same layout on both sides: one copy
+            OFB_CUDA(cudaMemcpyAsync(dst, src, fstride * (size_t)(count - 1) + (size_t)pitch * (h - 1) + w,
+                                     cudaMemcpyHostToDevice, ctx->copy_stream));
+            return OFB_OK;
+        }
+        for (int i = 0; i < count; ++i)
+            OFB_CUDA(cudaMemcpy2DAsync(dst + (size_t)i * fstride, fpitch, src + (size_t)i * image_stride, pitch, w, h,
+                                       cudaMemcpyHostToDevice, ctx->copy_stream));
+        return OFB_OK;
+    };
+    ofb_ctx* tw = ctx->twin;
+    uint64_t tw0 = 0;
+    if (use_twin) {
         // staged inputs (IMU samples, seed points) were enqueued on this context's stream
         OFB_CUDA(cudaEventRecord(ctx->ev_twin_fork, ctx->stream));
         OFB_CUDA(cudaStreamWaitEvent(tw->stream, ctx->ev_twin_fork, 0));
-        const uint64_t tw0 = tw->launches;
-        int ci = 0;
-        for (int c0 = 0; c0 < n_pairs; ++ci) {
-            const int left = n_pairs - c0;
-            const int n = left > 12 ? chunk : left > 4 ? 4 : left > 2 ? 2 : left;
-            ofb_ctx* c = (ci & 1) ? tw : ctx;
-            const int slot = (ci >> 1) & 1;
+        tw0 = tw->launches;
+    }
+    for (int c0 = 0, ci = 0, n = 0; c0 < n_pairs; c0 += n, ++ci) {
+        const int left = n_pairs - c0;
+        n = !staged ? (left < cap ? left : cap) : left > 12 ? 8 : left > 4 ? 4 : left > 2 ? 2 : left;
+        ofb_ctx* c = (ci & 1) ? tw : ctx;
+        const int slot = (ci >> 1) & 1;
+        if (staged) {
             if (seq) {
-                // frames c0 .. c0+n; frame c0 came with the previous sub-batch
+                // frames c0 .. c0+n; frame c0 came with the previous chunk
                 const int f0 = ci == 0 ? 0 : c0 + 1;
-                OFB_TRY(upload(d_frames + (size_t)f0 * stride_d, prev + (size_t)f0 * image_stride, c0 + n + 1 - f0));
+                OFB_TRY(upload(frames + (size_t)f0 * fstride, prev + (size_t)f0 * image_stride, c0 + n + 1 - f0));
             } else {
-                OFB_TRY(upload(d_prevf + (size_t)c0 * stride_d, prev + (size_t)c0 * image_stride, n));
-                OFB_TRY(upload(d_nextf + (size_t)c0 * stride_d, next + (size_t)c0 * image_stride, n));
+                OFB_TRY(upload(frames + (size_t)c0 * fstride, prev + (size_t)c0 * image_stride, n));
+                OFB_TRY(upload(frames + ((size_t)n_pairs + c0) * fstride, next + (size_t)c0 * image_stride, n));
             }
             if ((int)ctx->ev_piece.size() <= ci) {
                 cudaEvent_t e;
@@ -283,63 +298,22 @@ extern "C" int ofb_frame_pairs_fb(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const o
             }
             OFB_CUDA(cudaEventRecord(ctx->ev_piece[ci], ctx->copy_stream));
             OFB_CUDA(cudaStreamWaitEvent(c->stream, ctx->ev_piece[ci], 0));
-            // (c, slot) is reused every fourth sub-batch, on the same stream: stream order protects its upper levels
-            OFB_TRY(ofb_pyr_prepare(c, &c->pair_pyr[slot][0], d_prevf + (size_t)c0 * stride_d, w, h, pitch_d, stride_d,
-                                    seq ? n + 1 : n, seq ? chunk + 1 : chunk, cfg->max_level, false));
-            if (!seq)
-                OFB_TRY(ofb_pyr_prepare(c, &c->pair_pyr[slot][1], d_nextf + (size_t)c0 * stride_d, w, h, pitch_d, stride_d, n,
-                                        chunk, cfg->max_level, false));
-            OFB_TRY(run_pairs_chunk(c, cfg, cam, fb_max_err, c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
-                                    (const ofb_imu_sample*)dimu, counts_in, d_prev, d_next, d_stat, (ofb_pair_result*)o[3].dev, false));
-            c0 += n;
         }
+        // (c, slot) is reused every fourth chunk, on the same stream: stream order protects its upper levels
+        OFB_TRY(ofb_pyr_prepare(c, &c->pair_pyr[slot][0], fprev + (size_t)c0 * fstride, w, h, fpitch, fstride, n + extra,
+                                cap + extra, cfg->max_level, false));
+        if (!seq)
+            OFB_TRY(ofb_pyr_prepare(c, &c->pair_pyr[slot][1], fnext + (size_t)c0 * fstride, w, h, fpitch, fstride, n, cap,
+                                    cfg->max_level, false));
+        OFB_TRY(run_pairs_chunk(c, cfg, cam, fb_max_err, c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
+                                (const ofb_imu_sample*)dimu, counts_in, d_prev, d_next, d_stat, (ofb_pair_result*)o[3].dev,
+                                ctx->profile));
+    }
+    if (use_twin) {
         ctx->launches += tw->launches - tw0;
         OFB_CUDA(cudaEventRecord(ctx->ev_twin_join, tw->stream));
         OFB_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_twin_join, 0));
-        return ofb_finish_out(ctx, o, 4);
     }
-    // Resident frames: the batch is cut into chunks that alternate between this context and a twin context with its own
-    // stream and scratch. The lambda_min kernel (shared-memory heavy, issue bound) of one chunk and the LK kernel
-    // (register heavy, latency bound) of the other are then co-resident on the SMs instead of running back to back.
-    static const int twin_chunks = [] { const char* e = getenv("OFB_TWIN_CHUNKS"); return e ? atoi(e) : 2; }();
-    if (!host_frames && ofb_is_device_ptr(prev) && ofb_is_device_ptr(next) && !ctx->profile && twin_chunks >= 2 &&
-        n_pairs >= twin_chunks) {
-        if (!ctx->twin) {
-            OFB_TRY(ofb_ctx_create(ctx->device, &ctx->twin));
-            OFB_CUDA(cudaEventCreateWithFlags(&ctx->ev_twin_fork, cudaEventDisableTiming));
-            OFB_CUDA(cudaEventCreateWithFlags(&ctx->ev_twin_join, cudaEventDisableTiming));
-        }
-        ofb_ctx* tw = ctx->twin;
-        // staged inputs (IMU samples, seed points) were enqueued on this context's stream
-        OFB_CUDA(cudaEventRecord(ctx->ev_twin_fork, ctx->stream));
-        OFB_CUDA(cudaStreamWaitEvent(tw->stream, ctx->ev_twin_fork, 0));
-        const int per = (n_pairs + twin_chunks - 1) / twin_chunks;
-        const uint64_t tw0 = tw->launches;
-        int ci = 0;
-        for (int c0 = 0; c0 < n_pairs; c0 += per, ++ci) {
-            const int n = n_pairs - c0 < per ? n_pairs - c0 : per;
-            ofb_ctx* c = (ci & 1) ? tw : ctx;
-            const int slot = (ci >> 1) & 1;
-            OFB_TRY(ofb_pyr_prepare(c, &c->pair_pyr[slot][0], prev + (size_t)c0 * image_stride, w, h, pitch, image_stride,
-                                    seq ? n + 1 : n, seq ? per + 1 : per, cfg->max_level, false));
-            if (!seq)
-                OFB_TRY(ofb_pyr_prepare(c, &c->pair_pyr[slot][1], next + (size_t)c0 * image_stride, w, h, pitch, image_stride, n, per,
-                                        cfg->max_level, false));
-            OFB_TRY(run_pairs_chunk(c, cfg, cam, fb_max_err, c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
-                                    (const ofb_imu_sample*)dimu, counts_in, d_prev, d_next, d_stat, (ofb_pair_result*)o[3].dev, false));
-        }
-        ctx->launches += tw->launches - tw0;
-        OFB_CUDA(cudaEventRecord(ctx->ev_twin_join, tw->stream));
-        OFB_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_twin_join, 0));
-        return ofb_finish_out(ctx, o, 4);
-    }
-    // resident frames (or a small batch): one pass over the whole batch
-    OFB_TRY(ofb_pyr_prepare(ctx, &ctx->pair_pyr[0][0], prev, w, h, pitch, image_stride, seq ? n_pairs + 1 : n_pairs,
-                            seq ? n_pairs + 1 : n_pairs, cfg->max_level, false));
-    if (!seq)
-        OFB_TRY(ofb_pyr_prepare(ctx, &ctx->pair_pyr[0][1], next, w, h, pitch, image_stride, n_pairs, n_pairs, cfg->max_level, false));
-    OFB_TRY(run_pairs_chunk(ctx, cfg, cam, fb_max_err, ctx->pair_pyr[0][0], seq ? ctx->pair_pyr[0][0] : ctx->pair_pyr[0][1], n_pairs, 0,
-                            (const ofb_imu_sample*)dimu, counts_in, d_prev, d_next, d_stat, (ofb_pair_result*)o[3].dev, ctx->profile));
     int rc = ofb_finish_out(ctx, o, 4);
     if (rc == OFB_OK && ctx->profile) {
         // stage order: 0 pyramids, 1 lambda_min+NMS, 2 ordered selection, 3 LK, 4 solve

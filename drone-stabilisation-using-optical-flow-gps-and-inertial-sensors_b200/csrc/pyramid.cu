@@ -24,10 +24,7 @@ constexpr int PT_W = 64, PT_H = 32;                 // output tile
 constexpr int PS_W = 2 * PT_W + 32;                 // staged source columns: 2*X0-16 .. 2*X0+143 (10 x 16 bytes)
 constexpr int PS_H = 2 * PT_H + 3;                  // staged source rows:    2*Y0-2 .. 2*Y0+64
 constexpr int PS_PITCH = PS_W;                      // bytes, multiple of 16
-#ifndef OFB_PYR_THREADS
-#define OFB_PYR_THREADS 256
-#endif
-constexpr int PYR_THREADS = OFB_PYR_THREADS;        // threads of the two down-sampling kernels (the filter uses 128)
+constexpr int PYR_THREADS = 256;                    // threads of the two down-sampling kernels (the filter uses 128)
 
 __device__ __forceinline__ int refl101(int p, int len)
 {
@@ -361,15 +358,12 @@ static PFN_cuTensorMapEncodeTiled tensor_map_encoder()
     static bool tried = false;
     if (!tried) {
         tried = true;
-        const char* off = getenv("OFB_NO_TMA");
-        if (!(off && off[0] == '1')) {
-            void* f = nullptr;
-            cudaDriverEntryPointQueryResult q;
-            if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) == cudaSuccess &&
-                q == cudaDriverEntryPointSuccess)
-                fn = (PFN_cuTensorMapEncodeTiled)f;
-            else cudaGetLastError();
-        }
+        void* f = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) == cudaSuccess &&
+            q == cudaDriverEntryPointSuccess)
+            fn = (PFN_cuTensorMapEncodeTiled)f;
+        else cudaGetLastError();
     }
     return fn;
 }
@@ -405,8 +399,7 @@ int ofb_pyr_build_from(ofb_ctx* ctx, ofb_pyr* p, int first_level)
         // (the in-CTA double buffering pays once a CTA owns several tiles; a level with fewer than ~4 tiles per
         // resident CTA runs one tile per CTA and relies on the 5 co-resident CTAs to overlap copy and filter)
         long long grid = (long long)ctx->sm_count * (5 * 256 / PYR_THREADS);
-        static const int persist_min = [] { const char* e = getenv("OFB_PYR_PERSIST_MIN"); return e && atoi(e) > 0 ? atoi(e) : 4; }();
-        if (n_tiles < grid * persist_min) grid = n_tiles;
+        if (n_tiles < grid * 4) grid = n_tiles;
         if (grid == n_tiles) {
             // small level: latency-bound, one tile per CTA with direct loads
             dim3 g3(tiles_x, tiles_y, p->n_active);

@@ -254,10 +254,7 @@ lk_track_kernel(LKParams P, const float* __restrict__ prev_pts, float* __restric
 }
 
 // ================= register-resident fast path: winW <= 16, winH <= 15 (the reference uses 15x15) ============
-#ifndef OFB_LKF_WARPS
-#define OFB_LKF_WARPS 1
-#endif
-constexpr int LKF_WARPS = OFB_LKF_WARPS;
+constexpr int LKF_WARPS = 1;                 // one feature per CTA: see lk_track_fast2_kernel
 
 __device__ __forceinline__ int dp2a_lo(int w16x2, unsigned int bytes, int c)
 {
@@ -348,7 +345,7 @@ __device__ __forceinline__ unsigned int prmt(unsigned int a, unsigned int b, uns
 //     evaluation OpenCV uses is only needed there).
 // One feature = one warp = one CTA: no shared memory and no block barrier, and features differ in their number of Newton
 // steps -- with four warps per CTA the three that finished early kept their slots until the slowest one was done
-// (0.854 -> 0.805 ms per 128 pairs with one; -DOFB_LKF_WARPS=n for A/B builds). 32 CTAs per SM.
+// (0.854 -> 0.805 ms per 128 pairs with one). 32 CTAs per SM.
 // FB = the forward-backward check (ofb_pyrlk_fb): a feature whose forward track has status 1 is tracked back from
 // where it landed, in the same warp, and keeps status 1 only when the backward track has status 1 too and ends within
 // fb_thr of the starting point (max-norm of the fp32 difference, compared in fp64). next_pts and err are the forward

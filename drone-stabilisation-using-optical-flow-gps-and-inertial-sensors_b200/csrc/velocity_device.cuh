@@ -3,9 +3,7 @@
 #pragma once
 #include "math3.cuh"
 
-#ifndef OFB_SOLVE_THREADS
-#define OFB_SOLVE_THREADS 256
-#endif
+constexpr int OFB_SOLVE_THREADS = 256;   // threads of a one-CTA-per-frame solve
 
 struct OfbSolveOut { double v[3]; double s[3]; double res; int rank; int count; };
 

@@ -45,6 +45,21 @@ def as_list(p):
     return np.zeros((0, 2), np.float32) if p is None else np.asarray(p).reshape(-1, 2)
 
 
+def min_eig_map_unaligned(ofb200, ctx, img, bs):
+    """cornerMinEigenVal of a device copy of img that starts 1 byte past an aligned address and has an odd pitch: every
+    strip of the marching kernel then takes its general row loop (the lean loops need 4-byte-aligned rows)."""
+    import torch
+    h, w = img.shape
+    pitch = w + 1 + w % 2
+    host = np.zeros(1 + h * pitch, np.uint8)
+    host[1:].reshape(h, pitch)[:, :w] = img
+    dev = torch.from_numpy(host).cuda()
+    torch.cuda.synchronize()
+    out = np.empty((h, w), np.float32)
+    ofb200._lib.check(ctx.lib.ofb_min_eig_map(ctx.h, ofb200._lib.ptr(dev.data_ptr() + 1), w, h, pitch, bs, ofb200._lib.ptr(out)))
+    return out
+
+
 from tie_rule import TIE_REL, cv2_eig, explain_by_ties  # noqa: E402,F401
 
 
@@ -306,9 +321,10 @@ def test_two_kernel_variants_agree(ctx):
                             ofb200.goodFeaturesToTrack(img, 300, 0.01, 7, blockSize=bs, ctx=ctx),
                             ofb200.goodFeaturesToTrack(img, 0, 0.05, 3, mask=mask, blockSize=bs, ctx=ctx))
             fast, pts_fast, ptsm_fast = both()                      # marching kernel for blockSize 3, 7, 12
-            v1, pts_v1, ptsm_v1 = with_env("OFB_EIG_MARCH_V1", both)  # ... with its general row loop on every strip
-            assert np.array_equal(fast, v1) and np.array_equal(as_list(pts_fast), as_list(pts_v1))
-            assert np.array_equal(as_list(ptsm_fast), as_list(ptsm_v1))
+            # ... with its general row loop on every strip: unaligned rows (map), a mask that passes every pixel (list)
+            general = min_eig_map_unaligned(ofb200, ctx, img, bs)
+            pts_general = ofb200.goodFeaturesToTrack(img, 300, 0.01, 7, mask=np.full_like(img, 255), blockSize=bs, ctx=ctx)
+            assert np.array_equal(fast, general) and np.array_equal(as_list(pts_fast), as_list(pts_general))
             tile, pts_tile, ptsm_tile = with_env("OFB_EIG_TILE", both)
             gen, pts_gen, ptsm_gen = with_env("OFB_EIG_GENERIC", both)
             assert np.array_equal(fast, tile), (h, w, bs, np.abs(fast - tile).max(), np.argwhere(fast != tile)[:5])
@@ -342,19 +358,16 @@ def test_two_kernel_variants_agree(ctx):
 
 
 def test_marching_fast_rows_at_full_size(ctx):
-    """The lean row loop of the marching kernel (interior strips) against its general row loop at 1080p and at a size whose
-    band count / band height parity differs: identical maps, identical candidate-derived lists, with and without
-    a batch (bands get shorter as the batch grows)."""
+    """The lean row loops of the marching kernel against its general row loop at 1080p and at a size whose band count /
+    band height parity differs: identical maps (the general loop on unaligned rows), identical candidate-derived lists (the
+    general loop through a mask that passes every pixel), with and without a batch (bands get shorter as the batch grows)."""
     import ofb200
     for (h, w), seed, bs in [((1080, 1920), 71, 7), ((721, 1283), 72, 7), ((540, 960), 73, 3), ((487, 1001), 74, 12)]:
         img = synth.texture(h, w, seed)
-        run = lambda: (ofb200.cornerMinEigenVal(img, bs, ctx=ctx), ofb200.goodFeaturesToTrack(img, 1000, 0.01, 10, blockSize=bs, ctx=ctx))
-        fast_map, fast_pts = run()
-        os.environ["OFB_EIG_MARCH_V1"] = "1"
-        try:
-            ref_map, ref_pts = run()
-        finally:
-            os.environ["OFB_EIG_MARCH_V1"] = "0"
+        fast_map = ofb200.cornerMinEigenVal(img, bs, ctx=ctx)
+        fast_pts = ofb200.goodFeaturesToTrack(img, 1000, 0.01, 10, blockSize=bs, ctx=ctx)
+        ref_map = min_eig_map_unaligned(ofb200, ctx, img, bs)
+        ref_pts = ofb200.goodFeaturesToTrack(img, 1000, 0.01, 10, mask=np.full_like(img, 255), blockSize=bs, ctx=ctx)
         assert np.array_equal(fast_map, ref_map), (h, w, bs, np.argwhere(fast_map != ref_map)[:4])
         assert np.array_equal(as_list(fast_pts), as_list(ref_pts)), (h, w, bs)
     # batches: 1, 3 and 9 images of 720p through the fused path (feature lists per image must not depend on the batch)

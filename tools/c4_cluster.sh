@@ -11,4 +11,3 @@ done
 timeout 200 python bench.py --workload c4 --steps 50 --warmup 5 --no-cpu 2>/dev/null | python -c "
 import json,sys
 d=json.loads(sys.stdin.read().strip().split('\n')[-1]); print('default p50', d['value'], d['stage_ms_serial'], d['lifecycle_step'])"
-OFB_SELECT_TRACE=1 timeout 100 python bench.py --workload c4 --steps 3 --warmup 1 --no-cpu 2>&1 | grep "select trace" | tail -1

@@ -11,14 +11,10 @@ timeout 600 python bench.py --steps 10 --warmup 3 > gpurun_out/bench.log 2> gpur
 echo "bench exit $?" >> gpurun_out/bench.err
 tail -5 gpurun_out/pytest_gpu.log; tail -3 gpurun_out/smoke.log; tail -c 2500 gpurun_out/bench.log; tail -5 gpurun_out/bench.err
 if [ "$1" == "ncu" ]; then
-  # whole-batch launches (no twin-context chunking), 32 pairs per launch as in the bench
-  export OFB_TWIN_CHUNKS=0
+  # 32 pairs per call as in the bench (device frames: two 16-pair chunks, one on the context and one on its twin)
   PROF="python tools/profile_pairs.py --batch 32 --steps 2 --mc-trials 2000000"
   timeout 300 $PROF > gpurun_out/prof_plain.log 2>&1 &&
   timeout 900 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file gpurun_out/launches.csv $PROF > gpurun_out/ncu_list.log 2>&1
-  # launch list of the bench command itself (the same command line as the bench.log above, plus --no-cpu to keep
-  # the host-only CPU baseline out of the profiled run)
-  timeout 900 ncu --metrics gpu__time_duration.sum --clock-control none -c 20000 --csv --log-file gpurun_out/bench_launches.csv env -u OFB_TWIN_CHUNKS python bench.py --steps 10 --warmup 3 --no-cpu > gpurun_out/ncu_bench_list.log 2>&1
   timeout 1500 ncu --set full --clock-control none --import-source on -k regex:'eig_|lk_track|pyr_down|select_kernel|mc_sweep|pair_solve' -c 14 -f -o gpurun_out/prof $PROF > gpurun_out/ncu_full.log 2>&1
   timeout 900 ncu --set full --clock-control none --import-source on -k regex:'mc_sweep' -c 2 -f -o gpurun_out/prof_mc $PROF > gpurun_out/ncu_mc.log 2>&1
   # feature lifecycle: launch list and a full capture of its own kernels

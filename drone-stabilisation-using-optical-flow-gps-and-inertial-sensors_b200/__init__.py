@@ -19,7 +19,8 @@ from .velocity import (solve_lgs, solve_full, solve_lgs_batched, solve_lgs_modul
                        quaternion_to_rotation, plane_normal, body_to_world)
 from .vision import (goodFeaturesToTrack, calcOpticalFlowPyrLK, cornerMinEigenVal, buildPyramid, pyrDown, cvtColor,
                      Pyramid, make_pair_cfg, frame_pairs, frame_sequence, COLOR_BGR2GRAY, TERM_CRITERIA_COUNT, TERM_CRITERIA_EPS,
-                     undistortPoints, undistortPointsIter, make_camera, CAMERA_ITERATIONS, track_forward_backward)
+                     undistortPoints, undistortPointsIter, make_camera, CAMERA_ITERATIONS, track_forward_backward,
+                     gyro_predict)
 from .tracker import StreamTracker, FleetTracker, exclusion_mask
 from .simulation import of_simulation, feas_simulation, overlap, run_named_sweep, run_sweep, sorting_study, advect_points
 

@@ -49,6 +49,28 @@ __device__ __forceinline__ void ofb_undistort(const ofb_camera& c, double px, do
     }
 }
 
+// Normalised image coordinates -> pixel, OpenCV's forward lens model: cv2.projectPoints of the object point (x, y, 1)
+// with zero rvec / tvec, in cvProjectPoints2Internal's operation order (the zero rotation, translation and tilt terms
+// are exact identities there and are left out). The inverse of ofb_undistort where that converges.
+__device__ __forceinline__ void ofb_project(const ofb_camera& c, double x, double y, double& px, double& py)
+{
+    const int nd = c.n_dist;
+    const double k1 = nd ? c.dist[0] : 0.0, k2 = nd ? c.dist[1] : 0.0, p1 = nd ? c.dist[2] : 0.0, p2 = nd ? c.dist[3] : 0.0;
+    const double k3 = nd > 4 ? c.dist[4] : 0.0;
+    const double k4 = nd > 5 ? c.dist[5] : 0.0, k5 = nd > 5 ? c.dist[6] : 0.0, k6 = nd > 5 ? c.dist[7] : 0.0;
+    const double r2 = ofb_add(ofb_mul(x, x), ofb_mul(y, y));
+    const double r4 = ofb_mul(r2, r2), r6 = ofb_mul(r4, r2);
+    const double a1 = ofb_mul(2.0 * x, y);
+    const double a2 = ofb_add(r2, ofb_mul(2.0 * x, x)), a3 = ofb_add(r2, ofb_mul(2.0 * y, y));
+    // cdist = 1 + k1 r2 + k2 r4 + k3 r6,  icdist2 = 1 / (1 + k4 r2 + k5 r4 + k6 r6)
+    const double cdist = ofb_add(ofb_add(ofb_add(1.0, ofb_mul(k1, r2)), ofb_mul(k2, r4)), ofb_mul(k3, r6));
+    const double icdist2 = 1.0 / ofb_add(ofb_add(ofb_add(1.0, ofb_mul(k4, r2)), ofb_mul(k5, r4)), ofb_mul(k6, r6));
+    const double xd = ofb_add(ofb_add(ofb_mul(ofb_mul(x, cdist), icdist2), ofb_mul(p1, a1)), ofb_mul(p2, a2));
+    const double yd = ofb_add(ofb_add(ofb_mul(ofb_mul(y, cdist), icdist2), ofb_mul(p1, a3)), ofb_mul(p2, a1));
+    px = ofb_add(ofb_mul(xd, c.fx), c.cx);
+    py = ofb_add(ofb_mul(yd, c.fy), c.cy);
+}
+
 // Calibrated position and flow of one track: x = undistort(p_new), u = (x - undistort(p_old)) * rate.
 __device__ __forceinline__ double4 ofb_calibrate(const ofb_camera& c, float nx, float ny, float ox, float oy)
 {

@@ -15,6 +15,8 @@
 #include "pyrlk.cuh"
 #include "velocity_device.cuh"
 #include "camera.cuh"
+#include "gyro.cuh"
+#include <stddef.h>
 
 namespace {
 
@@ -80,10 +82,11 @@ pair_solve_cam_kernel(TrackLoader tl, ofb_camera cam, double4* __restrict__ xu, 
 }  // namespace
 
 // Stages 1b-4 for pairs [c0, c0+n) whose level-0 frames already sit in pp/pn (images 0..n-1 of each).
+// gyro (NULL: off): the pinhole model of the gyro prediction, with dcam the device copy of the camera (NULL: pinhole).
 // Sequence layout (pn == pp): pp holds n+1 consecutive frames of one stream, pair i = (image i, image i+1), so every
 // interior frame's pyramid is built once and serves as "next" of one pair and "prev" of the following one.
-static int run_pairs_chunk(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, double fb_max_err, ofb_pyr* pp, ofb_pyr* pn,
-                           int n, int c0,
+static int run_pairs_chunk(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, double fb_max_err,
+                           const GyroPinhole* gyro, const ofb_camera* dcam, ofb_pyr* pp, ofb_pyr* pn, int n, int c0,
                            const ofb_imu_sample* dimu, const int* counts_in, float* d_prev, float* d_next, uint8_t* d_stat,
                            ofb_pair_result* d_res, bool mark)
 {
@@ -142,9 +145,17 @@ static int run_pairs_chunk(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_came
     }
     STAGE_MARK(3);
     OFB_TRY(ctx->scratch[SC_ERR].reserve(sizeof(float) * (size_t)n * K));
+    int lk_flags = 0;
+    if (gyro) {
+        // LK starts from the rotation the gyro measured: the guesses go where LK writes its result
+        OFB_TRY(ofb_gyro_predict_device(ctx, *gyro, dcam, (const double*)((const char*)(dimu + c0) + offsetof(ofb_imu_sample, w)),
+                                        (int)(sizeof(ofb_imu_sample) / sizeof(double)), n, cp, counts, counts_stride, K,
+                                        (size_t)K, cn));
+        lk_flags = OFB_LK_USE_INITIAL_FLOW | OFB_LK_FB_INITIAL_FLOW;
+    }
     OFB_TRY(ofb_lk_device(ctx, pp, 0, 1, pn, seq ? 1 : 0, 1, n, cp, counts, counts_stride, K, (size_t)K, cfg->win_w, cfg->win_h,
-                          cfg->max_level, cfg->max_count, cfg->eps, 0, cfg->min_eig_thr, cn, cs, ctx->scratch[SC_ERR].as<float>(),
-                          fb_max_err));
+                          cfg->max_level, cfg->max_count, cfg->eps, lk_flags, cfg->min_eig_thr, cn, cs,
+                          ctx->scratch[SC_ERR].as<float>(), fb_max_err));
     STAGE_MARK(4);
     TrackLoader ld{cp, cn, cs, counts, counts_stride, (size_t)K, cfg->cx, cfg->cy, cfg->pos_scale, cfg->flow_scale};
     if (cam) {
@@ -183,9 +194,20 @@ extern "C" int ofb_frame_pairs_fb(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const o
                                   const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
                                   ofb_pair_result* results, float* prev_pts, float* next_pts, uint8_t* status)
 {
+    return ofb_frame_pairs_gyro(ctx, cfg, cam, fb_max_err, 0, n_pairs, prev, next, pitch, image_stride, imu, pts_in, n_in, results,
+                                prev_pts, next_pts, status);
+}
+
+extern "C" int ofb_frame_pairs_gyro(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, double fb_max_err,
+                                    int gyro_predict, int n_pairs, const uint8_t* prev, const uint8_t* next, int pitch,
+                                    size_t image_stride, const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
+                                    ofb_pair_result* results, float* prev_pts, float* next_pts, uint8_t* status)
+{
     OFB_REQUIRE(ctx && cfg && prev && next && imu && results, "frame_pairs: null argument");
     if (cam) OFB_TRY(ofb_camera_check(cam, "frame_pairs"));
     OFB_REQUIRE(ofb_fb_thr_ok(fb_max_err), "frame_pairs: fb_max_err must be >= 0 (0 = no forward-backward check)");
+    GyroPinhole gph{0.0, 0.0, 0.0, 0.0};
+    if (gyro_predict && !cam) OFB_TRY(ofb_gyro_pinhole(cfg, "frame_pairs", &gph));
     OFB_REQUIRE(n_pairs > 0 && n_pairs <= 65535, "frame_pairs: n_pairs must be in 1..65535");
     const int w = cfg->width, h = cfg->height, K = cfg->max_corners;
     OFB_REQUIRE(w > 0 && h > 0 && pitch >= w, "frame_pairs: bad image geometry");
@@ -208,6 +230,8 @@ extern "C" int ofb_frame_pairs_fb(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const o
     if (!d_stat) { OFB_TRY(ctx->scratch[SC_STAT].reserve(npts)); d_stat = ctx->scratch[SC_STAT].as<uint8_t>(); }
     const void* dimu;
     OFB_TRY(ofb_stage_in(ctx, SC_IN3, imu, sizeof(ofb_imu_sample) * n_pairs, &dimu));
+    const void* dcam = nullptr;                     // the prediction kernel reads the camera from device memory
+    if (gyro_predict && cam) OFB_TRY(ofb_stage_in(ctx, SC_IN5, cam, sizeof(ofb_camera), &dcam));
     const int* counts_in = nullptr;
     if (!cfg->detect) {
         const void* dn;
@@ -305,7 +329,8 @@ extern "C" int ofb_frame_pairs_fb(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const o
         if (!seq)
             OFB_TRY(ofb_pyr_prepare(c, &c->pair_pyr[slot][1], fnext + (size_t)c0 * fstride, w, h, fpitch, fstride, n, cap,
                                     cfg->max_level, false));
-        OFB_TRY(run_pairs_chunk(c, cfg, cam, fb_max_err, c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
+        OFB_TRY(run_pairs_chunk(c, cfg, cam, fb_max_err, gyro_predict ? &gph : nullptr, (const ofb_camera*)dcam,
+                                c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
                                 (const ofb_imu_sample*)dimu, counts_in, d_prev, d_next, d_stat, (ofb_pair_result*)o[3].dev,
                                 ctx->profile));
     }

@@ -110,7 +110,7 @@ lk_track_kernel(LKParams P, const float* __restrict__ prev_pts, float* __restric
             float sc = 1.f / (float)(1 << level);
             float ppx = ptx * sc, ppy = pty * sc;
             if (level == P.nlev - 1) {
-                if (!bwd && (P.flags & OFB_LK_USE_INITIAL_FLOW)) { nx = nx * sc; ny = ny * sc; }
+                if (bwd ? (P.flags & OFB_LK_FB_INITIAL_FLOW) : (P.flags & OFB_LK_USE_INITIAL_FLOW)) { nx = nx * sc; ny = ny * sc; }
                 else { nx = ppx; ny = ppy; }
             } else { nx = nx * 2.f; ny = ny * 2.f; }
             float px = ppx - hwx, py = ppy - hwy;
@@ -226,7 +226,11 @@ lk_track_kernel(LKParams P, const float* __restrict__ prev_pts, float* __restric
         }
         if (FB && pass == 0) {
             // the forward result is stored now and the starting point re-read at the end, so that neither stays in
-            // registers across the backward pass
+            // registers across the backward pass; likewise the initial flow g is re-read here, before the store
+            // overwrites it, rather than kept from the forward pass's load
+            float gx = 0.f, gy = 0.f;
+            const bool seed = (P.flags & OFB_LK_FB_INITIAL_FLOW) != 0;
+            if (seed) { gx = next_pts[2 * po]; gy = next_pts[2 * po + 1]; __syncwarp(); }
             if (lane == 0) {
                 OFB_DEV_ASSERT(feat >= 0 && feat < n && (gridDim.y == 1 || po < (size_t)(pair + 1) * pts_stride));
                 next_pts[2 * po] = nx; next_pts[2 * po + 1] = ny;
@@ -234,7 +238,9 @@ lk_track_kernel(LKParams P, const float* __restrict__ prev_pts, float* __restric
                 if (!st) { status[po] = 0; if (fb_err) fb_err[po] = INFINITY; }
             }
             if (!st) return;
+            const float p0x = ptx, p0y = pty;
             ptx = nx; pty = ny;
+            if (seed) { nx = nx + (p0x - gx); ny = ny + (p0y - gy); }     // backward initial flow p1 + (p0 - g)
         }
     }
     if (FB) {
@@ -377,7 +383,7 @@ lk_track_fast2_kernel(const __grid_constant__ LKParams P, const float* __restric
     const int pimg = P.prev_image0 + pair * P.prev_image_step, nimg = P.next_image0 + pair * P.next_image_step;
 
     // FB: pass 1 tracks back from the forward result (I and J swap roles; the level geometry is shared, both pyramids
-    // have one size), with no initial flow
+    // have one size), with no initial flow unless OFB_LK_FB_INITIAL_FLOW
 #pragma unroll
     for (int pass = 0; pass < (FB ? 2 : 1); ++pass) {
         const bool bwd = FB && pass == 1;
@@ -391,7 +397,7 @@ lk_track_fast2_kernel(const __grid_constant__ LKParams P, const float* __restric
             const float sc = __int_as_float((127 - level) << 23);        // 2^-level
             const float ppx = ptx * sc, ppy = pty * sc;
             if (level == P.nlev - 1) {
-                if (!bwd && (P.flags & OFB_LK_USE_INITIAL_FLOW)) { nx = nx * sc; ny = ny * sc; }
+                if (bwd ? (P.flags & OFB_LK_FB_INITIAL_FLOW) : (P.flags & OFB_LK_USE_INITIAL_FLOW)) { nx = nx * sc; ny = ny * sc; }
                 else { nx = ppx; ny = ppy; }
             } else { nx = nx * 2.f; ny = ny * 2.f; }
             const float px = ppx - hwx, py = ppy - hwy;
@@ -560,7 +566,11 @@ lk_track_fast2_kernel(const __grid_constant__ LKParams P, const float* __restric
         }
         if (FB && pass == 0) {
             // the forward result is stored now and the starting point re-read at the end, so that neither stays in
-            // registers across the backward pass
+            // registers across the backward pass; likewise the initial flow g is re-read here, before the store
+            // overwrites it, rather than kept from the forward pass's load
+            float gx = 0.f, gy = 0.f;
+            const bool seed = (P.flags & OFB_LK_FB_INITIAL_FLOW) != 0;
+            if (seed) { gx = next_pts[2 * po]; gy = next_pts[2 * po + 1]; __syncwarp(); }
             if (lane == 0) {
                 OFB_DEV_ASSERT(feat >= 0 && feat < n && (gridDim.y == 1 || po < (size_t)(pair + 1) * pts_stride));
                 next_pts[2 * po] = nx; next_pts[2 * po + 1] = ny;
@@ -568,7 +578,9 @@ lk_track_fast2_kernel(const __grid_constant__ LKParams P, const float* __restric
                 if (!st) { status[po] = 0; if (fb_err) fb_err[po] = INFINITY; }
             }
             if (!st) return;
+            const float p0x = ptx, p0y = pty;
             ptx = nx; pty = ny;
+            if (seed) { nx = nx + (p0x - gx); ny = ny + (p0y - gy); }     // backward initial flow p1 + (p0 - g)
         }
     }
     if (FB) {

@@ -20,6 +20,11 @@ struct LKParams {
     int prev_image0, prev_image_step, next_image0, next_image_step;   // image of pair p = image0 + p*step
 };
 
+// Internal LK flag (with OFB_LK_USE_INITIAL_FLOW and the forward-backward check): the backward pass starts from the
+// forward result displaced by the forward pass's initial flow reversed, p1 + (p0 - g), instead of p1. A guess that
+// carried the forward pass across a large motion is thereby given to the backward pass too.
+#define OFB_LK_FB_INITIAL_FLOW 256
+
 // Device-pointer core. counts (optional): per-pair feature count at counts[pair*counts_stride];
 // n_uniform = upper bound of the per-pair count (grid size).
 // fb_thr > 0: forward-backward check (ofb_pyrlk_fb) folded into status; fb_err (optional) gets the distance where both

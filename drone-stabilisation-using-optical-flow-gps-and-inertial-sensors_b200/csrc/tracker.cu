@@ -20,6 +20,8 @@
 #include "pyrlk.cuh"
 #include "velocity_device.cuh"
 #include "camera.cuh"
+#include "gyro.cuh"
+#include <stddef.h>
 
 struct ofb_tracker {
     ofb_ctx* ctx = nullptr;
@@ -65,6 +67,9 @@ struct ofb_tracker {
     // forward-backward check of the LK tracks (ofb_tracker_set_fb_check), 0 = off: a kernel argument, so captured graphs
     // hold the value they were captured with
     double fb_max_err = 0.0;
+    // gyro-predicted initial flow of the LK tracks (ofb_tracker_set_gyro_prediction): whether the prediction kernel is
+    // launched is decided when a step is enqueued, so a change drops the captured graphs
+    bool gyro = false;
     uint64_t graph_steps = 0;
 };
 
@@ -601,11 +606,22 @@ static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitc
     T.min_solve = cfg.min_solve; T.min_features = cfg.min_features; T.topup_mode = cfg.topup_mode; T.max_features = K;
     T.have_prev = t->have_prev ? 1 : 0;
     OFB_TRY(ofb_features_scratch(ctx, w, h, pc.min_distance, S, &T.feat_state, &T.cell_grid, &T.cell_stride));
-    // 2. track the stream's points from the kept frame into the new one
-    if (t->have_prev)
+    // 2. track the stream's points from the kept frame into the new one (with the gyro prediction: starting from where
+    //    this step's rotation moves them, predicted on the context's stream from this step's staged IMU samples)
+    if (t->have_prev) {
+        int lk_flags = 0;
+        if (t->gyro) {
+            GyroPinhole gph{0.0, 0.0, 0.0, 0.0};
+            if (!t->has_cam) OFB_TRY(ofb_gyro_pinhole(&pc, "tracker_step", &gph));
+            OFB_TRY(ofb_gyro_predict_device(ctx, gph, T.cam, (const double*)((const char*)dimu + offsetof(ofb_imu_sample, w)),
+                                            (int)(sizeof(ofb_imu_sample) / sizeof(double)), S, P, count, 1, cap, (size_t)cap,
+                                            t->nxt.as<float>()));
+            lk_flags = OFB_LK_USE_INITIAL_FLOW | OFB_LK_FB_INITIAL_FLOW;
+        }
         OFB_TRY(ofb_lk_device(ctx, t->pyr[t->cur ^ 1], 0, 1, t->pyr[t->cur], 0, 1, S, P, count, 1, cap, (size_t)cap, pc.win_w,
-                              pc.win_h, pc.max_level, pc.max_count, pc.eps, 0, pc.min_eig_thr, t->nxt.as<float>(),
+                              pc.win_h, pc.max_level, pc.max_count, pc.eps, lk_flags, pc.min_eig_thr, t->nxt.as<float>(),
                               t->status.as<uint8_t>(), t->err.as<float>(), t->fb_max_err));
+    }
     t->lk_recorded = false;
     if (early && t->have_prev) { OFB_CUDA(cudaEventRecord(t->ev_lk, ctx->stream)); t->lk_recorded = true; }
     // 3.+4. status filter, gates, solve; the compacted new positions become the point set (Pn)
@@ -771,6 +787,10 @@ extern "C" int ofb_tracker_step(ofb_tracker* t, const uint8_t* frames, int pitch
     const int S = t->cfg.n_streams, w = t->cfg.pair.width, h = t->cfg.pair.height, bpp = t->cfg.bgr_input ? 3 : 1;
     OFB_REQUIRE(pitch >= bpp * w, "tracker_step: pitch smaller than a row");
     OFB_REQUIRE(S == 1 || image_stride >= (size_t)pitch * (h - 1) + (size_t)bpp * w, "tracker_step: image_stride too small");
+    if (t->gyro && !t->has_cam) {
+        GyroPinhole gph;
+        OFB_TRY(ofb_gyro_pinhole(&t->cfg.pair, "tracker_step", &gph));
+    }
     OFB_CUDA(cudaSetDevice(ctx->device));
     // launch-bound case (a few small frames from host memory, only the result records wanted): replay a graph
     const char* genv = getenv("OFB_TRACKER_GRAPH");
@@ -824,6 +844,24 @@ extern "C" int ofb_tracker_set_fb_check(ofb_tracker* t, double fb_max_err)
             for (int j = 0; j < 2; ++j)
                 if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
         t->fb_max_err = fb_max_err;
+    }
+    return OFB_OK;
+}
+
+extern "C" int ofb_tracker_set_gyro_prediction(ofb_tracker* t, int enable)
+{
+    OFB_REQUIRE(t, "tracker_set_gyro_prediction: null tracker");
+    if (enable && !t->has_cam) {
+        GyroPinhole gph;
+        OFB_TRY(ofb_gyro_pinhole(&t->cfg.pair, "tracker_set_gyro_prediction", &gph));
+    }
+    if ((enable != 0) != t->gyro) {
+        // the prediction is a launch of the step and the LK flags are a launch argument: graphs captured before are
+        // rebuilt (no graph is in flight: a replayed step synchronises before it returns)
+        for (int i = 0; i < 2; ++i)
+            for (int j = 0; j < 2; ++j)
+                if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
+        t->gyro = enable != 0;
     }
     return OFB_OK;
 }

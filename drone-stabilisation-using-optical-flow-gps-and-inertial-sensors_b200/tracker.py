@@ -13,7 +13,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from .vision import _fb_threshold, as_camera, make_pair_cfg
+from .vision import _fb_threshold, _gyro_flag, as_camera, make_pair_cfg
 
 
 class StreamTracker:
@@ -32,13 +32,16 @@ class StreamTracker:
     borrow_frames: device-resident grey frames (CUDA tensors) are tracked in place instead of being copied into the
     tracker; pass a NEW tensor every step (the tracker keeps the previous one alive; do not overwrite it).
     camera: (K, D, rate[, iterations]) or vision.make_camera(...) -- see set_camera.
-    fb_threshold: None / 0 = off, T > 0 = forward-backward check of the LK tracks -- see set_fb_threshold."""
+    fb_threshold: None / 0 = off, T > 0 = forward-backward check of the LK tracks -- see set_fb_threshold.
+    gyro_prediction: LK starts from the rotation the step's gyro sample measured -- see set_gyro_prediction."""
 
     def __init__(self, width, height, max_features=100, min_features=20, n_streams=1, feature_params=None,
                  lk_params=None, topup="exp", mask_radius=30, bgr=False, variant="exp", principal=None,
                  scaling=1.0, flow_scaling=None, max_speed=0.0, dummy_value=float("nan"), gate=None, min_solve=3,
-                 min_eig_thr=1e-4, borrow_frames=False, v_init=None, camera=None, fb_threshold=None, ctx=None):
+                 min_eig_thr=1e-4, borrow_frames=False, v_init=None, camera=None, fb_threshold=None,
+                 gyro_prediction=False, ctx=None):
         fb = _fb_threshold(fb_threshold)
+        gyro = _gyro_flag(gyro_prediction)
         fp = dict(qualityLevel=0.01, minDistance=10, blockSize=7)
         fp.update(feature_params or {})
         lk = dict(winSize=(15, 15), maxLevel=3, criteria=(3, 20, 0.03))
@@ -74,10 +77,13 @@ class StreamTracker:
         cap = C.c_int()
         _lib.check(self.ctx.lib.ofb_tracker_capacity(self.h, C.byref(cap)))
         self.capacity = cap.value
+        self._has_cam = False
         if camera is not None:
             self.set_camera(camera)
         if fb:
             _lib.check(self.ctx.lib.ofb_tracker_set_fb_check(self.h, fb))
+        if gyro:
+            self.set_gyro_prediction(True)
 
     def close(self):
         if getattr(self, "h", None) and getattr(self.ctx, "h", None):
@@ -109,12 +115,24 @@ class StreamTracker:
         vision.CAMERA_ITERATIONS) instead of the pinhole principal / scaling / flow_scaling. None detaches it."""
         cam = as_camera(camera)
         _lib.check(self.ctx.lib.ofb_tracker_set_camera(self.h, C.byref(cam) if cam is not None else None))
+        self._has_cam = cam is not None
 
     def set_fb_threshold(self, threshold):
         """Forward-backward check of every stream's LK tracks from the next step on (vision.track_forward_backward): a
         point that does not return within `threshold` px of where it started counts as lost (status 0). None or 0
         turns it off."""
         _lib.check(self.ctx.lib.ofb_tracker_set_fb_check(self.h, _fb_threshold(threshold)))
+
+    def set_gyro_prediction(self, enable):
+        """Gyro prediction of every stream's LK tracks from the next step on (vision.gyro_predict): LK starts each point
+        from where the step's gyro rate imu["w"] rotates it over one frame, with the camera when one is set and the
+        pinhole principal / scaling / flow_scaling otherwise (dt = scaling / flow_scaling). False turns it off."""
+        on = _gyro_flag(enable)
+        p = self.cfg.pair
+        if on and not self._has_cam and (p.flow_scale == 0 or p.pos_scale == 0 or not np.isfinite(p.pos_scale / p.flow_scale)):
+            raise ValueError("gyro prediction with the pinhole needs flow_scaling != 0 and a finite, non-zero "
+                             "scaling / flow_scaling")
+        _lib.check(self.ctx.lib.ofb_tracker_set_gyro_prediction(self.h, on))
 
     def set_points(self, points):
         """points: one (N,2)/(N,1,2) array per stream (or a single array when n_streams == 1)."""
@@ -232,6 +250,13 @@ class FleetTracker:
         t = _fb_threshold(threshold)
         if self.local is not None:
             self.local.set_fb_threshold(t)
+
+    def set_gyro_prediction(self, enable):
+        """StreamTracker.set_gyro_prediction on this rank's streams (gyro_prediction=True at construction is passed to
+        the local tracker with the other keywords)"""
+        on = bool(_gyro_flag(enable))
+        if self.local is not None:
+            self.local.set_gyro_prediction(on)
 
     def gather_velocities(self):
         """(n_streams, 3) velocities of the last step on every rank; rows of streams that did not solve (or have not

@@ -323,6 +323,49 @@ def undistortPoints(src, cameraMatrix, distCoeffs, R=None, P=None, ctx=None):
     return undistortPointsIter(src, cameraMatrix, distCoeffs, R, P, (TERM_CRITERIA_COUNT, 5, 0), ctx=ctx)
 
 
+def gyro_predict(points, omega, camera=None, cfg=None, ctx=None, **pinhole):
+    """Where each pixel point lands when the camera rotates by the gyro rate `omega` (3 floats, rad per unit of time)
+    over one frame interval: the initial flow the velocity paths give LK with gyro_prediction=True (include/ofb200.h,
+    ofb_gyro_predict). points (N,2) / (N,1,2) -> (N,1,2) float32.
+    camera: (K, D, rate[, iterations]) or make_camera(...): the lens model, dt = 1 / rate. Otherwise the pinhole of
+    `cfg` (make_pair_cfg) or of make_pair_cfg's keywords in **pinhole (width, height, principal, pos_scale, flow_scale),
+    with dt = pos_scale / flow_scale."""
+    cam = as_camera(camera)
+    w = np.asarray(omega, dtype=np.float64).ravel()
+    if w.shape != (3,):
+        raise ValueError("omega must have 3 entries")
+    if cam is None:
+        if cfg is None:
+            pin = dict(pinhole)
+            width, height = pin.pop("width", 0), pin.pop("height", 0)
+            if pin.get("principal") is None and not (width and height):
+                raise ValueError("the pinhole needs cfg, or principal=, or width= and height=")
+            cfg = make_pair_cfg(width, height, 1, **pin)
+        elif pinhole:
+            raise ValueError("pass either cfg or pinhole keywords, not both")
+        if cfg.flow_scale == 0 or not np.isfinite(cfg.pos_scale / cfg.flow_scale) or cfg.pos_scale == 0:
+            raise ValueError("the pinhole needs flow_scale != 0 and a finite, non-zero pos_scale / flow_scale")
+    elif cfg is not None or pinhole:
+        raise ValueError("pass either camera or a pinhole, not both")
+    a = np.asarray(points)
+    if a.ndim not in (2, 3) or a.shape[-1] != 2 or (a.ndim == 3 and a.shape[1] != 1):
+        raise ValueError("points must be an (N,2) or (N,1,2) array")
+    pts = np.ascontiguousarray(a.reshape(-1, 2), dtype=np.float32)
+    out = np.empty_like(pts)
+    if len(pts):
+        ctx = ctx or _lib.default_context()
+        _lib.check(ctx.lib.ofb_gyro_predict(ctx.h, C.byref(cfg) if cfg is not None else None,
+                                            C.byref(cam) if cam is not None else None, _lib.ptr(pts), len(pts),
+                                            _lib.ptr(np.ascontiguousarray(w)), _lib.ptr(out)))
+    return out.reshape(-1, 1, 2)
+
+
+def _gyro_flag(gyro_prediction):
+    if not isinstance(gyro_prediction, (bool, np.bool_)):
+        raise ValueError("gyro_prediction must be True or False, got %r" % (gyro_prediction,))
+    return 1 if gyro_prediction else 0
+
+
 def make_pair_cfg(width, height, max_corners, quality=0.01, min_distance=10.0, block_size=7, win=(15, 15),
                   max_level=3, criteria=(3, 20, 0.03), min_eig_thr=1e-4, variant="node", principal=None,
                   pos_scale=1.0, flow_scale=1.0, detect=True):
@@ -342,7 +385,7 @@ def make_pair_cfg(width, height, max_corners, quality=0.01, min_distance=10.0, b
 
 
 def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, ctx=None, on_overflow="raise", camera=None,
-                fb_threshold=None):
+                fb_threshold=None, gyro_prediction=False):
     """Batched detect(+)track+solve. prev/nxt: (N,H,W) uint8 numpy arrays (host) or CUDA tensors;
     imu: structured array _lib.IMU_DTYPE (N,). Returns a structured array _lib.RESULT_DTYPE (N,)
     (and prev_pts, next_pts, status when want_tracks).
@@ -354,9 +397,16 @@ def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, 
     iterations default to CAMERA_ITERATIONS.
     fb_threshold: None / 0 = off; T > 0 = forward-backward check of every track (track_forward_backward): a track that
     does not return within T px counts as lost (status 0, not in n_tracked, not in the solve). It runs on pixel
-    positions, before the camera model."""
+    positions, before the camera model.
+    gyro_prediction: LK starts each track from where the pair's gyro rate imu["w"] rotates it (gyro_predict, with
+    `camera` or cfg's pinhole) instead of from the point itself; with fb_threshold the backward pass starts from
+    p1 + (p0 - guess)."""
     thr = _fb_threshold(fb_threshold)
+    gyro = _gyro_flag(gyro_prediction)
     cam = as_camera(camera)
+    if gyro and cam is None and (cfg.flow_scale == 0 or cfg.pos_scale == 0 or not np.isfinite(cfg.pos_scale / cfg.flow_scale)):
+        raise ValueError("gyro_prediction with the pinhole needs flow_scale != 0 and a finite, non-zero "
+                         "pos_scale / flow_scale")
     ctx = ctx or _lib.default_context()
     n = int(prev.shape[0])
     h, w = int(prev.shape[1]), int(prev.shape[2])
@@ -378,9 +428,9 @@ def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, 
     if pts_in is not None:
         pts_in = np.ascontiguousarray(pts_in, dtype=np.float32)
         n_in = np.ascontiguousarray(n_in, dtype=np.int32)
-    _lib.check(ctx.lib.ofb_frame_pairs_fb(ctx.h, C.byref(cfg), C.byref(cam) if cam is not None else None, thr, n,
-                                          _lib.ptr(prev), _lib.ptr(nxt), w, w * h, _lib.ptr(imu), _lib.ptr(pts_in), _lib.ptr(n_in),
-                                          _lib.ptr(res), _lib.ptr(pp), _lib.ptr(pn), _lib.ptr(st)))
+    _lib.check(ctx.lib.ofb_frame_pairs_gyro(ctx.h, C.byref(cfg), C.byref(cam) if cam is not None else None, thr, gyro, n,
+                                            _lib.ptr(prev), _lib.ptr(nxt), w, w * h, _lib.ptr(imu), _lib.ptr(pts_in),
+                                            _lib.ptr(n_in), _lib.ptr(res), _lib.ptr(pp), _lib.ptr(pn), _lib.ptr(st)))
     if on_overflow == "raise" and (res["flags"] & _lib.PAIR_OVERFLOW).any():
         bad = np.nonzero(res["flags"] & _lib.PAIR_OVERFLOW)[0]
         raise _lib.OfbError("frame_pairs: detector candidate buffer overflowed for pair(s) %s: the image has more than "
@@ -390,7 +440,8 @@ def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, 
     return res
 
 
-def frame_sequence(frames, imu, cfg, want_tracks=False, ctx=None, on_overflow="raise", camera=None, fb_threshold=None):
+def frame_sequence(frames, imu, cfg, want_tracks=False, ctx=None, on_overflow="raise", camera=None, fb_threshold=None,
+                   gyro_prediction=False):
     """One camera stream: frames (N+1,H,W) uint8 -> N consecutive pairs (frame i, frame i+1), as
     velocity_measurment_node:224-267 sees them (it keeps the previous callback's image). Passing the two views
     of ONE buffer lets the library upload every frame and build its pyramid once (`next == prev + image_stride`
@@ -398,5 +449,5 @@ def frame_sequence(frames, imu, cfg, want_tracks=False, ctx=None, on_overflow="r
     if isinstance(frames, np.ndarray):
         frames = np.ascontiguousarray(frames, dtype=np.uint8)
     return frame_pairs(frames[:-1], frames[1:], imu, cfg, want_tracks=want_tracks, ctx=ctx, on_overflow=on_overflow,
-                       camera=camera, fb_threshold=fb_threshold)
+                       camera=camera, fb_threshold=fb_threshold, gyro_prediction=gyro_prediction)
 

@@ -266,6 +266,29 @@ int ofb_frame_pairs_fb(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* 
                        const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
                        ofb_pair_result* results, float* prev_pts, float* next_pts, uint8_t* status);
 
+/* ---- gyro prediction: LK starts every point from where the rotation the gyro measured moves it, instead of from the
+ *      point itself. Rotational image motion does not depend on depth and is the large part of a drone's image motion
+ *      between two frames (a few rad/s at 30 fps move the whole image by tens to hundreds of pixels): beyond what the
+ *      pyramid captures from zero, LK loses points or converges to a wrong place with status 1. Rotation only, no
+ *      translation term. Per point, in fp64:
+ *        x = (p - c) * pos_scale, dt = pos_scale / flow_scale        (pinhole of ofb_pair_cfg), or
+ *        x = undistort(p) as the solve does, dt = 1 / cam->rate      (calibrated camera);
+ *        X' = exp([w dt]x) (x, y, 1), x' = X'_xy / X'_z               (to first order X' - X = dt (w x X): the sign
+ *                                                                     convention of the solve's gyro term);
+ *        guess = c + x' / pos_scale, or cv2.projectPoints of (x', y', 1) with zero rvec / tvec (calibrated camera);
+ *      guess = p when w = 0, X'_z <= 0 or any value is not finite (e.g. a NaN gyro sample). With the forward-backward check
+ *      the backward pass starts from p1 + (p0 - guess). */
+/* The predictor alone: guess_out[i] for pts[i] (n x 2 float32, host or device) under the gyro rate w3 (3 doubles,
+ * host or device). cam == NULL uses cfg's pinhole (then flow_scale must be non-zero and pos_scale / flow_scale finite). */
+int ofb_gyro_predict(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, const float* pts, int n,
+                     const double w3[3], float* guess_out);
+/* ofb_frame_pairs_fb with gyro_predict != 0: pair i's LK starts from the prediction under imu[i].w. gyro_predict == 0
+ * is exactly ofb_frame_pairs_fb. */
+int ofb_frame_pairs_gyro(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, double fb_max_err, int gyro_predict,
+                         int n_pairs, const uint8_t* prev, const uint8_t* next, int pitch, size_t image_stride,
+                         const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
+                         ofb_pair_result* results, float* prev_pts, float* next_pts, uint8_t* status);
+
 /* ---- feature lifecycle around the tracker (SURVEY 8f-2): the point set of every camera stream stays on the
  *      device between frames. One step does what the reference's per-frame loops do around the tracker
  *      (flight_experiments/evaluate_exp.py:97-120, velocity_measurment_node:129-172 and 224-260,
@@ -370,6 +393,10 @@ int ofb_tracker_set_camera(ofb_tracker* trk, const ofb_camera* cam);
  * off (the default). A point that fails it counts as lost (status 0): it leaves the set before the gates, the solve
  * and the top-up. A change of the value rebuilds the captured CUDA graphs. */
 int ofb_tracker_set_fb_check(ofb_tracker* trk, double fb_max_err);
+/* Gyro prediction (see ofb_gyro_predict) of every stream's LK tracks from the next ofb_tracker_step on, from the step's
+ * IMU sample w, with the tracker's camera when one is set and the pinhole of its configuration otherwise; 0 turns it off
+ * (the default). A change rebuilds the captured CUDA graphs. */
+int ofb_tracker_set_gyro_prediction(ofb_tracker* trk, int enable);
 /* the exclusion mask OFB_TOPUP_APPEND_MASKED would use for `n` points (n x 2 float32): mask_out h x w u8
  * (1 = allowed, 0 = inside a circle). Exposed for parity tests against cv2.circle. */
 int ofb_tracker_render_mask(ofb_ctx* ctx, const float* pts, int n, int radius, int w, int h, uint8_t* mask_out);

@@ -61,6 +61,11 @@ class TrackResult(C.Structure):
                 ("n_added", C.c_int), ("n_points", C.c_int)]
 
 
+class EgoResult(C.Structure):
+    _fields_ = [("v", C.c_double * 3), ("w", C.c_double * 3), ("s", C.c_double * 6), ("res", C.c_double),
+                ("rank", C.c_int), ("flags", C.c_int)]
+
+
 class McStep(C.Structure):
     _fields_ = [("v", C.c_double * 3), ("w", C.c_double * 3), ("n", C.c_double * 3), ("t", C.c_double * 3),
                 ("height", C.c_double),
@@ -80,6 +85,9 @@ RESULT_DTYPE = np.dtype([("v", "<f8", 3), ("s", "<f8", 3), ("res", "<f8"), ("ran
 TRACK_RESULT_DTYPE = np.dtype([("v", "<f8", 3), ("s", "<f8", 3), ("res", "<f8"), ("rank", "<i4"), ("flags", "<i4"),
                                ("n_prev", "<i4"), ("n_tracked", "<i4"), ("n_kept", "<i4"), ("n_added", "<i4"),
                                ("n_points", "<i4")], align=True)
+EGO_RESULT_DTYPE = np.dtype([("v", "<f8", 3), ("w", "<f8", 3), ("s", "<f8", 6), ("res", "<f8"), ("rank", "<i4"),
+                             ("flags", "<i4")], align=True)
+EGO_SOLVED = 1
 TOPUP_APPEND_MASKED, TOPUP_APPEND, TOPUP_REPLACE = 0, 1, 2
 TOPUP_MODES = {"node": TOPUP_APPEND_MASKED, "exp": TOPUP_APPEND, "module": TOPUP_REPLACE}
 GATE_NONE, GATE_R_GE, GATE_R_LE = 0, 1, 2
@@ -146,6 +154,12 @@ _SIGNATURES = {
     "ofb_frame_pairs_gyro": (i32, [vp, C.POINTER(PairCfg), C.POINTER(Camera), f64, i32, i32, vp, vp, i32, sz, vp, vp, vp, vp, vp, vp,
                                    vp]),
     "ofb_tracker_set_gyro_prediction": (i32, [vp, i32]),
+    "ofb_solve_ego_motion": (i32, [vp, i32, vp, vp, i32, f64, vp, vp, vp]),
+    "ofb_solve_ego_motion_batched": (i32, [vp, i32, vp, vp, vp, i32, vp, vp, vp, vp]),
+    "ofb_frame_pairs_ego": (i32, [vp, C.POINTER(PairCfg), C.POINTER(Camera), f64, i32, i32, vp, vp, i32, sz, vp, vp, vp, vp, vp, vp,
+                                  vp, vp]),
+    "ofb_tracker_set_ego_motion": (i32, [vp, i32]),
+    "ofb_tracker_step_ego": (i32, [vp, vp, i32, sz, vp, vp, vp, vp, vp, vp, vp, vp]),
     "ofb_mc_sweep": (i32, [vp, vp, i32, i32, vp, vp, i32, u64, u64, u64, i32, vp, vp, vp]),
     "ofb_mc_sweep_multi": (i32, [vp, i32, vp, i32, i32, vp, vp, i32, u64, u64, u64, i32, vp]),
     "ofb_mc_feas": (i32, [vp, vp, i32, vp, vp, u64, u64, u64, vp]),

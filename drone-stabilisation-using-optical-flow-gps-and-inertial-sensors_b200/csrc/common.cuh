@@ -140,7 +140,8 @@ enum {
     SC_CAND, SC_CANDCNT, SC_SEL, SC_GRID, SC_PTS0, SC_PTS1, SC_STAT, SC_ERR,
     SC_MC0, SC_MC1, SC_MC2, SC_TMP0, SC_TMP1,
     SC_FRAMES,                                               // device staging of host frames (ofb_frame_pairs)
-    SC_CALIB                                                 // calibrated tracks of ofb_frame_pairs_cam
+    SC_CALIB,                                                // calibrated tracks of ofb_frame_pairs_cam
+    SC_EGO                                                   // staged ego-motion records (frame pairs, tracker)
 };
 
 struct ofb_pyr {

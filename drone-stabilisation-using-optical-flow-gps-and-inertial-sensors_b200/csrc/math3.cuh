@@ -119,6 +119,61 @@ OFB_HD void ofb_jacobi3(const double M[6], double ev[3], double q[3][3])
     }
 }
 
+// Cyclic Jacobi eigen-decomposition of an N x N symmetric matrix a (overwritten: its diagonal holds the eigenvalues on
+// return, unsorted), eigenvectors in the columns of v (v[row][col]). Same rotation and stopping rule as ofb_jacobi3.
+// Every index is a compile-time constant once the loops are unrolled, so both matrices stay in registers.
+template <int N>
+OFB_HD void ofb_jacobi_n(double (&a)[N][N], double (&v)[N][N])
+{
+#pragma unroll
+    for (int i = 0; i < N; ++i)
+#pragma unroll
+        for (int j = 0; j < N; ++j) v[i][j] = i == j ? 1.0 : 0.0;
+    for (int sweep = 0; sweep < 16; ++sweep) {
+        double off = 0.0, diag = 0.0;
+#pragma unroll
+        for (int p = 0; p < N; ++p) {
+            diag += fabs(a[p][p]);
+#pragma unroll
+            for (int r = p + 1; r < N; ++r) off += fabs(a[p][r]);
+        }
+        if (off <= 1e-300 || off <= 1e-18 * diag) break;
+#pragma unroll
+        for (int p = 0; p < N - 1; ++p)
+#pragma unroll
+            for (int r = p + 1; r < N; ++r) {
+                const double apq = a[p][r];
+                if (apq == 0.0) continue;
+                const double d = a[r][r] - a[p][p], two = 2.0 * apq;
+                const double sg = (d == 0.0 || ((d > 0.0) == (apq > 0.0))) ? 1.0 : -1.0;
+                const double t = sg * fabs(two) / (fabs(d) + sqrt(d * d + two * two));
+#ifdef __CUDA_ARCH__
+                const double c = rsqrt(t * t + 1.0), s = t * c;
+#else
+                const double c = 1.0 / sqrt(t * t + 1.0), s = t * c;
+#endif
+#pragma unroll
+                for (int k = 0; k < N; ++k) {
+                    const double akp = a[k][p], akq = a[k][r];
+                    a[k][p] = c * akp - s * akq;
+                    a[k][r] = s * akp + c * akq;
+                }
+#pragma unroll
+                for (int k = 0; k < N; ++k) {
+                    const double apk = a[p][k], aqk = a[r][k];
+                    a[p][k] = c * apk - s * aqk;
+                    a[r][k] = s * apk + c * aqk;
+                }
+#pragma unroll
+                for (int k = 0; k < N; ++k) {
+                    const double vkp = v[k][p], vkq = v[k][r];
+                    v[k][p] = c * vkp - s * vkq;
+                    v[k][r] = s * vkp + c * vkq;
+                }
+            }
+    }
+}
+
 // Solve M v = g for SPD M by the adjugate (cofactors); returns det.
 OFB_HD double ofb_solve_sym3(const double M[6], const double g[3], double v[3])
 {

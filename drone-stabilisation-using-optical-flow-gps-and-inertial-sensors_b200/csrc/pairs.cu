@@ -38,9 +38,11 @@ struct TrackLoader {
     __device__ bool dist(int, int, double&) const { return false; }
 };
 
-template <class Loader>
+// EGO: the ego-motion solve of the pair follows on the same points (ego[f]); EGO = false is the velocity solve alone
+template <bool EGO, class Loader>
 __device__ __forceinline__ void pair_solve(const Loader& ld, int variant, const ofb_imu_sample* __restrict__ imu,
-                                           ofb_pair_result* __restrict__ out, const FeatImageState* __restrict__ det)
+                                           ofb_pair_result* __restrict__ out, const FeatImageState* __restrict__ det,
+                                           ofb_ego_result* __restrict__ ego)
 {
     int f = blockIdx.x;
     const ofb_imu_sample& s = imu[f];
@@ -54,21 +56,27 @@ __device__ __forceinline__ void pair_solve(const Loader& ld, int variant, const 
         r.flags = (det && det[f].overflow) ? OFB_PAIR_OVERFLOW : 0;     // detector ran out of candidate slots
         out[f] = r;
     }
+    if (EGO) {
+        const OfbEgoOut e = ofb_block_solve_ego(ld, f, variant, s.d, s.n, s.t);
+        if (threadIdx.x == 0) ego[f] = ofb_ego_record(e, OFB_EGO_SOLVED);
+    }
 }
 
+template <bool EGO>
 __global__ void __launch_bounds__(OFB_SOLVE_THREADS)
 pair_solve_kernel(TrackLoader ld, int variant, const ofb_imu_sample* __restrict__ imu, ofb_pair_result* __restrict__ out,
-                  const FeatImageState* __restrict__ det)
+                  const FeatImageState* __restrict__ det, ofb_ego_result* __restrict__ ego)
 {
-    pair_solve(ld, variant, imu, out, det);
+    pair_solve<EGO>(ld, variant, imu, out, det, ego);
 }
 
 // With a calibrated camera: every tracked point is undistorted once into xu (the solve reads each point twice), then
 // solved from there.
+template <bool EGO>
 __global__ void __launch_bounds__(OFB_SOLVE_THREADS)
 pair_solve_cam_kernel(TrackLoader tl, ofb_camera cam, double4* __restrict__ xu, int variant,
                       const ofb_imu_sample* __restrict__ imu, ofb_pair_result* __restrict__ out,
-                      const FeatImageState* __restrict__ det)
+                      const FeatImageState* __restrict__ det, ofb_ego_result* __restrict__ ego)
 {
     const int f = blockIdx.x, n = tl.end(f);
     for (int i = threadIdx.x; i < n; i += blockDim.x) {
@@ -76,19 +84,20 @@ pair_solve_cam_kernel(TrackLoader tl, ofb_camera cam, double4* __restrict__ xu, 
         if (tl.status[o]) xu[o] = ofb_calibrate(cam, tl.next[2 * o], tl.next[2 * o + 1], tl.prev[2 * o], tl.prev[2 * o + 1]);
     }
     __syncthreads();
-    pair_solve(CalibLoader{xu, tl.stride, tl.status, tl.counts, tl.counts_stride, 0}, variant, imu, out, det);
+    pair_solve<EGO>(CalibLoader{xu, tl.stride, tl.status, tl.counts, tl.counts_stride, 0}, variant, imu, out, det, ego);
 }
 
 }  // namespace
 
 // Stages 1b-4 for pairs [c0, c0+n) whose level-0 frames already sit in pp/pn (images 0..n-1 of each).
 // gyro (NULL: off): the pinhole model of the gyro prediction, with dcam the device copy of the camera (NULL: pinhole).
+// d_ego (NULL: off): the pairs' ego-motion records, solved in the velocity solve's kernel.
 // Sequence layout (pn == pp): pp holds n+1 consecutive frames of one stream, pair i = (image i, image i+1), so every
 // interior frame's pyramid is built once and serves as "next" of one pair and "prev" of the following one.
 static int run_pairs_chunk(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, double fb_max_err,
                            const GyroPinhole* gyro, const ofb_camera* dcam, ofb_pyr* pp, ofb_pyr* pn, int n, int c0,
                            const ofb_imu_sample* dimu, const int* counts_in, float* d_prev, float* d_next, uint8_t* d_stat,
-                           ofb_pair_result* d_res, bool mark)
+                           ofb_pair_result* d_res, ofb_ego_result* d_ego, bool mark)
 {
     const bool seq = pn == pp;
     const int w = cfg->width, h = cfg->height, K = cfg->max_corners;
@@ -158,12 +167,15 @@ static int run_pairs_chunk(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_came
                           ctx->scratch[SC_ERR].as<float>(), fb_max_err));
     STAGE_MARK(4);
     TrackLoader ld{cp, cn, cs, counts, counts_stride, (size_t)K, cfg->cx, cfg->cy, cfg->pos_scale, cfg->flow_scale};
+    ofb_ego_result* ego = d_ego ? d_ego + c0 : nullptr;
     if (cam) {
         OFB_TRY(ctx->scratch[SC_CALIB].reserve(sizeof(double4) * (size_t)n * K));
-        pair_solve_cam_kernel<<<n, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, *cam, ctx->scratch[SC_CALIB].as<double4>(), cfg->variant,
-                                                                       dimu + c0, d_res + c0, st);
+        auto kern = d_ego ? pair_solve_cam_kernel<true> : pair_solve_cam_kernel<false>;
+        kern<<<n, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, *cam, ctx->scratch[SC_CALIB].as<double4>(), cfg->variant, dimu + c0,
+                                                       d_res + c0, st, ego);
     } else {
-        pair_solve_kernel<<<n, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, cfg->variant, dimu + c0, d_res + c0, st);
+        auto kern = d_ego ? pair_solve_kernel<true> : pair_solve_kernel<false>;
+        kern<<<n, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, cfg->variant, dimu + c0, d_res + c0, st, ego);
     }
     OFB_LAUNCH_CHECK(ctx);
     STAGE_MARK(5);
@@ -203,6 +215,16 @@ extern "C" int ofb_frame_pairs_gyro(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const
                                     size_t image_stride, const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
                                     ofb_pair_result* results, float* prev_pts, float* next_pts, uint8_t* status)
 {
+    return ofb_frame_pairs_ego(ctx, cfg, cam, fb_max_err, gyro_predict, n_pairs, prev, next, pitch, image_stride, imu, pts_in, n_in,
+                               results, nullptr, prev_pts, next_pts, status);
+}
+
+extern "C" int ofb_frame_pairs_ego(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, double fb_max_err,
+                                   int gyro_predict, int n_pairs, const uint8_t* prev, const uint8_t* next, int pitch,
+                                   size_t image_stride, const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
+                                   ofb_pair_result* results, ofb_ego_result* ego, float* prev_pts, float* next_pts,
+                                   uint8_t* status)
+{
     OFB_REQUIRE(ctx && cfg && prev && next && imu && results, "frame_pairs: null argument");
     if (cam) OFB_TRY(ofb_camera_check(cam, "frame_pairs"));
     OFB_REQUIRE(ofb_fb_thr_ok(fb_max_err), "frame_pairs: fb_max_err must be >= 0 (0 = no forward-backward check)");
@@ -218,11 +240,12 @@ extern "C" int ofb_frame_pairs_gyro(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const
     OFB_REQUIRE(n_pairs == 1 || image_stride >= (size_t)pitch * (h - 1) + w, "frame_pairs: image_stride too small");
     OFB_CUDA(cudaSetDevice(ctx->device));
     const size_t npts = (size_t)n_pairs * K;
-    OutStage o[4];
+    OutStage o[5];
     OFB_TRY(ofb_stage_out(ctx, SC_PTS0, prev_pts, sizeof(float) * 2 * npts, &o[0]));
     OFB_TRY(ofb_stage_out(ctx, SC_PTS1, next_pts, sizeof(float) * 2 * npts, &o[1]));
     OFB_TRY(ofb_stage_out(ctx, SC_STAT, status, npts, &o[2]));
     OFB_TRY(ofb_stage_out(ctx, SC_OUT3, results, sizeof(ofb_pair_result) * n_pairs, &o[3]));
+    OFB_TRY(ofb_stage_out(ctx, SC_EGO, ego, sizeof(ofb_ego_result) * n_pairs, &o[4]));
     // optional outputs still need device storage when the caller passes NULL
     float* d_prev = (float*)o[0].dev; float* d_next = (float*)o[1].dev; uint8_t* d_stat = (uint8_t*)o[2].dev;
     if (!d_prev) { OFB_TRY(ctx->scratch[SC_PTS0].reserve(sizeof(float) * 2 * npts)); d_prev = ctx->scratch[SC_PTS0].as<float>(); }
@@ -332,14 +355,14 @@ extern "C" int ofb_frame_pairs_gyro(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const
         OFB_TRY(run_pairs_chunk(c, cfg, cam, fb_max_err, gyro_predict ? &gph : nullptr, (const ofb_camera*)dcam,
                                 c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
                                 (const ofb_imu_sample*)dimu, counts_in, d_prev, d_next, d_stat, (ofb_pair_result*)o[3].dev,
-                                ctx->profile));
+                                (ofb_ego_result*)o[4].dev, ctx->profile));
     }
     if (use_twin) {
         ctx->launches += tw->launches - tw0;
         OFB_CUDA(cudaEventRecord(ctx->ev_twin_join, tw->stream));
         OFB_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_twin_join, 0));
     }
-    int rc = ofb_finish_out(ctx, o, 4);
+    int rc = ofb_finish_out(ctx, o, ego ? 5 : 4);
     if (rc == OFB_OK && ctx->profile) {
         // stage order: 0 pyramids, 1 lambda_min+NMS, 2 ordered selection, 3 LK, 4 solve
         OFB_CUDA(cudaEventSynchronize(ctx->stage_ev[5]));

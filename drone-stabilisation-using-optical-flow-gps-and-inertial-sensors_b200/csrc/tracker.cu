@@ -70,6 +70,10 @@ struct ofb_tracker {
     // gyro-predicted initial flow of the LK tracks (ofb_tracker_set_gyro_prediction): whether the prediction kernel is
     // launched is decided when a step is enqueued, so a change drops the captured graphs
     bool gyro = false;
+    // ego-motion solve after the velocity solve (ofb_tracker_set_ego_motion): which kernel is launched is decided when a
+    // step is enqueued, so a change drops the captured graphs; records the caller did not ask for go to ego_buf
+    bool ego = false;
+    DevBuf ego_buf;
     uint64_t graph_steps = 0;
 };
 
@@ -121,14 +125,16 @@ __device__ __forceinline__ double r_tilde_point(double px, double py, double ux,
     return r;
 }
 
+// EGO: the ego-motion solve of the stream follows the velocity solve on the same kept points (ego[s], zero with flags 0
+// when the stream did not solve); EGO = false is the velocity solve alone.
 // PART 0: filter + solve in one launch. PART 1: the filter alone (compaction, gates, counts, top-up decision -- all the next
 // step's LK needs); PART 2: the solve of a stream an earlier PART 1 launch compacted. The split lets the solve run beside
 // the next frame's LK on a stream of its own: nothing but the NEXT filter (its r_tilde gate uses the solved velocity) and
 // the reader of the result record depend on it.
-template <int PART>
+template <int PART, bool EGO = false>
 __global__ void __launch_bounds__(OFB_SOLVE_THREADS)
 track_filter_solve_kernel(TrackerDev T, const ofb_imu_sample* __restrict__ imu, const double* __restrict__ v_prior,
-                          ofb_track_result* __restrict__ out)
+                          ofb_track_result* __restrict__ out, ofb_ego_result* __restrict__ ego)
 {
     const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     __shared__ int wtot[OFB_SOLVE_THREADS / 32];
@@ -222,6 +228,15 @@ track_filter_solve_kernel(TrackerDev T, const ofb_imu_sample* __restrict__ imu, 
             o = ofb_block_solve(ld, s, T.variant, im.d, im.n, im.w, im.t, vp);
         }
     }
+    OfbEgoOut e;
+    if (EGO && PART != 1 && solve) {
+        if (T.cam) {
+            e = ofb_block_solve_ego(CalibLoader{T.calib, (size_t)T.cap, nullptr, nullptr, 0, kept}, s, T.variant, im.d, im.n, im.t);
+        } else {
+            KeptLoader ld{T.kept_prev, T.kept_next, kept, (size_t)T.cap, T.cx, T.cy, T.ps, T.fs};
+            e = ofb_block_solve_ego(ld, s, T.variant, im.d, im.n, im.t);
+        }
+    }
     // the detector's per-image state and (for streams that will top up) its min-distance cell grid start clean
     if (PART != 2 && kept <= T.min_features)
         for (size_t i = tid; i < T.cell_stride; i += OFB_SOLVE_THREADS) T.cell_grid[(size_t)s * T.cell_stride + i] = -1;
@@ -232,6 +247,10 @@ track_filter_solve_kernel(TrackerDev T, const ofb_imu_sample* __restrict__ imu, 
             r.res = solve ? o.res : 0.0; r.rank = solve ? o.rank : 0;
             r.flags = solve ? OFB_TRACK_SOLVED : 0;
             if (solve) { T.vlast[3 * s] = o.v[0]; T.vlast[3 * s + 1] = o.v[1]; T.vlast[3 * s + 2] = o.v[2]; }
+            if (EGO) {
+                if (solve) ego[s] = ofb_ego_record(e, OFB_EGO_SOLVED);
+                else { ofb_ego_result z = {}; ego[s] = z; }
+            }
         }
         if (PART != 2) {
             FeatImageState z; z.max_key = 0; z.n_cand = 0; z.n_out = 0; z.overflow = 0;
@@ -452,7 +471,7 @@ extern "C" int ofb_tracker_destroy(ofb_tracker* t)
     if (t->ev_lk) cudaEventDestroy(t->ev_lk);
     if (t->ev_pyr) cudaEventDestroy(t->ev_pyr);
     DevBuf* bufs[] = {&t->counts, &t->nxt, &t->status, &t->err, &t->kept_prev, &t->det, &t->vlast, &t->mask, &t->hw, &t->bgr, &t->dev_io,
-                      &t->cam_dev, &t->calib};
+                      &t->cam_dev, &t->calib, &t->ego_buf};
     for (DevBuf* b : bufs) b->release();
     delete t;
     return OFB_OK;
@@ -504,16 +523,22 @@ static cudaError_t tracker_join_solve(ofb_tracker* t)
 // One step, launch by launch, on ctx->stream (also the body that is captured into a graph).
 static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitch, size_t image_stride,
                                  const ofb_imu_sample* imu, const double* v_prior, ofb_track_result* results,
-                                 float* pts_out, int* n_out, float* kept_prev, float* kept_next)
+                                 float* pts_out, int* n_out, float* kept_prev, float* kept_next, ofb_ego_result* ego)
 {
     ofb_ctx* ctx = t->ctx;
     const ofb_tracker_cfg& cfg = t->cfg;
     const ofb_pair_cfg& pc = cfg.pair;
     const int S = cfg.n_streams, w = pc.width, h = pc.height, K = pc.max_corners, cap = t->cap;
     const size_t np = (size_t)S * cap;
-    OutStage o[2];
+    OutStage o[3];
     OFB_TRY(ofb_stage_out(ctx, SC_OUT3, results, sizeof(ofb_track_result) * S, &o[0]));
     OFB_TRY(ofb_stage_out(ctx, SC_OUT2, n_out, sizeof(int) * S, &o[1]));
+    OFB_TRY(ofb_stage_out(ctx, SC_EGO, ego, sizeof(ofb_ego_result) * S, &o[2]));
+    ofb_ego_result* d_ego = (ofb_ego_result*)o[2].dev;
+    if (t->ego && !d_ego) {
+        OFB_TRY(t->ego_buf.reserve(sizeof(ofb_ego_result) * S));
+        d_ego = t->ego_buf.as<ofb_ego_result>();
+    }
     const void *dimu, *dvp = nullptr;
     OFB_TRY(ofb_stage_in(ctx, SC_IN3, imu, sizeof(ofb_imu_sample) * S, &dimu));
     if (v_prior) OFB_TRY(ofb_stage_in(ctx, SC_IN4, v_prior, sizeof(double) * 3 * S, &dvp));
@@ -631,7 +656,7 @@ static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitc
     {
         const char* se = getenv("OFB_TRACKER_SPLIT_SOLVE");
         split = early && t->have_prev && ofb_is_device_ptr(results) && ofb_is_device_ptr(imu) && (!v_prior || ofb_is_device_ptr(v_prior)) &&
-                !(se && se[0] == '0');
+                (!ego || ofb_is_device_ptr(ego)) && !(se && se[0] == '0');
     }
     if (split) {
         if (!t->sol_stream) {
@@ -642,18 +667,20 @@ static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitc
             ctx->aux_join.push_back(std::make_pair(t->sol_stream, t->ev_sol_join));
         }
         track_filter_solve_kernel<1><<<S, OFB_SOLVE_THREADS, 0, ctx->stream>>>(T, (const ofb_imu_sample*)dimu, (const double*)dvp,
-                                                                               (ofb_track_result*)o[0].dev);
+                                                                               (ofb_track_result*)o[0].dev, nullptr);
         OFB_LAUNCH_CHECK(ctx);
         OFB_CUDA(cudaEventRecord(t->ev_filt, ctx->stream));
         OFB_CUDA(cudaStreamWaitEvent(t->sol_stream, t->ev_filt, 0));
-        track_filter_solve_kernel<2><<<S, OFB_SOLVE_THREADS, 0, t->sol_stream>>>(T, (const ofb_imu_sample*)dimu, (const double*)dvp,
-                                                                                 (ofb_track_result*)o[0].dev);
+        auto kern = t->ego ? track_filter_solve_kernel<2, true> : track_filter_solve_kernel<2>;
+        kern<<<S, OFB_SOLVE_THREADS, 0, t->sol_stream>>>(T, (const ofb_imu_sample*)dimu, (const double*)dvp, (ofb_track_result*)o[0].dev,
+                                                         d_ego);
         OFB_LAUNCH_CHECK(ctx);
         OFB_CUDA(cudaEventRecord(t->ev_sol, t->sol_stream));
         t->sol_pending = true;
     } else {
-        track_filter_solve_kernel<0><<<S, OFB_SOLVE_THREADS, 0, ctx->stream>>>(T, (const ofb_imu_sample*)dimu, (const double*)dvp,
-                                                                               (ofb_track_result*)o[0].dev);
+        auto kern = t->ego ? track_filter_solve_kernel<0, true> : track_filter_solve_kernel<0>;
+        kern<<<S, OFB_SOLVE_THREADS, 0, ctx->stream>>>(T, (const ofb_imu_sample*)dimu, (const double*)dvp, (ofb_track_result*)o[0].dev,
+                                                       d_ego);
         OFB_LAUNCH_CHECK(ctx);
     }
     bool host_out = false;
@@ -693,7 +720,7 @@ static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitc
     t->cur ^= 1;
     t->have_prev = true;
     t->launches_end = ctx->launches; t->async_end = ctx->async_writes;
-    int rc = ofb_finish_out(ctx, o, 2);
+    int rc = ofb_finish_out(ctx, o, 3);
     if (rc == OFB_OK && host_out) OFB_CUDA(cudaStreamSynchronize(ctx->stream));
     return rc;
 }
@@ -710,7 +737,7 @@ static uint64_t scratch_signature(const ofb_ctx* ctx)
 // Steady-state step replayed from a captured CUDA graph. Returns OFB_E_UNSUPPORTED when the graph could not be
 // built (the caller then runs the step launch by launch; nothing has executed and the tracker state is unchanged).
 static int tracker_step_graph(ofb_tracker* t, const uint8_t* frames, int pitch, size_t image_stride,
-                              const ofb_imu_sample* imu, const double* v_prior, ofb_track_result* results)
+                              const ofb_imu_sample* imu, const double* v_prior, ofb_track_result* results, ofb_ego_result* ego)
 {
     ofb_ctx* ctx = t->ctx;
     const int S = t->cfg.n_streams, w = t->cfg.pair.width, h = t->cfg.pair.height;
@@ -718,10 +745,11 @@ static int tracker_step_graph(ofb_tracker* t, const uint8_t* frames, int pitch, 
     const size_t off_imu = (fbytes * S + 255) & ~(size_t)255, off_vp = off_imu + sizeof(ofb_imu_sample) * S;
     const size_t in_bytes = off_vp + sizeof(double) * 3 * S;
     const size_t d_vp = sizeof(ofb_imu_sample) * S, d_res = d_vp + sizeof(double) * 3 * S;
+    const size_t d_ego = d_res + sizeof(ofb_track_result) * S, out_bytes = sizeof(ofb_track_result) * S;
     if (!t->pin_in.p) {                 // fixed sizes: allocated once, the addresses are baked into the graphs
         OFB_TRY(t->pin_in.reserve(in_bytes));
-        OFB_TRY(t->pin_out.reserve(sizeof(ofb_track_result) * S));
-        OFB_TRY(t->dev_io.reserve(d_res + sizeof(ofb_track_result) * S));
+        OFB_TRY(t->pin_out.reserve(out_bytes + sizeof(ofb_ego_result) * S));    // results | ego records
+        OFB_TRY(t->dev_io.reserve(d_ego + sizeof(ofb_ego_result) * S));
     }
     uint8_t* pin = (uint8_t*)t->pin_in.p;
     uint8_t* dio = t->dev_io.as<uint8_t>();
@@ -750,8 +778,11 @@ static int tracker_step_graph(ofb_tracker* t, const uint8_t* frames, int pitch, 
             cudaMemcpyAsync(dio + d_vp, pin + off_vp, sizeof(double) * 3 * S, cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess) rc = OFB_E_CUDA;
         if (rc == OFB_OK)
             rc = tracker_step_launches(t, pin, (int)row, fbytes, (const ofb_imu_sample*)dio, v_prior ? (const double*)(dio + d_vp) : nullptr,
-                                       (ofb_track_result*)(dio + d_res), nullptr, nullptr, nullptr, nullptr);
-        if (rc == OFB_OK && cudaMemcpyAsync(t->pin_out.p, dio + d_res, sizeof(ofb_track_result) * S, cudaMemcpyDeviceToHost,
+                                       (ofb_track_result*)(dio + d_res), nullptr, nullptr, nullptr, nullptr,
+                                       t->ego ? (ofb_ego_result*)(dio + d_ego) : nullptr);
+        // the ego records follow the results in dev_io and pin_out: one copy brings both back
+        const size_t copy_bytes = out_bytes + (t->ego ? sizeof(ofb_ego_result) * S : 0);
+        if (rc == OFB_OK && cudaMemcpyAsync(t->pin_out.p, dio + d_res, copy_bytes, cudaMemcpyDeviceToHost,
                                             ctx->stream) != cudaSuccess) rc = OFB_E_CUDA;
         const cudaError_t e = cudaStreamEndCapture(ctx->stream, &g);
         const uint64_t captured = ctx->launches - l0;
@@ -774,7 +805,8 @@ static int tracker_step_graph(ofb_tracker* t, const uint8_t* frames, int pitch, 
     ctx->launches += t->glaunches[par][hp];
     t->pcur ^= 1; t->cur ^= 1; t->graph_steps++;
     OFB_CUDA(cudaStreamSynchronize(ctx->stream));
-    memcpy(results, t->pin_out.p, sizeof(ofb_track_result) * S);
+    memcpy(results, t->pin_out.p, out_bytes);
+    if (ego) memcpy(ego, (const uint8_t*)t->pin_out.p + out_bytes, sizeof(ofb_ego_result) * S);
     return OFB_OK;
 }
 
@@ -782,7 +814,15 @@ extern "C" int ofb_tracker_step(ofb_tracker* t, const uint8_t* frames, int pitch
                                 const ofb_imu_sample* imu, const double* v_prior, ofb_track_result* results,
                                 float* pts_out, int* n_out, float* kept_prev, float* kept_next)
 {
+    return ofb_tracker_step_ego(t, frames, pitch, image_stride, imu, v_prior, results, pts_out, n_out, kept_prev, kept_next, nullptr);
+}
+
+extern "C" int ofb_tracker_step_ego(ofb_tracker* t, const uint8_t* frames, int pitch, size_t image_stride,
+                                    const ofb_imu_sample* imu, const double* v_prior, ofb_track_result* results,
+                                    float* pts_out, int* n_out, float* kept_prev, float* kept_next, ofb_ego_result* ego)
+{
     OFB_REQUIRE(t && frames && imu && results, "tracker_step: null argument");
+    OFB_REQUIRE(!ego || t->ego, "tracker_step: ego records need ofb_tracker_set_ego_motion(trk, 1)");
     ofb_ctx* ctx = t->ctx;
     const int S = t->cfg.n_streams, w = t->cfg.pair.width, h = t->cfg.pair.height, bpp = t->cfg.bgr_input ? 3 : 1;
     OFB_REQUIRE(pitch >= bpp * w, "tracker_step: pitch smaller than a row");
@@ -797,13 +837,13 @@ extern "C" int ofb_tracker_step(ofb_tracker* t, const uint8_t* frames, int pitch
     const bool graphs_on = !(genv && genv[0] == '0');
     if (graphs_on && t->graph_ok && t->have_prev && t->plain_steps >= 3 && !pts_out && !n_out && !kept_prev && !kept_next &&
         (size_t)S * bpp * w * h <= ((size_t)16 << 20) && !ofb_is_device_ptr(frames) && !ofb_is_device_ptr(imu) &&
-        !ofb_is_device_ptr(results) && !(v_prior && ofb_is_device_ptr(v_prior))) {
-        const int rc = tracker_step_graph(t, frames, pitch, image_stride, imu, v_prior, results);
+        !ofb_is_device_ptr(results) && !(v_prior && ofb_is_device_ptr(v_prior)) && !(ego && ofb_is_device_ptr(ego))) {
+        const int rc = tracker_step_graph(t, frames, pitch, image_stride, imu, v_prior, results, ego);
         if (rc != OFB_E_UNSUPPORTED) return rc;
         t->graph_ok = false;            // this build / driver cannot capture the step: stay on plain launches
     }
     t->plain_steps++;
-    return tracker_step_launches(t, frames, pitch, image_stride, imu, v_prior, results, pts_out, n_out, kept_prev, kept_next);
+    return tracker_step_launches(t, frames, pitch, image_stride, imu, v_prior, results, pts_out, n_out, kept_prev, kept_next, ego);
 }
 
 extern "C" int ofb_tracker_set_camera(ofb_tracker* t, const ofb_camera* cam)
@@ -862,6 +902,22 @@ extern "C" int ofb_tracker_set_gyro_prediction(ofb_tracker* t, int enable)
             for (int j = 0; j < 2; ++j)
                 if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
         t->gyro = enable != 0;
+    }
+    return OFB_OK;
+}
+
+extern "C" int ofb_tracker_set_ego_motion(ofb_tracker* t, int enable)
+{
+    OFB_REQUIRE(t, "tracker_set_ego_motion: null tracker");
+    OFB_REQUIRE(!enable || t->cfg.pair.variant != OFB_VARIANT_MODULE,
+                "tracker_set_ego_motion: the MODULE variant has no gyro term to estimate");
+    if ((enable != 0) != t->ego) {
+        // the solve kernel is chosen when a step is enqueued: graphs captured before are rebuilt (no graph is in flight: a
+        // replayed step synchronises before it returns)
+        for (int i = 0; i < 2; ++i)
+            for (int j = 0; j < 2; ++j)
+                if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
+        t->ego = enable != 0;
     }
     return OFB_OK;
 }

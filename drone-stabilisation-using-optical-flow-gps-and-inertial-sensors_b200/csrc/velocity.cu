@@ -51,6 +51,15 @@ solve_velocity_kernel(Loader ld, int variant, const double* __restrict__ d_arr, 
     }
 }
 
+__global__ void __launch_bounds__(OFB_SOLVE_THREADS)
+solve_ego_kernel(PointsF64 ld, int variant, const double* __restrict__ d_arr, const double* __restrict__ n_arr,
+                 const double* __restrict__ t_arr, ofb_ego_result* __restrict__ out)
+{
+    const int f = blockIdx.x;
+    const OfbEgoOut o = ofb_block_solve_ego(ld, f, variant, d_arr[f], n_arr + 3 * (size_t)f, t_arr ? t_arr + 3 * (size_t)f : nullptr);
+    if (threadIdx.x == 0) out[f] = ofb_ego_record(o, OFB_EGO_SOLVED);
+}
+
 __global__ void generate_flow_kernel(const double* __restrict__ x, int n, double3 v, double3 w, double d,
                                      double3 nrm, double* __restrict__ u)
 {
@@ -227,6 +236,50 @@ extern "C" int ofb_solve_velocity(ofb_ctx* ctx, int variant, const double* x, co
     double dummy[2] = {0, 0};
     return ofb_solve_velocity_batched(ctx, variant, n ? x : dummy, n ? u : dummy, offsets, 1, &d, n3, w3, t3,
                                       v_out, res, rank, s_out);
+}
+
+extern "C" int ofb_solve_ego_motion_batched(ofb_ctx* ctx, int variant, const double* x, const double* u, const int* offsets,
+                                            int n_frames, const double* d, const double* n3, const double* t3, ofb_ego_result* out)
+{
+    OFB_REQUIRE(ctx && x && u && offsets && d && n3 && out, "solve_ego_motion_batched: null argument");
+    OFB_REQUIRE(variant >= 0 && variant <= 2, "solve_ego_motion: unknown variant %d (MODULE has no gyro term to estimate)", variant);
+    OFB_REQUIRE(n_frames > 0, "solve_ego_motion_batched: n_frames must be positive");
+    OFB_CUDA(cudaSetDevice(ctx->device));
+    std::vector<int> hoff(n_frames + 1);
+    if (ofb_is_device_ptr(offsets)) {
+        OFB_CUDA(cudaMemcpyAsync(hoff.data(), offsets, sizeof(int) * (n_frames + 1), cudaMemcpyDeviceToHost, ctx->stream));
+        OFB_CUDA(cudaStreamSynchronize(ctx->stream));
+    } else memcpy(hoff.data(), offsets, sizeof(int) * (n_frames + 1));
+    OFB_REQUIRE(hoff[0] >= 0, "solve_ego_motion_batched: offsets[0] = %d is negative", hoff[0]);
+    for (int f = 0; f < n_frames; ++f)
+        OFB_REQUIRE(hoff[f + 1] >= hoff[f], "solve_ego_motion_batched: offsets must be non-decreasing (offsets[%d] = %d > offsets[%d] = %d)",
+                    f, hoff[f], f + 1, hoff[f + 1]);
+    const int total = hoff[n_frames];
+    const void *dx, *du, *doff, *dd, *dn, *dt = nullptr;
+    OFB_TRY(ofb_stage_in(ctx, SC_IN0, x, sizeof(double) * 2 * (size_t)total, &dx));
+    OFB_TRY(ofb_stage_in(ctx, SC_IN1, u, sizeof(double) * 2 * (size_t)total, &du));
+    OFB_TRY(ofb_stage_in(ctx, SC_IN2, offsets, sizeof(int) * (n_frames + 1), &doff));
+    OFB_TRY(ofb_stage_in(ctx, SC_IN3, d, sizeof(double) * n_frames, &dd));
+    OFB_TRY(ofb_stage_in(ctx, SC_IN4, n3, sizeof(double) * 3 * n_frames, &dn));
+    if (t3) OFB_TRY(ofb_stage_in(ctx, SC_TMP0, t3, sizeof(double) * 3 * n_frames, &dt));
+    OutStage o;
+    OFB_TRY(ofb_stage_out(ctx, SC_OUT0, out, sizeof(ofb_ego_result) * n_frames, &o));
+    PointsF64 ld{(const double*)dx, (const double*)du, (const int*)doff, 0};
+    solve_ego_kernel<<<n_frames, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, variant, (const double*)dd, (const double*)dn,
+                                                                       (const double*)dt, (ofb_ego_result*)o.dev);
+    OFB_LAUNCH_CHECK(ctx);
+    return ofb_finish_out(ctx, &o, 1);
+}
+
+extern "C" int ofb_solve_ego_motion(ofb_ctx* ctx, int variant, const double* x, const double* u, int n, double d,
+                                    const double n3[3], const double t3[3], ofb_ego_result* out)
+{
+    OFB_REQUIRE(ctx && n3 && out, "solve_ego_motion: null argument");
+    OFB_REQUIRE(n >= 0, "solve_ego_motion: negative point count");
+    OFB_REQUIRE(n == 0 || (x && u), "solve_ego_motion: null points");
+    int offsets[2] = {0, n};
+    double dummy[2] = {0, 0};
+    return ofb_solve_ego_motion_batched(ctx, variant, n ? x : dummy, n ? u : dummy, offsets, 1, &d, n3, t3, out);
 }
 
 extern "C" int ofb_generate_flow(ofb_ctx* ctx, const double* x, int n, const double v3[3], const double w3[3],

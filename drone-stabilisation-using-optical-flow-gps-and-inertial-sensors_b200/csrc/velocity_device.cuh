@@ -160,3 +160,136 @@ __device__ OfbSolveOut ofb_block_solve(const Loader& ld, int f, int variant, dou
     o.v[0] = v[0]; o.v[1] = v[1]; o.v[2] = v[2];
     return o;
 }
+
+// Ego-motion solve: the angular rate is estimated together with the velocity instead of being taken from the gyro.
+// Moving the gyro term of ofb_point_terms to the left side makes every point's block linear in (v', w):
+//   X = (x, y, 1), C = [X]x, P = |X|^2 I - X X^T = C^T C, u3 = (ux, uy, 0), v' = v + w x t
+//   A_i = [ wA C , d wb P ],  b_i = d wb C u3        (wA, wb: the variant weights of ofb_point_terms; MODULE has no
+//                                                      gyro term and is not accepted)
+// The normal-equation blocks have closed forms (C X = 0, C P = |X|^2 C, P^2 = |X|^2 P):
+//   A^T A: vv = wA^2 P, vw = -wA d wb |X|^2 C, ww = d^2 wb^2 |X|^2 P;   A^T b: v = wA d wb P u3, w = d^2 wb^2 |X|^2 C u3
+// C is antisymmetric with entries (-1, y, -x) above the diagonal, so vw needs three sums: 6 + 3 + 6 + 6 + a count =
+// 22 fp64 accumulators per thread. The 6x6 system is decomposed by one warp (ofb_jacobi_n<6>, the other warps wait);
+// the pseudo-inverse keeps the eigenpairs of A^T A that pass ofb_block_solve's rank rule; a second pass sums the
+// residual r_i = X x (wA v' - d wb (X x w) - d wb u3) = A_i (v', w) - b_i.
+struct OfbEgoOut { double v[3]; double w[3]; double s[6]; double res; int rank; int count; };
+
+template <class Loader>
+__device__ OfbEgoOut ofb_block_solve_ego(const Loader& ld, int f, int variant, double d, const double* n3g, const double* t3g)
+{
+    __shared__ double red[22 * 32];
+    __shared__ double sol[6 + 6 + 1];                // (v', w), s descending, rank
+    const double n3[3] = {n3g[0], n3g[1], n3g[2]};
+    const bool sim = variant == OFB_VARIANT_SIM;
+    const int i0 = ld.begin(f), i1 = ld.end(f);
+    double acc[22];
+#pragma unroll
+    for (int k = 0; k < 22; ++k) acc[k] = 0.0;
+    for (int i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+        double px, py, ux, uy;
+        if (!ld.load(f, i, px, py, ux, uy)) continue;
+        const double nx = n3[0] * px + n3[1] * py + n3[2];
+        const double wA = sim ? nx : 1.0, e = sim ? d : d / nx;           // e = d wb
+        const double xx = px * px, yy = py * py, xy = px * py, r2 = xx + yy + 1.0;
+        // P packed as (xx, xy, xz, yy, yz, zz)
+        const double P[6] = {yy + 1.0, -xy, -px, xx + 1.0, -py, xx + yy};
+        const double a2 = wA * wA, e2r = e * e * r2;
+#pragma unroll
+        for (int k = 0; k < 6; ++k) { acc[k] += a2 * P[k]; acc[9 + k] += e2r * P[k]; }
+        const double kc = -wA * e * r2;                                    // vw = kc C
+        acc[6] += kc; acc[7] += kc * py; acc[8] += kc * px;
+        const double s = px * ux + py * uy, we = wA * e;                   // P u3 = r2 u3 - X (X . u3)
+        acc[15] += we * (r2 * ux - px * s);
+        acc[16] += we * (r2 * uy - py * s);
+        acc[17] += we * (-s);
+        acc[18] += e2r * (-uy);                                            // C u3 = X x u3
+        acc[19] += e2r * ux;
+        acc[20] += e2r * (px * uy - py * ux);
+        acc[21] += 1.0;
+    }
+    ofb_block_sum<22>(acc, red);
+    OfbEgoOut o;
+    o.count = (int)(acc[21] + 0.5);
+    if (threadIdx.x < 32) {
+        const double k0 = acc[6], k1 = acc[7], k2 = acc[8];
+        // vw block = sum kc C, C = [[0, -1, y], [1, 0, -x], [-y, x, 0]]
+        double a[6][6] = {
+            {acc[0], acc[1], acc[2], 0.0, -k0, k1},
+            {acc[1], acc[3], acc[4], k0, 0.0, -k2},
+            {acc[2], acc[4], acc[5], -k1, k2, 0.0},
+            {0.0, k0, -k1, acc[9], acc[10], acc[11]},
+            {-k0, 0.0, k2, acc[10], acc[12], acc[13]},
+            {k1, -k2, 0.0, acc[11], acc[13], acc[14]}};
+        double q[6][6];
+        ofb_jacobi_n<6>(a, q);
+        double ev[6], smax = 0.0;
+#pragma unroll
+        for (int k = 0; k < 6; ++k) { ev[k] = a[k][k]; smax = fmax(smax, ev[k] > 0 ? sqrt(ev[k]) : 0.0); }
+        // numpy lstsq's rank rule (rcond=None), floored as in ofb_block_solve
+        const double rows = 3.0 * (double)o.count;
+        double rc = 2.220446049250313e-16 * (rows > 6.0 ? rows : 6.0);
+        if (rc < 1e-7) rc = 1e-7;
+        double x[6] = {0, 0, 0, 0, 0, 0}, sk[6];
+        int rank = 0;
+#pragma unroll
+        for (int k = 0; k < 6; ++k) {
+            sk[k] = ev[k] > 0 ? sqrt(ev[k]) : 0.0;
+            if (sk[k] > rc * smax && smax > 0) {
+                ++rank;
+                double c = 0.0;
+#pragma unroll
+                for (int j = 0; j < 6; ++j) c += q[j][k] * acc[15 + j];
+                c /= ev[k];
+#pragma unroll
+                for (int j = 0; j < 6; ++j) x[j] += c * q[j][k];
+            }
+        }
+#pragma unroll
+        for (int i = 0; i < 5; ++i)                                        // descending, fixed compare-exchange order
+#pragma unroll
+            for (int j = 0; j < 5 - i; ++j) {
+                const double hi = fmax(sk[j], sk[j + 1]), lo = fmin(sk[j], sk[j + 1]);
+                sk[j] = hi; sk[j + 1] = lo;
+            }
+        if (threadIdx.x == 0) {
+#pragma unroll
+            for (int k = 0; k < 6; ++k) { sol[k] = x[k]; sol[6 + k] = sk[k]; }
+            sol[12] = (double)rank;
+        }
+    }
+    __syncthreads();
+    const double vp[3] = {sol[0], sol[1], sol[2]}, w[3] = {sol[3], sol[4], sol[5]};
+    double r[1] = {0};
+    for (int i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+        double px, py, ux, uy;
+        if (!ld.load(f, i, px, py, ux, uy)) continue;
+        const double nx = n3[0] * px + n3[1] * py + n3[2];
+        const double wA = sim ? nx : 1.0, e = sim ? d : d / nx;
+        const double cx = py * w[2] - w[1], cy = w[0] - px * w[2], cz = px * w[1] - py * w[0];   // X x w
+        const double ax = wA * vp[0] - e * (cx + ux), ay = wA * vp[1] - e * (cy + uy), az = wA * vp[2] - e * cz;
+        const double rx = py * az - ay, ry = ax - px * az, rz = px * ay - py * ax;
+        r[0] += rx * rx + ry * ry + rz * rz;
+    }
+    ofb_block_sum<1>(r, red);
+    o.res = r[0];
+    o.rank = (int)sol[12];
+    for (int k = 0; k < 3; ++k) { o.v[k] = vp[k]; o.w[k] = w[k]; }
+    for (int k = 0; k < 6; ++k) o.s[k] = sol[6 + k];
+    // lever arm: v = v' - w x t with the estimated rate (EXP, SIM); NODE has none
+    if (variant != OFB_VARIANT_NODE && t3g) {
+        o.v[0] -= w[1] * t3g[2] - w[2] * t3g[1];
+        o.v[1] -= w[2] * t3g[0] - w[0] * t3g[2];
+        o.v[2] -= w[0] * t3g[1] - w[1] * t3g[0];
+    }
+    return o;
+}
+
+// the C ABI record of a solve
+__device__ __forceinline__ ofb_ego_result ofb_ego_record(const OfbEgoOut& o, int flags)
+{
+    ofb_ego_result r;
+    for (int k = 0; k < 3; ++k) { r.v[k] = o.v[k]; r.w[k] = o.w[k]; }
+    for (int k = 0; k < 6; ++k) r.s[k] = o.s[k];
+    r.res = o.res; r.rank = o.rank; r.flags = flags;
+    return r;
+}

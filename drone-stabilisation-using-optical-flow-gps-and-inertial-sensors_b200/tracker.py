@@ -13,7 +13,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from .vision import _fb_threshold, _gyro_flag, as_camera, make_pair_cfg
+from .vision import _ego_flag, _fb_threshold, _gyro_flag, as_camera, make_pair_cfg
 
 
 class StreamTracker:
@@ -33,15 +33,17 @@ class StreamTracker:
     tracker; pass a NEW tensor every step (the tracker keeps the previous one alive; do not overwrite it).
     camera: (K, D, rate[, iterations]) or vision.make_camera(...) -- see set_camera.
     fb_threshold: None / 0 = off, T > 0 = forward-backward check of the LK tracks -- see set_fb_threshold.
-    gyro_prediction: LK starts from the rotation the step's gyro sample measured -- see set_gyro_prediction."""
+    gyro_prediction: LK starts from the rotation the step's gyro sample measured -- see set_gyro_prediction.
+    ego_motion: every stream's angular rate is also estimated from its kept points -- see set_ego_motion."""
 
     def __init__(self, width, height, max_features=100, min_features=20, n_streams=1, feature_params=None,
                  lk_params=None, topup="exp", mask_radius=30, bgr=False, variant="exp", principal=None,
                  scaling=1.0, flow_scaling=None, max_speed=0.0, dummy_value=float("nan"), gate=None, min_solve=3,
                  min_eig_thr=1e-4, borrow_frames=False, v_init=None, camera=None, fb_threshold=None,
-                 gyro_prediction=False, ctx=None):
+                 gyro_prediction=False, ego_motion=False, ctx=None):
         fb = _fb_threshold(fb_threshold)
         gyro = _gyro_flag(gyro_prediction)
+        ego = _ego_flag(ego_motion)
         fp = dict(qualityLevel=0.01, minDistance=10, blockSize=7)
         fp.update(feature_params or {})
         lk = dict(winSize=(15, 15), maxLevel=3, criteria=(3, 20, 0.03))
@@ -84,6 +86,9 @@ class StreamTracker:
             _lib.check(self.ctx.lib.ofb_tracker_set_fb_check(self.h, fb))
         if gyro:
             self.set_gyro_prediction(True)
+        self.ego_motion = False
+        if ego:
+            self.set_ego_motion(True)
 
     def close(self):
         if getattr(self, "h", None) and getattr(self.ctx, "h", None):
@@ -134,6 +139,14 @@ class StreamTracker:
                              "scaling / flow_scaling")
         _lib.check(self.ctx.lib.ofb_tracker_set_gyro_prediction(self.h, on))
 
+    def set_ego_motion(self, enable):
+        """Ego-motion solve of every stream from the next step on (velocity.solve_ego_motion on the kept points, right
+        after the velocity solve): step(..., want_ego=True) returns its _lib.EGO_RESULT_DTYPE records. The standard
+        records do not change. Not available for variant="module" (no gyro term). False turns it off."""
+        on = _ego_flag(enable)
+        _lib.check(self.ctx.lib.ofb_tracker_set_ego_motion(self.h, 1 if on else 0))
+        self.ego_motion = on
+
     def set_points(self, points):
         """points: one (N,2)/(N,1,2) array per stream (or a single array when n_streams == 1)."""
         if self.n_streams == 1 and not isinstance(points, (list, tuple)):
@@ -150,10 +163,13 @@ class StreamTracker:
             cnt[s] = len(p)
         _lib.check(self.ctx.lib.ofb_tracker_set_points(self.h, _lib.ptr(buf), _lib.ptr(cnt)))
 
-    def step(self, frames, imu, v_prior=None, want_points=False, want_kept=False):
+    def step(self, frames, imu, v_prior=None, want_points=False, want_kept=False, want_ego=False):
         """frames: (H,W) / (S,H,W) uint8 (or (...,3) BGR when bgr=True), NumPy or CUDA tensor; imu: _lib.IMU_DTYPE
         (S,). Returns the _lib.TRACK_RESULT_DTYPE records (S,); with want_points additionally the list of (N,1,2)
-        float32 point sets after the step; with want_kept the lists of (old, new) positions the solve used."""
+        float32 point sets after the step; with want_kept the lists of (old, new) positions the solve used; with
+        want_ego (needs set_ego_motion) the _lib.EGO_RESULT_DTYPE records (S,), last."""
+        if want_ego and not self.ego_motion:
+            raise ValueError("want_ego needs ego-motion: StreamTracker(..., ego_motion=True) or set_ego_motion(True)")
         S, h, w = self.n_streams, self.height, self.width
         shape = tuple(frames.shape)
         tail = (h, w, 3) if self.bgr else (h, w)
@@ -175,6 +191,7 @@ class StreamTracker:
         if v_prior is not None:
             v_prior = np.ascontiguousarray(v_prior, dtype=np.float64).reshape(S, 3)
         res = np.zeros(S, _lib.TRACK_RESULT_DTYPE)
+        ego = np.zeros(S, _lib.EGO_RESULT_DTYPE) if want_ego else None
         pts = cnt = kp = kn = None
         if want_points:
             pts = np.zeros((S, self.capacity, 2), np.float32)
@@ -182,15 +199,17 @@ class StreamTracker:
         if want_kept:
             kp = np.zeros((S, self.capacity, 2), np.float32)
             kn = np.zeros((S, self.capacity, 2), np.float32)
-        _lib.check(self.ctx.lib.ofb_tracker_step(self.h, _lib.ptr(frames), bpp * w, bpp * w * h, _lib.ptr(imu),
-                                                 _lib.ptr(v_prior), _lib.ptr(res), _lib.ptr(pts), _lib.ptr(cnt),
-                                                 _lib.ptr(kp), _lib.ptr(kn)))
+        _lib.check(self.ctx.lib.ofb_tracker_step_ego(self.h, _lib.ptr(frames), bpp * w, bpp * w * h, _lib.ptr(imu),
+                                                     _lib.ptr(v_prior), _lib.ptr(res), _lib.ptr(pts), _lib.ptr(cnt),
+                                                     _lib.ptr(kp), _lib.ptr(kn), _lib.ptr(ego)))
         out = [res]
         if want_points:
             out.append([pts[s, :cnt[s]].reshape(-1, 1, 2).copy() for s in range(S)])
         if want_kept:
             out.append([kp[s, :res["n_kept"][s]].copy() for s in range(S)])
             out.append([kn[s, :res["n_kept"][s]].copy() for s in range(S)])
+        if want_ego:
+            out.append(ego)
         return out[0] if len(out) == 1 else tuple(out)
 
 
@@ -257,6 +276,13 @@ class FleetTracker:
         on = bool(_gyro_flag(enable))
         if self.local is not None:
             self.local.set_gyro_prediction(on)
+
+    def set_ego_motion(self, enable):
+        """StreamTracker.set_ego_motion on this rank's streams (ego_motion=True at construction is passed to the local
+        tracker with the other keywords)"""
+        on = _ego_flag(enable)
+        if self.local is not None:
+            self.local.set_ego_motion(on)
 
     def gather_velocities(self):
         """(n_streams, 3) velocities of the last step on every rank; rows of streams that did not solve (or have not

@@ -132,6 +132,53 @@ def solve_lgs_batched(x, u, offsets, d, n, omega, t=None, variant="node", ctx=No
     return v, res, rank, s
 
 
+def _ego_variant(variant):
+    if variant not in _lib.VARIANTS:
+        raise ValueError("ego-motion variant must be one of %s (module has no gyro term)" % sorted(_lib.VARIANTS))
+    return _lib.VARIANTS[variant]
+
+
+def solve_ego_motion(x, u, d, n, t=None, variant="node", ctx=None):
+    """The angular rate estimated from the flow together with the velocity (include/ofb200.h, ofb_solve_ego_motion):
+    np.linalg.lstsq on the 3N x 6 system in (v', omega), v' = v + omega x t. No gyro sample is used.
+    Returns (v (3,), omega (3,), res (1,)|(0,), rank, s (6,)); res follows lstsq (only for rank 6 and 3N > 6)."""
+    var = _ego_variant(variant)
+    x = _pts(x, "x")
+    u = _pts(u, "u")
+    if len(x) != len(u):
+        raise ValueError("x and u must have the same number of rows")
+    n3 = _vec3(n, "n")
+    t3 = _vec3(t, "t") if t is not None else None
+    ctx = ctx or _lib.default_context()
+    rec = np.zeros(1, _lib.EGO_RESULT_DTYPE)
+    _lib.check(ctx.lib.ofb_solve_ego_motion(ctx.h, var, _lib.ptr(x), _lib.ptr(u), len(x), _scalar(d), _lib.ptr(n3),
+                                            _lib.ptr(t3), _lib.ptr(rec)))
+    r = rec[0]
+    res = np.array([r["res"]]) if (r["rank"] == 6 and 3 * len(x) > 6) else np.array([])
+    return r["v"].copy(), r["w"].copy(), res, int(r["rank"]), r["s"].copy()
+
+
+def solve_ego_motion_batched(x, u, offsets, d, n, t=None, variant="node", ctx=None):
+    """Many frames at once, frame f on rows offsets[f]:offsets[f+1] -> _lib.EGO_RESULT_DTYPE records (F,)."""
+    var = _ego_variant(variant)
+    x = _pts(x, "x")
+    u = _pts(u, "u")
+    offsets = np.ascontiguousarray(offsets, dtype=np.int32)
+    F = len(offsets) - 1
+    if F < 1 or offsets[0] < 0 or np.any(np.diff(offsets) < 0):
+        raise ValueError("offsets must be a non-decreasing sequence of at least two non-negative row indices")
+    if len(x) != len(u) or len(x) < offsets[-1]:
+        raise ValueError("x and u must have the same number of rows, at least offsets[-1] = %d" % offsets[-1])
+    d = np.ascontiguousarray(np.broadcast_to(np.asarray(d, dtype=np.float64).reshape(-1), (F,)))
+    n3 = np.ascontiguousarray(np.broadcast_to(np.asarray(n, dtype=np.float64), (F, 3)))
+    t3 = None if t is None else np.ascontiguousarray(np.broadcast_to(np.asarray(t, dtype=np.float64), (F, 3)))
+    out = np.zeros(F, _lib.EGO_RESULT_DTYPE)
+    ctx = ctx or _lib.default_context()
+    _lib.check(ctx.lib.ofb_solve_ego_motion_batched(ctx.h, var, _lib.ptr(x), _lib.ptr(u), _lib.ptr(offsets), F, _lib.ptr(d),
+                                                    _lib.ptr(n3), _lib.ptr(t3), _lib.ptr(out)))
+    return out
+
+
 def generate_test_data(x, v, omega, d, n, t=None, ctx=None):
     ctx = ctx or _lib.default_context()
     x = _pts(x, "x")

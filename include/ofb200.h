@@ -144,6 +144,33 @@ int ofb_solve_velocity_batched(ofb_ctx* ctx, int variant, const double* x, const
 int ofb_solve_velocity_module(ofb_ctx* ctx, const double* x, const double* u, int n, int ld, const double* dist,
                               const double n3[3], const double* v_prior,
                               double v_out[3], double* res, int* rank, double s_out[3]);
+/* ---- ego-motion solve: the angular rate estimated from the flow together with the velocity, instead of taken from the
+ *      gyro. For a plane at height d with normal n the flow model is linear in (v', w) together, v' = v + w x t:
+ *        X = (x, y, 1), C = [X]x, P = |X|^2 I - X X^T (= C^T C), u3 = (ux, uy, 0)
+ *        A_i = [ wA C , d wb P ],  b_i = d wb C u3
+ *        SIM: wA = n.X, wb = 1;   NODE / EXP: wA = 1, wb = 1 / (n.X)      (the weights of ofb_solve_velocity)
+ *      solved as np.linalg.lstsq on the stacked 3N x 6 system: the pseudo-inverse over the eigenpairs of A^T A that pass
+ *      the rank rule of ofb_solve_velocity (s_k > eps * max(3N, 6) * s_max, the factor floored at 1e-7). Then v = v' - w x t
+ *      for EXP and SIM (NODE has no lever arm). imu.w - w is the gyro's error: bias, or an IMU sample taken at another time
+ *      than the frame. The model is instantaneous: at rotations of ~0.1 rad per frame the second-order rotational flow
+ *      biases w by several percent and goes into the velocity. MODULE (no gyro term) returns OFB_E_INVALID. */
+#define OFB_EGO_SOLVED 1            /* ofb_ego_result.flags: the solve ran for this frame (tracker: as OFB_TRACK_SOLVED) */
+typedef struct {
+    double v[3];     /* velocity, lever arm removed with the estimated rate */
+    double w[3];     /* estimated angular rate */
+    double s[6];     /* singular values of A, descending */
+    double res;      /* sum of squared residuals of the 3N x 6 system (as lstsq: meaningful when rank == 6 and 3N > 6) */
+    int    rank;
+    int    flags;    /* OFB_EGO_* */
+} ofb_ego_result;
+/* x, u: n x 2 float64 (host or device), d: height, n3: plane normal, t3: lever arm (may be NULL: zero); out: one record */
+int ofb_solve_ego_motion(ofb_ctx* ctx, int variant, const double* x, const double* u, int n, double d,
+                         const double n3[3], const double t3[3], ofb_ego_result* out);
+/* n_frames problems as ofb_solve_velocity_batched (offsets may be device memory); d[n_frames], n3 / t3 n_frames x 3,
+ * out[n_frames] */
+int ofb_solve_ego_motion_batched(ofb_ctx* ctx, int variant, const double* x, const double* u, const int* offsets,
+                                 int n_frames, const double* d, const double* n3, const double* t3, ofb_ego_result* out);
+
 /* generate_test_data: simulation.py:7-12 (t3 != NULL) / velocity_measurment_node:25-29 (t3 NULL) */
 int ofb_generate_flow(ofb_ctx* ctx, const double* x, int n, const double v3[3], const double w3[3],
                       double d, const double n3[3], const double* t3, double* u_out);
@@ -288,6 +315,14 @@ int ofb_frame_pairs_gyro(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera
                          int n_pairs, const uint8_t* prev, const uint8_t* next, int pitch, size_t image_stride,
                          const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
                          ofb_pair_result* results, float* prev_pts, float* next_pts, uint8_t* status);
+/* ofb_frame_pairs_gyro plus the ego-motion solve (see ofb_solve_ego_motion) of every pair: ego[n_pairs] (host or device)
+ * from the same tracked points as the pair's velocity solve (status 1 after the forward-backward check, undistorted when
+ * cam is set), in the same kernel. ego == NULL is exactly ofb_frame_pairs_gyro; the results and tracks do not depend
+ * on it. */
+int ofb_frame_pairs_ego(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, double fb_max_err, int gyro_predict,
+                        int n_pairs, const uint8_t* prev, const uint8_t* next, int pitch, size_t image_stride,
+                        const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
+                        ofb_pair_result* results, ofb_ego_result* ego, float* prev_pts, float* next_pts, uint8_t* status);
 
 /* ---- feature lifecycle around the tracker (SURVEY 8f-2): the point set of every camera stream stays on the
  *      device between frames. One step does what the reference's per-frame loops do around the tracker
@@ -397,6 +432,16 @@ int ofb_tracker_set_fb_check(ofb_tracker* trk, double fb_max_err);
  * IMU sample w, with the tracker's camera when one is set and the pinhole of its configuration otherwise; 0 turns it off
  * (the default). A change rebuilds the captured CUDA graphs. */
 int ofb_tracker_set_gyro_prediction(ofb_tracker* trk, int enable);
+/* Ego-motion solve (see ofb_solve_ego_motion) of every stream from the next ofb_tracker_step on, on the kept points,
+ * right after the velocity solve and under the same condition (the record is zero with flags 0 when the stream did not
+ * solve). The standard records, tracks and point sets do not change. MODULE trackers return OFB_E_INVALID. A change
+ * rebuilds the captured CUDA graphs. 0 turns it off (the default). */
+int ofb_tracker_set_ego_motion(ofb_tracker* trk, int enable);
+/* ofb_tracker_step plus ego[n_streams] (host or device, may be NULL): the step's ego-motion records. ego != NULL needs
+ * ofb_tracker_set_ego_motion(trk, 1). The records complete under the rule of the result records. */
+int ofb_tracker_step_ego(ofb_tracker* trk, const uint8_t* frames, int pitch, size_t image_stride,
+                         const ofb_imu_sample* imu, const double* v_prior, ofb_track_result* results,
+                         float* pts_out, int* n_out, float* kept_prev, float* kept_next, ofb_ego_result* ego);
 /* the exclusion mask OFB_TOPUP_APPEND_MASKED would use for `n` points (n x 2 float32): mask_out h x w u8
  * (1 = allowed, 0 = inside a circle). Exposed for parity tests against cv2.circle. */
 int ofb_tracker_render_mask(ofb_ctx* ctx, const float* pts, int n, int radius, int w, int h, uint8_t* mask_out);

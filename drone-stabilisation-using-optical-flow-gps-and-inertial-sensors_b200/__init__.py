@@ -16,7 +16,8 @@ from ._lib import Context, OfbError, default_context
 from . import of_library, velocity, vision, simulation, tracker, replay
 from .of_library import pix_trans, r_tilde, static_immobile, initialize_ft
 from .velocity import (solve_lgs, solve_full, solve_lgs_batched, solve_lgs_module, generate_test_data, feasibility,
-                       quaternion_to_rotation, plane_normal, body_to_world, solve_ego_motion, solve_ego_motion_batched)
+                       quaternion_to_rotation, plane_normal, body_to_world, solve_ego_motion, solve_ego_motion_batched,
+                       solve_velocity_robust, solve_velocity_robust_batched)
 from .vision import (goodFeaturesToTrack, calcOpticalFlowPyrLK, cornerMinEigenVal, buildPyramid, pyrDown, cvtColor,
                      Pyramid, make_pair_cfg, frame_pairs, frame_sequence, COLOR_BGR2GRAY, TERM_CRITERIA_COUNT, TERM_CRITERIA_EPS,
                      undistortPoints, undistortPointsIter, make_camera, CAMERA_ITERATIONS, track_forward_backward,

@@ -66,6 +66,15 @@ class EgoResult(C.Structure):
                 ("rank", C.c_int), ("flags", C.c_int)]
 
 
+class RobustCfg(C.Structure):
+    _fields_ = [("c", C.c_double), ("iterations", C.c_int)]
+
+
+class RobustResult(C.Structure):
+    _fields_ = [("v", C.c_double * 3), ("s", C.c_double * 3), ("res", C.c_double), ("scale", C.c_double),
+                ("rank", C.c_int), ("n_inliers", C.c_int), ("iterations", C.c_int), ("flags", C.c_int)]
+
+
 class McStep(C.Structure):
     _fields_ = [("v", C.c_double * 3), ("w", C.c_double * 3), ("n", C.c_double * 3), ("t", C.c_double * 3),
                 ("height", C.c_double),
@@ -88,6 +97,10 @@ TRACK_RESULT_DTYPE = np.dtype([("v", "<f8", 3), ("s", "<f8", 3), ("res", "<f8"),
 EGO_RESULT_DTYPE = np.dtype([("v", "<f8", 3), ("w", "<f8", 3), ("s", "<f8", 6), ("res", "<f8"), ("rank", "<i4"),
                              ("flags", "<i4")], align=True)
 EGO_SOLVED = 1
+ROBUST_RESULT_DTYPE = np.dtype([("v", "<f8", 3), ("s", "<f8", 3), ("res", "<f8"), ("scale", "<f8"), ("rank", "<i4"),
+                                ("n_inliers", "<i4"), ("iterations", "<i4"), ("flags", "<i4")], align=True)
+ROBUST_SOLVED = 1
+ROBUST_DEFAULT_C, ROBUST_DEFAULT_ITERATIONS = 4.0, 10
 TOPUP_APPEND_MASKED, TOPUP_APPEND, TOPUP_REPLACE = 0, 1, 2
 TOPUP_MODES = {"node": TOPUP_APPEND_MASKED, "exp": TOPUP_APPEND, "module": TOPUP_REPLACE}
 GATE_NONE, GATE_R_GE, GATE_R_LE = 0, 1, 2
@@ -160,6 +173,12 @@ _SIGNATURES = {
                                   vp, vp]),
     "ofb_tracker_set_ego_motion": (i32, [vp, i32]),
     "ofb_tracker_step_ego": (i32, [vp, vp, i32, sz, vp, vp, vp, vp, vp, vp, vp, vp]),
+    "ofb_solve_velocity_robust": (i32, [vp, i32, vp, vp, i32, f64, vp, vp, vp, C.POINTER(RobustCfg), vp, vp]),
+    "ofb_solve_velocity_robust_batched": (i32, [vp, i32, vp, vp, vp, i32, vp, vp, vp, vp, C.POINTER(RobustCfg), vp, vp]),
+    "ofb_frame_pairs_robust": (i32, [vp, C.POINTER(PairCfg), C.POINTER(Camera), f64, i32, i32, vp, vp, i32, sz, vp, vp, vp, vp, vp,
+                                     C.POINTER(RobustCfg), vp, vp, vp, vp]),
+    "ofb_tracker_set_robust": (i32, [vp, C.POINTER(RobustCfg)]),
+    "ofb_tracker_step_robust": (i32, [vp, vp, i32, sz, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
     "ofb_mc_sweep": (i32, [vp, vp, i32, i32, vp, vp, i32, u64, u64, u64, i32, vp, vp, vp]),
     "ofb_mc_sweep_multi": (i32, [vp, i32, vp, i32, i32, vp, vp, i32, u64, u64, u64, i32, vp]),
     "ofb_mc_feas": (i32, [vp, vp, i32, vp, vp, u64, u64, u64, vp]),
@@ -194,6 +213,31 @@ def check(rc):
     if rc == OFB_E_NOMEM:
         raise MemoryError(msg)
     raise OfbError("libofb200 error %d: %s" % (rc, msg))
+
+
+def robust_cfg(robust):
+    """The robust-solve setting from its Python forms: None / False -> None (off), True -> the defaults (c = 4, 10
+    iterations), (c, iterations) -> those. Raises ValueError for anything else, c not finite or < 1.5, or iterations
+    outside 0..64."""
+    if robust is None or robust is False or (isinstance(robust, np.bool_) and not robust):
+        return None
+    if robust is True or isinstance(robust, np.bool_):
+        c, k = ROBUST_DEFAULT_C, ROBUST_DEFAULT_ITERATIONS
+    else:
+        try:
+            c, k = robust
+        except (TypeError, ValueError):
+            raise ValueError("robust must be None, False, True or (c, iterations), got %r" % (robust,)) from None
+    if isinstance(c, (bool, np.bool_)) or not isinstance(c, (int, float, np.integer, np.floating)):
+        raise ValueError("robust c must be a number, got %r" % (c,))
+    if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)):
+        raise ValueError("robust iterations must be an integer, got %r" % (k,))
+    c, k = float(c), int(k)
+    if not (np.isfinite(c) and c >= 1.5):
+        raise ValueError("robust c must be finite and >= 1.5, got %r" % c)
+    if not 0 <= k <= 64:
+        raise ValueError("robust iterations must be in 0..64, got %d" % k)
+    return RobustCfg(c, k)
 
 
 def ptr(a):

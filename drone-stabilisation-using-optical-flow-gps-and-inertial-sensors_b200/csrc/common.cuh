@@ -87,7 +87,7 @@ struct PinBuf {
 #define OFB_DEV_ASSERT(c) ((void)0)
 #endif
 
-enum { OFB_NSCRATCH = 26, OFB_NSTAGES = 5, OFB_NSTAGE_EV = 6, OFB_NFUNC_SLOTS = 32 };
+enum { OFB_NSCRATCH = 27, OFB_NSTAGES = 5, OFB_NSTAGE_EV = 6, OFB_NFUNC_SLOTS = 32 };
 
 struct ofb_ctx {
     int device = 0;
@@ -141,7 +141,8 @@ enum {
     SC_MC0, SC_MC1, SC_MC2, SC_TMP0, SC_TMP1,
     SC_FRAMES,                                               // device staging of host frames (ofb_frame_pairs)
     SC_CALIB,                                                // calibrated tracks of ofb_frame_pairs_cam
-    SC_EGO                                                   // staged ego-motion records (frame pairs, tracker)
+    SC_EGO,                                                  // staged ego-motion records (frame pairs, tracker)
+    SC_ROBUST                                                // staged robust velocity records (frame pairs, tracker)
 };
 
 struct ofb_pyr {

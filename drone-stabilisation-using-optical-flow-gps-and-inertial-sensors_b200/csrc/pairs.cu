@@ -62,21 +62,43 @@ __device__ __forceinline__ void pair_solve(const Loader& ld, int variant, const 
     }
 }
 
-template <bool EGO>
+// ROBUST: pair_solve, then the robust velocity solve of the pair on the same points (rob[f]). The ROBUST kernels see their
+// loader through a type of their own: the solve functions they instantiate, and the shared arrays inside them, are then
+// not shared with the ROBUST = false kernels, which keep their machine code.
+template <class L> struct RobustPass : L {};
+
+template <bool EGO, class Loader>
+__device__ __forceinline__ void pair_solve_robust(const Loader& ld, int variant, const ofb_imu_sample* __restrict__ imu,
+                                                  ofb_pair_result* __restrict__ out, const FeatImageState* __restrict__ det,
+                                                  ofb_ego_result* __restrict__ ego, const ofb_robust_cfg& rcfg,
+                                                  ofb_robust_result* __restrict__ rob)
+{
+    const RobustPass<Loader> rl{ld};
+    pair_solve<EGO>(rl, variant, imu, out, det, ego);
+    const int f = blockIdx.x;
+    const ofb_imu_sample& s = imu[f];
+    const OfbRobustOut r = ofb_block_solve_robust(rl, f, variant, s.d, s.n, s.w, s.t, rcfg.c, rcfg.iterations);
+    if (threadIdx.x == 0) rob[f] = ofb_robust_record(r, OFB_ROBUST_SOLVED);
+}
+
+template <bool EGO, bool ROBUST = false>
 __global__ void __launch_bounds__(OFB_SOLVE_THREADS)
 pair_solve_kernel(TrackLoader ld, int variant, const ofb_imu_sample* __restrict__ imu, ofb_pair_result* __restrict__ out,
-                  const FeatImageState* __restrict__ det, ofb_ego_result* __restrict__ ego)
+                  const FeatImageState* __restrict__ det, ofb_ego_result* __restrict__ ego, ofb_robust_cfg rcfg,
+                  ofb_robust_result* __restrict__ rob)
 {
-    pair_solve<EGO>(ld, variant, imu, out, det, ego);
+    if constexpr (ROBUST) pair_solve_robust<EGO>(ld, variant, imu, out, det, ego, rcfg, rob);
+    else pair_solve<EGO>(ld, variant, imu, out, det, ego);
 }
 
 // With a calibrated camera: every tracked point is undistorted once into xu (the solve reads each point twice), then
 // solved from there.
-template <bool EGO>
+template <bool EGO, bool ROBUST = false>
 __global__ void __launch_bounds__(OFB_SOLVE_THREADS)
 pair_solve_cam_kernel(TrackLoader tl, ofb_camera cam, double4* __restrict__ xu, int variant,
                       const ofb_imu_sample* __restrict__ imu, ofb_pair_result* __restrict__ out,
-                      const FeatImageState* __restrict__ det, ofb_ego_result* __restrict__ ego)
+                      const FeatImageState* __restrict__ det, ofb_ego_result* __restrict__ ego, ofb_robust_cfg rcfg,
+                      ofb_robust_result* __restrict__ rob)
 {
     const int f = blockIdx.x, n = tl.end(f);
     for (int i = threadIdx.x; i < n; i += blockDim.x) {
@@ -84,20 +106,25 @@ pair_solve_cam_kernel(TrackLoader tl, ofb_camera cam, double4* __restrict__ xu, 
         if (tl.status[o]) xu[o] = ofb_calibrate(cam, tl.next[2 * o], tl.next[2 * o + 1], tl.prev[2 * o], tl.prev[2 * o + 1]);
     }
     __syncthreads();
-    pair_solve<EGO>(CalibLoader{xu, tl.stride, tl.status, tl.counts, tl.counts_stride, 0}, variant, imu, out, det, ego);
+    if constexpr (ROBUST)
+        pair_solve_robust<EGO>(CalibLoader{xu, tl.stride, tl.status, tl.counts, tl.counts_stride, 0}, variant, imu, out, det, ego,
+                               rcfg, rob);
+    else pair_solve<EGO>(CalibLoader{xu, tl.stride, tl.status, tl.counts, tl.counts_stride, 0}, variant, imu, out, det, ego);
 }
 
 }  // namespace
 
 // Stages 1b-4 for pairs [c0, c0+n) whose level-0 frames already sit in pp/pn (images 0..n-1 of each).
 // gyro (NULL: off): the pinhole model of the gyro prediction, with dcam the device copy of the camera (NULL: pinhole).
-// d_ego (NULL: off): the pairs' ego-motion records, solved in the velocity solve's kernel.
+// d_ego (NULL: off): the pairs' ego-motion records, solved in the velocity solve's kernel; d_rob (NULL: off) likewise
+// the robust records under rcfg.
 // Sequence layout (pn == pp): pp holds n+1 consecutive frames of one stream, pair i = (image i, image i+1), so every
 // interior frame's pyramid is built once and serves as "next" of one pair and "prev" of the following one.
 static int run_pairs_chunk(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, double fb_max_err,
                            const GyroPinhole* gyro, const ofb_camera* dcam, ofb_pyr* pp, ofb_pyr* pn, int n, int c0,
                            const ofb_imu_sample* dimu, const int* counts_in, float* d_prev, float* d_next, uint8_t* d_stat,
-                           ofb_pair_result* d_res, ofb_ego_result* d_ego, bool mark)
+                           ofb_pair_result* d_res, ofb_ego_result* d_ego, const ofb_robust_cfg& rcfg, ofb_robust_result* d_rob,
+                           bool mark)
 {
     const bool seq = pn == pp;
     const int w = cfg->width, h = cfg->height, K = cfg->max_corners;
@@ -168,14 +195,17 @@ static int run_pairs_chunk(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_came
     STAGE_MARK(4);
     TrackLoader ld{cp, cn, cs, counts, counts_stride, (size_t)K, cfg->cx, cfg->cy, cfg->pos_scale, cfg->flow_scale};
     ofb_ego_result* ego = d_ego ? d_ego + c0 : nullptr;
+    ofb_robust_result* rob = d_rob ? d_rob + c0 : nullptr;
     if (cam) {
         OFB_TRY(ctx->scratch[SC_CALIB].reserve(sizeof(double4) * (size_t)n * K));
-        auto kern = d_ego ? pair_solve_cam_kernel<true> : pair_solve_cam_kernel<false>;
+        auto kern = d_ego ? (d_rob ? pair_solve_cam_kernel<true, true> : pair_solve_cam_kernel<true>)
+                          : (d_rob ? pair_solve_cam_kernel<false, true> : pair_solve_cam_kernel<false>);
         kern<<<n, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, *cam, ctx->scratch[SC_CALIB].as<double4>(), cfg->variant, dimu + c0,
-                                                       d_res + c0, st, ego);
+                                                       d_res + c0, st, ego, rcfg, rob);
     } else {
-        auto kern = d_ego ? pair_solve_kernel<true> : pair_solve_kernel<false>;
-        kern<<<n, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, cfg->variant, dimu + c0, d_res + c0, st, ego);
+        auto kern = d_ego ? (d_rob ? pair_solve_kernel<true, true> : pair_solve_kernel<true>)
+                          : (d_rob ? pair_solve_kernel<false, true> : pair_solve_kernel<false>);
+        kern<<<n, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, cfg->variant, dimu + c0, d_res + c0, st, ego, rcfg, rob);
     }
     OFB_LAUNCH_CHECK(ctx);
     STAGE_MARK(5);
@@ -225,7 +255,23 @@ extern "C" int ofb_frame_pairs_ego(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const 
                                    ofb_pair_result* results, ofb_ego_result* ego, float* prev_pts, float* next_pts,
                                    uint8_t* status)
 {
+    return ofb_frame_pairs_robust(ctx, cfg, cam, fb_max_err, gyro_predict, n_pairs, prev, next, pitch, image_stride, imu, pts_in,
+                                  n_in, results, ego, nullptr, nullptr, prev_pts, next_pts, status);
+}
+
+extern "C" int ofb_frame_pairs_robust(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, double fb_max_err,
+                                      int gyro_predict, int n_pairs, const uint8_t* prev, const uint8_t* next, int pitch,
+                                      size_t image_stride, const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
+                                      ofb_pair_result* results, ofb_ego_result* ego, const ofb_robust_cfg* robust,
+                                      ofb_robust_result* rob, float* prev_pts, float* next_pts, uint8_t* status)
+{
     OFB_REQUIRE(ctx && cfg && prev && next && imu && results, "frame_pairs: null argument");
+    ofb_robust_cfg rcfg{0.0, 0};
+    if (rob) {
+        OFB_REQUIRE(cfg->variant >= 0 && cfg->variant <= 2, "frame_pairs: unknown variant");
+        OFB_TRY(ofb_robust_check(robust, "frame_pairs"));
+        rcfg = *robust;
+    }
     if (cam) OFB_TRY(ofb_camera_check(cam, "frame_pairs"));
     OFB_REQUIRE(ofb_fb_thr_ok(fb_max_err), "frame_pairs: fb_max_err must be >= 0 (0 = no forward-backward check)");
     GyroPinhole gph{0.0, 0.0, 0.0, 0.0};
@@ -240,12 +286,13 @@ extern "C" int ofb_frame_pairs_ego(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const 
     OFB_REQUIRE(n_pairs == 1 || image_stride >= (size_t)pitch * (h - 1) + w, "frame_pairs: image_stride too small");
     OFB_CUDA(cudaSetDevice(ctx->device));
     const size_t npts = (size_t)n_pairs * K;
-    OutStage o[5];
+    OutStage o[6];
     OFB_TRY(ofb_stage_out(ctx, SC_PTS0, prev_pts, sizeof(float) * 2 * npts, &o[0]));
     OFB_TRY(ofb_stage_out(ctx, SC_PTS1, next_pts, sizeof(float) * 2 * npts, &o[1]));
     OFB_TRY(ofb_stage_out(ctx, SC_STAT, status, npts, &o[2]));
     OFB_TRY(ofb_stage_out(ctx, SC_OUT3, results, sizeof(ofb_pair_result) * n_pairs, &o[3]));
     OFB_TRY(ofb_stage_out(ctx, SC_EGO, ego, sizeof(ofb_ego_result) * n_pairs, &o[4]));
+    OFB_TRY(ofb_stage_out(ctx, SC_ROBUST, rob, sizeof(ofb_robust_result) * n_pairs, &o[5]));
     // optional outputs still need device storage when the caller passes NULL
     float* d_prev = (float*)o[0].dev; float* d_next = (float*)o[1].dev; uint8_t* d_stat = (uint8_t*)o[2].dev;
     if (!d_prev) { OFB_TRY(ctx->scratch[SC_PTS0].reserve(sizeof(float) * 2 * npts)); d_prev = ctx->scratch[SC_PTS0].as<float>(); }
@@ -355,14 +402,14 @@ extern "C" int ofb_frame_pairs_ego(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const 
         OFB_TRY(run_pairs_chunk(c, cfg, cam, fb_max_err, gyro_predict ? &gph : nullptr, (const ofb_camera*)dcam,
                                 c->pair_pyr[slot][0], seq ? c->pair_pyr[slot][0] : c->pair_pyr[slot][1], n, c0,
                                 (const ofb_imu_sample*)dimu, counts_in, d_prev, d_next, d_stat, (ofb_pair_result*)o[3].dev,
-                                (ofb_ego_result*)o[4].dev, ctx->profile));
+                                (ofb_ego_result*)o[4].dev, rcfg, (ofb_robust_result*)o[5].dev, ctx->profile));
     }
     if (use_twin) {
         ctx->launches += tw->launches - tw0;
         OFB_CUDA(cudaEventRecord(ctx->ev_twin_join, tw->stream));
         OFB_CUDA(cudaStreamWaitEvent(ctx->stream, ctx->ev_twin_join, 0));
     }
-    int rc = ofb_finish_out(ctx, o, ego ? 5 : 4);
+    int rc = ofb_finish_out(ctx, o, 6);
     if (rc == OFB_OK && ctx->profile) {
         // stage order: 0 pyramids, 1 lambda_min+NMS, 2 ordered selection, 3 LK, 4 solve
         OFB_CUDA(cudaEventSynchronize(ctx->stage_ev[5]));

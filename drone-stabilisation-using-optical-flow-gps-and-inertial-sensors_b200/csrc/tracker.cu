@@ -74,6 +74,11 @@ struct ofb_tracker {
     // step is enqueued, so a change drops the captured graphs; records the caller did not ask for go to ego_buf
     bool ego = false;
     DevBuf ego_buf;
+    // robust velocity solve after them (ofb_tracker_set_robust), as ego: the setting is a kernel argument, so any change
+    // drops the captured graphs; records the caller did not ask for go to rob_buf
+    bool robust = false;
+    ofb_robust_cfg rcfg = {0.0, 0};
+    DevBuf rob_buf;
     uint64_t graph_steps = 0;
 };
 
@@ -126,15 +131,17 @@ __device__ __forceinline__ double r_tilde_point(double px, double py, double ux,
 }
 
 // EGO: the ego-motion solve of the stream follows the velocity solve on the same kept points (ego[s], zero with flags 0
-// when the stream did not solve); EGO = false is the velocity solve alone.
+// when the stream did not solve); ROBUST: then the robust velocity solve under rcfg (rob[s], likewise). Both false is
+// the velocity solve alone.
 // PART 0: filter + solve in one launch. PART 1: the filter alone (compaction, gates, counts, top-up decision -- all the next
 // step's LK needs); PART 2: the solve of a stream an earlier PART 1 launch compacted. The split lets the solve run beside
 // the next frame's LK on a stream of its own: nothing but the NEXT filter (its r_tilde gate uses the solved velocity) and
 // the reader of the result record depend on it.
-template <int PART, bool EGO = false>
+template <int PART, bool EGO = false, bool ROBUST = false>
 __global__ void __launch_bounds__(OFB_SOLVE_THREADS)
 track_filter_solve_kernel(TrackerDev T, const ofb_imu_sample* __restrict__ imu, const double* __restrict__ v_prior,
-                          ofb_track_result* __restrict__ out, ofb_ego_result* __restrict__ ego)
+                          ofb_track_result* __restrict__ out, ofb_ego_result* __restrict__ ego, ofb_robust_cfg rcfg,
+                          ofb_robust_result* __restrict__ rob)
 {
     const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     __shared__ int wtot[OFB_SOLVE_THREADS / 32];
@@ -237,6 +244,16 @@ track_filter_solve_kernel(TrackerDev T, const ofb_imu_sample* __restrict__ imu, 
             e = ofb_block_solve_ego(ld, s, T.variant, im.d, im.n, im.t);
         }
     }
+    OfbRobustOut rb;
+    if (ROBUST && PART != 1 && solve) {
+        if (T.cam) {
+            rb = ofb_block_solve_robust(CalibLoader{T.calib, (size_t)T.cap, nullptr, nullptr, 0, kept}, s, T.variant, im.d, im.n, im.w,
+                                        im.t, rcfg.c, rcfg.iterations);
+        } else {
+            KeptLoader ld{T.kept_prev, T.kept_next, kept, (size_t)T.cap, T.cx, T.cy, T.ps, T.fs};
+            rb = ofb_block_solve_robust(ld, s, T.variant, im.d, im.n, im.w, im.t, rcfg.c, rcfg.iterations);
+        }
+    }
     // the detector's per-image state and (for streams that will top up) its min-distance cell grid start clean
     if (PART != 2 && kept <= T.min_features)
         for (size_t i = tid; i < T.cell_stride; i += OFB_SOLVE_THREADS) T.cell_grid[(size_t)s * T.cell_stride + i] = -1;
@@ -250,6 +267,10 @@ track_filter_solve_kernel(TrackerDev T, const ofb_imu_sample* __restrict__ imu, 
             if (EGO) {
                 if (solve) ego[s] = ofb_ego_record(e, OFB_EGO_SOLVED);
                 else { ofb_ego_result z = {}; ego[s] = z; }
+            }
+            if (ROBUST) {
+                if (solve) rob[s] = ofb_robust_record(rb, OFB_ROBUST_SOLVED);
+                else { ofb_robust_result z = {}; rob[s] = z; }
             }
         }
         if (PART != 2) {
@@ -471,7 +492,7 @@ extern "C" int ofb_tracker_destroy(ofb_tracker* t)
     if (t->ev_lk) cudaEventDestroy(t->ev_lk);
     if (t->ev_pyr) cudaEventDestroy(t->ev_pyr);
     DevBuf* bufs[] = {&t->counts, &t->nxt, &t->status, &t->err, &t->kept_prev, &t->det, &t->vlast, &t->mask, &t->hw, &t->bgr, &t->dev_io,
-                      &t->cam_dev, &t->calib, &t->ego_buf};
+                      &t->cam_dev, &t->calib, &t->ego_buf, &t->rob_buf};
     for (DevBuf* b : bufs) b->release();
     delete t;
     return OFB_OK;
@@ -523,21 +544,28 @@ static cudaError_t tracker_join_solve(ofb_tracker* t)
 // One step, launch by launch, on ctx->stream (also the body that is captured into a graph).
 static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitch, size_t image_stride,
                                  const ofb_imu_sample* imu, const double* v_prior, ofb_track_result* results,
-                                 float* pts_out, int* n_out, float* kept_prev, float* kept_next, ofb_ego_result* ego)
+                                 float* pts_out, int* n_out, float* kept_prev, float* kept_next, ofb_ego_result* ego,
+                                 ofb_robust_result* rob)
 {
     ofb_ctx* ctx = t->ctx;
     const ofb_tracker_cfg& cfg = t->cfg;
     const ofb_pair_cfg& pc = cfg.pair;
     const int S = cfg.n_streams, w = pc.width, h = pc.height, K = pc.max_corners, cap = t->cap;
     const size_t np = (size_t)S * cap;
-    OutStage o[3];
+    OutStage o[4];
     OFB_TRY(ofb_stage_out(ctx, SC_OUT3, results, sizeof(ofb_track_result) * S, &o[0]));
     OFB_TRY(ofb_stage_out(ctx, SC_OUT2, n_out, sizeof(int) * S, &o[1]));
     OFB_TRY(ofb_stage_out(ctx, SC_EGO, ego, sizeof(ofb_ego_result) * S, &o[2]));
+    OFB_TRY(ofb_stage_out(ctx, SC_ROBUST, rob, sizeof(ofb_robust_result) * S, &o[3]));
     ofb_ego_result* d_ego = (ofb_ego_result*)o[2].dev;
     if (t->ego && !d_ego) {
         OFB_TRY(t->ego_buf.reserve(sizeof(ofb_ego_result) * S));
         d_ego = t->ego_buf.as<ofb_ego_result>();
+    }
+    ofb_robust_result* d_rob = (ofb_robust_result*)o[3].dev;
+    if (t->robust && !d_rob) {
+        OFB_TRY(t->rob_buf.reserve(sizeof(ofb_robust_result) * S));
+        d_rob = t->rob_buf.as<ofb_robust_result>();
     }
     const void *dimu, *dvp = nullptr;
     OFB_TRY(ofb_stage_in(ctx, SC_IN3, imu, sizeof(ofb_imu_sample) * S, &dimu));
@@ -656,7 +684,7 @@ static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitc
     {
         const char* se = getenv("OFB_TRACKER_SPLIT_SOLVE");
         split = early && t->have_prev && ofb_is_device_ptr(results) && ofb_is_device_ptr(imu) && (!v_prior || ofb_is_device_ptr(v_prior)) &&
-                (!ego || ofb_is_device_ptr(ego)) && !(se && se[0] == '0');
+                (!ego || ofb_is_device_ptr(ego)) && (!rob || ofb_is_device_ptr(rob)) && !(se && se[0] == '0');
     }
     if (split) {
         if (!t->sol_stream) {
@@ -667,20 +695,22 @@ static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitc
             ctx->aux_join.push_back(std::make_pair(t->sol_stream, t->ev_sol_join));
         }
         track_filter_solve_kernel<1><<<S, OFB_SOLVE_THREADS, 0, ctx->stream>>>(T, (const ofb_imu_sample*)dimu, (const double*)dvp,
-                                                                               (ofb_track_result*)o[0].dev, nullptr);
+                                                                               (ofb_track_result*)o[0].dev, nullptr, t->rcfg, nullptr);
         OFB_LAUNCH_CHECK(ctx);
         OFB_CUDA(cudaEventRecord(t->ev_filt, ctx->stream));
         OFB_CUDA(cudaStreamWaitEvent(t->sol_stream, t->ev_filt, 0));
-        auto kern = t->ego ? track_filter_solve_kernel<2, true> : track_filter_solve_kernel<2>;
+        auto kern = t->ego ? (t->robust ? track_filter_solve_kernel<2, true, true> : track_filter_solve_kernel<2, true>)
+                           : (t->robust ? track_filter_solve_kernel<2, false, true> : track_filter_solve_kernel<2>);
         kern<<<S, OFB_SOLVE_THREADS, 0, t->sol_stream>>>(T, (const ofb_imu_sample*)dimu, (const double*)dvp, (ofb_track_result*)o[0].dev,
-                                                         d_ego);
+                                                         d_ego, t->rcfg, d_rob);
         OFB_LAUNCH_CHECK(ctx);
         OFB_CUDA(cudaEventRecord(t->ev_sol, t->sol_stream));
         t->sol_pending = true;
     } else {
-        auto kern = t->ego ? track_filter_solve_kernel<0, true> : track_filter_solve_kernel<0>;
+        auto kern = t->ego ? (t->robust ? track_filter_solve_kernel<0, true, true> : track_filter_solve_kernel<0, true>)
+                           : (t->robust ? track_filter_solve_kernel<0, false, true> : track_filter_solve_kernel<0>);
         kern<<<S, OFB_SOLVE_THREADS, 0, ctx->stream>>>(T, (const ofb_imu_sample*)dimu, (const double*)dvp, (ofb_track_result*)o[0].dev,
-                                                       d_ego);
+                                                       d_ego, t->rcfg, d_rob);
         OFB_LAUNCH_CHECK(ctx);
     }
     bool host_out = false;
@@ -720,7 +750,7 @@ static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitc
     t->cur ^= 1;
     t->have_prev = true;
     t->launches_end = ctx->launches; t->async_end = ctx->async_writes;
-    int rc = ofb_finish_out(ctx, o, 3);
+    int rc = ofb_finish_out(ctx, o, 4);
     if (rc == OFB_OK && host_out) OFB_CUDA(cudaStreamSynchronize(ctx->stream));
     return rc;
 }
@@ -737,7 +767,8 @@ static uint64_t scratch_signature(const ofb_ctx* ctx)
 // Steady-state step replayed from a captured CUDA graph. Returns OFB_E_UNSUPPORTED when the graph could not be
 // built (the caller then runs the step launch by launch; nothing has executed and the tracker state is unchanged).
 static int tracker_step_graph(ofb_tracker* t, const uint8_t* frames, int pitch, size_t image_stride,
-                              const ofb_imu_sample* imu, const double* v_prior, ofb_track_result* results, ofb_ego_result* ego)
+                              const ofb_imu_sample* imu, const double* v_prior, ofb_track_result* results, ofb_ego_result* ego,
+                              ofb_robust_result* rob)
 {
     ofb_ctx* ctx = t->ctx;
     const int S = t->cfg.n_streams, w = t->cfg.pair.width, h = t->cfg.pair.height;
@@ -746,10 +777,11 @@ static int tracker_step_graph(ofb_tracker* t, const uint8_t* frames, int pitch, 
     const size_t in_bytes = off_vp + sizeof(double) * 3 * S;
     const size_t d_vp = sizeof(ofb_imu_sample) * S, d_res = d_vp + sizeof(double) * 3 * S;
     const size_t d_ego = d_res + sizeof(ofb_track_result) * S, out_bytes = sizeof(ofb_track_result) * S;
+    const size_t ego_bytes = sizeof(ofb_ego_result) * S, d_rob = d_ego + ego_bytes, rob_bytes = sizeof(ofb_robust_result) * S;
     if (!t->pin_in.p) {                 // fixed sizes: allocated once, the addresses are baked into the graphs
         OFB_TRY(t->pin_in.reserve(in_bytes));
-        OFB_TRY(t->pin_out.reserve(out_bytes + sizeof(ofb_ego_result) * S));    // results | ego records
-        OFB_TRY(t->dev_io.reserve(d_ego + sizeof(ofb_ego_result) * S));
+        OFB_TRY(t->pin_out.reserve(out_bytes + ego_bytes + rob_bytes));    // results | ego records | robust records
+        OFB_TRY(t->dev_io.reserve(d_rob + rob_bytes));
     }
     uint8_t* pin = (uint8_t*)t->pin_in.p;
     uint8_t* dio = t->dev_io.as<uint8_t>();
@@ -779,9 +811,10 @@ static int tracker_step_graph(ofb_tracker* t, const uint8_t* frames, int pitch, 
         if (rc == OFB_OK)
             rc = tracker_step_launches(t, pin, (int)row, fbytes, (const ofb_imu_sample*)dio, v_prior ? (const double*)(dio + d_vp) : nullptr,
                                        (ofb_track_result*)(dio + d_res), nullptr, nullptr, nullptr, nullptr,
-                                       t->ego ? (ofb_ego_result*)(dio + d_ego) : nullptr);
-        // the ego records follow the results in dev_io and pin_out: one copy brings both back
-        const size_t copy_bytes = out_bytes + (t->ego ? sizeof(ofb_ego_result) * S : 0);
+                                       t->ego ? (ofb_ego_result*)(dio + d_ego) : nullptr,
+                                       t->robust ? (ofb_robust_result*)(dio + d_rob) : nullptr);
+        // the ego and robust records follow the results in dev_io and pin_out: one copy brings them all back
+        const size_t copy_bytes = out_bytes + (t->robust ? ego_bytes + rob_bytes : t->ego ? ego_bytes : 0);
         if (rc == OFB_OK && cudaMemcpyAsync(t->pin_out.p, dio + d_res, copy_bytes, cudaMemcpyDeviceToHost,
                                             ctx->stream) != cudaSuccess) rc = OFB_E_CUDA;
         const cudaError_t e = cudaStreamEndCapture(ctx->stream, &g);
@@ -806,7 +839,8 @@ static int tracker_step_graph(ofb_tracker* t, const uint8_t* frames, int pitch, 
     t->pcur ^= 1; t->cur ^= 1; t->graph_steps++;
     OFB_CUDA(cudaStreamSynchronize(ctx->stream));
     memcpy(results, t->pin_out.p, out_bytes);
-    if (ego) memcpy(ego, (const uint8_t*)t->pin_out.p + out_bytes, sizeof(ofb_ego_result) * S);
+    if (ego) memcpy(ego, (const uint8_t*)t->pin_out.p + out_bytes, ego_bytes);
+    if (rob) memcpy(rob, (const uint8_t*)t->pin_out.p + out_bytes + ego_bytes, rob_bytes);
     return OFB_OK;
 }
 
@@ -821,8 +855,18 @@ extern "C" int ofb_tracker_step_ego(ofb_tracker* t, const uint8_t* frames, int p
                                     const ofb_imu_sample* imu, const double* v_prior, ofb_track_result* results,
                                     float* pts_out, int* n_out, float* kept_prev, float* kept_next, ofb_ego_result* ego)
 {
+    return ofb_tracker_step_robust(t, frames, pitch, image_stride, imu, v_prior, results, pts_out, n_out, kept_prev, kept_next, ego,
+                                   nullptr);
+}
+
+extern "C" int ofb_tracker_step_robust(ofb_tracker* t, const uint8_t* frames, int pitch, size_t image_stride,
+                                       const ofb_imu_sample* imu, const double* v_prior, ofb_track_result* results,
+                                       float* pts_out, int* n_out, float* kept_prev, float* kept_next, ofb_ego_result* ego,
+                                       ofb_robust_result* rob)
+{
     OFB_REQUIRE(t && frames && imu && results, "tracker_step: null argument");
     OFB_REQUIRE(!ego || t->ego, "tracker_step: ego records need ofb_tracker_set_ego_motion(trk, 1)");
+    OFB_REQUIRE(!rob || t->robust, "tracker_step: robust records need ofb_tracker_set_robust");
     ofb_ctx* ctx = t->ctx;
     const int S = t->cfg.n_streams, w = t->cfg.pair.width, h = t->cfg.pair.height, bpp = t->cfg.bgr_input ? 3 : 1;
     OFB_REQUIRE(pitch >= bpp * w, "tracker_step: pitch smaller than a row");
@@ -837,13 +881,15 @@ extern "C" int ofb_tracker_step_ego(ofb_tracker* t, const uint8_t* frames, int p
     const bool graphs_on = !(genv && genv[0] == '0');
     if (graphs_on && t->graph_ok && t->have_prev && t->plain_steps >= 3 && !pts_out && !n_out && !kept_prev && !kept_next &&
         (size_t)S * bpp * w * h <= ((size_t)16 << 20) && !ofb_is_device_ptr(frames) && !ofb_is_device_ptr(imu) &&
-        !ofb_is_device_ptr(results) && !(v_prior && ofb_is_device_ptr(v_prior)) && !(ego && ofb_is_device_ptr(ego))) {
-        const int rc = tracker_step_graph(t, frames, pitch, image_stride, imu, v_prior, results, ego);
+        !ofb_is_device_ptr(results) && !(v_prior && ofb_is_device_ptr(v_prior)) && !(ego && ofb_is_device_ptr(ego)) &&
+        !(rob && ofb_is_device_ptr(rob))) {
+        const int rc = tracker_step_graph(t, frames, pitch, image_stride, imu, v_prior, results, ego, rob);
         if (rc != OFB_E_UNSUPPORTED) return rc;
         t->graph_ok = false;            // this build / driver cannot capture the step: stay on plain launches
     }
     t->plain_steps++;
-    return tracker_step_launches(t, frames, pitch, image_stride, imu, v_prior, results, pts_out, n_out, kept_prev, kept_next, ego);
+    return tracker_step_launches(t, frames, pitch, image_stride, imu, v_prior, results, pts_out, n_out, kept_prev, kept_next, ego,
+                                 rob);
 }
 
 extern "C" int ofb_tracker_set_camera(ofb_tracker* t, const ofb_camera* cam)
@@ -918,6 +964,26 @@ extern "C" int ofb_tracker_set_ego_motion(ofb_tracker* t, int enable)
             for (int j = 0; j < 2; ++j)
                 if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
         t->ego = enable != 0;
+    }
+    return OFB_OK;
+}
+
+extern "C" int ofb_tracker_set_robust(ofb_tracker* t, const ofb_robust_cfg* cfg)
+{
+    OFB_REQUIRE(t, "tracker_set_robust: null tracker");
+    if (cfg) {
+        OFB_REQUIRE(t->cfg.pair.variant != OFB_VARIANT_MODULE, "tracker_set_robust: the MODULE variant is not supported");
+        OFB_TRY(ofb_robust_check(cfg, "tracker_set_robust"));
+    }
+    const bool on = cfg != nullptr;
+    if (on != t->robust || (on && (cfg->c != t->rcfg.c || cfg->iterations != t->rcfg.iterations))) {
+        // the kernel and its setting are chosen when a step is enqueued: graphs captured before are rebuilt (no graph is in
+        // flight: a replayed step synchronises before it returns)
+        for (int i = 0; i < 2; ++i)
+            for (int j = 0; j < 2; ++j)
+                if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
+        t->robust = on;
+        t->rcfg = on ? *cfg : ofb_robust_cfg{0.0, 0};
     }
     return OFB_OK;
 }

@@ -60,6 +60,17 @@ solve_ego_kernel(PointsF64 ld, int variant, const double* __restrict__ d_arr, co
     if (threadIdx.x == 0) out[f] = ofb_ego_record(o, OFB_EGO_SOLVED);
 }
 
+__global__ void __launch_bounds__(OFB_SOLVE_THREADS)
+solve_robust_kernel(PointsF64 ld, int variant, const double* __restrict__ d_arr, const double* __restrict__ n_arr,
+                    const double* __restrict__ w_arr, const double* __restrict__ t_arr, ofb_robust_cfg cfg,
+                    ofb_robust_result* __restrict__ out, double* __restrict__ wout)
+{
+    const int f = blockIdx.x;
+    const OfbRobustOut o = ofb_block_solve_robust(ld, f, variant, d_arr[f], n_arr + 3 * (size_t)f, w_arr + 3 * (size_t)f,
+                                                  t_arr ? t_arr + 3 * (size_t)f : nullptr, cfg.c, cfg.iterations, wout);
+    if (threadIdx.x == 0) out[f] = ofb_robust_record(o, OFB_ROBUST_SOLVED);
+}
+
 __global__ void generate_flow_kernel(const double* __restrict__ x, int n, double3 v, double3 w, double d,
                                      double3 nrm, double* __restrict__ u)
 {
@@ -280,6 +291,58 @@ extern "C" int ofb_solve_ego_motion(ofb_ctx* ctx, int variant, const double* x, 
     int offsets[2] = {0, n};
     double dummy[2] = {0, 0};
     return ofb_solve_ego_motion_batched(ctx, variant, n ? x : dummy, n ? u : dummy, offsets, 1, &d, n3, t3, out);
+}
+
+extern "C" int ofb_solve_velocity_robust_batched(ofb_ctx* ctx, int variant, const double* x, const double* u, const int* offsets,
+                                                 int n_frames, const double* d, const double* n3, const double* w3, const double* t3,
+                                                 const ofb_robust_cfg* cfg, ofb_robust_result* out, double* weights_out)
+{
+    OFB_REQUIRE(ctx && x && u && offsets && d && n3 && w3 && out, "solve_velocity_robust_batched: null argument");
+    OFB_REQUIRE(variant >= 0 && variant <= 2, "solve_velocity_robust: unknown variant %d (MODULE is not supported)", variant);
+    OFB_TRY(ofb_robust_check(cfg, "solve_velocity_robust"));
+    OFB_REQUIRE(n_frames > 0, "solve_velocity_robust_batched: n_frames must be positive");
+    OFB_CUDA(cudaSetDevice(ctx->device));
+    std::vector<int> hoff(n_frames + 1);
+    if (ofb_is_device_ptr(offsets)) {
+        OFB_CUDA(cudaMemcpyAsync(hoff.data(), offsets, sizeof(int) * (n_frames + 1), cudaMemcpyDeviceToHost, ctx->stream));
+        OFB_CUDA(cudaStreamSynchronize(ctx->stream));
+    } else memcpy(hoff.data(), offsets, sizeof(int) * (n_frames + 1));
+    OFB_REQUIRE(hoff[0] >= 0, "solve_velocity_robust_batched: offsets[0] = %d is negative", hoff[0]);
+    for (int f = 0; f < n_frames; ++f)
+        OFB_REQUIRE(hoff[f + 1] >= hoff[f], "solve_velocity_robust_batched: offsets must be non-decreasing (offsets[%d] = %d > offsets[%d] = %d)",
+                    f, hoff[f], f + 1, hoff[f + 1]);
+    const int total = hoff[n_frames];
+    const void *dx, *du, *doff, *dd, *dn, *dw, *dt = nullptr;
+    OFB_TRY(ofb_stage_in(ctx, SC_IN0, x, sizeof(double) * 2 * (size_t)total, &dx));
+    OFB_TRY(ofb_stage_in(ctx, SC_IN1, u, sizeof(double) * 2 * (size_t)total, &du));
+    OFB_TRY(ofb_stage_in(ctx, SC_IN2, offsets, sizeof(int) * (n_frames + 1), &doff));
+    OFB_TRY(ofb_stage_in(ctx, SC_IN3, d, sizeof(double) * n_frames, &dd));
+    OFB_TRY(ofb_stage_in(ctx, SC_IN4, n3, sizeof(double) * 3 * n_frames, &dn));
+    OFB_TRY(ofb_stage_in(ctx, SC_IN5, w3, sizeof(double) * 3 * n_frames, &dw));
+    if (t3) OFB_TRY(ofb_stage_in(ctx, SC_TMP0, t3, sizeof(double) * 3 * n_frames, &dt));
+    OutStage o[2];
+    OFB_TRY(ofb_stage_out(ctx, SC_OUT0, out, sizeof(ofb_robust_result) * n_frames, &o[0]));
+    OFB_TRY(ofb_stage_out(ctx, SC_OUT1, weights_out, sizeof(double) * (size_t)total, &o[1]));
+    if (o[1].dev) OFB_CUDA(cudaMemsetAsync(o[1].dev, 0, sizeof(double) * (size_t)total, ctx->stream));   // rows in no frame
+    PointsF64 ld{(const double*)dx, (const double*)du, (const int*)doff, 0};
+    solve_robust_kernel<<<n_frames, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, variant, (const double*)dd, (const double*)dn,
+                                                                          (const double*)dw, (const double*)dt, *cfg,
+                                                                          (ofb_robust_result*)o[0].dev, (double*)o[1].dev);
+    OFB_LAUNCH_CHECK(ctx);
+    return ofb_finish_out(ctx, o, 2);
+}
+
+extern "C" int ofb_solve_velocity_robust(ofb_ctx* ctx, int variant, const double* x, const double* u, int n, double d,
+                                         const double n3[3], const double w3[3], const double t3[3], const ofb_robust_cfg* cfg,
+                                         ofb_robust_result* out, double* weights_out)
+{
+    OFB_REQUIRE(ctx && n3 && w3 && out, "solve_velocity_robust: null argument");
+    OFB_REQUIRE(n >= 0, "solve_velocity_robust: negative point count");
+    OFB_REQUIRE(n == 0 || (x && u), "solve_velocity_robust: null points");
+    int offsets[2] = {0, n};
+    double dummy[2] = {0, 0};
+    return ofb_solve_velocity_robust_batched(ctx, variant, n ? x : dummy, n ? u : dummy, offsets, 1, &d, n3, w3, t3, cfg, out,
+                                             n ? weights_out : nullptr);
 }
 
 extern "C" int ofb_generate_flow(ofb_ctx* ctx, const double* x, int n, const double v3[3], const double w3[3],

@@ -66,6 +66,45 @@ __device__ __forceinline__ void ofb_block_sum(double (&acc)[K], double* smem /* 
     }
 }
 
+// ofb_block_solve's lstsq step and residual term for the robust solve below, which must reproduce the plain solve bit for
+// bit. ofb_block_solve keeps its own inline copy: calling these from it changes its machine code.
+// numpy lstsq (rcond=None) of the normal equations acc[0..5] v = d acc[6..8] (M packed xx, xy, xz, yy, yz, zz) of
+// acc[9] points (3 rows each): sets o.count, o.s and o.rank, returns the solution in v.
+__device__ __forceinline__ void ofb_lstsq3(const double (&acc)[10], double d, OfbSolveOut& o, double (&v)[3])
+{
+    o.count = (int)(acc[9] + 0.5);
+    double M[6] = {acc[0], acc[1], acc[2], acc[3], acc[4], acc[5]};
+    double ev[3], q[3][3];
+    ofb_jacobi3(M, ev, q);
+    // numpy lstsq (rcond=None): singular values below eps*max(M,N)*s_max are treated as zero.
+    // s comes from eig(A^T A), so it cannot resolve below ~1e-8*s_max; use 1e-7 as the floor.
+    double rows = 3.0 * (double)o.count;
+    double rc = 2.220446049250313e-16 * (rows > 3.0 ? rows : 3.0);
+    if (rc < 1e-7) rc = 1e-7;
+    double smax = ev[0] > 0 ? sqrt(ev[0]) : 0.0;
+    int rank = 0;
+    v[0] = v[1] = v[2] = 0.0;
+    for (int k = 0; k < 3; ++k) {
+        double sk = ev[k] > 0 ? sqrt(ev[k]) : 0.0;
+        o.s[k] = sk;
+        if (sk > rc * smax && smax > 0) {
+            ++rank;
+            double c = (q[k][0] * acc[6] + q[k][1] * acc[7] + q[k][2] * acc[8]) * d / ev[k];
+            v[0] += c * q[k][0]; v[1] += c * q[k][1]; v[2] += c * q[k][2];
+        }
+    }
+    o.rank = rank;
+}
+
+// ||A_i v - d b_i||^2 of one point (the residual of the plain solve's second pass)
+__device__ __forceinline__ double ofb_point_res2(const OfbPointTerms& t, double px, double py, double d, const double (&v)[3])
+{
+    double rx = t.wA * (py * v[2] - v[1]) - d * t.wb * t.bx;
+    double ry = t.wA * (v[0] - px * v[2]) - d * t.wb * t.by;
+    double rz = t.wA * (px * v[1] - py * v[0]) - d * t.wb * t.bz;
+    return rx * rx + ry * ry + rz * rz;
+}
+
 // Loader concept: begin(f), end(f), load(f, i, px, py, ux, uy) -> bool (false = point skipped),
 // dist(f, i, d) -> bool (MODULE variant: true = per-point distance supplied by the caller, false = derive it from the
 // prior velocity `vprior` with the 4-argument r_tilde).
@@ -292,4 +331,166 @@ __device__ __forceinline__ ofb_ego_result ofb_ego_record(const OfbEgoOut& o, int
     for (int k = 0; k < 6; ++k) r.s[k] = o.s[k];
     r.res = o.res; r.rank = o.rank; r.flags = flags;
     return r;
+}
+
+// Robust velocity solve: iteratively reweighted least squares with Tukey's biweight and a median scale.
+//   iteration 0: the plain solve (ofb_block_solve's v' before the lever arm, bit for bit), all weights 1;
+//   iteration k = 1..K: rho_i = ||r_i(v'_{k-1})|| (fp64; r_i = wA (X x v') - d wb beta_i, the plain solve's residual),
+//     sigma = the lower median of (float)rho_i (rank floor((N-1)/2), exact), tau = c sigma; tau 0 or not finite: stop,
+//     keeping v'_{k-1} and its weights (an exact fit of at least half the points);
+//     w_i = (1 - (rho_i / tau)^2)^2 for rho_i < tau, else 0; v'_k = lstsq of the weighted normal equations, 3 N_in rows.
+// Each weight multiplies its point's terms, so a weight of 1 changes nothing. The median is a radix select over the
+// fp32 keys (the bits of non-negative floats sort as unsigned integers): 4 passes of 8 bits, each recomputing rho_i from
+// the loader, counting into a shared-memory histogram with integer atomics and picking the digit by a warp scan. So
+// there is no cap on N and no per-point scratch, and the result does not depend on the order of the atomics.
+// Per iteration that is 5 passes over the points (4 select passes and the weighted accumulation); one more pass at the
+// end sums res = sum w_i rho_i(v'_K)^2 with the last solve's weights (and writes them to wout when given).
+struct OfbRobustOut { double v[3]; double s[3]; double res; double scale; int rank; int n_inliers; int iterations; };
+
+__device__ __forceinline__ double ofb_tukey_weight(double rho, double tau)
+{
+    if (!(rho < tau)) return 0.0;
+    const double q = rho / tau, a = 1.0 - __dmul_rn(q, q);      // rounded as NumPy rounds (no fused multiply-add)
+    return a * a;
+}
+
+template <class Loader>
+__device__ OfbRobustOut ofb_block_solve_robust(const Loader& ld, int f, int variant, double d, const double* n3g,
+                                               const double* w3g, const double* t3g, double c, int iterations,
+                                               double* __restrict__ wout = nullptr)
+{
+    __shared__ double red[11 * 32];
+    __shared__ unsigned hist[256];
+    __shared__ unsigned sel[2];                      // selected key prefix, rank left inside it
+    const double n3[3] = {n3g[0], n3g[1], n3g[2]};
+    const double w3[3] = {w3g[0], w3g[1], w3g[2]};
+    const int i0 = ld.begin(f), i1 = ld.end(f);
+    // weighted normal equations with weights from (vw, tau); tau = 0: all weights 1 (the plain solve)
+    auto solve = [&](const double (&vw)[3], double tau, OfbSolveOut& o, double (&v)[3]) {
+        double acc[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+        for (int i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+            double px, py, ux, uy;
+            if (!ld.load(f, i, px, py, ux, uy)) continue;
+            const OfbPointTerms t = ofb_point_terms(variant, px, py, ux, uy, n3, w3);
+            double om = 1.0;
+            if (tau > 0.0) {
+                om = ofb_tukey_weight(sqrt(ofb_point_res2(t, px, py, d, vw)), tau);
+                if (om == 0.0) continue;
+            }
+            const double w2 = t.wA * t.wA * om;
+            const double xx = px * px, yy = py * py;
+            acc[0] += w2 * (yy + 1.0);
+            acc[1] += w2 * (-px * py);
+            acc[2] += w2 * (-px);
+            acc[3] += w2 * (xx + 1.0);
+            acc[4] += w2 * (-py);
+            acc[5] += w2 * (xx + yy);
+            const double s = -t.wA * t.wb * om;
+            acc[6] += s * (py * t.bz - t.by);
+            acc[7] += s * (t.bx - px * t.bz);
+            acc[8] += s * (px * t.by - py * t.bx);
+            acc[9] += 1.0;
+        }
+        ofb_block_sum<10>(acc, red);
+        ofb_lstsq3(acc, d, o, v);
+    };
+    // the key of rank m (0-based, ascending) of (float)rho_i(vk)
+    auto select = [&](const double (&vk)[3], unsigned m) -> unsigned {
+        unsigned prefix = 0u, rank = m;
+        for (int shift = 24; shift >= 0; shift -= 8) {
+            const unsigned hi = shift == 24 ? 0u : 0xffffffffu << (shift + 8);
+            for (int b = threadIdx.x; b < 256; b += blockDim.x) hist[b] = 0u;
+            __syncthreads();
+            for (int i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+                double px, py, ux, uy;
+                if (!ld.load(f, i, px, py, ux, uy)) continue;
+                const OfbPointTerms t = ofb_point_terms(variant, px, py, ux, uy, n3, w3);
+                const unsigned key = __float_as_uint((float)sqrt(ofb_point_res2(t, px, py, d, vk)));
+                if ((key & hi) == prefix) atomicAdd(&hist[(key >> shift) & 255u], 1u);
+            }
+            __syncthreads();
+            if (threadIdx.x < 32) {                  // lane l holds bins 8l .. 8l+7
+                const int lane = threadIdx.x;
+                unsigned cnt[8], sum = 0u;
+#pragma unroll
+                for (int j = 0; j < 8; ++j) { cnt[j] = hist[8 * lane + j]; sum += cnt[j]; }
+                unsigned incl = sum;
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) {
+                    const unsigned y = __shfl_up_sync(0xffffffffu, incl, o);
+                    if (lane >= o) incl += y;
+                }
+                unsigned cum = incl - sum;
+                if (rank >= cum && rank < incl) {
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) {
+                        if (rank < cum + cnt[j]) { sel[0] = prefix | ((unsigned)(8 * lane + j) << shift); sel[1] = rank - cum; break; }
+                        cum += cnt[j];
+                    }
+                }
+            }
+            __syncthreads();
+            prefix = sel[0]; rank = sel[1];
+        }
+        return prefix;
+    };
+    OfbRobustOut r;
+    OfbSolveOut o;
+    double vk[3], vprev[3] = {0.0, 0.0, 0.0};
+    solve(vprev, 0.0, o, vk);
+    const int n = o.count;
+    double tau_last = 0.0;                           // tau of the weights of the last solve (0: all weights 1)
+    r.scale = 0.0; r.iterations = 0;
+    for (int k = 1; k <= iterations && n > 0; ++k) {
+        const double sigma = (double)__uint_as_float(select(vk, (unsigned)(n - 1) / 2u));
+        const double tau = c * sigma;
+        if (!(tau > 0.0) || !isfinite(tau)) break;
+        OfbSolveOut ok;
+        double vn[3];
+        solve(vk, tau, ok, vn);
+        for (int j = 0; j < 3; ++j) { vprev[j] = vk[j]; vk[j] = vn[j]; }
+        o = ok; tau_last = tau; r.scale = sigma; r.iterations = k;
+    }
+    // last pass: res with the last solve's weights (from vprev and tau_last)
+    double acc[1] = {0.0};
+    for (int i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
+        double px, py, ux, uy;
+        double om = 0.0;
+        if (ld.load(f, i, px, py, ux, uy)) {
+            const OfbPointTerms t = ofb_point_terms(variant, px, py, ux, uy, n3, w3);
+            om = tau_last > 0.0 ? ofb_tukey_weight(sqrt(ofb_point_res2(t, px, py, d, vprev)), tau_last) : 1.0;
+            if (om != 0.0) acc[0] += om * ofb_point_res2(t, px, py, d, vk);
+        }
+        if (wout) wout[i] = om;
+    }
+    ofb_block_sum<1>(acc, red);
+    r.res = acc[0];
+    r.rank = o.rank; r.n_inliers = o.count;
+    for (int k = 0; k < 3; ++k) { r.s[k] = o.s[k]; r.v[k] = vk[k]; }
+    // lever arm: v = v' - w x t (EXP, SIM); NODE has none
+    if (variant != OFB_VARIANT_NODE && t3g) {
+        r.v[0] -= w3[1] * t3g[2] - w3[2] * t3g[1];
+        r.v[1] -= w3[2] * t3g[0] - w3[0] * t3g[2];
+        r.v[2] -= w3[0] * t3g[1] - w3[1] * t3g[0];
+    }
+    return r;
+}
+
+// the C ABI record of a robust solve
+__device__ __forceinline__ ofb_robust_result ofb_robust_record(const OfbRobustOut& o, int flags)
+{
+    ofb_robust_result r;
+    for (int k = 0; k < 3; ++k) { r.v[k] = o.v[k]; r.s[k] = o.s[k]; }
+    r.res = o.res; r.scale = o.scale;
+    r.rank = o.rank; r.n_inliers = o.n_inliers; r.iterations = o.iterations; r.flags = flags;
+    return r;
+}
+
+// host-side check of a robust setting: c finite and >= 1.5 (so that at least half the points keep a weight), 0..64 iterations
+static inline int ofb_robust_check(const ofb_robust_cfg* r, const char* who)
+{
+    OFB_REQUIRE(r, "%s: null robust setting", who);
+    OFB_REQUIRE(r->c >= 1.5 && r->c < HUGE_VAL, "%s: robust c must be finite and >= 1.5 (got %g)", who, r->c);
+    OFB_REQUIRE(r->iterations >= 0 && r->iterations <= 64, "%s: robust iterations must be in 0..64 (got %d)", who, r->iterations);
+    return OFB_OK;
 }

@@ -34,16 +34,18 @@ class StreamTracker:
     camera: (K, D, rate[, iterations]) or vision.make_camera(...) -- see set_camera.
     fb_threshold: None / 0 = off, T > 0 = forward-backward check of the LK tracks -- see set_fb_threshold.
     gyro_prediction: LK starts from the rotation the step's gyro sample measured -- see set_gyro_prediction.
-    ego_motion: every stream's angular rate is also estimated from its kept points -- see set_ego_motion."""
+    ego_motion: every stream's angular rate is also estimated from its kept points -- see set_ego_motion.
+    robust: None / False, True or (c, iterations): the robust velocity solve of every stream -- see set_robust."""
 
     def __init__(self, width, height, max_features=100, min_features=20, n_streams=1, feature_params=None,
                  lk_params=None, topup="exp", mask_radius=30, bgr=False, variant="exp", principal=None,
                  scaling=1.0, flow_scaling=None, max_speed=0.0, dummy_value=float("nan"), gate=None, min_solve=3,
                  min_eig_thr=1e-4, borrow_frames=False, v_init=None, camera=None, fb_threshold=None,
-                 gyro_prediction=False, ego_motion=False, ctx=None):
+                 gyro_prediction=False, ego_motion=False, robust=None, ctx=None):
         fb = _fb_threshold(fb_threshold)
         gyro = _gyro_flag(gyro_prediction)
         ego = _ego_flag(ego_motion)
+        rcfg = _lib.robust_cfg(robust)
         fp = dict(qualityLevel=0.01, minDistance=10, blockSize=7)
         fp.update(feature_params or {})
         lk = dict(winSize=(15, 15), maxLevel=3, criteria=(3, 20, 0.03))
@@ -89,6 +91,9 @@ class StreamTracker:
         self.ego_motion = False
         if ego:
             self.set_ego_motion(True)
+        self.robust = None
+        if rcfg is not None:
+            self.set_robust((rcfg.c, rcfg.iterations))
 
     def close(self):
         if getattr(self, "h", None) and getattr(self.ctx, "h", None):
@@ -147,6 +152,16 @@ class StreamTracker:
         _lib.check(self.ctx.lib.ofb_tracker_set_ego_motion(self.h, 1 if on else 0))
         self.ego_motion = on
 
+    def set_robust(self, robust):
+        """Robust velocity solve of every stream from the next step on (velocity.solve_velocity_robust on the kept
+        points, after the velocity and ego-motion solves): step(..., want_robust=True) returns its
+        _lib.ROBUST_RESULT_DTYPE records. None / False turns it off, True uses c = 4 and 10 iterations, (c, iterations)
+        sets them. The standard records, the point sets and the r_tilde gate's prior (the plain velocity) do not
+        change. Not available for variant="module"."""
+        cfg = _lib.robust_cfg(robust)
+        _lib.check(self.ctx.lib.ofb_tracker_set_robust(self.h, C.byref(cfg) if cfg is not None else None))
+        self.robust = None if cfg is None else (cfg.c, cfg.iterations)
+
     def set_points(self, points):
         """points: one (N,2)/(N,1,2) array per stream (or a single array when n_streams == 1)."""
         if self.n_streams == 1 and not isinstance(points, (list, tuple)):
@@ -163,13 +178,16 @@ class StreamTracker:
             cnt[s] = len(p)
         _lib.check(self.ctx.lib.ofb_tracker_set_points(self.h, _lib.ptr(buf), _lib.ptr(cnt)))
 
-    def step(self, frames, imu, v_prior=None, want_points=False, want_kept=False, want_ego=False):
+    def step(self, frames, imu, v_prior=None, want_points=False, want_kept=False, want_ego=False, want_robust=False):
         """frames: (H,W) / (S,H,W) uint8 (or (...,3) BGR when bgr=True), NumPy or CUDA tensor; imu: _lib.IMU_DTYPE
         (S,). Returns the _lib.TRACK_RESULT_DTYPE records (S,); with want_points additionally the list of (N,1,2)
         float32 point sets after the step; with want_kept the lists of (old, new) positions the solve used; with
-        want_ego (needs set_ego_motion) the _lib.EGO_RESULT_DTYPE records (S,), last."""
+        want_ego (needs set_ego_motion) the _lib.EGO_RESULT_DTYPE records (S,); with want_robust (needs set_robust) the
+        _lib.ROBUST_RESULT_DTYPE records (S,), last."""
         if want_ego and not self.ego_motion:
             raise ValueError("want_ego needs ego-motion: StreamTracker(..., ego_motion=True) or set_ego_motion(True)")
+        if want_robust and self.robust is None:
+            raise ValueError("want_robust needs the robust solve: StreamTracker(..., robust=True) or set_robust(True)")
         S, h, w = self.n_streams, self.height, self.width
         shape = tuple(frames.shape)
         tail = (h, w, 3) if self.bgr else (h, w)
@@ -192,6 +210,7 @@ class StreamTracker:
             v_prior = np.ascontiguousarray(v_prior, dtype=np.float64).reshape(S, 3)
         res = np.zeros(S, _lib.TRACK_RESULT_DTYPE)
         ego = np.zeros(S, _lib.EGO_RESULT_DTYPE) if want_ego else None
+        rob = np.zeros(S, _lib.ROBUST_RESULT_DTYPE) if want_robust else None
         pts = cnt = kp = kn = None
         if want_points:
             pts = np.zeros((S, self.capacity, 2), np.float32)
@@ -199,9 +218,9 @@ class StreamTracker:
         if want_kept:
             kp = np.zeros((S, self.capacity, 2), np.float32)
             kn = np.zeros((S, self.capacity, 2), np.float32)
-        _lib.check(self.ctx.lib.ofb_tracker_step_ego(self.h, _lib.ptr(frames), bpp * w, bpp * w * h, _lib.ptr(imu),
-                                                     _lib.ptr(v_prior), _lib.ptr(res), _lib.ptr(pts), _lib.ptr(cnt),
-                                                     _lib.ptr(kp), _lib.ptr(kn), _lib.ptr(ego)))
+        _lib.check(self.ctx.lib.ofb_tracker_step_robust(self.h, _lib.ptr(frames), bpp * w, bpp * w * h, _lib.ptr(imu),
+                                                        _lib.ptr(v_prior), _lib.ptr(res), _lib.ptr(pts), _lib.ptr(cnt),
+                                                        _lib.ptr(kp), _lib.ptr(kn), _lib.ptr(ego), _lib.ptr(rob)))
         out = [res]
         if want_points:
             out.append([pts[s, :cnt[s]].reshape(-1, 1, 2).copy() for s in range(S)])
@@ -210,6 +229,8 @@ class StreamTracker:
             out.append([kn[s, :res["n_kept"][s]].copy() for s in range(S)])
         if want_ego:
             out.append(ego)
+        if want_robust:
+            out.append(rob)
         return out[0] if len(out) == 1 else tuple(out)
 
 
@@ -283,6 +304,13 @@ class FleetTracker:
         on = _ego_flag(enable)
         if self.local is not None:
             self.local.set_ego_motion(on)
+
+    def set_robust(self, robust):
+        """StreamTracker.set_robust on this rank's streams (robust=... at construction is passed to the local tracker
+        with the other keywords)"""
+        cfg = _lib.robust_cfg(robust)
+        if self.local is not None:
+            self.local.set_robust(None if cfg is None else (cfg.c, cfg.iterations))
 
     def gather_velocities(self):
         """(n_streams, 3) velocities of the last step on every rank; rows of streams that did not solve (or have not

@@ -179,6 +179,58 @@ def solve_ego_motion_batched(x, u, offsets, d, n, t=None, variant="node", ctx=No
     return out
 
 
+def _robust_args(variant, c, iterations):
+    if variant not in _lib.VARIANTS:
+        raise ValueError("robust variant must be one of %s (module is not supported)" % sorted(_lib.VARIANTS))
+    return _lib.VARIANTS[variant], _lib.robust_cfg((c, iterations))
+
+
+def solve_velocity_robust(x, u, d, n, omega, t=None, variant="node", c=4.0, iterations=10, want_weights=False, ctx=None):
+    """Robust velocity solve (include/ofb200.h, ofb_solve_velocity_robust): iteratively reweighted least squares with
+    Tukey's biweight, tau = c x the lower median of the point residual norms, `iterations` reweighted solves after the
+    plain one (0 is the plain solve). Returns the _lib.ROBUST_RESULT_DTYPE record, and with want_weights also every
+    point's weight in the last solve (N,)."""
+    var, cfg = _robust_args(variant, c, iterations)
+    x = _pts(x, "x")
+    u = _pts(u, "u")
+    if len(x) != len(u):
+        raise ValueError("x and u must have the same number of rows")
+    n3, w3 = _vec3(n, "n"), _vec3(omega, "omega")
+    t3 = _vec3(t, "t") if t is not None else None
+    ctx = ctx or _lib.default_context()
+    rec = np.zeros(1, _lib.ROBUST_RESULT_DTYPE)
+    wts = np.zeros(len(x)) if want_weights else None
+    _lib.check(ctx.lib.ofb_solve_velocity_robust(ctx.h, var, _lib.ptr(x), _lib.ptr(u), len(x), _scalar(d), _lib.ptr(n3),
+                                                 _lib.ptr(w3), _lib.ptr(t3), C.byref(cfg), _lib.ptr(rec), _lib.ptr(wts)))
+    return (rec[0], wts) if want_weights else rec[0]
+
+
+def solve_velocity_robust_batched(x, u, offsets, d, n, omega, t=None, variant="node", c=4.0, iterations=10,
+                                  want_weights=False, ctx=None):
+    """Many frames at once, frame f on rows offsets[f]:offsets[f+1] -> _lib.ROBUST_RESULT_DTYPE records (F,), and with
+    want_weights the weights of every row (rows in no frame get 0)."""
+    var, cfg = _robust_args(variant, c, iterations)
+    x = _pts(x, "x")
+    u = _pts(u, "u")
+    offsets = np.ascontiguousarray(offsets, dtype=np.int32)
+    F = len(offsets) - 1
+    if F < 1 or offsets[0] < 0 or np.any(np.diff(offsets) < 0):
+        raise ValueError("offsets must be a non-decreasing sequence of at least two non-negative row indices")
+    if len(x) != len(u) or len(x) < offsets[-1]:
+        raise ValueError("x and u must have the same number of rows, at least offsets[-1] = %d" % offsets[-1])
+    d = np.ascontiguousarray(np.broadcast_to(np.asarray(d, dtype=np.float64).reshape(-1), (F,)))
+    n3 = np.ascontiguousarray(np.broadcast_to(np.asarray(n, dtype=np.float64), (F, 3)))
+    w3 = np.ascontiguousarray(np.broadcast_to(np.asarray(omega, dtype=np.float64), (F, 3)))
+    t3 = None if t is None else np.ascontiguousarray(np.broadcast_to(np.asarray(t, dtype=np.float64), (F, 3)))
+    out = np.zeros(F, _lib.ROBUST_RESULT_DTYPE)
+    wts = np.zeros(int(offsets[-1])) if want_weights else None
+    ctx = ctx or _lib.default_context()
+    _lib.check(ctx.lib.ofb_solve_velocity_robust_batched(ctx.h, var, _lib.ptr(x), _lib.ptr(u), _lib.ptr(offsets), F,
+                                                         _lib.ptr(d), _lib.ptr(n3), _lib.ptr(w3), _lib.ptr(t3),
+                                                         C.byref(cfg), _lib.ptr(out), _lib.ptr(wts if wts is None or len(wts) else None)))
+    return (out, wts) if want_weights else out
+
+
 def generate_test_data(x, v, omega, d, n, t=None, ctx=None):
     ctx = ctx or _lib.default_context()
     x = _pts(x, "x")

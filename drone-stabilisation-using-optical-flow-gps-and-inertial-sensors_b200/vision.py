@@ -391,7 +391,7 @@ def _ego_flag(ego_motion):
 
 
 def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, ctx=None, on_overflow="raise", camera=None,
-                fb_threshold=None, gyro_prediction=False, ego_motion=False):
+                fb_threshold=None, gyro_prediction=False, ego_motion=False, robust=None):
     """Batched detect(+)track+solve. prev/nxt: (N,H,W) uint8 numpy arrays (host) or CUDA tensors;
     imu: structured array _lib.IMU_DTYPE (N,). Returns a structured array _lib.RESULT_DTYPE (N,)
     (and prev_pts, next_pts, status when want_tracks).
@@ -409,9 +409,13 @@ def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, 
     p1 + (p0 - guess).
     ego_motion: also estimate every pair's angular rate from its tracks together with the velocity (velocity.
     solve_ego_motion on the points the pair's solve uses; the gyro sample is not used there): the _lib.EGO_RESULT_DTYPE
-    records (N,) are appended as the last element of the return. The standard results do not change."""
+    records (N,) are appended as the last element of the return. The standard results do not change.
+    robust: None / False = off; True = the robust velocity solve (velocity.solve_velocity_robust, c = 4, 10 iterations)
+    of every pair on the points its solve uses; (c, iterations) sets them. The _lib.ROBUST_RESULT_DTYPE records (N,)
+    are appended as the last element of the return, after the ego records. The standard results do not change."""
     thr = _fb_threshold(fb_threshold)
     ego_on = _ego_flag(ego_motion)
+    rcfg = _lib.robust_cfg(robust)
     gyro = _gyro_flag(gyro_prediction)
     cam = as_camera(camera)
     if gyro and cam is None and (cfg.flow_scale == 0 or cfg.pos_scale == 0 or not np.isfinite(cfg.pos_scale / cfg.flow_scale)):
@@ -430,6 +434,7 @@ def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, 
         raise ValueError("one IMU sample per pair is required")
     res = np.zeros(n, _lib.RESULT_DTYPE)
     ego = np.zeros(n, _lib.EGO_RESULT_DTYPE) if ego_on else None
+    rob = np.zeros(n, _lib.ROBUST_RESULT_DTYPE) if rcfg is not None else None
     K = cfg.max_corners
     pp = pn = st = None
     if want_tracks:
@@ -439,10 +444,11 @@ def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, 
     if pts_in is not None:
         pts_in = np.ascontiguousarray(pts_in, dtype=np.float32)
         n_in = np.ascontiguousarray(n_in, dtype=np.int32)
-    _lib.check(ctx.lib.ofb_frame_pairs_ego(ctx.h, C.byref(cfg), C.byref(cam) if cam is not None else None, thr, gyro, n,
-                                           _lib.ptr(prev), _lib.ptr(nxt), w, w * h, _lib.ptr(imu), _lib.ptr(pts_in),
-                                           _lib.ptr(n_in), _lib.ptr(res), _lib.ptr(ego), _lib.ptr(pp), _lib.ptr(pn),
-                                           _lib.ptr(st)))
+    _lib.check(ctx.lib.ofb_frame_pairs_robust(ctx.h, C.byref(cfg), C.byref(cam) if cam is not None else None, thr, gyro, n,
+                                              _lib.ptr(prev), _lib.ptr(nxt), w, w * h, _lib.ptr(imu), _lib.ptr(pts_in),
+                                              _lib.ptr(n_in), _lib.ptr(res), _lib.ptr(ego),
+                                              C.byref(rcfg) if rcfg is not None else None, _lib.ptr(rob), _lib.ptr(pp),
+                                              _lib.ptr(pn), _lib.ptr(st)))
     if on_overflow == "raise" and (res["flags"] & _lib.PAIR_OVERFLOW).any():
         bad = np.nonzero(res["flags"] & _lib.PAIR_OVERFLOW)[0]
         raise _lib.OfbError("frame_pairs: detector candidate buffer overflowed for pair(s) %s: the image has more than "
@@ -450,11 +456,13 @@ def frame_pairs(prev, nxt, imu, cfg, pts_in=None, n_in=None, want_tracks=False, 
     out = (res, pp, pn, st) if want_tracks else (res,)
     if ego_on:
         out = out + (ego,)
+    if rob is not None:
+        out = out + (rob,)
     return out if len(out) > 1 else out[0]
 
 
 def frame_sequence(frames, imu, cfg, want_tracks=False, ctx=None, on_overflow="raise", camera=None, fb_threshold=None,
-                   gyro_prediction=False, ego_motion=False):
+                   gyro_prediction=False, ego_motion=False, robust=None):
     """One camera stream: frames (N+1,H,W) uint8 -> N consecutive pairs (frame i, frame i+1), as
     velocity_measurment_node:224-267 sees them (it keeps the previous callback's image). Passing the two views
     of ONE buffer lets the library upload every frame and build its pyramid once (`next == prev + image_stride`
@@ -462,5 +470,6 @@ def frame_sequence(frames, imu, cfg, want_tracks=False, ctx=None, on_overflow="r
     if isinstance(frames, np.ndarray):
         frames = np.ascontiguousarray(frames, dtype=np.uint8)
     return frame_pairs(frames[:-1], frames[1:], imu, cfg, want_tracks=want_tracks, ctx=ctx, on_overflow=on_overflow,
-                       camera=camera, fb_threshold=fb_threshold, gyro_prediction=gyro_prediction, ego_motion=ego_motion)
+                       camera=camera, fb_threshold=fb_threshold, gyro_prediction=gyro_prediction, ego_motion=ego_motion,
+                       robust=robust)
 

@@ -171,6 +171,49 @@ int ofb_solve_ego_motion(ofb_ctx* ctx, int variant, const double* x, const doubl
 int ofb_solve_ego_motion_batched(ofb_ctx* ctx, int variant, const double* x, const double* u, const int* offsets,
                                  int n_frames, const double* d, const double* n3, const double* t3, ofb_ego_result* out);
 
+/* ---- robust velocity solve: iteratively reweighted least squares with Tukey's biweight and a median scale, so that a
+ *      group of points that is consistent but not the ground plane (a moving object, a roof, water) does not move the
+ *      velocity by as much as the group weighs. On the points of ofb_solve_velocity, with its terms wA, wb, beta_i and
+ *      v' = v + w x t, every point has the residual r_i(v') = wA (X x v') - d wb beta_i (a 3-vector):
+ *        iteration 0: the plain solve (v' of ofb_solve_velocity bit for bit), all weights 1;
+ *        iteration k = 1..K: rho_i = |r_i(v'_{k-1})| (fp64), sigma = the lower median of the fp32 values (float)rho_i
+ *          (0-based rank floor((N-1)/2), exact), tau = c sigma. tau 0 or not finite (an exact fit of at least half the
+ *          points): stop and keep v'_{k-1} and its weights. Else w_i = (1 - (rho_i/tau)^2)^2 for rho_i < tau, 0 beyond,
+ *          and v'_k = np.linalg.lstsq on the sqrt(w_i)-scaled rows of the N_in points with w_i > 0 (the rank rule of
+ *          ofb_solve_velocity with 3 N_in rows).
+ *      Then v = v'_K - w x t for EXP and SIM (NODE has no lever arm). For residuals isotropic in the plane normal to X the
+ *      median |r| is ~1.18 of their standard deviation, so c = 4 is about Tukey's 4.685. With c >= 1.5 every point at or
+ *      below the median keeps a positive weight. Limits: the start is least squares, so the solve breaks down as the
+ *      outliers approach half the points (40 % moving points are still rejected with the defaults on synthetic data, 45 %
+ *      no longer); a second plane close to the ground has nearly the ground's flow and is kept. The cost is 5 passes over
+ *      the points per iteration (4 passes of the median's radix select and the weighted accumulation). Deterministic: no
+ *      random draws, and the same input gives the same record bit for bit. MODULE returns OFB_E_INVALID. */
+typedef struct {
+    double c;            /* tuning constant, finite and >= 1.5 (default 4) */
+    int    iterations;   /* reweighted solves K, 0 .. 64 (default 10); 0 is the plain solve */
+} ofb_robust_cfg;
+#define OFB_ROBUST_SOLVED 1         /* ofb_robust_result.flags: the solve ran for this frame (tracker: as OFB_TRACK_SOLVED) */
+typedef struct {
+    double v[3];         /* velocity, lever arm removed with the gyro rate */
+    double s[3];         /* singular values of the last weighted system, descending */
+    double res;          /* sum w_i rho_i(v'_K)^2 with the weights of the last solve */
+    double scale;        /* sigma of the last completed iteration (0 when none ran) */
+    int    rank;         /* rank of the last weighted system */
+    int    n_inliers;    /* points with w_i > 0 in the last solve (N when none ran) */
+    int    iterations;   /* reweighted solves actually done (< K after the stop rule) */
+    int    flags;        /* OFB_ROBUST_* */
+} ofb_robust_result;
+/* As ofb_solve_velocity (x, u: n x 2 float64, host or device); out: one record; weights_out (n, host or device, may be
+ * NULL): w_i of the last solve for every point (all 1 when no reweighted solve ran). */
+int ofb_solve_velocity_robust(ofb_ctx* ctx, int variant, const double* x, const double* u, int n, double d,
+                              const double n3[3], const double w3[3], const double t3[3], const ofb_robust_cfg* cfg,
+                              ofb_robust_result* out, double* weights_out);
+/* n_frames problems as ofb_solve_velocity_batched (offsets may be device memory); out[n_frames]; weights_out
+ * (offsets[n_frames] rows, may be NULL): rows in no frame are set to 0. */
+int ofb_solve_velocity_robust_batched(ofb_ctx* ctx, int variant, const double* x, const double* u, const int* offsets,
+                                      int n_frames, const double* d, const double* n3, const double* w3, const double* t3,
+                                      const ofb_robust_cfg* cfg, ofb_robust_result* out, double* weights_out);
+
 /* generate_test_data: simulation.py:7-12 (t3 != NULL) / velocity_measurment_node:25-29 (t3 NULL) */
 int ofb_generate_flow(ofb_ctx* ctx, const double* x, int n, const double v3[3], const double w3[3],
                       double d, const double n3[3], const double* t3, double* u_out);
@@ -323,6 +366,15 @@ int ofb_frame_pairs_ego(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera*
                         int n_pairs, const uint8_t* prev, const uint8_t* next, int pitch, size_t image_stride,
                         const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
                         ofb_pair_result* results, ofb_ego_result* ego, float* prev_pts, float* next_pts, uint8_t* status);
+/* ofb_frame_pairs_ego plus the robust velocity solve (see ofb_solve_velocity_robust) of every pair: rob[n_pairs] (host or
+ * device) from the same tracked points as the pair's velocity solve, in the same kernel, after it and the ego-motion
+ * solve. robust must be set when rob is; rob == NULL is exactly ofb_frame_pairs_ego. The results, tracks and ego records
+ * do not depend on it. */
+int ofb_frame_pairs_robust(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_camera* cam, double fb_max_err, int gyro_predict,
+                           int n_pairs, const uint8_t* prev, const uint8_t* next, int pitch, size_t image_stride,
+                           const ofb_imu_sample* imu, const float* pts_in, const int* n_in,
+                           ofb_pair_result* results, ofb_ego_result* ego, const ofb_robust_cfg* robust,
+                           ofb_robust_result* rob, float* prev_pts, float* next_pts, uint8_t* status);
 
 /* ---- feature lifecycle around the tracker (SURVEY 8f-2): the point set of every camera stream stays on the
  *      device between frames. One step does what the reference's per-frame loops do around the tracker
@@ -442,6 +494,18 @@ int ofb_tracker_set_ego_motion(ofb_tracker* trk, int enable);
 int ofb_tracker_step_ego(ofb_tracker* trk, const uint8_t* frames, int pitch, size_t image_stride,
                          const ofb_imu_sample* imu, const double* v_prior, ofb_track_result* results,
                          float* pts_out, int* n_out, float* kept_prev, float* kept_next, ofb_ego_result* ego);
+/* Robust velocity solve (see ofb_solve_velocity_robust) of every stream from the next ofb_tracker_step on, on the kept
+ * points, after the velocity and ego-motion solves and under the same condition (the record is zero with flags 0 when
+ * the stream did not solve). cfg == NULL turns it off (the default). The standard records, tracks and point sets do not
+ * change, and the r_tilde gate keeps using the plain velocity. MODULE trackers return OFB_E_INVALID. A change rebuilds
+ * the captured CUDA graphs. */
+int ofb_tracker_set_robust(ofb_tracker* trk, const ofb_robust_cfg* cfg);
+/* ofb_tracker_step_ego plus rob[n_streams] (host or device, may be NULL): the step's robust records. rob != NULL needs
+ * ofb_tracker_set_robust. The records complete under the rule of the result records. */
+int ofb_tracker_step_robust(ofb_tracker* trk, const uint8_t* frames, int pitch, size_t image_stride,
+                            const ofb_imu_sample* imu, const double* v_prior, ofb_track_result* results,
+                            float* pts_out, int* n_out, float* kept_prev, float* kept_next, ofb_ego_result* ego,
+                            ofb_robust_result* rob);
 /* the exclusion mask OFB_TOPUP_APPEND_MASKED would use for `n` points (n x 2 float32): mask_out h x w u8
  * (1 = allowed, 0 = inside a circle). Exposed for parity tests against cv2.circle. */
 int ofb_tracker_render_mask(ofb_ctx* ctx, const float* pts, int n, int radius, int w, int h, uint8_t* mask_out);

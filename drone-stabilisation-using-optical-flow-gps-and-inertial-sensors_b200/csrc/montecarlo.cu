@@ -356,9 +356,16 @@ __global__ void minmax_final_kernel(double* part, int nblocks)
         part[0] = lo; part[1] = hi;
     }
 }
+// Edge k of numpy.linspace(lo, hi, bins + 1), bit for bit: k * ((hi - lo) / bins) + lo, rounded after the product and
+// after the sum (the intrinsics keep nvcc from contracting the two into one FMA); the last edge is hi itself.
+__device__ __forceinline__ double linspace_edge(double lo, double hi, double step, int k, int bins)
+{
+    return k == bins ? hi : __dadd_rn(__dmul_rn((double)k, step), lo);
+}
+
 // numpy.histogram semantics for uniform bins over [lo,hi]: bin = floor((x-lo)/(hi-lo)*bins), x==hi
 // falls in the last bin, values outside are dropped; the computed index is then corrected against the
-// actual edges lo + k*(hi-lo)/bins the way numpy does.
+// actual linspace edges the way numpy does, so a sample on an edge lands where numpy puts it.
 __global__ void histogram_kernel(const double* __restrict__ data, size_t n, double lo, double hi, int bins,
                                  unsigned long long* __restrict__ counts)
 {
@@ -366,14 +373,13 @@ __global__ void histogram_kernel(const double* __restrict__ data, size_t n, doub
     for (int i = threadIdx.x; i < bins; i += blockDim.x) sh[i] = 0;
     __syncthreads();
     double norm = (double)bins / (hi - lo);
+    double step = (hi - lo) / bins;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
         double v = data[i];
         if (!(v >= lo && v <= hi)) continue;
         int b = (int)((v - lo) * norm);
         if (b >= bins) b = bins - 1;
-        // edge correction (numpy: linspace edges)
-        double e0 = lo + (hi - lo) * ((double)b / bins), e1 = lo + (hi - lo) * ((double)(b + 1) / bins);
-        if (b + 1 == bins) e1 = hi;
+        double e0 = linspace_edge(lo, hi, step, b, bins), e1 = linspace_edge(lo, hi, step, b + 1, bins);
         if (v < e0 && b > 0) --b;
         else if (v >= e1 && b + 1 < bins) ++b;
         atomicAdd(&sh[b], 1u);
@@ -386,8 +392,10 @@ __global__ void histogram_kernel(const double* __restrict__ data, size_t n, doub
 int validate_steps(const ofb_mc_step* steps, int n_steps, int total_points)
 {
     for (int i = 0; i < n_steps; ++i) {
-        OFB_REQUIRE(steps[i].n_points > 0 && steps[i].n_points <= OFB_MC_MAX_POINTS,
-                    "mc: step %d has %d points (1..%d supported)", i, steps[i].n_points, OFB_MC_MAX_POINTS);
+        // one point leaves the 3x3 normal matrix singular (its own ray is in the null space): at least two
+        OFB_REQUIRE(steps[i].n_points >= 2 && steps[i].n_points <= OFB_MC_MAX_POINTS,
+                    "mc: step %d has %d points (2..%d supported: one point does not determine the velocity)", i,
+                    steps[i].n_points, OFB_MC_MAX_POINTS);
         OFB_REQUIRE(steps[i].pos_offset >= 0 && steps[i].pos_offset + steps[i].n_points <= total_points,
                     "mc: step %d point range outside pos/true_flow", i);
         OFB_REQUIRE(steps[i].height != 0.0, "mc: step %d has zero height", i);
@@ -546,6 +554,7 @@ extern "C" int ofb_histogram(ofb_ctx* ctx, const double* data, size_t n, double 
 {
     OFB_REQUIRE(ctx && data && counts_out, "histogram: null argument");
     OFB_REQUIRE(bins > 0 && bins <= 4096, "histogram: bins must be in 1..4096");
+    OFB_REQUIRE(isfinite(lo) && isfinite(hi), "histogram: range [%g, %g] is not finite", lo, hi);
     OFB_REQUIRE(hi >= lo, "histogram: max must be larger than min");
     OFB_CUDA(cudaSetDevice(ctx->device));
     if (hi == lo) { lo -= 0.5; hi += 0.5; }   // numpy widens a degenerate range

@@ -63,6 +63,8 @@ def make_step(linear_velocity, angular_velocity, height_above_gr, normal_vector,
             raise ValueError("%s must be >= 0 (numpy.random.normal rejects negative scales)" % name)
         setattr(s, name, val)
     s.true_vel[:] = _v3(true_vel)
+    if int(n_points) < 2:
+        raise ValueError("a step needs at least 2 points: with one, the velocity solve is singular (got %d)" % n_points)
     s.n_points = int(n_points)
     s.pos_offset = int(pos_offset)
     return s
@@ -302,12 +304,17 @@ def overlap(data1, data2, ctx=None, distributed=False, group=None):
     """simulation.py:124-136: common 100-bin histogram over the pooled range, sum of bin-wise minima.
     distributed=True: data1/data2 are this rank's SHARDS of the two samples (e.g. the v_obs dumps of its trial range);
     the range is merged with all-reduce(min/max), the bin counts with all-reduce(sum), and every rank returns the
-    overlap of the full samples."""
-    ctx = ctx or _lib.default_context()
+    overlap of the full samples.
+    Like numpy.histogram's autodetected range, a NaN or infinite sample raises ValueError (on every rank when
+    distributed: a shard with one reports the range (-inf, inf), which the merge hands to all)."""
     d1 = np.ascontiguousarray(data1, dtype=np.float64).reshape(-1)
     d2 = np.ascontiguousarray(data2, dtype=np.float64).reshape(-1)
-    los, his = [], []
-    for d in (d1, d2):
+    finite = bool(np.isfinite(d1).all() and np.isfinite(d2).all())
+    if not finite and not distributed:
+        raise ValueError("overlap: the data are not finite (NaN or inf), so neither is their range")
+    ctx = ctx or _lib.default_context()
+    los, his = ([], []) if finite else ([-np.inf], [np.inf])
+    for d in (d1, d2) if finite else ():
         if len(d):
             lo, hi = C.c_double(), C.c_double()
             _lib.check(ctx.lib.ofb_minmax(ctx.h, _lib.ptr(d), len(d), C.byref(lo), C.byref(hi)))
@@ -318,8 +325,10 @@ def overlap(data1, data2, ctx=None, distributed=False, group=None):
         import torch.distributed as dist
         dev = torch.device("cuda", ctx.device) if dist.get_backend(group) == "nccl" else None
         lo, hi = merge_range(min(los) if los else np.inf, max(his) if his else -np.inf, group, dev)
-        if not np.isfinite(lo):
-            return 0
+        if lo == np.inf:
+            return 0                                    # every shard empty
+        if not (np.isfinite(lo) and np.isfinite(hi)):
+            raise ValueError("overlap: the data are not finite (NaN or inf), so neither is their range")
     else:
         if not los:
             return 0

@@ -513,7 +513,8 @@ int ofb_tracker_render_mask(ofb_ctx* ctx, const float* pts, int n, int radius, i
 /* ---- stage 5: Monte-Carlo error propagation. Replaces of_simulation (simulation.py:36-66),
  *      feas_simulation (simulation.py:70-104) and the per-step np.mean/np.std of the sweep
  *      drivers (e.g. simulation.py:183-202). One ofb_mc_step = one call of of_simulation. */
-#define OFB_MC_MAX_POINTS 256
+#define OFB_MC_MAX_POINTS 256            /* n_points of a step: 2..OFB_MC_MAX_POINTS. One point leaves the 3x3 normal
+                                            matrix singular (the point's own ray is in its null space): rejected. */
 typedef struct {
     double v[3], w[3], n[3], t[3];       /* truth: linear/angular velocity, normal, lever arm */
     double height;

@@ -49,6 +49,14 @@ def test_sweep_construction_matches_reference_parameters():
         sim.build_sweep("nope", pts)
     with pytest.raises(ValueError):
         sim.make_step([1, 1, 1], [1, 1, 1], 1.0, [0, 0, 1], [0, 0, 0], 5, 0, -1.0, 0, 0, 0, 0, 0)
+    for n_points in (1, 0):                             # one point: the velocity solve is singular
+        with pytest.raises(ValueError, match="at least 2"):
+            sim.make_step([1, 1, 1], [1, 1, 1], 1.0, [0, 0, 1], [0, 0, 0], n_points, 0, 0, 0, 0, 0, 0, 0)
+    for bad in (np.nan, np.inf):                        # numpy.histogram refuses a non-finite autodetected range
+        with pytest.raises(ValueError, match="finite"):
+            sim.overlap(np.array([0.0, bad]), np.array([1.0]))
+        with pytest.raises(ValueError):
+            vo.overlap(np.array([0.0, bad]), np.array([1.0]))
     d = sim.centred_points(pts)
     assert abs(d[:, 0].mean()) < 1e-15 and d[:, 0].std() == pytest.approx(pts[:, 0].std() * 1.27)
 

@@ -79,20 +79,3 @@ __device__ __forceinline__ double4 ofb_calibrate(const ofb_camera& c, float nx, 
     ofb_undistort(c, (double)ox, (double)oy, xo, yo);
     return make_double4(xn, yn, (xn - xo) * c.rate, (yn - yo) * c.rate);
 }
-
-// ofb_block_solve loader over tracks calibrated once beforehand (the solve reads every point twice): xu[f*stride + i]
-// = (x, y, ux, uy); a point is used when status is NULL or status[f*stride + i] != 0; points per frame from
-// counts[f*counts_stride] (counts NULL: n).
-struct CalibLoader {
-    const double4* xu; size_t stride; const uint8_t* status; const int* counts; int counts_stride; int n;
-    __device__ int begin(int) const { return 0; }
-    __device__ int end(int f) const { return counts ? counts[(size_t)f * counts_stride] : n; }
-    __device__ bool load(int f, int i, double& px, double& py, double& ux, double& uy) const {
-        const size_t o = (size_t)f * stride + i;
-        if (status && !status[o]) return false;
-        const double4 v = xu[o];
-        px = v.x; py = v.y; ux = v.z; uy = v.w;
-        return true;
-    }
-    __device__ bool dist(int, int, double&) const { return false; }
-};

@@ -17,36 +17,29 @@
 #include "camera.cuh"
 #include "gyro.cuh"
 #include <stddef.h>
+#include <type_traits>
 
 namespace {
 
-struct TrackLoader {
-    const float* prev; const float* next; const uint8_t* status;
-    const int* counts; int counts_stride; size_t stride;
-    double cx, cy, ps, fs;
-    __device__ int begin(int) const { return 0; }
-    __device__ int end(int f) const { return counts[(size_t)f * counts_stride]; }
-    __device__ bool load(int f, int i, double& px, double& py, double& ux, double& uy) const {
-        size_t o = (size_t)f * stride + i;
-        if (!status[o]) return false;                       // new_pos[status==1]  (node:134, evaluate_exp.py:99)
-        float nx = next[2 * o], ny = next[2 * o + 1];
-        float dx = nx - prev[2 * o], dy = ny - prev[2 * o + 1];   // flow formed in fp32 as cv2 arrays are (node:136)
-        px = ((double)nx - cx) * ps; py = ((double)ny - cy) * ps;  // node:232-233
-        ux = (double)dx * fs; uy = (double)dy * fs;                // node:235
-        return true;
-    }
-    __device__ bool dist(int, int, double&) const { return false; }
-};
-
-// EGO: the ego-motion solve of the pair follows on the same points (ego[f]); EGO = false is the velocity solve alone
-template <bool EGO, class Loader>
-__device__ __forceinline__ void pair_solve(const Loader& ld, int variant, const ofb_imu_sample* __restrict__ imu,
-                                           ofb_pair_result* __restrict__ out, const FeatImageState* __restrict__ det,
-                                           ofb_ego_result* __restrict__ ego)
+// One CTA per pair: the velocity solve; with EGO the ego-motion solve and with ROBUST the robust velocity solve of the pair
+// follow on the same points (ego[f], rob[f]). CALIB: every tracked point is undistorted once into ld.xu first.
+template <bool EGO, bool ROBUST, bool CALIB>
+__global__ void __launch_bounds__(OFB_SOLVE_THREADS)
+pair_solve_kernel(TrackLoader<CALIB> ld, ofb_camera cam, int variant, const ofb_imu_sample* __restrict__ imu,
+                  ofb_pair_result* __restrict__ out, const FeatImageState* __restrict__ det, ofb_ego_result* __restrict__ ego,
+                  ofb_robust_cfg rcfg, ofb_robust_result* __restrict__ rob)
 {
-    int f = blockIdx.x;
+    const int f = blockIdx.x;
+    if (CALIB) {
+        const int n = ld.end(f);
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            const size_t o = (size_t)f * ld.stride + i;
+            if (ld.status[o]) ld.xu[o] = ofb_calibrate(cam, ld.next[2 * o], ld.next[2 * o + 1], ld.prev[2 * o], ld.prev[2 * o + 1]);
+        }
+        __syncthreads();
+    }
     const ofb_imu_sample& s = imu[f];
-    OfbSolveOut o = ofb_block_solve(ld, f, variant, s.d, s.n, s.w, s.t);
+    const OfbSolveOut o = ofb_block_solve(ld, f, variant, s.d, s.n, s.w, s.t);
     if (threadIdx.x == 0) {
         ofb_pair_result r;
         for (int k = 0; k < 3; ++k) { r.v[k] = o.v[k]; r.s[k] = o.s[k]; }
@@ -60,56 +53,10 @@ __device__ __forceinline__ void pair_solve(const Loader& ld, int variant, const 
         const OfbEgoOut e = ofb_block_solve_ego(ld, f, variant, s.d, s.n, s.t);
         if (threadIdx.x == 0) ego[f] = ofb_ego_record(e, OFB_EGO_SOLVED);
     }
-}
-
-// ROBUST: pair_solve, then the robust velocity solve of the pair on the same points (rob[f]). The ROBUST kernels see their
-// loader through a type of their own: the solve functions they instantiate, and the shared arrays inside them, are then
-// not shared with the ROBUST = false kernels, which keep their machine code.
-template <class L> struct RobustPass : L {};
-
-template <bool EGO, class Loader>
-__device__ __forceinline__ void pair_solve_robust(const Loader& ld, int variant, const ofb_imu_sample* __restrict__ imu,
-                                                  ofb_pair_result* __restrict__ out, const FeatImageState* __restrict__ det,
-                                                  ofb_ego_result* __restrict__ ego, const ofb_robust_cfg& rcfg,
-                                                  ofb_robust_result* __restrict__ rob)
-{
-    const RobustPass<Loader> rl{ld};
-    pair_solve<EGO>(rl, variant, imu, out, det, ego);
-    const int f = blockIdx.x;
-    const ofb_imu_sample& s = imu[f];
-    const OfbRobustOut r = ofb_block_solve_robust(rl, f, variant, s.d, s.n, s.w, s.t, rcfg.c, rcfg.iterations);
-    if (threadIdx.x == 0) rob[f] = ofb_robust_record(r, OFB_ROBUST_SOLVED);
-}
-
-template <bool EGO, bool ROBUST = false>
-__global__ void __launch_bounds__(OFB_SOLVE_THREADS)
-pair_solve_kernel(TrackLoader ld, int variant, const ofb_imu_sample* __restrict__ imu, ofb_pair_result* __restrict__ out,
-                  const FeatImageState* __restrict__ det, ofb_ego_result* __restrict__ ego, ofb_robust_cfg rcfg,
-                  ofb_robust_result* __restrict__ rob)
-{
-    if constexpr (ROBUST) pair_solve_robust<EGO>(ld, variant, imu, out, det, ego, rcfg, rob);
-    else pair_solve<EGO>(ld, variant, imu, out, det, ego);
-}
-
-// With a calibrated camera: every tracked point is undistorted once into xu (the solve reads each point twice), then
-// solved from there.
-template <bool EGO, bool ROBUST = false>
-__global__ void __launch_bounds__(OFB_SOLVE_THREADS)
-pair_solve_cam_kernel(TrackLoader tl, ofb_camera cam, double4* __restrict__ xu, int variant,
-                      const ofb_imu_sample* __restrict__ imu, ofb_pair_result* __restrict__ out,
-                      const FeatImageState* __restrict__ det, ofb_ego_result* __restrict__ ego, ofb_robust_cfg rcfg,
-                      ofb_robust_result* __restrict__ rob)
-{
-    const int f = blockIdx.x, n = tl.end(f);
-    for (int i = threadIdx.x; i < n; i += blockDim.x) {
-        const size_t o = (size_t)f * tl.stride + i;
-        if (tl.status[o]) xu[o] = ofb_calibrate(cam, tl.next[2 * o], tl.next[2 * o + 1], tl.prev[2 * o], tl.prev[2 * o + 1]);
+    if (ROBUST) {
+        const OfbRobustOut r = ofb_block_solve_robust(ld, f, variant, s.d, s.n, s.w, s.t, rcfg.c, rcfg.iterations);
+        if (threadIdx.x == 0) rob[f] = ofb_robust_record(r, OFB_ROBUST_SOLVED);
     }
-    __syncthreads();
-    if constexpr (ROBUST)
-        pair_solve_robust<EGO>(CalibLoader{xu, tl.stride, tl.status, tl.counts, tl.counts_stride, 0}, variant, imu, out, det, ego,
-                               rcfg, rob);
-    else pair_solve<EGO>(CalibLoader{xu, tl.stride, tl.status, tl.counts, tl.counts_stride, 0}, variant, imu, out, det, ego);
 }
 
 }  // namespace
@@ -193,20 +140,21 @@ static int run_pairs_chunk(ofb_ctx* ctx, const ofb_pair_cfg* cfg, const ofb_came
                           cfg->max_level, cfg->max_count, cfg->eps, lk_flags, cfg->min_eig_thr, cn, cs,
                           ctx->scratch[SC_ERR].as<float>(), fb_max_err));
     STAGE_MARK(4);
-    TrackLoader ld{cp, cn, cs, counts, counts_stride, (size_t)K, cfg->cx, cfg->cy, cfg->pos_scale, cfg->flow_scale};
-    ofb_ego_result* ego = d_ego ? d_ego + c0 : nullptr;
-    ofb_robust_result* rob = d_rob ? d_rob + c0 : nullptr;
+    double4* xu = nullptr;
     if (cam) {
         OFB_TRY(ctx->scratch[SC_CALIB].reserve(sizeof(double4) * (size_t)n * K));
-        auto kern = d_ego ? (d_rob ? pair_solve_cam_kernel<true, true> : pair_solve_cam_kernel<true>)
-                          : (d_rob ? pair_solve_cam_kernel<false, true> : pair_solve_cam_kernel<false>);
-        kern<<<n, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, *cam, ctx->scratch[SC_CALIB].as<double4>(), cfg->variant, dimu + c0,
-                                                       d_res + c0, st, ego, rcfg, rob);
-    } else {
-        auto kern = d_ego ? (d_rob ? pair_solve_kernel<true, true> : pair_solve_kernel<true>)
-                          : (d_rob ? pair_solve_kernel<false, true> : pair_solve_kernel<false>);
-        kern<<<n, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, cfg->variant, dimu + c0, d_res + c0, st, ego, rcfg, rob);
+        xu = ctx->scratch[SC_CALIB].as<double4>();
     }
+    auto launch = [&](auto calib) {
+        constexpr bool C = decltype(calib)::value;
+        const TrackLoader<C> ld{cp, cn, cs, counts, counts_stride, 0, (size_t)K, cfg->cx, cfg->cy, cfg->pos_scale, cfg->flow_scale, xu};
+        auto kern = d_ego ? (d_rob ? pair_solve_kernel<true, true, C> : pair_solve_kernel<true, false, C>)
+                          : (d_rob ? pair_solve_kernel<false, true, C> : pair_solve_kernel<false, false, C>);
+        kern<<<n, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, cam ? *cam : ofb_camera{}, cfg->variant, dimu + c0, d_res + c0, st,
+                                                       d_ego ? d_ego + c0 : nullptr, rcfg, d_rob ? d_rob + c0 : nullptr);
+    };
+    if (cam) launch(std::true_type{});
+    else launch(std::false_type{});
     OFB_LAUNCH_CHECK(ctx);
     STAGE_MARK(5);
 #undef STAGE_MARK

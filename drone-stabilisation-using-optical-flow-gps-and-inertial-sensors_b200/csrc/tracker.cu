@@ -22,6 +22,7 @@
 #include "camera.cuh"
 #include "gyro.cuh"
 #include <stddef.h>
+#include <type_traits>
 
 struct ofb_tracker {
     ofb_ctx* ctx = nullptr;
@@ -100,22 +101,6 @@ struct TrackerDev {
     FeatImageState* feat_state; int* cell_grid; size_t cell_stride; // detector scratch, reset here instead of by memsets
 };
 
-struct KeptLoader {
-    const float* prev; const float* next; int n; size_t stride;
-    double cx, cy, ps, fs;
-    __device__ int begin(int) const { return 0; }
-    __device__ int end(int) const { return n; }
-    __device__ bool load(int f, int i, double& px, double& py, double& ux, double& uy) const {
-        size_t o = (size_t)f * stride + i;
-        float nx = next[2 * o], ny = next[2 * o + 1];
-        float dx = nx - prev[2 * o], dy = ny - prev[2 * o + 1];     // fp32 flow, as cv2's float32 arrays (node:136)
-        px = ((double)nx - cx) * ps; py = ((double)ny - cy) * ps;    // node:232-233
-        ux = (double)dx * fs; uy = (double)dy * fs;                  // node:235
-        return true;
-    }
-    __device__ bool dist(int, int, double&) const { return false; }   // MODULE: distances from the prior velocity
-};
-
 // of.r_tilde (of_library.py:365-386, 5-argument form), feasibility value only
 __device__ __forceinline__ double r_tilde_point(double px, double py, double ux, double uy, const double n3[3],
                                                 const double v[3])
@@ -132,12 +117,12 @@ __device__ __forceinline__ double r_tilde_point(double px, double py, double ux,
 
 // EGO: the ego-motion solve of the stream follows the velocity solve on the same kept points (ego[s], zero with flags 0
 // when the stream did not solve); ROBUST: then the robust velocity solve under rcfg (rob[s], likewise). Both false is
-// the velocity solve alone.
+// the velocity solve alone. CALIB (a camera is attached): the solves read the kept points' calibrated values (T.calib).
 // PART 0: filter + solve in one launch. PART 1: the filter alone (compaction, gates, counts, top-up decision -- all the next
 // step's LK needs); PART 2: the solve of a stream an earlier PART 1 launch compacted. The split lets the solve run beside
 // the next frame's LK on a stream of its own: nothing but the NEXT filter (its r_tilde gate uses the solved velocity) and
 // the reader of the result record depend on it.
-template <int PART, bool EGO = false, bool ROBUST = false>
+template <int PART, bool EGO = false, bool ROBUST = false, bool CALIB = false>
 __global__ void __launch_bounds__(OFB_SOLVE_THREADS)
 track_filter_solve_kernel(TrackerDev T, const ofb_imu_sample* __restrict__ imu, const double* __restrict__ v_prior,
                           ofb_track_result* __restrict__ out, ofb_ego_result* __restrict__ ego, ofb_robust_cfg rcfg,
@@ -217,43 +202,18 @@ track_filter_solve_kernel(TrackerDev T, const ofb_imu_sample* __restrict__ imu, 
             T.calib[o] = ofb_calibrate(*T.cam, T.kept_next[2 * o], T.kept_next[2 * o + 1], T.kept_prev[2 * o], T.kept_prev[2 * o + 1]);
         }
     if (PART != 2) {
-        // tracked: every lane of a warp holds its warp's total; sum over warps
+        // tracked: every lane of a warp holds its warp's total; the record takes the sum over warps
         if (lane == 0) wtot[warp] = tracked;
-        __syncthreads();
-        tracked = 0;
-#pragma unroll
-        for (int k = 0; k < OFB_SOLVE_THREADS / 32; ++k) tracked += wtot[k];
-        __syncthreads();                                              // kept_* visible to the whole CTA
+        __syncthreads();                                              // wtot and kept_* visible to the whole CTA
     }
-    OfbSolveOut o;
     const bool solve = T.have_prev && kept >= T.min_solve && kept > 0;
-    if (PART != 1 && solve) {                                         // vp: MODULE's per-point distances (of_module.py:125)
-        if (T.cam) {
-            o = ofb_block_solve(CalibLoader{T.calib, (size_t)T.cap, nullptr, nullptr, 0, kept}, s, T.variant, im.d, im.n, im.w, im.t, vp);
-        } else {
-            KeptLoader ld{T.kept_prev, T.kept_next, kept, (size_t)T.cap, T.cx, T.cy, T.ps, T.fs};
-            o = ofb_block_solve(ld, s, T.variant, im.d, im.n, im.w, im.t, vp);
-        }
-    }
+    const TrackLoader<CALIB> ld{T.kept_prev, T.kept_next, nullptr, nullptr, 0, kept, (size_t)T.cap, T.cx, T.cy, T.ps, T.fs, T.calib};
+    OfbSolveOut o;                                                    // vp: MODULE's per-point distances (of_module.py:125)
+    if (PART != 1 && solve) o = ofb_block_solve(ld, s, T.variant, im.d, im.n, im.w, im.t, vp);
     OfbEgoOut e;
-    if (EGO && PART != 1 && solve) {
-        if (T.cam) {
-            e = ofb_block_solve_ego(CalibLoader{T.calib, (size_t)T.cap, nullptr, nullptr, 0, kept}, s, T.variant, im.d, im.n, im.t);
-        } else {
-            KeptLoader ld{T.kept_prev, T.kept_next, kept, (size_t)T.cap, T.cx, T.cy, T.ps, T.fs};
-            e = ofb_block_solve_ego(ld, s, T.variant, im.d, im.n, im.t);
-        }
-    }
+    if (EGO && PART != 1 && solve) e = ofb_block_solve_ego(ld, s, T.variant, im.d, im.n, im.t);
     OfbRobustOut rb;
-    if (ROBUST && PART != 1 && solve) {
-        if (T.cam) {
-            rb = ofb_block_solve_robust(CalibLoader{T.calib, (size_t)T.cap, nullptr, nullptr, 0, kept}, s, T.variant, im.d, im.n, im.w,
-                                        im.t, rcfg.c, rcfg.iterations);
-        } else {
-            KeptLoader ld{T.kept_prev, T.kept_next, kept, (size_t)T.cap, T.cx, T.cy, T.ps, T.fs};
-            rb = ofb_block_solve_robust(ld, s, T.variant, im.d, im.n, im.w, im.t, rcfg.c, rcfg.iterations);
-        }
-    }
+    if (ROBUST && PART != 1 && solve) rb = ofb_block_solve_robust(ld, s, T.variant, im.d, im.n, im.w, im.t, rcfg.c, rcfg.iterations);
     // the detector's per-image state and (for streams that will top up) its min-distance cell grid start clean
     if (PART != 2 && kept <= T.min_features)
         for (size_t i = tid; i < T.cell_stride; i += OFB_SOLVE_THREADS) T.cell_grid[(size_t)s * T.cell_stride + i] = -1;
@@ -276,6 +236,9 @@ track_filter_solve_kernel(TrackerDev T, const ofb_imu_sample* __restrict__ imu, 
         if (PART != 2) {
             FeatImageState z; z.max_key = 0; z.n_cand = 0; z.n_out = 0; z.overflow = 0;
             T.feat_state[s] = z;
+            tracked = 0;
+#pragma unroll
+            for (int k = 0; k < OFB_SOLVE_THREADS / 32; ++k) tracked += wtot[k];
             r.n_prev = n; r.n_tracked = tracked; r.n_kept = kept; r.n_added = 0; r.n_points = kept;
             const int need = kept <= T.min_features;
             T.kept[s] = kept;
@@ -699,19 +662,24 @@ static int tracker_step_launches(ofb_tracker* t, const uint8_t* frames, int pitc
         OFB_LAUNCH_CHECK(ctx);
         OFB_CUDA(cudaEventRecord(t->ev_filt, ctx->stream));
         OFB_CUDA(cudaStreamWaitEvent(t->sol_stream, t->ev_filt, 0));
-        auto kern = t->ego ? (t->robust ? track_filter_solve_kernel<2, true, true> : track_filter_solve_kernel<2, true>)
-                           : (t->robust ? track_filter_solve_kernel<2, false, true> : track_filter_solve_kernel<2>);
-        kern<<<S, OFB_SOLVE_THREADS, 0, t->sol_stream>>>(T, (const ofb_imu_sample*)dimu, (const double*)dvp, (ofb_track_result*)o[0].dev,
-                                                         d_ego, t->rcfg, d_rob);
-        OFB_LAUNCH_CHECK(ctx);
+    }
+    // the solve: in one launch with the filter, or (split) on the solve stream behind the filter launched above; CALIB when
+    // a camera is attached (attaching or detaching one drops the captured graphs)
+    auto launch = [&](auto calib) {
+        constexpr bool C = decltype(calib)::value;
+        auto kern = split ? (t->ego ? (t->robust ? track_filter_solve_kernel<2, true, true, C> : track_filter_solve_kernel<2, true, false, C>)
+                                    : (t->robust ? track_filter_solve_kernel<2, false, true, C> : track_filter_solve_kernel<2, false, false, C>))
+                          : (t->ego ? (t->robust ? track_filter_solve_kernel<0, true, true, C> : track_filter_solve_kernel<0, true, false, C>)
+                                    : (t->robust ? track_filter_solve_kernel<0, false, true, C> : track_filter_solve_kernel<0, false, false, C>));
+        kern<<<S, OFB_SOLVE_THREADS, 0, split ? t->sol_stream : ctx->stream>>>(T, (const ofb_imu_sample*)dimu, (const double*)dvp,
+                                                                               (ofb_track_result*)o[0].dev, d_ego, t->rcfg, d_rob);
+    };
+    if (t->has_cam) launch(std::true_type{});
+    else launch(std::false_type{});
+    OFB_LAUNCH_CHECK(ctx);
+    if (split) {
         OFB_CUDA(cudaEventRecord(t->ev_sol, t->sol_stream));
         t->sol_pending = true;
-    } else {
-        auto kern = t->ego ? (t->robust ? track_filter_solve_kernel<0, true, true> : track_filter_solve_kernel<0, true>)
-                           : (t->robust ? track_filter_solve_kernel<0, false, true> : track_filter_solve_kernel<0>);
-        kern<<<S, OFB_SOLVE_THREADS, 0, ctx->stream>>>(T, (const ofb_imu_sample*)dimu, (const double*)dvp, (ofb_track_result*)o[0].dev,
-                                                       d_ego, t->rcfg, d_rob);
-        OFB_LAUNCH_CHECK(ctx);
     }
     bool host_out = false;
     auto copy_out = [&](float* dst, const float* src) -> int {
@@ -892,6 +860,15 @@ extern "C" int ofb_tracker_step_robust(ofb_tracker* t, const uint8_t* frames, in
                                  rob);
 }
 
+// A setting that changes what a step launches, or a launch argument, makes the graphs captured before it stale: they are
+// rebuilt on the next eligible step (no graph is in flight: a replayed step synchronises before it returns).
+static void tracker_drop_graphs(ofb_tracker* t)
+{
+    for (int i = 0; i < 2; ++i)
+        for (int j = 0; j < 2; ++j)
+            if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
+}
+
 extern "C" int ofb_tracker_set_camera(ofb_tracker* t, const ofb_camera* cam)
 {
     OFB_REQUIRE(t, "tracker_set_camera: null tracker");
@@ -909,11 +886,8 @@ extern "C" int ofb_tracker_set_camera(ofb_tracker* t, const ofb_camera* cam)
         OFB_CUDA(cudaMemcpyAsync(t->cam_dev.p, &t->cam_host, sizeof(ofb_camera), cudaMemcpyHostToDevice, ctx->stream));
     }
     if (t->has_cam != (cam != nullptr)) {
-        // attaching or detaching changes the filter kernel's arguments: graphs captured before are rebuilt (no graph is in
-        // flight: a replayed step synchronises before it returns)
-        for (int i = 0; i < 2; ++i)
-            for (int j = 0; j < 2; ++j)
-                if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
+        // attaching or detaching changes the solve kernel and the filter kernel's arguments
+        tracker_drop_graphs(t);
         t->has_cam = cam != nullptr;
     }
     return OFB_OK;
@@ -924,11 +898,8 @@ extern "C" int ofb_tracker_set_fb_check(ofb_tracker* t, double fb_max_err)
     OFB_REQUIRE(t, "tracker_set_fb_check: null tracker");
     OFB_REQUIRE(ofb_fb_thr_ok(fb_max_err), "tracker_set_fb_check: fb_max_err must be >= 0 (0 = off)");
     if (fb_max_err != t->fb_max_err) {
-        // the threshold is an argument of the LK launch: graphs captured with the old value are rebuilt (no graph is in
-        // flight: a replayed step synchronises before it returns)
-        for (int i = 0; i < 2; ++i)
-            for (int j = 0; j < 2; ++j)
-                if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
+        // the threshold is an argument of the LK launch
+        tracker_drop_graphs(t);
         t->fb_max_err = fb_max_err;
     }
     return OFB_OK;
@@ -942,11 +913,8 @@ extern "C" int ofb_tracker_set_gyro_prediction(ofb_tracker* t, int enable)
         OFB_TRY(ofb_gyro_pinhole(&t->cfg.pair, "tracker_set_gyro_prediction", &gph));
     }
     if ((enable != 0) != t->gyro) {
-        // the prediction is a launch of the step and the LK flags are a launch argument: graphs captured before are
-        // rebuilt (no graph is in flight: a replayed step synchronises before it returns)
-        for (int i = 0; i < 2; ++i)
-            for (int j = 0; j < 2; ++j)
-                if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
+        // the prediction is a launch of the step and the LK flags are a launch argument
+        tracker_drop_graphs(t);
         t->gyro = enable != 0;
     }
     return OFB_OK;
@@ -958,11 +926,8 @@ extern "C" int ofb_tracker_set_ego_motion(ofb_tracker* t, int enable)
     OFB_REQUIRE(!enable || t->cfg.pair.variant != OFB_VARIANT_MODULE,
                 "tracker_set_ego_motion: the MODULE variant has no gyro term to estimate");
     if ((enable != 0) != t->ego) {
-        // the solve kernel is chosen when a step is enqueued: graphs captured before are rebuilt (no graph is in flight: a
-        // replayed step synchronises before it returns)
-        for (int i = 0; i < 2; ++i)
-            for (int j = 0; j < 2; ++j)
-                if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
+        // the solve kernel is chosen when a step is enqueued
+        tracker_drop_graphs(t);
         t->ego = enable != 0;
     }
     return OFB_OK;
@@ -977,11 +942,8 @@ extern "C" int ofb_tracker_set_robust(ofb_tracker* t, const ofb_robust_cfg* cfg)
     }
     const bool on = cfg != nullptr;
     if (on != t->robust || (on && (cfg->c != t->rcfg.c || cfg->iterations != t->rcfg.iterations))) {
-        // the kernel and its setting are chosen when a step is enqueued: graphs captured before are rebuilt (no graph is in
-        // flight: a replayed step synchronises before it returns)
-        for (int i = 0; i < 2; ++i)
-            for (int j = 0; j < 2; ++j)
-                if (t->gexec[i][j]) { cudaGraphExecDestroy(t->gexec[i][j]); t->gexec[i][j] = nullptr; }
+        // the kernel and its setting are chosen when a step is enqueued
+        tracker_drop_graphs(t);
         t->robust = on;
         t->rcfg = on ? *cfg : ofb_robust_cfg{0.0, 0};
     }

@@ -29,9 +29,8 @@ struct PointsF64 {          // x,u as n x ld doubles, frame f covers [offsets[f]
     __device__ bool dist(int, int i, double& d) const { if (!dists) return false; d = dists[i]; return true; }
 };
 
-template <class Loader>
 __global__ void __launch_bounds__(OFB_SOLVE_THREADS)
-solve_velocity_kernel(Loader ld, int variant, const double* __restrict__ d_arr, const double* __restrict__ n_arr,
+solve_velocity_kernel(PointsF64 ld, int variant, const double* __restrict__ d_arr, const double* __restrict__ n_arr,
                       const double* __restrict__ w_arr, const double* __restrict__ t_arr, int d_stride, int imu_stride,
                       double* __restrict__ v_out, double* __restrict__ res_out, int* __restrict__ rank_out,
                       double* __restrict__ s_out, int* __restrict__ count_out, const double* __restrict__ vprior_arr)
@@ -158,6 +157,35 @@ __global__ void feasibility_kernel(const double* __restrict__ x, double3 v, cons
 
 inline double3 d3(const double* p) { return make_double3(p[0], p[1], p[2]); }
 
+// The device inputs of a batched solve. x and u hold offsets[n_frames] rows.
+struct BatchIn { const void *x, *u, *offsets, *d, *n3, *w3, *t3; int total; };
+
+// Copies the offsets to the host (they size the point copies), checks them and stages x, u, offsets, d, n3 and the
+// optional w3 and t3 (NULL: not staged). `who` prefixes the error messages.
+int stage_batch(ofb_ctx* ctx, const char* who, const double* x, const double* u, const int* offsets, int n_frames,
+                const double* d, const double* n3, const double* w3, const double* t3, BatchIn* in)
+{
+    std::vector<int> hoff(n_frames + 1);
+    if (ofb_is_device_ptr(offsets)) {
+        OFB_CUDA(cudaMemcpyAsync(hoff.data(), offsets, sizeof(int) * (n_frames + 1), cudaMemcpyDeviceToHost, ctx->stream));
+        OFB_CUDA(cudaStreamSynchronize(ctx->stream));
+    } else memcpy(hoff.data(), offsets, sizeof(int) * (n_frames + 1));
+    OFB_REQUIRE(hoff[0] >= 0, "%s: offsets[0] = %d is negative", who, hoff[0]);
+    for (int f = 0; f < n_frames; ++f)
+        OFB_REQUIRE(hoff[f + 1] >= hoff[f], "%s: offsets must be non-decreasing (offsets[%d] = %d > offsets[%d] = %d)", who, f, hoff[f],
+                    f + 1, hoff[f + 1]);
+    *in = BatchIn{};
+    in->total = hoff[n_frames];
+    OFB_TRY(ofb_stage_in(ctx, SC_IN0, x, sizeof(double) * 2 * (size_t)in->total, &in->x));
+    OFB_TRY(ofb_stage_in(ctx, SC_IN1, u, sizeof(double) * 2 * (size_t)in->total, &in->u));
+    OFB_TRY(ofb_stage_in(ctx, SC_IN2, offsets, sizeof(int) * (n_frames + 1), &in->offsets));
+    OFB_TRY(ofb_stage_in(ctx, SC_IN3, d, sizeof(double) * n_frames, &in->d));
+    OFB_TRY(ofb_stage_in(ctx, SC_IN4, n3, sizeof(double) * 3 * n_frames, &in->n3));
+    if (w3) OFB_TRY(ofb_stage_in(ctx, SC_IN5, w3, sizeof(double) * 3 * n_frames, &in->w3));
+    if (t3) OFB_TRY(ofb_stage_in(ctx, SC_TMP0, t3, sizeof(double) * 3 * n_frames, &in->t3));
+    return OFB_OK;
+}
+
 }  // namespace
 
 extern "C" int ofb_solve_velocity_batched(ofb_ctx* ctx, int variant, const double* x, const double* u,
@@ -169,34 +197,16 @@ extern "C" int ofb_solve_velocity_batched(ofb_ctx* ctx, int variant, const doubl
     OFB_REQUIRE(variant >= 0 && variant <= 2, "solve_velocity: unknown variant %d", variant);
     OFB_REQUIRE(n_frames > 0, "solve_velocity_batched: n_frames must be positive");
     OFB_CUDA(cudaSetDevice(ctx->device));
-    // offsets are needed on the host to size the copies
-    std::vector<int> hoff(n_frames + 1);
-    if (ofb_is_device_ptr(offsets)) {
-        OFB_CUDA(cudaMemcpyAsync(hoff.data(), offsets, sizeof(int) * (n_frames + 1), cudaMemcpyDeviceToHost, ctx->stream));
-        OFB_CUDA(cudaStreamSynchronize(ctx->stream));
-    } else memcpy(hoff.data(), offsets, sizeof(int) * (n_frames + 1));
-    OFB_REQUIRE(hoff[0] >= 0, "solve_velocity_batched: offsets[0] = %d is negative", hoff[0]);
-    for (int f = 0; f < n_frames; ++f)
-        OFB_REQUIRE(hoff[f + 1] >= hoff[f], "solve_velocity_batched: offsets must be non-decreasing (offsets[%d] = %d > offsets[%d] = %d)",
-                    f, hoff[f], f + 1, hoff[f + 1]);
-    int total = hoff[n_frames];                       // x and u must hold at least this many rows
-    const void *dx, *du, *doff, *dd, *dn, *dw, *dt = nullptr;
-    OFB_TRY(ofb_stage_in(ctx, SC_IN0, x, sizeof(double) * 2 * (size_t)total, &dx));
-    OFB_TRY(ofb_stage_in(ctx, SC_IN1, u, sizeof(double) * 2 * (size_t)total, &du));
-    OFB_TRY(ofb_stage_in(ctx, SC_IN2, offsets, sizeof(int) * (n_frames + 1), &doff));
-    OFB_TRY(ofb_stage_in(ctx, SC_IN3, d, sizeof(double) * n_frames, &dd));
-    OFB_TRY(ofb_stage_in(ctx, SC_IN4, n3, sizeof(double) * 3 * n_frames, &dn));
-    OFB_TRY(ofb_stage_in(ctx, SC_IN5, w3, sizeof(double) * 3 * n_frames, &dw));
-    if (t3) OFB_TRY(ofb_stage_in(ctx, SC_TMP0, t3, sizeof(double) * 3 * n_frames, &dt));
+    BatchIn in;
+    OFB_TRY(stage_batch(ctx, "solve_velocity_batched", x, u, offsets, n_frames, d, n3, w3, t3, &in));
     OutStage o[4];
     OFB_TRY(ofb_stage_out(ctx, SC_OUT0, v_out, sizeof(double) * 3 * n_frames, &o[0]));
     OFB_TRY(ofb_stage_out(ctx, SC_OUT1, res, sizeof(double) * n_frames, &o[1]));
     OFB_TRY(ofb_stage_out(ctx, SC_OUT2, rank, sizeof(int) * n_frames, &o[2]));
     OFB_TRY(ofb_stage_out(ctx, SC_OUT3, s_out, sizeof(double) * 3 * n_frames, &o[3]));
-    PointsF64 ld{(const double*)dx, (const double*)du, (const int*)doff, 0};
-    if (total == 0 && !dx) { ld.x = ld.u = nullptr; }
-    solve_velocity_kernel<PointsF64><<<n_frames, OFB_SOLVE_THREADS, 0, ctx->stream>>>(
-        ld, variant, (const double*)dd, (const double*)dn, (const double*)dw, (const double*)dt, 1, 3,
+    const PointsF64 ld{(const double*)in.x, (const double*)in.u, (const int*)in.offsets, 0};
+    solve_velocity_kernel<<<n_frames, OFB_SOLVE_THREADS, 0, ctx->stream>>>(
+        ld, variant, (const double*)in.d, (const double*)in.n3, (const double*)in.w3, (const double*)in.t3, 1, 3,
         (double*)o[0].dev, (double*)o[1].dev, (int*)o[2].dev, (double*)o[3].dev, nullptr, nullptr);
     OFB_LAUNCH_CHECK(ctx);
     return ofb_finish_out(ctx, o, 4);
@@ -229,7 +239,7 @@ extern "C" int ofb_solve_velocity_module(ofb_ctx* ctx, const double* x, const do
     OFB_TRY(ofb_stage_out(ctx, SC_OUT3, s_out, sizeof(double) * 3, &o[3]));
     PointsF64 ldr{(const double*)dx, (const double*)du, nullptr, n};
     ldr.ld = ld; ldr.dists = (const double*)dd;
-    solve_velocity_kernel<PointsF64><<<1, OFB_SOLVE_THREADS, 0, ctx->stream>>>(
+    solve_velocity_kernel<<<1, OFB_SOLVE_THREADS, 0, ctx->stream>>>(
         ldr, OFB_VARIANT_MODULE, nullptr, (const double*)dn, (const double*)dw, nullptr, 1, 3,
         (double*)o[0].dev, (double*)o[1].dev, (int*)o[2].dev, (double*)o[3].dev, nullptr, (const double*)dvp);
     OFB_LAUNCH_CHECK(ctx);
@@ -256,28 +266,13 @@ extern "C" int ofb_solve_ego_motion_batched(ofb_ctx* ctx, int variant, const dou
     OFB_REQUIRE(variant >= 0 && variant <= 2, "solve_ego_motion: unknown variant %d (MODULE has no gyro term to estimate)", variant);
     OFB_REQUIRE(n_frames > 0, "solve_ego_motion_batched: n_frames must be positive");
     OFB_CUDA(cudaSetDevice(ctx->device));
-    std::vector<int> hoff(n_frames + 1);
-    if (ofb_is_device_ptr(offsets)) {
-        OFB_CUDA(cudaMemcpyAsync(hoff.data(), offsets, sizeof(int) * (n_frames + 1), cudaMemcpyDeviceToHost, ctx->stream));
-        OFB_CUDA(cudaStreamSynchronize(ctx->stream));
-    } else memcpy(hoff.data(), offsets, sizeof(int) * (n_frames + 1));
-    OFB_REQUIRE(hoff[0] >= 0, "solve_ego_motion_batched: offsets[0] = %d is negative", hoff[0]);
-    for (int f = 0; f < n_frames; ++f)
-        OFB_REQUIRE(hoff[f + 1] >= hoff[f], "solve_ego_motion_batched: offsets must be non-decreasing (offsets[%d] = %d > offsets[%d] = %d)",
-                    f, hoff[f], f + 1, hoff[f + 1]);
-    const int total = hoff[n_frames];
-    const void *dx, *du, *doff, *dd, *dn, *dt = nullptr;
-    OFB_TRY(ofb_stage_in(ctx, SC_IN0, x, sizeof(double) * 2 * (size_t)total, &dx));
-    OFB_TRY(ofb_stage_in(ctx, SC_IN1, u, sizeof(double) * 2 * (size_t)total, &du));
-    OFB_TRY(ofb_stage_in(ctx, SC_IN2, offsets, sizeof(int) * (n_frames + 1), &doff));
-    OFB_TRY(ofb_stage_in(ctx, SC_IN3, d, sizeof(double) * n_frames, &dd));
-    OFB_TRY(ofb_stage_in(ctx, SC_IN4, n3, sizeof(double) * 3 * n_frames, &dn));
-    if (t3) OFB_TRY(ofb_stage_in(ctx, SC_TMP0, t3, sizeof(double) * 3 * n_frames, &dt));
+    BatchIn in;
+    OFB_TRY(stage_batch(ctx, "solve_ego_motion_batched", x, u, offsets, n_frames, d, n3, nullptr, t3, &in));
     OutStage o;
     OFB_TRY(ofb_stage_out(ctx, SC_OUT0, out, sizeof(ofb_ego_result) * n_frames, &o));
-    PointsF64 ld{(const double*)dx, (const double*)du, (const int*)doff, 0};
-    solve_ego_kernel<<<n_frames, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, variant, (const double*)dd, (const double*)dn,
-                                                                       (const double*)dt, (ofb_ego_result*)o.dev);
+    const PointsF64 ld{(const double*)in.x, (const double*)in.u, (const int*)in.offsets, 0};
+    solve_ego_kernel<<<n_frames, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, variant, (const double*)in.d, (const double*)in.n3,
+                                                                       (const double*)in.t3, (ofb_ego_result*)o.dev);
     OFB_LAUNCH_CHECK(ctx);
     return ofb_finish_out(ctx, &o, 1);
 }
@@ -302,31 +297,15 @@ extern "C" int ofb_solve_velocity_robust_batched(ofb_ctx* ctx, int variant, cons
     OFB_TRY(ofb_robust_check(cfg, "solve_velocity_robust"));
     OFB_REQUIRE(n_frames > 0, "solve_velocity_robust_batched: n_frames must be positive");
     OFB_CUDA(cudaSetDevice(ctx->device));
-    std::vector<int> hoff(n_frames + 1);
-    if (ofb_is_device_ptr(offsets)) {
-        OFB_CUDA(cudaMemcpyAsync(hoff.data(), offsets, sizeof(int) * (n_frames + 1), cudaMemcpyDeviceToHost, ctx->stream));
-        OFB_CUDA(cudaStreamSynchronize(ctx->stream));
-    } else memcpy(hoff.data(), offsets, sizeof(int) * (n_frames + 1));
-    OFB_REQUIRE(hoff[0] >= 0, "solve_velocity_robust_batched: offsets[0] = %d is negative", hoff[0]);
-    for (int f = 0; f < n_frames; ++f)
-        OFB_REQUIRE(hoff[f + 1] >= hoff[f], "solve_velocity_robust_batched: offsets must be non-decreasing (offsets[%d] = %d > offsets[%d] = %d)",
-                    f, hoff[f], f + 1, hoff[f + 1]);
-    const int total = hoff[n_frames];
-    const void *dx, *du, *doff, *dd, *dn, *dw, *dt = nullptr;
-    OFB_TRY(ofb_stage_in(ctx, SC_IN0, x, sizeof(double) * 2 * (size_t)total, &dx));
-    OFB_TRY(ofb_stage_in(ctx, SC_IN1, u, sizeof(double) * 2 * (size_t)total, &du));
-    OFB_TRY(ofb_stage_in(ctx, SC_IN2, offsets, sizeof(int) * (n_frames + 1), &doff));
-    OFB_TRY(ofb_stage_in(ctx, SC_IN3, d, sizeof(double) * n_frames, &dd));
-    OFB_TRY(ofb_stage_in(ctx, SC_IN4, n3, sizeof(double) * 3 * n_frames, &dn));
-    OFB_TRY(ofb_stage_in(ctx, SC_IN5, w3, sizeof(double) * 3 * n_frames, &dw));
-    if (t3) OFB_TRY(ofb_stage_in(ctx, SC_TMP0, t3, sizeof(double) * 3 * n_frames, &dt));
+    BatchIn in;
+    OFB_TRY(stage_batch(ctx, "solve_velocity_robust_batched", x, u, offsets, n_frames, d, n3, w3, t3, &in));
     OutStage o[2];
     OFB_TRY(ofb_stage_out(ctx, SC_OUT0, out, sizeof(ofb_robust_result) * n_frames, &o[0]));
-    OFB_TRY(ofb_stage_out(ctx, SC_OUT1, weights_out, sizeof(double) * (size_t)total, &o[1]));
-    if (o[1].dev) OFB_CUDA(cudaMemsetAsync(o[1].dev, 0, sizeof(double) * (size_t)total, ctx->stream));   // rows in no frame
-    PointsF64 ld{(const double*)dx, (const double*)du, (const int*)doff, 0};
-    solve_robust_kernel<<<n_frames, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, variant, (const double*)dd, (const double*)dn,
-                                                                          (const double*)dw, (const double*)dt, *cfg,
+    OFB_TRY(ofb_stage_out(ctx, SC_OUT1, weights_out, sizeof(double) * (size_t)in.total, &o[1]));
+    if (o[1].dev) OFB_CUDA(cudaMemsetAsync(o[1].dev, 0, sizeof(double) * (size_t)in.total, ctx->stream));   // rows in no frame
+    const PointsF64 ld{(const double*)in.x, (const double*)in.u, (const int*)in.offsets, 0};
+    solve_robust_kernel<<<n_frames, OFB_SOLVE_THREADS, 0, ctx->stream>>>(ld, variant, (const double*)in.d, (const double*)in.n3,
+                                                                          (const double*)in.w3, (const double*)in.t3, *cfg,
                                                                           (ofb_robust_result*)o[0].dev, (double*)o[1].dev);
     OFB_LAUNCH_CHECK(ctx);
     return ofb_finish_out(ctx, o, 2);

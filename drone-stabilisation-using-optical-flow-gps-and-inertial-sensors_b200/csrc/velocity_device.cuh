@@ -66,8 +66,27 @@ __device__ __forceinline__ void ofb_block_sum(double (&acc)[K], double* smem /* 
     }
 }
 
-// ofb_block_solve's lstsq step and residual term for the robust solve below, which must reproduce the plain solve bit for
-// bit. ofb_block_solve keeps its own inline copy: calling these from it changes its machine code.
+// Adds one point's contribution, weighted by om, to the normal equations acc[0..5] v = d acc[6..8] and the count acc[9].
+// The plain solve passes om = 1, which multiplies exactly.
+__device__ __forceinline__ void ofb_normal_add(double (&acc)[10], const OfbPointTerms& t, double px, double py, double om)
+{
+    const double w2 = t.wA * t.wA * om;
+    const double xx = px * px, yy = py * py;
+    // |X|^2 I - X X^T
+    acc[0] += w2 * (yy + 1.0);      // xx
+    acc[1] += w2 * (-px * py);      // xy
+    acc[2] += w2 * (-px);           // xz
+    acc[3] += w2 * (xx + 1.0);      // yy
+    acc[4] += w2 * (-py);           // yz
+    acc[5] += w2 * (xx + yy);       // zz
+    // A^T b = -wA wb (X x beta)
+    const double s = -t.wA * t.wb * om;
+    acc[6] += s * (py * t.bz - t.by);
+    acc[7] += s * (t.bx - px * t.bz);
+    acc[8] += s * (px * t.by - py * t.bx);
+    acc[9] += 1.0;
+}
+
 // numpy lstsq (rcond=None) of the normal equations acc[0..5] v = d acc[6..8] (M packed xx, xy, xz, yy, yz, zz) of
 // acc[9] points (3 rows each): sets o.count, o.s and o.rank, returns the solution in v.
 __device__ __forceinline__ void ofb_lstsq3(const double (&acc)[10], double d, OfbSolveOut& o, double (&v)[3])
@@ -108,6 +127,38 @@ __device__ __forceinline__ double ofb_point_res2(const OfbPointTerms& t, double 
 // Loader concept: begin(f), end(f), load(f, i, px, py, ux, uy) -> bool (false = point skipped),
 // dist(f, i, d) -> bool (MODULE variant: true = per-point distance supplied by the caller, false = derive it from the
 // prior velocity `vprior` with the 4-argument r_tilde).
+
+// Loader over LK tracks (frame pairs, tracker): point i of frame f sits at o = f*stride + i, and is used when status is
+// NULL or status[o] != 0; points per frame from counts[f*counts_stride] (counts NULL: n). CALIB: xu[o] holds the point's
+// (x, y, ux, uy) of a calibrated camera, undistorted once before the solves (they read every point several times);
+// otherwise the pinhole model maps the track. CALIB is a compile-time choice: behind a runtime branch nvcc contracts the
+// pinhole flow scale differently into the solves' sums, and the pinhole results would change in the last bit.
+template <bool CALIB>
+struct TrackLoader {
+    const float* prev; const float* next;                            // (x, y) pairs
+    const uint8_t* status;
+    const int* counts; int counts_stride; int n; size_t stride;
+    double cx, cy, ps, fs;
+    double4* xu;
+    __device__ int begin(int) const { return 0; }
+    __device__ int end(int f) const { return counts ? counts[(size_t)f * counts_stride] : n; }
+    __device__ bool load(int f, int i, double& px, double& py, double& ux, double& uy) const {
+        const size_t o = (size_t)f * stride + i;
+        if (status && !status[o]) return false;                      // new_pos[status==1]  (node:134, evaluate_exp.py:99)
+        if constexpr (CALIB) {
+            const double4 v = xu[o];
+            px = v.x; py = v.y; ux = v.z; uy = v.w;
+        } else {
+            const float nx = next[2 * o], ny = next[2 * o + 1];
+            const float dx = nx - prev[2 * o], dy = ny - prev[2 * o + 1];   // flow formed in fp32 as cv2 arrays are (node:136)
+            px = ((double)nx - cx) * ps; py = ((double)ny - cy) * ps;         // node:232-233
+            ux = (double)dx * fs; uy = (double)dy * fs;                       // node:235
+        }
+        return true;
+    }
+    __device__ bool dist(int, int, double&) const { return false; }  // MODULE: distances from the prior velocity
+};
+
 template <class Loader>
 __device__ OfbSolveOut ofb_block_solve(const Loader& ld, int f, int variant, double d, const double* n3g,
                                        const double* w3g, const double* t3g, const double* vprior = nullptr)
@@ -136,57 +187,18 @@ __device__ OfbSolveOut ofb_block_solve(const Loader& ld, int f, int variant, dou
     for (int i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
         double px, py, ux, uy;
         if (!ld.load(f, i, px, py, ux, uy)) continue;
-        OfbPointTerms t = ofb_point_terms(variant, px, py, ux, uy, n3, w3, inv_dist(i, px, py, ux, uy));
-        double w2 = t.wA * t.wA;
-        double xx = px * px, yy = py * py;
-        // |X|^2 I - X X^T
-        acc[0] += w2 * (yy + 1.0);      // xx
-        acc[1] += w2 * (-px * py);      // xy
-        acc[2] += w2 * (-px);           // xz
-        acc[3] += w2 * (xx + 1.0);      // yy
-        acc[4] += w2 * (-py);           // yz
-        acc[5] += w2 * (xx + yy);       // zz
-        // A^T b = -wA wb (X x beta)
-        double s = -t.wA * t.wb;
-        acc[6] += s * (py * t.bz - t.by);
-        acc[7] += s * (t.bx - px * t.bz);
-        acc[8] += s * (px * t.by - py * t.bx);
-        acc[9] += 1.0;
+        ofb_normal_add(acc, ofb_point_terms(variant, px, py, ux, uy, n3, w3, inv_dist(i, px, py, ux, uy)), px, py, 1.0);
     }
     ofb_block_sum<10>(acc, red);
     OfbSolveOut o;
-    o.count = (int)(acc[9] + 0.5);
-    double M[6] = {acc[0], acc[1], acc[2], acc[3], acc[4], acc[5]};
-    double ev[3], q[3][3];
-    ofb_jacobi3(M, ev, q);
-    // numpy lstsq (rcond=None): singular values below eps*max(M,N)*s_max are treated as zero.
-    // s comes from eig(A^T A), so it cannot resolve below ~1e-8*s_max; use 1e-7 as the floor.
-    double rows = 3.0 * (double)o.count;
-    double rc = 2.220446049250313e-16 * (rows > 3.0 ? rows : 3.0);
-    if (rc < 1e-7) rc = 1e-7;
-    double smax = ev[0] > 0 ? sqrt(ev[0]) : 0.0;
-    int rank = 0;
-    double v[3] = {0, 0, 0};
-    for (int k = 0; k < 3; ++k) {
-        double sk = ev[k] > 0 ? sqrt(ev[k]) : 0.0;
-        o.s[k] = sk;
-        if (sk > rc * smax && smax > 0) {
-            ++rank;
-            double c = (q[k][0] * acc[6] + q[k][1] * acc[7] + q[k][2] * acc[8]) * d / ev[k];
-            v[0] += c * q[k][0]; v[1] += c * q[k][1]; v[2] += c * q[k][2];
-        }
-    }
-    o.rank = rank;
+    double v[3];
+    ofb_lstsq3(acc, d, o, v);
     // second pass: residual sum ||A_i v - d b_i||^2
     double r[1] = {0};
     for (int i = i0 + threadIdx.x; i < i1; i += blockDim.x) {
         double px, py, ux, uy;
         if (!ld.load(f, i, px, py, ux, uy)) continue;
-        OfbPointTerms t = ofb_point_terms(variant, px, py, ux, uy, n3, w3, inv_dist(i, px, py, ux, uy));
-        double rx = t.wA * (py * v[2] - v[1]) - d * t.wb * t.bx;
-        double ry = t.wA * (v[0] - px * v[2]) - d * t.wb * t.by;
-        double rz = t.wA * (px * v[1] - py * v[0]) - d * t.wb * t.bz;
-        r[0] += rx * rx + ry * ry + rz * rz;
+        r[0] += ofb_point_res2(ofb_point_terms(variant, px, py, ux, uy, n3, w3, inv_dist(i, px, py, ux, uy)), px, py, d, v);
     }
     ofb_block_sum<1>(r, red);
     o.res = r[0];
@@ -377,19 +389,7 @@ __device__ OfbRobustOut ofb_block_solve_robust(const Loader& ld, int f, int vari
                 om = ofb_tukey_weight(sqrt(ofb_point_res2(t, px, py, d, vw)), tau);
                 if (om == 0.0) continue;
             }
-            const double w2 = t.wA * t.wA * om;
-            const double xx = px * px, yy = py * py;
-            acc[0] += w2 * (yy + 1.0);
-            acc[1] += w2 * (-px * py);
-            acc[2] += w2 * (-px);
-            acc[3] += w2 * (xx + 1.0);
-            acc[4] += w2 * (-py);
-            acc[5] += w2 * (xx + yy);
-            const double s = -t.wA * t.wb * om;
-            acc[6] += s * (py * t.bz - t.by);
-            acc[7] += s * (t.bx - px * t.bz);
-            acc[8] += s * (px * t.by - py * t.bx);
-            acc[9] += 1.0;
+            ofb_normal_add(acc, t, px, py, om);
         }
         ofb_block_sum<10>(acc, red);
         ofb_lstsq3(acc, d, o, v);

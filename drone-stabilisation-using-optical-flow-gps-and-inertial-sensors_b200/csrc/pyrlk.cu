@@ -12,7 +12,7 @@
 // Scharr gradients of the (win+1)^2 footprint are formed there once, and the template patch and its
 // two interpolated gradients are kept in shared memory as int16 for the iterations. Each iteration
 // stages the (win+1)^2 window of J (reflect-101 fix-up only for windows that touch the border,
-// a warp-uniform branch), accumulates the mismatch vector in exact int32 per lane, reduces it with
+// a warp-uniform branch), accumulates the mismatch vector in exact int64 per lane, reduces it with
 // 64-bit shuffles and solves the 2x2 system redundantly in every lane's registers. OpenCV builds
 // full-frame Scharr images per level; here gradients are formed only under the windows, so the
 // derivative images (the largest share of OpenCV's LK time, SURVEY 6) never exist.
@@ -140,6 +140,8 @@ lk_track_kernel(LKParams P, const float* __restrict__ prev_pts, float* __restric
                 ders[i] = gx; ders[DW * DH + i] = gy;
             }
             __syncwarp();
+            // a lane sums at most ceil(4096 / 32) = 128 products of gradients |I'| <= 16 * 255 = 4080:
+            // 128 * 4080^2 = 2,130,739,200 < 2^31, so the A sums stay exact in int32
             int iA11 = 0, iA12 = 0, iA22 = 0;
             for (int i = lane; i < npx; i += 32) {
                 int y = i / winW, x = i - y * winW;
@@ -178,14 +180,16 @@ lk_track_kernel(LKParams P, const float* __restrict__ prev_pts, float* __restric
                 __syncwarp();
                 stage_block(J, w, h, jpitch, jx, jy, DW, DH, reg, RP, lane);
                 __syncwarp();
-                int ib1 = 0, ib2 = 0;
+                // |diff| <= 8160 (Q5) times |I'| <= 4080 over up to 128 pixels reaches 4.26e9: past 2048 window pixels
+                // (64 per lane) an int32 lane partial can wrap, so b is summed in 64 bits
+                long long ib1 = 0, ib2 = 0;
                 for (int i = lane; i < npx; i += 32) {
                     int y = i / winW, x = i - y * winW;
                     const uint8_t* s0 = reg + y * RP + x;
                     const uint8_t* s1 = s0 + RP;
                     int jv = ((int)s0[0] * w00 + (int)s0[1] * w01 + (int)s1[0] * w10 + (int)s1[1] * w11 + (1 << 8)) >> 9;
                     int diff = jv - (int)pat[i];
-                    ib1 += diff * (int)pat[npx + i];
+                    ib1 += diff * (int)pat[npx + i];        // (each product fits int32: |diff * I'| <= 3.33e7)
                     ib2 += diff * (int)pat[2 * npx + i];
                 }
                 float b1 = (float)warp_sum_ll(ib1) * FLT_SCALE;
@@ -275,8 +279,10 @@ __device__ __forceinline__ int dp2a_hi(int w16x2, unsigned int bytes, int c)
     return d;
 }
 
-// Column index reflected into [0, len): exact reflect-101 for p in [-len, 2*len) (two folds), which covers every
-// patch position the tracker can reach (|offset| <= window + 9 columns, len > window).
+// Column index reflected into [0, len): exact reflect-101 for |p| <= 3*len - 3 (three folds), then clamped. The kernel
+// reads columns -winW - 1 .. len + winW, so it is exact for winW <= 2*len - 3: on every level above 0 (len > winW
+// there, by OpenCV's window cut) and on level 0 images that are wide enough; ofb_lk_device sends narrower level 0
+// images to lk_track_kernel.
 __device__ __forceinline__ int refl_col(int p, int len)
 {
     p = p < 0 ? -p : p;
@@ -660,7 +666,8 @@ int ofb_lk_device(ofb_ctx* ctx, const ofb_pyr* prev, int prev_image0, int prev_s
     P.next_image0 = next_image0; P.next_image_step = next_step;
     if (n_uniform <= 0) return OFB_OK;
     const char* env = getenv("OFB_LK_GENERIC");      // parity tests cross-check the two kernels
-    if (win_w <= 16 && win_h <= 15 && !(env && env[0] == '1')) {
+    const bool narrow = win_w > 2 * prev->w[0] - 3;  // refl_col is not exact over the columns the fast kernel reads
+    if (win_w <= 16 && win_h <= 15 && !narrow && !(env && env[0] == '1')) {
         dim3 fgrid(ofb_div_up(n_uniform, LKF_WARPS), n_pairs);
         if (fb)
             lk_track_fast2_kernel<true><<<fgrid, LKF_WARPS * 32, 0, ctx->stream>>>(P, prev_pts, next_pts, status, err, counts,

@@ -108,7 +108,13 @@ def good_features(img, max_corners, quality, min_distance, mask=None, block_size
     return select_features(min_eig_map(img, block_size), max_corners, quality, min_distance, mask)
 
 
-def pyrlk(prev, nxt, prev_pts, win=(21, 21), max_level=3, criteria=(3, 30, 0.01), min_eig_thr=1e-4):
+ORC_LK_EXACT_SUMS = 1 << 16
+
+
+def pyrlk(prev, nxt, prev_pts, win=(21, 21), max_level=3, criteria=(3, 30, 0.01), min_eig_thr=1e-4, exact_sums=False):
+    """calcOpticalFlowPyrLK. exact_sums=False: OpenCV's fp32 running sums; True: A, b and the error summed exactly
+    in int64 and rounded to fp32 once, the arithmetic of the device kernels. As cv2, a criteria type without
+    TERM_CRITERIA_COUNT (1) means 30 iterations and one without TERM_CRITERIA_EPS (2) eps = 0.01."""
     prev = np.ascontiguousarray(prev, dtype=np.uint8)
     nxt = np.ascontiguousarray(nxt, dtype=np.uint8)
     h, w = prev.shape
@@ -117,7 +123,9 @@ def pyrlk(prev, nxt, prev_pts, win=(21, 21), max_level=3, criteria=(3, 30, 0.01)
     out = np.zeros((n, 2), np.float32)
     st = np.zeros(n, np.uint8)
     err = np.zeros(n, np.float32)
-    _, count, eps = criteria
-    lib().orc_pyrlk(_u8(prev), _u8(nxt), w, h, w, _f32(p), n, win[0], win[1], max_level, int(count),
-                    float(eps), 0, min_eig_thr, _f32(out), _u8(st), _f32(err))
+    typ, count, eps = criteria
+    count = int(count) if int(typ) & 1 else 30
+    eps = float(eps) if int(typ) & 2 else 0.01
+    lib().orc_pyrlk(_u8(prev), _u8(nxt), w, h, w, _f32(p), n, win[0], win[1], max_level, count,
+                    eps, ORC_LK_EXACT_SUMS if exact_sums else 0, min_eig_thr, _f32(out), _u8(st), _f32(err))
     return out.reshape(-1, 1, 2), st.reshape(-1, 1), err.reshape(-1, 1)

@@ -320,12 +320,18 @@ static inline void bil_weights(float a, float b, int* w00, int* w01, int* w10, i
     *w11 = (1 << W_BITS) - *w00 - *w01 - *w10;
 }
 
+/* flags: ORC_LK_EXACT_SUMS sums A, b and the L1 error as exact int64 integers and rounds each sum to fp32 once, as
+ * the device kernels do (their per-lane partials are exact integers, reduced in 64 bits); the error is then scaled by
+ * the fp32 reciprocal of 32 * win_w * win_h, as there. Without it the sums are OpenCV's running fp32 additions in
+ * window order and the error is divided, as lkpyramid.cpp does. */
+#define ORC_LK_EXACT_SUMS (1 << 16)
+
 ORC_API int orc_pyrlk(const uint8_t* prev, const uint8_t* next, int w, int h, int pitch,
                       const float* prev_pts, int n, int win_w, int win_h, int max_level,
                       int max_count, double eps_in, int flags, double min_eig_thr,
                       float* next_pts, uint8_t* status, float* err)
 {
-    (void)flags;
+    const int exact = (flags & ORC_LK_EXACT_SUMS) != 0;
     if (max_count < 0) max_count = 0; if (max_count > 100) max_count = 100;
     double e = eps_in < 0 ? 0 : eps_in > 10 ? 10 : eps_in;
     double eps = e * e;
@@ -361,6 +367,7 @@ ORC_API int orc_pyrlk(const uint8_t* prev, const uint8_t* next, int w, int h, in
             float a = px - ix, b = py - iy;
             int w00, w01, w10, w11; bil_weights(a, b, &w00, &w01, &w10, &w11);
             float A11 = 0, A12 = 0, A22 = 0;
+            long long iA11 = 0, iA12 = 0, iA22 = 0;
             for (int y = 0; y < win_h; ++y)
                 for (int x = 0; x < win_w; ++x) {
                     int X = ix + x, Y = iy + y;
@@ -371,8 +378,10 @@ ORC_API int orc_pyrlk(const uint8_t* prev, const uint8_t* next, int w, int h, in
                     int gy = (der_pad(I, I->dy, X, Y) * w00 + der_pad(I, I->dy, X + 1, Y) * w01 +
                               der_pad(I, I->dy, X, Y + 1) * w10 + der_pad(I, I->dy, X + 1, Y + 1) * w11 + (1 << (W_BITS1 - 1))) >> W_BITS1;
                     Ip[y * win_w + x] = (int16_t)iv; Dx[y * win_w + x] = (int16_t)gx; Dy[y * win_w + x] = (int16_t)gy;
-                    A11 += (float)(gx * gx); A12 += (float)(gx * gy); A22 += (float)(gy * gy);
+                    if (exact) { iA11 += gx * gx; iA12 += gx * gy; iA22 += gy * gy; }
+                    else { A11 += (float)(gx * gx); A12 += (float)(gx * gy); A22 += (float)(gy * gy); }
                 }
+            if (exact) { A11 = (float)iA11; A12 = (float)iA12; A22 = (float)iA22; }
             A11 *= FLT_SCALE; A12 *= FLT_SCALE; A22 *= FLT_SCALE;
             float D = A11 * A22 - A12 * A12;
             float minEig = (A22 + A11 - sqrtf((A11 - A22) * (A11 - A22) + 4.f * A12 * A12)) / (float)(2 * win_w * win_h);
@@ -392,15 +401,17 @@ ORC_API int orc_pyrlk(const uint8_t* prev, const uint8_t* next, int w, int h, in
                 a = qx - jx; b = qy - jy;
                 bil_weights(a, b, &w00, &w01, &w10, &w11);
                 float b1 = 0, b2 = 0;
+                long long ib1 = 0, ib2 = 0;
                 for (int y = 0; y < win_h; ++y)
                     for (int x = 0; x < win_w; ++x) {
                         int X = jx + x, Y = jy + y;
                         int jv = (img_pad(J, X, Y) * w00 + img_pad(J, X + 1, Y) * w01 +
                                   img_pad(J, X, Y + 1) * w10 + img_pad(J, X + 1, Y + 1) * w11 + (1 << (W_BITS - 5 - 1))) >> (W_BITS - 5);
                         int diff = jv - Ip[y * win_w + x];
-                        b1 += (float)(diff * Dx[y * win_w + x]);
-                        b2 += (float)(diff * Dy[y * win_w + x]);
+                        if (exact) { ib1 += diff * Dx[y * win_w + x]; ib2 += diff * Dy[y * win_w + x]; }
+                        else { b1 += (float)(diff * Dx[y * win_w + x]); b2 += (float)(diff * Dy[y * win_w + x]); }
                     }
+                if (exact) { b1 = (float)ib1; b2 = (float)ib2; }
                 b1 *= FLT_SCALE; b2 *= FLT_SCALE;
                 float dx = (float)((A12 * b2 - A22 * b1) * D);
                 float dy = (float)((A12 * b1 - A11 * b2) * D);
@@ -420,14 +431,16 @@ ORC_API int orc_pyrlk(const uint8_t* prev, const uint8_t* next, int w, int h, in
                 a = rx - jx; b = ry - jy;
                 bil_weights(a, b, &w00, &w01, &w10, &w11);
                 float errval = 0;
+                long long ierr = 0;
                 for (int y = 0; y < win_h; ++y)
                     for (int x = 0; x < win_w; ++x) {
                         int X = jx + x, Y = jy + y;
                         int jv = (img_pad(J, X, Y) * w00 + img_pad(J, X + 1, Y) * w01 +
                                   img_pad(J, X, Y + 1) * w10 + img_pad(J, X + 1, Y + 1) * w11 + (1 << (W_BITS - 5 - 1))) >> (W_BITS - 5);
-                        errval += (float)abs(jv - Ip[y * win_w + x]);
+                        if (exact) ierr += abs(jv - Ip[y * win_w + x]);
+                        else errval += (float)abs(jv - Ip[y * win_w + x]);
                     }
-                err[i] = errval * 1.f / (32 * win_w * win_h);
+                err[i] = exact ? (float)ierr * (1.f / (float)(32 * win_w * win_h)) : errval * 1.f / (32 * win_w * win_h);
             }
         }
     }

@@ -137,3 +137,71 @@ def test_feature_lists_vs_live_cv2_with_tie_rule():
         d_exact = np.abs(io.min_eig_map(img, bs) - e).max() / e.max()
         d_f32 = np.abs(io.min_eig_map(img, bs, fp32_sums=True) - e).max() / e.max()
         assert d_exact <= 2e-6 and d_f32 <= 4e-6, (bs, d_exact, d_f32)
+
+
+def _lk_edge_cases():
+    import lk_edge_cases as lc
+    tex = lc.texture_scene()
+    for win in lc.FAST_WINDOWS + lc.BOUNDARY_WINDOWS + lc.GENERIC_WINDOWS:
+        yield "texture", tex, win, 3, lc.CRIT, 1e-4, False
+    wide = lc.wide_scene()
+    for win in lc.SMEM_WINDOWS:
+        yield "wide", wide, win, 3, lc.CRIT, 1e-4, False
+    for cell in lc.CHECKER_CELLS:
+        for shift in lc.CHECKER_SHIFTS:
+            board = lc.checkerboard(cell, shift)
+            for win in lc.CHECKER_WINDOWS:
+                for ml in (0, 2):
+                    yield ("checkerboard", cell, shift), board, win, ml, lc.CRIT, 1e-4, lc.chaotic_checkerboard(cell, shift)
+    for h, w in lc.TINY_SIZES:
+        tiny = lc.tiny_scene(h, w)
+        for win in lc.TINY_WINDOWS:
+            for ml in (0, 3):
+                yield ("tiny", h, w), tiny, win, ml, lc.CRIT, 1e-4, False
+    crit = lc.criteria_scene()
+    for c, me in lc.CRITERIA_CASES:
+        for win in ((15, 15), (21, 21)):
+            yield "criteria", crit, win, 3, c, me, False
+    for (h, w), seed in (((1080, 1920), 44), ((97, 1003), 45)):
+        scene = lc.depth_scene(h, w, seed)
+        for win in ((15, 15), (21, 21), (3, 41), (61, 3)):
+            for ml in list(range(9)) + [20]:
+                yield ("depth", h, w), scene, win, ml, lc.CRIT, 1e-4, False
+
+
+def test_lk_edge_inputs_pinned_to_cv2():
+    """The inputs of test_gpu_lk_edges.py, oracle against cv2 4.13: identical status everywhere; positions within
+    5e-3 px and errors within lk_edge_cases.err_tol except at the points whose Newton path fp32 rounding decides
+    (the two summation modes of the oracle part there by more than 5e-3; at most 1 % of the tracked points, or 2),
+    status only on the checkerboards moved by half their period. The exact-sum mode is pinned to the default one
+    by the same rule."""
+    import lk_edge_cases as lc
+    n = 0
+    for what, (a, b, pts), win, ml, crit, me, chaotic in _lk_edge_cases():
+        what = (what, win, ml, crit, me)
+        ref = cv2.calcOpticalFlowPyrLK(a, b, pts, None, winSize=win, maxLevel=ml, criteria=crit, minEigThreshold=me)
+        plain = io.pyrlk(a, b, pts, win, ml, crit, me)
+        exact = io.pyrlk(a, b, pts, win, ml, crit, me, exact_sums=True)
+        decided = lc.rounding_decided(plain, exact)
+        if chaotic:
+            assert np.array_equal(plain[1], ref[1]) and np.array_equal(exact[1], ref[1]), what
+        else:
+            lc.assert_close_to(plain, ref, decided, what)
+            lc.assert_close_to(exact, plain, decided, what)
+        n += 1
+    assert n == 19 + 4 + 64 + 132 + 30 + 80
+
+
+def test_lk_exact_sums_mode_where_fp32_sums_are_exact():
+    """Windows of at most 8 pixels with gradients and differences of a few grey levels: every fp32 partial sum is an
+    integer below 2^24, so OpenCV's running sums are exact and both oracle modes must agree to the bit (the error
+    aside, which the default mode divides by 32 * npx and the exact one multiplies by its fp32 reciprocal)."""
+    rng = np.random.default_rng(3)
+    a = (rng.random((40, 50)) * 4).astype(np.uint8) + 100
+    b = np.roll(a, 1, axis=1)
+    pts = np.stack(np.meshgrid(np.arange(5, 45, 3.3), np.arange(5, 35, 2.7)), -1).astype(np.float32).reshape(-1, 1, 2)
+    for win in ((3, 3), (4, 3)):
+        plain = io.pyrlk(a, b, pts, win, 0, (3, 30, 0.01), 0.0)
+        exact = io.pyrlk(a, b, pts, win, 0, (3, 30, 0.01), 0.0, exact_sums=True)
+        assert np.array_equal(plain[0], exact[0]) and np.array_equal(plain[1], exact[1])
+        assert np.abs(plain[2] - exact[2]).max() <= 1e-6 * np.abs(plain[2]).max()
